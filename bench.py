@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- SD v1.5 UNet denoise hot path on B200 (BASELINE.json configs[1]).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl reference] [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
 One "step" = one denoising iteration of the 50-step DDIM + classifier-free-guidance sampler for B
@@ -348,7 +348,7 @@ class _PerCallSampler:
         B = self.B
         self.x2[:B].copy_(self.latents)
         self.x2[B:].copy_(self.latents)
-        eps2 = self.unet(self.x2, t, self.ctx).sample
+        eps2 = self.eps = self.unet(self.x2, t, self.ctx).sample
         self.sch.step_cfg(eps2, t, self.latents, 7.5, out=self.nxt)
         self.latents, self.nxt = self.nxt, self.latents
         eng = next(iter(self.unet._engines.values()))
@@ -369,6 +369,24 @@ class _PerCallSampler:
         self.step()
         out_host.copy_(self.latents, non_blocking=True)
         torch.cuda.current_stream().synchronize()
+
+
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir, tensors):
+    """Write each tensor as out_dir/<name>.npy in float32, so that two builds run with the same arguments can be compared output
+    for output.  When the tensors hold more than DUMP_BYTES together, each is replaced by the same seeded sample of its flattened
+    elements (ascending indices), sized so that the files stay within DUMP_BYTES."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: v.detach().float().cpu().numpy() for k, v in tensors.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    for name, a in arrays.items():
+        if total > DUMP_BYTES:
+            keep = a.size * (DUMP_BYTES - 256 * len(arrays)) // total          # 256: room for each .npy header
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, keep, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def run_ours(args):
@@ -445,6 +463,9 @@ def run_ours(args):
         ms = e0.elapsed_time(e1)
         eager_launches = ops.launch_count() - launches0
         gpu_launches = eager_launches + smp.kernels_per_step * (0 if idle else args.steps)
+        if args.dump_outputs and rank == 0:
+            # the step below (end to end) keeps updating the same buffers: keep what the last timed step returned
+            dump_outputs(args.dump_outputs, {"latents": smp.latents, "noise_pred": smp.eps})
 
         # ---- end to end through the public API with host buffers (H2D + D2H inside the timed region): every step copies the
         # latents and the text context out of pinned host memory, projects the context, runs the step and copies the new
@@ -1052,7 +1073,12 @@ def main():
     ap.add_argument("--no-train-legs", action="store_true", help="skip the fine-tuning sub-records (configs 3 / 4) of the default line")
     ap.add_argument("--no-elementwise", action="store_true", help="skip the elementwise GB/s sub-record")
     ap.add_argument("--dump-ops", default=None, help="write the per-launch timing table to this file")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="sampling workload: write what the last timed step returned (rank 0) as DIR/latents.npy (the new "
+                         "latents) and DIR/noise_pred.npy (the UNet's [uncond | cond] noise prediction), float32")
     args = ap.parse_args()
+    if args.dump_outputs and (args.workload != "sample" or args.impl != "b200sd"):
+        ap.error("--dump-outputs covers the sampling workload of the b200sd implementation")
     if args.workload == "sweep":
         if args.gpus > 1 and "RANK" not in os.environ:
             cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", f"--nproc-per-node={args.gpus}",

@@ -64,7 +64,9 @@ def test_gemm_args_struct_layout_matches_header(built):
 
 
 def test_sass_is_blackwell_native(built):
-    out = subprocess.run(["cuobjdump", "-sass", built.LIB_PATH], capture_output=True, text=True).stdout
+    from b200sd import build
+    cuobjdump = os.path.join(os.path.dirname(build.NVCC), "cuobjdump")     # the toolkit that compiled the library
+    out = subprocess.run([cuobjdump, "-sass", built.LIB_PATH], capture_output=True, text=True).stdout
     for mnem in ("UTCHMMA", "UTMALDG", "LDTM"):   # tcgen05.mma, TMA load, tcgen05.ld
         assert mnem in out, mnem
 

@@ -203,6 +203,31 @@ def test_bench_config_dicts_of_both_arms_are_one_function():
     assert '"config": sample_config(' in src_ours
 
 
+def test_bench_dump_outputs_writes_float32_within_its_budget(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: float32 .npy files named after the outputs, whole when they fit; beyond DUMP_BYTES the same
+    seeded sample of every output, so that two runs (two builds) stay comparable element for element."""
+    import importlib.util
+    import numpy as np
+    spec = importlib.util.spec_from_file_location("bench_mod3", os.path.join(os.path.dirname(os.path.dirname(__file__)), "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    lat = torch.randn(2, 4, 8, 8, dtype=torch.float64)
+    eps = torch.randn(4, 4, 8, 8, dtype=torch.bfloat16)
+    bench.dump_outputs(str(tmp_path / "whole"), {"latents": lat, "noise_pred": eps})
+    a, b = np.load(tmp_path / "whole" / "latents.npy"), np.load(tmp_path / "whole" / "noise_pred.npy")
+    assert a.dtype == b.dtype == np.float32 and a.shape == (2, 4, 8, 8) and b.shape == (4, 4, 8, 8)
+    assert np.array_equal(a, lat.float().numpy()) and np.array_equal(b, eps.float().numpy())
+    monkeypatch.setattr(bench, "DUMP_BYTES", 4000)           # the two outputs hold 6144 bytes
+    for d in ("s1", "s2"):
+        bench.dump_outputs(str(tmp_path / d), {"latents": lat, "noise_pred": eps})
+    files = [tmp_path / d / f"{n}.npy" for d in ("s1", "s2") for n in ("latents", "noise_pred")]
+    assert sum(os.path.getsize(f) for f in files[:2]) <= 4000
+    s = [np.load(f) for f in files]
+    assert np.array_equal(s[0], s[2]) and np.array_equal(s[1], s[3])
+    assert s[0].dtype == s[1].dtype == np.float32 and 0 < s[0].size < lat.numel() and 0 < s[1].size < eps.numel()
+    assert np.isin(s[0], lat.float().numpy()).all() and np.isin(s[1], eps.float().numpy()).all()
+
+
 def test_pipeline_wrapper_save_load_layout(tmp_path):
     """finetune_sd.py:517-537 builds StableDiffusionPipeline(text_encoder=, vae=, unet=, tokenizer=, scheduler=, safety_checker=,
     feature_extractor=) and save_pretrained()s it; utils.py:187-191 loads it back with safety_checker=None: the diffusers directory
