@@ -30,6 +30,7 @@ from torch.autograd.function import once_differentiable
 
 from . import ops
 from ._lib import B200SDError
+from .plan import Builder, Plan, capture, run_plan
 from .train import F32, BF16, FlatParams
 
 _CONFIG_DEFAULTS = dict(vocab_size=49408, hidden_size=768, intermediate_size=3072, num_hidden_layers=12, num_attention_heads=12,
@@ -117,14 +118,14 @@ class ClipFlat(FlatParams):
         add(tm.final_layer_norm.weight, "vec"); add(tm.final_layer_norm.bias, "vec")
 
 
-class ClipEngine:
+class ClipEngine(Builder):
     """Forward launch plan (keeps what the backward needs: ~30 MB at 16 prompts) and backward launch plan for a fixed number
     of prompts; each is captured into a CUDA graph on first use."""
 
     def __init__(self, model, flat, B, S, device, train_weights):
-        self.model, self.flat, self.B, self.S, self.device, self.train_weights = model, flat, B, S, device, train_weights
-        self.fwd, self.bwd = [], []
-        self._keep = []
+        super().__init__(device)
+        self.model, self.flat, self.B, self.S, self.train_weights = model, flat, B, S, train_weights
+        self.fwd, self.bwd = Plan(), Plan()
         self.fwd_graph = self.bwd_graph = None
         self.use_graph = True
         self.forward_generation = 0
@@ -141,23 +142,6 @@ class ClipEngine:
 
     def _new(self, rows, cols, dtype=BF16):
         return torch.empty(rows, cols, dtype=dtype, device=self.device)
-
-    def _gemm(self, a0, w, out, **kw):
-        args = ops.gemm(a0, w, out, launch=False, **kw)
-        self._keep.append((a0, w, out, kw))
-        self.fwd.append(lambda a=args: ops.gemm_run(a))
-
-    def _dgrad(self, dy, w, out, **kw):
-        args = ops.gemm_dgrad(dy, w, out, launch=False, **kw)
-        self._keep.append((dy, w, out, kw))
-        self.bwd.append(lambda a=args: ops.check(ops.lib().b200sd_gemm_dgrad(ops.C.byref(a), ops._stream()), "gemm_dgrad"))
-
-    def _wgrad(self, dy, x, dw):
-        if not self.train_weights:
-            return
-        args = ops.gemm_wgrad(dy, x, dw, launch=False)
-        self._keep.append((dy, x, dw))
-        self.bwd.append(lambda a=args: ops.check(ops.lib().b200sd_gemm_wgrad(ops.C.byref(a), ops._stream()), "gemm_wgrad"))
 
     def _build(self):
         m, flat, B, S, dev = self.model, self.flat, self.B, self.S, self.device
@@ -184,13 +168,13 @@ class ClipEngine:
             n1, qkv, at = self._new(M, C), self._new(M, 3 * C), self._new(M, C)
             x1, n2, u, g, x2 = self._new(M, C, F32), self._new(M, C), self._new(M, I), self._new(M, I), self._new(M, C, F32)
             Fp.append(lambda x=x, L=L, n1=n1: ops.layernorm(x, self.P(L.layer_norm1.weight), self.P(L.layer_norm1.bias), n1, eps))
-            self._gemm(n1, w_qkv, qkv, bias=b_qkv)
+            self.gemm(Fp, n1, w_qkv, qkv, bias=b_qkv)
             Fp.append(lambda qkv=qkv, at=at: ops.causal_attention(qkv, at, B, heads, S, d, scale))
-            self._gemm(at, wb(a.out_proj.weight), x1, bias=self.P(a.out_proj.bias), residual=x)
+            self.gemm(Fp, at, wb(a.out_proj.weight), x1, bias=self.P(a.out_proj.bias), residual=x)
             Fp.append(lambda x1=x1, L=L, n2=n2: ops.layernorm(x1, self.P(L.layer_norm2.weight), self.P(L.layer_norm2.bias), n2, eps))
-            self._gemm(n2, wb(L.mlp.fc1.weight), u, bias=self.P(L.mlp.fc1.bias))
+            self.gemm(Fp, n2, wb(L.mlp.fc1.weight), u, bias=self.P(L.mlp.fc1.bias))
             Fp.append(lambda u=u, g=g: ops.quick_gelu_fwd(u, g))
-            self._gemm(g, wb(L.mlp.fc2.weight), x2, bias=self.P(L.mlp.fc2.bias), residual=x1)
+            self.gemm(Fp, g, wb(L.mlp.fc2.weight), x2, bias=self.P(L.mlp.fc2.bias), residual=x1)
             layers.append((L, x, n1, qkv, at, x1, n2, u, g, w_qkv))
             x = x2
         lnf = tm.final_layer_norm
@@ -208,25 +192,25 @@ class ClipEngine:
             wb = lambda p: flat.reg(p).wb
             # x' = fc2(g) + x1
             Bp.append(lambda L=L: ops.grad_prep(dx, d16, self.G(L.mlp.fc2.bias)))
-            self._wgrad(d16, g, self.G(L.mlp.fc2.weight))
-            self._dgrad(d16, wb(L.mlp.fc2.weight), dg)
+            self.wgrad(Bp, d16, g, self.G(L.mlp.fc2.weight))
+            self.dgrad(Bp, d16, wb(L.mlp.fc2.weight), dg)
             Bp.append(lambda u=u: ops.quick_gelu_bwd(u, dg, du))
             if tw:
                 Bp.append(lambda L=L: ops.grad_prep(du, None, self.G(L.mlp.fc1.bias)))
-            self._wgrad(du, n2, self.G(L.mlp.fc1.weight))
-            self._dgrad(du, wb(L.mlp.fc1.weight), dn)
+            self.wgrad(Bp, du, n2, self.G(L.mlp.fc1.weight))
+            self.dgrad(Bp, du, wb(L.mlp.fc1.weight), dn)
             Bp.append(lambda x1=x1, L=L: ops.layernorm_bwd(x1, self.P(L.layer_norm2.weight), dn, dx, self.G(L.layer_norm2.weight),
                                                           self.G(L.layer_norm2.bias), eps))
             # x1 = out_proj(attention) + x
             Bp.append(lambda a=a: ops.grad_prep(dx, d16, self.G(a.out_proj.bias)))
-            self._wgrad(d16, at, self.G(a.out_proj.weight))
-            self._dgrad(d16, wb(a.out_proj.weight), da)
+            self.wgrad(Bp, d16, at, self.G(a.out_proj.weight))
+            self.dgrad(Bp, d16, wb(a.out_proj.weight), da)
             Bp.append(lambda qkv=qkv: ops.causal_attention_bwd(qkv, da, dqkv, B, heads, S, d, scale))
             if tw:
                 g_bqkv = flat.span([a.q_proj.bias, a.k_proj.bias, a.v_proj.bias], "grad")
                 Bp.append(lambda gb=g_bqkv: ops.grad_prep(dqkv, None, gb))
-                self._wgrad(dqkv, n1, flat.span([a.q_proj.weight, a.k_proj.weight, a.v_proj.weight], "grad"))
-            self._dgrad(dqkv, w_qkv, dn)
+                self.wgrad(Bp, dqkv, n1, flat.span([a.q_proj.weight, a.k_proj.weight, a.v_proj.weight], "grad"))
+            self.dgrad(Bp, dqkv, w_qkv, dn)
             Bp.append(lambda xin=xin, L=L: ops.layernorm_bwd(xin, self.P(L.layer_norm1.weight), dn, dx, self.G(L.layer_norm1.weight),
                                                             self.G(L.layer_norm1.bias), eps))
         if tw:
@@ -238,17 +222,10 @@ class ClipEngine:
         g = getattr(self, which)
         if g is not None:
             g.replay()
-            return
-        for op in plan:              # the first call runs eagerly: it IS this call's result (the backward ACCUMULATES gradients,
-            op()                     # so it must run exactly once) and does the lazy one-time setup outside any capture
-        if not self.use_graph:
-            return
-        torch.cuda.current_stream().synchronize()
-        g = torch.cuda.CUDAGraph()
-        with torch.cuda.graph(g, capture_error_mode="thread_local"):      # backward plans are captured on autograd's thread
-            for op in plan:
-                op()
-        setattr(self, which, g)
+        elif self.use_graph:
+            setattr(self, which, capture(plan, "thread_local")[0])      # backward plans are captured on autograd's thread
+        else:
+            run_plan(plan)
 
     def run_forward(self, ids):
         with torch.cuda.device(self.device):

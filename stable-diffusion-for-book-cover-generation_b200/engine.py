@@ -15,69 +15,28 @@ Data flow per block (SURVEY.md App. A.2), each arrow = one kernel:
 """
 from __future__ import annotations
 
-import ctypes as C
-
 import os
-
-import weakref
 
 import torch
 
 from . import ops
-from ._lib import check, lib
+from .plan import Builder, ContextKey, Plan, Pool, capture, profile_plan, run_plan
 
 
-class _Pool:
-    """Size-keyed free lists of bf16 row-major buffers; safe because all work is stream-ordered."""
-
-    def __init__(self, device):
-        self.device = device
-        self.free = {}
-        self.total = 0
-
-    def get(self, rows, cols, dtype=torch.bfloat16):
-        key = (rows * cols, dtype)
-        lst = self.free.get(key)
-        if lst:
-            return lst.pop().view(rows, cols)
-        self.total += rows * cols * (2 if dtype == torch.bfloat16 else 4)
-        return torch.empty(rows, cols, dtype=dtype, device=self.device)
-
-    def put(self, t):
-        self.free.setdefault((t.numel(), t.dtype), []).append(t)
-
-
-class _Plan(list):
-    """List of launch closures + parallel metadata (kind, algorithmic flops) for profiling."""
-
-    def __init__(self):
-        super().__init__()
-        self.meta = []
-
-    def append(self, fn, kind="other", flops=0.0, name=""):
-        super().append(fn)
-        self.meta.append((kind, float(flops), name))
-
-
-class Engine:
+class Engine(Builder):
     def __init__(self, model, N, H, W, S_ctx, device, io=None):
+        super().__init__(device)
         self.model, self.N, self.H, self.W, self.S = model, N, H, W, S_ctx
-        self.device = device
         self._io = io           # LanedEngine: (in_sample, in_t, out) views of the parent's static buffers
         cfg = model.config
         self.heads = cfg.attention_head_dim
         self.ctx_dim = cfg.cross_attention_dim
-        self.plan = _Plan()     # main plan (per step)
-        self.ctx_plan = _Plan() # context K/V projections (once per context)
-        self.pool = _Pool(device)
+        self.plan = Plan()      # main plan (per step)
+        self.ctx_plan = Plan()  # context K/V projections (once per context)
         self.graph = None
-        self._ctx_key = None
-        self._keep = []
+        self._ctx_key = ContextKey()
         self.debug = False      # when True (eager runs only) every tapped activation is cloned
         self.debug_out = {}
-        # GroupNorm statistics from the producing GEMM's epilogue (B200SD_GN_FROM_GEMM=0: always the stand-alone kernel)
-        self.gn_from_gemm = os.environ.get("B200SD_GN_FROM_GEMM", "1") != "0"
-        self._gn_parts = {}     # id(activation buffer) -> ops.GnParts describing its CURRENT contents (plan-build time)
         self.prefetch_kblocks = int(os.environ.get("B200SD_PREFETCH", "0"))     # k-blocks of the next layer staged in L2 (0 = off)
         self.prefetch_weights = self.prefetch_kblocks > 0
         self._prev_gemm, self._first_w = None, None
@@ -85,20 +44,8 @@ class Engine:
             self._build()
 
     # -- plan-building helpers --------------------------------------------------------------------
-    def _gemm(self, plan, a0, w, out, **kw):
-        rb = kw.pop("rowbias_ptr", None)
-        gn_hw = kw.pop("gn_hw", 0)    # > 0: `out` feeds a GroupNorm -- have the epilogue emit its column statistics
-        args = ops.gemm(a0, w, out, launch=False, **kw)
-        if rb is not None:
-            args.rowbias, args.ldrb, args.rows_per_image = rb[0], rb[1], rb[2]
-        self._gn_parts.pop(id(out), None)      # whatever statistics described this (pooled) buffer are stale now
-        if gn_hw > 0 and self.gn_from_gemm:
-            parts = ops.gemm_attach_gn_parts(args, gn_hw, self.device)
-            if parts is not None:
-                self._gn_parts[id(out)] = parts
-                self._keep.append(parts)       # the captured launch writes into parts.buf on every replay: it must outlive
-                #                                its entry in _gn_parts (popped when the pooled buffer is produced again)
-        self._keep.append((a0, w, out, kw))
+    def gemm(self, plan, a0, w, out, **kw):
+        args = super().gemm(plan, a0, w, out, **kw)
         if plan is self.plan and self.prefetch_weights:
             # the weights of THIS layer are what the PREVIOUS tensor-core launch pulls into L2 while it runs: every layer's weights
             # are cold in HBM when its kernel starts (1.7 GB stream through a 126 MB L2 once per step)
@@ -107,9 +54,7 @@ class Engine:
             else:
                 self._first_w = w
             self._prev_gemm = args
-        kind = "conv3x3" if args.conv_taps == 9 else "gemm"
-        plan.append(lambda a=args: ops.gemm_run(a), kind, 2.0 * args.M * args.N * args.K,
-                    f"{kind} M{args.M} N{args.N} K{args.K}")
+        return args
 
     def _prefetch_bytes(self, w):
         """How much of the next layer's weights the previous launch stages in L2.  Staging ALL of it was measured slower (the
@@ -119,19 +64,6 @@ class Engine:
         if w.dim() == 3:
             return min(total, self.prefetch_kblocks * w.shape[1] * w.shape[2] * w.element_size())
         return total if self.prefetch_kblocks >= 1000 else 0
-
-    def _groupnorm(self, x, skip, g, b, out, hw, eps, silu, raw_out=None):
-        """Plan one GroupNorm(+SiLU, + concat): from the producers' epilogue statistics when every source has them."""
-        N = self.N
-        p0 = self._gn_parts.get(id(x))
-        p1 = self._gn_parts.get(id(skip)) if skip is not None else None
-        C = x.shape[-1] + (skip.shape[-1] if skip is not None else 0)
-        if p0 is not None and (skip is None or p1 is not None) and ops.gn_parts_supported(C, 32):
-            self._keep.append((p0, p1))
-            self.plan.append(lambda: ops.groupnorm_silu_parts(x, skip, p0, p1, g, b, out, N, hw, 32, eps, silu, raw_out=raw_out),
-                             "groupnorm", 0, "groupnorm (stats from GEMM)")
-        else:
-            self.plan.append(lambda: ops.groupnorm_silu(x, skip, g, b, out, N, hw, 32, eps, silu, raw_out=raw_out), "groupnorm")
 
     def _tap(self, name, t, h, w):
         """Debug probe: snapshot activation `t` ([N*h*w, C] NHWC) as NCHW fp32 under `name`."""
@@ -144,7 +76,8 @@ class Engine:
         m, Wp, N, dev = self.model, self.model._packed, self.N, self.device
         cfg = m.config
         boc = cfg.block_out_channels
-        P, pool = self.plan, self.pool
+        P, pool = self.plan, Pool(dev)
+        self.pool = pool
         f32 = dict(dtype=torch.float32, device=dev)
 
         # static inputs
@@ -161,7 +94,7 @@ class Engine:
         t_sin = torch.empty(N, boc[0], **f32)
         t_h = torch.empty(N, temb_dim, **f32)
         t_emb = torch.empty(N, temb_dim, **f32)
-        n_tp = Wp["tproj"]["n"]
+        tp_off, n_tp = m._tproj_offsets()
         self.tproj = torch.empty(N, n_tp, **f32)
         te = Wp["temb"]
         P.append(lambda: ops.timestep_embedding(self.in_t, boc[0], out=t_sin), "time_embed")
@@ -174,8 +107,8 @@ class Engine:
         if self.large_batch:
             a16 = torch.empty(N, temb_dim, dtype=torch.bfloat16, device=dev)
             P.append(lambda: ops.cast_act(t_emb, a16, silu=True), "time_embed")
-            self._gemm(P, a16, Wp["tproj"]["w"], self.tproj, bias=Wp["tproj"]["b"])
-            self.plan.meta[-1] = ("time_embed", self.plan.meta[-1][1], "time_emb_proj x22 (tensor cores)")
+            self.gemm(P, a16, Wp["tproj"]["w"], self.tproj, bias=Wp["tproj"]["b"], kind="time_embed",
+                      name="time_emb_proj x22 (tensor cores)")
         else:
             P.append(lambda: ops.small_linear(t_emb, Wp["tproj"]["w"], Wp["tproj"]["b"], silu_in=True, out=self.tproj), "time_embed", 0, "time_emb_proj x22")
 
@@ -189,16 +122,7 @@ class Engine:
         #                       bf16 appears only where a tensor is a tensor-core operand
         x = pool.get(N * h * w, boc[0], F32)
         P.append(lambda x=x: ops.conv_in(self.in_sample, Wp["conv_in"]["w"], Wp["conv_in"]["b"], x), "conv_io", 0, "conv_in")
-
         self._tap("conv_in", x, h, w)
-        skips = [(x, boc[0])]
-        skip_refs = {id(x): 1}
-
-        def release(t):
-            # a buffer may be both the running activation and a pending skip
-            if skip_refs.get(id(t), 0) > 0:
-                return
-            pool.put(t)
 
         def resnet(prefix, r, x, skip, h, w):
             wr = Wp[prefix]
@@ -206,22 +130,22 @@ class Engine:
             cin, cout = r.cin, r.cout
             t1 = pool.get(M, cin)
             raw = pool.get(M, cin) if "wsc" in wr else None   # bf16 copy of [x|skip]: operand of the 1x1 shortcut
-            self._groupnorm(x, skip, wr["g1"], wr["b1"], t1, h * w, cfg.norm_eps, True, raw_out=raw)
+            self.groupnorm(P, x, skip, wr["g1"], wr["b1"], t1, N, h * w, cfg.norm_eps, True, raw_out=raw)
             hbuf = pool.get(M, cout, F32)
-            rb = (self.tproj.data_ptr() + m._tproj_off[prefix] * 4, n_tp, h * w)
-            self._gemm(P, t1, wr["w1"], hbuf, bias=wr["cb1"], conv=(N, h, w), rowbias_ptr=rb, gn_hw=h * w)
+            rb = (self.tproj.data_ptr() + tp_off[prefix] * 4, n_tp, h * w)
+            self.gemm(P, t1, wr["w1"], hbuf, bias=wr["cb1"], conv=(N, h, w), rowbias_ptr=rb, gn_hw=h * w)
             pool.put(t1)
             t2 = pool.get(M, cout)
-            self._groupnorm(hbuf, None, wr["g2"], wr["b2"], t2, h * w, cfg.norm_eps, True)
+            self.groupnorm(P, hbuf, None, wr["g2"], wr["b2"], t2, N, h * w, cfg.norm_eps, True)
             pool.put(hbuf)
             if "wsc" in wr:
                 sc = pool.get(M, cout, F32)
-                self._gemm(P, raw, wr["wsc"], sc, bias=wr["bsc"])
+                self.gemm(P, raw, wr["wsc"], sc, bias=wr["bsc"])
                 pool.put(raw)
             else:
                 sc = x
             y = pool.get(M, cout, F32)
-            self._gemm(P, t2, wr["w2"], y, bias=wr["cb2"], residual=sc, conv=(N, h, w), gn_hw=h * w)
+            self.gemm(P, t2, wr["w2"], y, bias=wr["cb2"], residual=sc, conv=(N, h, w), gn_hw=h * w)
             pool.put(t2)
             if sc is not x:
                 pool.put(sc)
@@ -236,120 +160,77 @@ class Engine:
             scale = d ** -0.5
             # context K/V: hoisted out of the per-step plan
             kv = torch.empty(N * self.S, 2 * Cc, dtype=torch.bfloat16, device=dev)
-            self._gemm(self.ctx_plan, self.in_ctx, wa["w_kv2"], kv)
+            self.gemm(self.ctx_plan, self.in_ctx, wa["w_kv2"], kv)
             t = pool.get(M, Cc)
-            self._groupnorm(x, None, wa["gn_g"], wa["gn_b"], t, h * w, 1e-6, False)
+            self.groupnorm(P, x, None, wa["gn_g"], wa["gn_b"], t, N, h * w, 1e-6, False)
             hs = pool.get(M, Cc, F32)
-            self._gemm(P, t, wa["w_in"], hs, bias=wa["b_in"])
+            self.gemm(P, t, wa["w_in"], hs, bias=wa["b_in"])
             # self attention
             P.append(lambda: ops.layernorm(hs, wa["ln1_g"], wa["ln1_b"], t), "layernorm")
             qkv = pool.get(M, 3 * Cc)
-            self._gemm(P, t, wa["w_qkv"], qkv)
+            self.gemm(P, t, wa["w_qkv"], qkv)
             P.append(lambda: ops.attention(qkv, qkv, qkv, t, N, self.heads, h * w, h * w, d, scale, ldq=3 * Cc,
                                            ldk=3 * Cc, ldv=3 * Cc, ldo=Cc, q_off=0, k_off=Cc, v_off=2 * Cc, ws=self.attn_ws),
                      "attention", 4.0 * N * self.heads * (h * w) * (h * w) * d, f"self-attn S{h * w} d{d}")
             pool.put(qkv)
-            self._gemm(P, t, wa["w_o1"], hs, bias=wa["b_o1"], residual=hs)
+            self.gemm(P, t, wa["w_o1"], hs, bias=wa["b_o1"], residual=hs)
             # cross attention
             P.append(lambda: ops.layernorm(hs, wa["ln2_g"], wa["ln2_b"], t), "layernorm")
             q = pool.get(M, Cc)
-            self._gemm(P, t, wa["w_q2"], q)
+            self.gemm(P, t, wa["w_q2"], q)
             P.append(lambda: ops.attention(q, kv, kv, t, N, self.heads, h * w, self.S, d, scale, ldq=Cc, ldk=2 * Cc,
                                            ldv=2 * Cc, ldo=Cc, k_off=0, v_off=Cc, ws=self.attn_ws),
                      "attention", 4.0 * N * self.heads * (h * w) * self.S * d, f"cross-attn S{h * w} d{d}")
             pool.put(q)
-            self._gemm(P, t, wa["w_o2"], hs, bias=wa["b_o2"], residual=hs)
+            self.gemm(P, t, wa["w_o2"], hs, bias=wa["b_o2"], residual=hs)
             # GEGLU feed-forward
             P.append(lambda: ops.layernorm(hs, wa["ln3_g"], wa["ln3_b"], t), "layernorm")
             ff = pool.get(M, 4 * Cc)
-            self._gemm(P, t, wa["w_ff1"], ff, bias=wa["b_ff1"], epilogue=ops.EPI_GEGLU, block_n=wa["ff_tile"])
+            self.gemm(P, t, wa["w_ff1"], ff, bias=wa["b_ff1"], epilogue=ops.EPI_GEGLU, block_n=wa["ff_tile"])
             # last residual add of the block: its only consumer is proj_out's A operand -> write bf16 directly
-            self._gemm(P, ff, wa["w_ff2"], t, bias=wa["b_ff2"], residual=hs)
+            self.gemm(P, ff, wa["w_ff2"], t, bias=wa["b_ff2"], residual=hs)
             pool.put(ff)
             y = pool.get(M, Cc, F32)
-            self._gemm(P, t, wa["w_out"], y, bias=wa["b_out"], residual=x, gn_hw=h * w)
+            self.gemm(P, t, wa["w_out"], y, bias=wa["b_out"], residual=x, gn_hw=h * w)
             pool.put(t)
             pool.put(hs)
             self._tap(prefix, y, h, w)
             return y
 
-        def push_skip(t, c):
-            skips.append((t, c))
-            skip_refs[id(t)] = skip_refs.get(id(t), 0) + 1
+        def downsample(prefix, _s, x, h, w):
+            Cc = x.shape[1]
+            col = pool.get(N * (h // 2) * (w // 2), 9 * Cc)
+            P.append(lambda x=x, col=col, h=h, w=w: ops.im2col_s2(x, col, N, h, w), "resample", 0, "im2col_s2")
+            h, w = h // 2, w // 2
+            y = pool.get(N * h * w, Cc, F32)
+            self.gemm(P, col, Wp[prefix]["w"], y, bias=Wp[prefix]["b"], gn_hw=h * w)
+            pool.put(col)
+            self._tap(prefix, y, h, w)
+            return y
 
-        # ---- down ----
-        for i, b in enumerate(m.down_blocks):
-            for j, r in enumerate(b.resnets):
-                y = resnet(f"down{i}.res{j}", r, x, None, h, w)
-                release(x)
-                x = y
-                if hasattr(b, "attentions"):
-                    y = xformer(f"down{i}.attn{j}", b.attentions[j], x, h, w)
-                    release(x)
-                    x = y
-                push_skip(x, r.cout)
-            if hasattr(b, "downsamplers"):
-                wd = Wp[f"down{i}.ds"]
-                Cc = boc[i]
-                col = pool.get(N * (h // 2) * (w // 2), 9 * Cc)
-                P.append(lambda x=x, col=col, h=h, w=w: ops.im2col_s2(x, col, N, h, w), "resample", 0, "im2col_s2")
-                h, w = h // 2, w // 2
-                y = pool.get(N * h * w, Cc, F32)
-                self._gemm(P, col, wd["w"], y, bias=wd["b"], gn_hw=h * w)
-                pool.put(col)
-                release(x)
-                x = y
-                self._tap(f"down{i}.ds", x, h, w)
-                push_skip(x, Cc)
+        def upsample(prefix, _s, x, h, w):
+            Cc = x.shape[1]
+            up = pool.get(N * 4 * h * w, Cc)
+            P.append(lambda x=x, up=up, h=h, w=w: ops.upsample2x(x, up, N, h, w), "resample", 0, "upsample2x")
+            h, w = 2 * h, 2 * w
+            y = pool.get(N * h * w, Cc, F32)
+            self.gemm(P, up, Wp[prefix]["w"], y, bias=Wp[prefix]["b"], conv=(N, h, w), gn_hw=h * w)
+            pool.put(up)
+            self._tap(prefix, y, h, w)
+            return y
 
-        # ---- mid ----
-        y = resnet("mid.res0", m.mid_block.resnets[0], x, None, h, w)
-        release(x)
-        x = y
-        y = xformer("mid.attn0", m.mid_block.attentions[0], x, h, w)
-        release(x)
-        x = y
-        y = resnet("mid.res1", m.mid_block.resnets[1], x, None, h, w)
-        release(x)
-        x = y
-
-        # ---- up ----
-        for i, b in enumerate(m.up_blocks):
-            for j, r in enumerate(b.resnets):
-                skip, _c = skips.pop()
-                y = resnet(f"up{i}.res{j}", r, x, skip, h, w)
-                skip_refs[id(skip)] -= 1
-                release(skip)
-                release(x)
-                x = y
-                if hasattr(b, "attentions"):
-                    y = xformer(f"up{i}.attn{j}", b.attentions[j], x, h, w)
-                    release(x)
-                    x = y
-            if hasattr(b, "upsamplers"):
-                wu = Wp[f"up{i}.us"]
-                Cc = x.shape[1]
-                up = pool.get(N * 4 * h * w, Cc)
-                P.append(lambda x=x, up=up, h=h, w=w: ops.upsample2x(x, up, N, h, w), "resample", 0, "upsample2x")
-                release(x)
-                h, w = 2 * h, 2 * w
-                y = pool.get(N * h * w, Cc, F32)
-                self._gemm(P, up, wu["w"], y, bias=wu["b"], conv=(N, h, w), gn_hw=h * w)
-                pool.put(up)
-                x = y
-                self._tap(f"up{i}.us", x, h, w)
+        x, h, w = m._walk(x, h, w, resnet=resnet, xformer=xformer, downsample=downsample, upsample=upsample, release=pool.put)
 
         # ---- out ----
         wo = Wp["conv_out"]
         t = pool.get(N * h * w, boc[0])
-        self._groupnorm(x, None, wo["g"], wo["beta"], t, h * w, cfg.norm_eps, True)
+        self.groupnorm(P, x, None, wo["g"], wo["beta"], t, N, h * w, cfg.norm_eps, True)
         if self.large_batch and boc[0] % 64 == 0 and cfg.out_channels <= 4:
             # conv_out (320 -> 4) as an implicit GEMM on the tensor cores: [x | x] . [w_hi | w_lo] per tap (fp32-accurate weights),
             # the 4 channels padded to a 32-wide tile, then bias + NHWC -> NCHW.  The CUDA-core kernel is latency-bound at CFG batch 2
             # (32 us) and stops scaling beyond (267 us at batch 16).
             tmp = pool.get(N * h * w, 32, F32)
-            self._gemm(P, t, wo["w_tc"], tmp, a1=t, conv=(N, h, w))
-            self.plan.meta[-1] = ("conv_io", self.plan.meta[-1][1], "conv_out (tensor cores)")
+            self.gemm(P, t, wo["w_tc"], tmp, a1=t, conv=(N, h, w), kind="conv_io", name="conv_out (tensor cores)")
             P.append(lambda tmp=tmp: ops.nhwc_bias_to_nchw(tmp, wo["b"], self.out), "conv_io", 0, "conv_out: bias + NCHW")
         else:
             P.append(lambda t=t: ops.conv_out(t, wo["w"], wo["b"], self.out), "conv_io", 0, "conv_out")
@@ -360,20 +241,11 @@ class Engine:
     # -- execution --------------------------------------------------------------------------------
     def set_context(self, ctx):
         """Project the (constant-over-steps) text context to every cross-attention's K/V once."""
-        # Cache hit only for the SAME live tensor object at the same version.  (The key used to be (data_ptr, version, shape):
-        # a new context tensor that the caching allocator placed at the freed address of the previous one -- same shape,
-        # version 0 -- was then taken for the old one and sampled with stale K/V.)
-        ref = self._ctx_key[0]() if self._ctx_key is not None else None
-        if ref is ctx and self._ctx_key[1] == ctx._version:
+        if self._ctx_key.matches(ctx):
             return
         self.in_ctx.copy_(ctx.reshape(self.N * self.S, self.ctx_dim))
-        for op in self.ctx_plan:
-            op()
-        self._ctx_key = (weakref.ref(ctx), ctx._version)
-
-    def _run_plan(self):
-        for op in self.plan:
-            op()
+        run_plan(self.ctx_plan)
+        self._ctx_key.set(ctx)
 
     def run(self, sample, timestep, ctx, use_graph=True):
         with torch.cuda.device(self.device):
@@ -384,71 +256,13 @@ class Engine:
             else:
                 self.in_t.fill_(float(timestep))
             if not use_graph:
-                self._run_plan()
+                run_plan(self.plan)
+            elif self.graph is None:
+                self.graph, self.kernels_per_graph = capture(self.plan)
             else:
-                if self.graph is None:
-                    self._run_plan()  # warm-up: lazy one-time setup (func attributes, workspaces) outside capture
-                    torch.cuda.current_stream().synchronize()
-                    g = torch.cuda.CUDAGraph()
-                    before = ops.launch_count()
-                    with torch.cuda.graph(g):
-                        self._run_plan()
-                    self.kernels_per_graph = ops.launch_count() - before
-                    self.graph = g
                 self.graph.replay()
             return self.out.clone()
 
     def profile(self, iters=5):
-        """Per-launch device time of every plan entry measured INSIDE the step (see profile_plan)."""
+        """Per-launch device time of every plan entry measured INSIDE the step (see plan.profile_plan)."""
         return profile_plan(self.plan, self.device, iters)
-
-
-def profile_plan(plan, device, iters=5):
-    """Per-launch device time of every entry of a launch plan measured INSIDE the step: the whole plan is captured once more
-    into a CUDA graph with an external event-record node (b200sd_timer_record) between consecutive entries, and the replays are
-    read back per entry.  Every kernel therefore runs under the conditions of the real step -- its weights streaming cold from
-    HBM, its input left in L2 by its true predecessor, no host launch gaps.  (The first version replayed each entry four
-    times back to back in a graph of its own: warm weights, optimistic.)  Returns ({kind: [ms, flops, launches]} per step,
-    [(name, ms, flops)] per entry, ms of the whole instrumented replay)."""
-    with torch.cuda.device(device):
-        entries = [(op, meta) for op, meta in zip(plan, plan.meta) if meta[0] != "tap"]
-        n = len(entries)
-        check(lib().b200sd_timer_reserve(n + 1), "timer_reserve")
-
-        def run_all():
-            for op, _m in entries:
-                op()
-        run_all()
-        torch.cuda.synchronize()
-        side = torch.cuda.Stream()
-        g = torch.cuda.CUDAGraph()
-        with torch.cuda.graph(g, stream=side):
-            sh = torch.cuda.current_stream().cuda_stream
-            for i, (op, _meta) in enumerate(entries):
-                check(lib().b200sd_timer_record(i, sh), "timer_record")
-                op()
-            check(lib().b200sd_timer_record(n, sh), "timer_record")
-        torch.cuda.synchronize()
-        times = [0.0] * n
-        total = 0.0
-        ms = C.c_float(0.0)
-        g.replay()          # warm-up replay of the instrumented graph
-        torch.cuda.synchronize()
-        for _ in range(iters):
-            g.replay()
-            torch.cuda.synchronize()
-            for i in range(n):
-                check(lib().b200sd_timer_elapsed_ms(i, i + 1, C.byref(ms)), "timer_elapsed")
-                times[i] += ms.value / iters
-            check(lib().b200sd_timer_elapsed_ms(0, n, C.byref(ms)), "timer_elapsed")
-            total += ms.value / iters
-        acc, per_op = {}, []
-        for t, (op, (kind, flops, name)) in zip(times, entries):
-            a = acc.setdefault(kind, [0.0, 0.0, 0])
-            a[0] += t
-            a[1] += flops
-            a[2] += 1
-            per_op.append((name or kind, t, flops))
-        run_all()
-        torch.cuda.synchronize()
-    return acc, per_op, total

@@ -16,11 +16,11 @@ attention: an accuracy path, selected with `unet.set_precision("fp32")`.
 """
 from __future__ import annotations
 
-import weakref
-
 import torch
 
 from . import ops
+from .engine import Engine
+from .plan import Builder
 
 F32, BF16 = torch.float32, torch.bfloat16
 
@@ -44,17 +44,10 @@ def _pack_lin(w):       # (out, in[,1,1]) -> W1 [out][2 in] = [hi | hi], W2 [out
     return torch.cat([hi, hi], dim=1).contiguous(), lo.contiguous()
 
 
-class EngineF32:
-    def __init__(self, model, N, H, W, S_ctx, device):
-        self.model, self.N, self.H, self.W, self.S, self.device = model, N, H, W, S_ctx, device
-        cfg = model.config
-        self.heads, self.ctx_dim = cfg.attention_head_dim, cfg.cross_attention_dim
-        self.plan, self.ctx_plan = [], []
-        self.graph = None
-        self._ctx_key = None
-        self._keep = []
-        with torch.cuda.device(device):
-            self._build()
+class EngineF32(Engine):
+    """Engine's inputs, context cache and execution over the fp32-accuracy plan built below."""
+
+    gemm = Builder.gemm     # no L2 weight prefetch chain (Engine.gemm): every contraction here is a pair of launches
 
     def _buf(self, rows, cols, dtype=F32):
         return torch.empty(rows, cols, dtype=dtype, device=self.device)
@@ -65,13 +58,8 @@ class EngineF32:
     def _gemm2(self, plan, a_hi, a_lo, w12, out, *, bias=None, residual=None, conv=None, rowbias_ptr=None):
         """out (fp32) = A W^T (+bias +rowbias +residual) to ~fp32 accuracy: two launches of the bf16 tensor-core GEMM"""
         w1, w2 = w12
-        args1 = ops.gemm(a_hi, w1, out, a1=a_lo, bias=bias, residual=residual, conv=conv, launch=False)
-        if rowbias_ptr is not None:
-            args1.rowbias, args1.ldrb, args1.rows_per_image = rowbias_ptr
-        args2 = ops.gemm(a_hi, w2, out, residual=out, conv=conv, launch=False)
-        self._keep.append((a_hi, a_lo, w1, w2, out, bias, residual))
-        plan.append(lambda: ops.gemm_run(args1))
-        plan.append(lambda: ops.gemm_run(args2))
+        self.gemm(plan, a_hi, w1, out, a1=a_lo, bias=bias, residual=residual, conv=conv, rowbias_ptr=rowbias_ptr)
+        self.gemm(plan, a_hi, w2, out, residual=out, conv=conv)
 
     def _build(self):
         m, N, dev = self.model, self.N, self.device
@@ -94,11 +82,7 @@ class EngineF32:
         resnets = list(m._iter_resnets())
         tp_w = torch.cat([f32p(r.time_emb_proj.weight) for _, r in resnets], 0)
         tp_b = torch.cat([f32p(r.time_emb_proj.bias) for _, r in resnets], 0)
-        n_tp = tp_w.shape[0]
-        tp_off, o = {}, 0
-        for prefix, r in resnets:
-            tp_off[prefix] = o
-            o += r.cout
+        tp_off, n_tp = m._tproj_offsets()
         temb_dim = boc[0] * 4
         t_sin = self._buf(N, boc[0])
         t_h = self._buf(N, temb_dim)
@@ -196,42 +180,27 @@ class EngineF32:
                 P.append(lambda: ops.upsample2x(xl, ol, N, h, w))
             return oh, ol
 
+        def downsample(_prefix, s, x, h, w):
+            ds = s.conv
+            ch, cl = resample(x, h, w, True)
+            y = self._buf(N * (h // 2) * (w // 2), x.shape[1])
+            wp = ds.weight.detach().permute(0, 2, 3, 1).reshape(ds.weight.shape[0], -1)      # [Cout][9*Cin] matches im2col order
+            self._gemm2(P, ch, cl, _pack_lin(wp), y, bias=f32p(ds.bias))
+            return y
+
+        def upsample(_prefix, s, x, h, w):
+            us = s.conv
+            uh, ul = resample(x, h, w, False)
+            y = self._buf(N * 4 * h * w, x.shape[1])
+            self._gemm2(P, uh, ul, _pack_conv(us.weight), y, bias=f32p(us.bias), conv=(N, 2 * h, 2 * w))
+            return y
+
         # ---- forward graph ----
         h, w = self.H, self.W
         x = self._buf(N * h * w, boc[0])
         ci_w, ci_b = f32p(m.conv_in.weight.detach().permute(0, 2, 3, 1).reshape(boc[0], -1)), f32p(m.conv_in.bias)
         P.append(lambda x=x: ops.conv_in(self.in_sample, ci_w, ci_b, x))
-        skips = [x]
-        for i, b in enumerate(m.down_blocks):
-            for j, r in enumerate(b.resnets):
-                x = resnet(f"down{i}.res{j}", r, x, None, h, w)
-                if hasattr(b, "attentions"):
-                    x = xformer(f"down{i}.attn{j}", b.attentions[j], x, h, w)
-                skips.append(x)
-            if hasattr(b, "downsamplers"):
-                ds = b.downsamplers[0].conv
-                ch, cl = resample(x, h, w, True)
-                h, w = h // 2, w // 2
-                y = self._buf(N * h * w, x.shape[1])
-                wp = ds.weight.detach().permute(0, 2, 3, 1).reshape(ds.weight.shape[0], -1)      # [Cout][9*Cin] matches im2col order
-                self._gemm2(P, ch, cl, _pack_lin(wp), y, bias=f32p(ds.bias))
-                x = y
-                skips.append(x)
-        x = resnet("mid.res0", m.mid_block.resnets[0], x, None, h, w)
-        x = xformer("mid.attn0", m.mid_block.attentions[0], x, h, w)
-        x = resnet("mid.res1", m.mid_block.resnets[1], x, None, h, w)
-        for i, b in enumerate(m.up_blocks):
-            for j, r in enumerate(b.resnets):
-                x = resnet(f"up{i}.res{j}", r, x, skips.pop(), h, w)
-                if hasattr(b, "attentions"):
-                    x = xformer(f"up{i}.attn{j}", b.attentions[j], x, h, w)
-            if hasattr(b, "upsamplers"):
-                us = b.upsamplers[0].conv
-                uh, ul = resample(x, h, w, False)
-                h, w = 2 * h, 2 * w
-                y = self._buf(N * h * w, x.shape[1])
-                self._gemm2(P, uh, ul, _pack_conv(us.weight), y, bias=f32p(us.bias), conv=(N, h, w))
-                x = y
+        x, h, w = m._walk(x, h, w, resnet=resnet, xformer=xformer, downsample=downsample, upsample=upsample, release=lambda t: None)
         # ---- out: GroupNorm+SiLU -> (hi, lo); the 4-channel conv is linear, so conv(hi) + conv(lo) with fp32 weights ----
         th, tl = self._pair(N * h * w, boc[0])
         go, bo = f32p(m.conv_norm_out.weight), f32p(m.conv_norm_out.bias)
@@ -243,42 +212,3 @@ class EngineF32:
         P.append(lambda: ops.conv_out(th, co_w, co_b, self.out))
         P.append(lambda: ops.conv_out(tl, co_w, zero_b, out_lo))
         P.append(lambda: self.out.add_(out_lo))
-
-    # -- execution --------------------------------------------------------------------------------
-    def set_context(self, ctx):
-        # Cache hit only for the SAME live tensor object at the same version.  (The key used to be (data_ptr, version, shape):
-        # a new context tensor that the caching allocator placed at the freed address of the previous one -- same shape,
-        # version 0 -- was then taken for the old one and sampled with stale K/V.)
-        ref = self._ctx_key[0]() if self._ctx_key is not None else None
-        if ref is ctx and self._ctx_key[1] == ctx._version:
-            return
-        self.in_ctx.copy_(ctx.reshape(self.N * self.S, self.ctx_dim))
-        for op in self.ctx_plan:
-            op()
-        self._ctx_key = (weakref.ref(ctx), ctx._version)
-
-    def run(self, sample, timestep, ctx, use_graph=True):
-        with torch.cuda.device(self.device):
-            self.set_context(ctx)
-            self.in_sample.copy_(sample)
-            if torch.is_tensor(timestep):
-                self.in_t.copy_(timestep.to(device=self.device, dtype=F32).reshape(-1).expand(self.N))
-            else:
-                self.in_t.fill_(float(timestep))
-            if not use_graph:
-                for op in self.plan:
-                    op()
-            else:
-                if self.graph is None:
-                    for op in self.plan:
-                        op()
-                    torch.cuda.current_stream().synchronize()
-                    g = torch.cuda.CUDAGraph()
-                    before = ops.launch_count()
-                    with torch.cuda.graph(g):
-                        for op in self.plan:
-                            op()
-                    self.kernels_per_graph = ops.launch_count() - before
-                    self.graph = g
-                self.graph.replay()
-            return self.out.clone()

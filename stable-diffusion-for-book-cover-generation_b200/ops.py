@@ -67,6 +67,10 @@ def attention_workspace_bytes(batch, heads, Skv, d) -> int:
     return int(lib().b200sd_attention_workspace_bytes(batch, heads, Skv, d))
 
 
+def attention_bwd_workspace_bytes(batch, heads, Sq) -> int:
+    return int(lib().b200sd_attention_bwd_workspace_bytes(batch, heads, Sq))
+
+
 def launch_count() -> int:
     return int(lib().b200sd_launch_count())
 
@@ -113,6 +117,24 @@ def cfg_plms_step(eps_u, eps_c, x, hist, weights, guidance, cx, ce, out=None, ep
                                      len(hist), w, x.numel(), float(guidance), float(cx), float(ce), _dt(eps_u), _dt(x),
                                      _stream()), "cfg_plms_step")
     return out
+
+
+def sampler_advance(t_table, cursor, in_t):
+    """in_t[:] = t_table[cursor[0]]; cursor[0] += 1 (device-side step index of a captured denoising loop)"""
+    check(lib().b200sd_sampler_advance(_p(t_table), t_table.numel(), _p(cursor), _p(in_t), in_t.numel(), _stream()),
+          "sampler_advance")
+
+
+def cfg_ddim_step_table(eps_u, eps_c, x, out, guidance, coef_table, cursor):
+    """cfg_ddim_step() with the coefficients read from coef_table[cursor[0]] (fp32 tensors)"""
+    check(lib().b200sd_cfg_ddim_step_table(_p(eps_u), _p(eps_c), _p(x), _p(out), None, x.numel(), float(guidance), _p(coef_table),
+                                           _p(cursor), F32, F32, _stream()), "cfg_ddim_step_table")
+
+
+def cfg_plms_step_table(eps_u, eps_c, x, saved, ring, guidance, coef_table, cursor):
+    """cfg_plms_step() with weights, eps-ring slots and saved-sample flags read from coef_table[cursor[0]]; x is updated in place"""
+    check(lib().b200sd_cfg_plms_step_table(_p(eps_u), _p(eps_c), _p(x), _p(saved), _p(ring), x.numel(), float(guidance),
+                                           _p(coef_table), _p(cursor), _stream()), "cfg_plms_step_table")
 
 
 def add_noise(x0, noise, timesteps, sa_table, sb_table, out=None):
@@ -239,7 +261,7 @@ def gemm(a0, w, out, *, a1=None, bias=None, rowbias=None, residual=None, conv=No
     args.workspace, args.workspace_bytes = _p(ws), ws.numel()
     if not launch:
         return args
-    check(lib().b200sd_gemm(C.byref(args), _stream()), "gemm")
+    gemm_run(args)
     return out
 
 
@@ -317,8 +339,12 @@ def gemm_dgrad(dy, w, out, *, residual=None, conv=None, Cin=None, block_n=0, lau
     a.pair = pair
     if not launch:
         return a
-    check(lib().b200sd_gemm_dgrad(C.byref(a), _stream()), "gemm_dgrad")
+    gemm_dgrad_run(a)
     return out
+
+
+def gemm_dgrad_run(args):
+    check(lib().b200sd_gemm_dgrad(C.byref(args), _stream()), "gemm_dgrad")
 
 
 def gemm_wgrad(dy, x, dw, *, conv=None, lddw=0, block_n=0, split_k=0, launch=True):
@@ -336,8 +362,12 @@ def gemm_wgrad(dy, x, dw, *, conv=None, lddw=0, block_n=0, split_k=0, launch=Tru
     a.block_n, a.split_k = block_n, split_k
     if not launch:
         return a
-    check(lib().b200sd_gemm_wgrad(C.byref(a), _stream()), "gemm_wgrad")
+    gemm_wgrad_run(a)
     return dw
+
+
+def gemm_wgrad_run(args):
+    check(lib().b200sd_gemm_wgrad(C.byref(args), _stream()), "gemm_wgrad")
 
 
 def geglu_tile(N):
@@ -436,7 +466,7 @@ def attention_bwd(q, k, v, out, dout, lse, dq, dk, dv, batch, heads, Sq, Skv, d,
                   ws=None):
     """dq/dk/dv (bf16) of attention(); q/k/v and dq/dk/dv may be column slices (buffer + element offset)."""
     _chk(q, k, v, out, dout, lse, dq, dk, dv)
-    need = int(lib().b200sd_attention_bwd_workspace_bytes(batch, heads, Sq))
+    need = attention_bwd_workspace_bytes(batch, heads, Sq)
     if ws is None or ws.numel() < need:
         ws = _workspace("attn_bwd", need, q.device, zero=False)
     check(lib().b200sd_attention_bwd(q.data_ptr() + q_off * 2, k.data_ptr() + k_off * 2, v.data_ptr() + v_off * 2,

@@ -26,14 +26,14 @@ the new latents -- what bench.py reports as `e2e`.
 """
 from __future__ import annotations
 
-import ctypes as C
 import os
 
 import torch
 
 from . import ops
-from ._lib import B200SDError, check, lib
+from ._lib import B200SDError
 from .engine import Engine
+from .plan import run_plan
 
 
 def default_lanes(batch_images: int) -> int:
@@ -129,28 +129,21 @@ class CapturedSampler:
             eng = self.engines[l]
             lo, hi = self._slices[l]
             eng.in_ctx.copy_(self.ctx[lo:hi].reshape(-1, self.ctx.shape[-1]))
-            for op in eng.ctx_plan:
-                op()
+            run_plan(eng.ctx_plan)
         self._fork_join(lane)
 
     def _step_ops(self):
-        check(lib().b200sd_sampler_advance(self.t_table.data_ptr(), self.n_steps, self.cursor.data_ptr(), self.in_t.data_ptr(),
-                                           self.in_t.numel(), ops._stream()), "sampler_advance")
+        ops.sampler_advance(self.t_table, self.cursor, self.in_t)
         if self.lanes == 1:
             self.x2[:self.B].copy_(self.latents)
             self.x2[self.B:].copy_(self.latents)
-        self._fork_join(lambda l: self.engines[l]._run_plan())
+        self._fork_join(lambda l: run_plan(self.engines[l].plan))
         B = self.B
         if self.plms:
-            check(lib().b200sd_cfg_plms_step_table(self.eps[:B].data_ptr(), self.eps[B:].data_ptr(), self.latents.data_ptr(),
-                                                   self.saved.data_ptr(), self.ring.data_ptr(), self.latents.numel(), self.guidance,
-                                                   self.coef_table.data_ptr(), self.cursor.data_ptr(), ops._stream()),
-                  "cfg_plms_step_table")
+            ops.cfg_plms_step_table(self.eps[:B], self.eps[B:], self.latents, self.saved, self.ring, self.guidance, self.coef_table,
+                                    self.cursor)
             return
-        check(lib().b200sd_cfg_ddim_step_table(self.eps[:B].data_ptr(), self.eps[B:].data_ptr(), self.latents.data_ptr(),
-                                               self.latents.data_ptr(), None, self.latents.numel(), self.guidance,
-                                               self.coef_table.data_ptr(), self.cursor.data_ptr(), ops.F32, ops.F32,
-                                               ops._stream()), "cfg_ddim_step_table")
+        ops.cfg_ddim_step_table(self.eps[:B], self.eps[B:], self.latents, self.latents, self.guidance, self.coef_table, self.cursor)
 
     def _capture(self, body):
         """Warm up `body` on the capture stream (lazy one-time setup: function attributes, per-stream workspaces), then capture."""

@@ -25,6 +25,7 @@ import torch
 
 from . import ops
 from ._lib import B200SDError
+from .plan import Builder, Plan, Pool
 
 F32, BF16 = torch.float32, torch.bfloat16
 _ALIGN = 64  # elements: every region starts 128-byte aligned in the bf16 buffer (TMA needs 16)
@@ -228,40 +229,19 @@ class FlatParams:
                    else (r.param.data.data_ptr(), r.param.dtype) == r.src for r in self.order[:4] + self.order[-4:])
 
 
-class _Pool:
-    """scratch buffers for the backward: size-keyed free lists (all work is stream-ordered)"""
-
-    def __init__(self, device):
-        self.device, self.free, self.total = device, {}, 0
-
-    def get(self, rows, cols, dtype=BF16):
-        lst = self.free.get((rows * cols, dtype))
-        if lst:
-            return lst.pop().view(rows, cols)
-        self.total += rows * cols * (2 if dtype == BF16 else 4)
-        return torch.empty(rows, cols, dtype=dtype, device=self.device)
-
-    def put(self, *ts):
-        for t in ts:
-            if t is not None:
-                self.free.setdefault((t.numel(), t.dtype), []).append(t)
-
-
-class TrainEngine:
+class TrainEngine(Builder):
     def __init__(self, model, flat: FlatParams, N, H, W, S_ctx, device, train_weights=True, ctx_grad=False):
+        super().__init__(device)
         self.model, self.flat = model, flat
-        self.N, self.H, self.W, self.S, self.device = N, H, W, S_ctx, device
+        self.N, self.H, self.W, self.S = N, H, W, S_ctx
         self.train_weights, self.ctx_grad = train_weights, ctx_grad
         cfg = model.config
         self.heads, self.ctx_dim = cfg.attention_head_dim, cfg.cross_attention_dim
-        self.fwd, self.bwd = [], []
+        self.fwd, self.bwd = Plan(), Plan()
         self.ready_marks = []   # (number of backward entries executed, offset): flat.grad[offset:] is final
         self.saved_bytes = 0
-        self._keep = []
         self._gi = {}      # id(activation) -> [grad buffer, initialised?]
-        self._gn_parts = {}   # id(fp32 activation) -> ops.GnParts written by the GEMM that produced it
-        self.gn_from_gemm = __import__("os").environ.get("B200SD_TRAIN_GN_FROM_GEMM", "1") != "0"
-        self.pool = _Pool(device)
+        self.pool = Pool(device)
         with torch.cuda.device(device):
             self._build()
 
@@ -269,45 +249,6 @@ class TrainEngine:
     def _new(self, rows, cols, dtype=BF16):
         self.saved_bytes += rows * cols * (2 if dtype == BF16 else 4)
         return torch.empty(rows, cols, dtype=dtype, device=self.device)
-
-    def _gemm(self, plan, a0, w, out, **kw):
-        rb = kw.pop("rowbias_ptr", None)
-        gn_hw = kw.pop("gn_hw", 0)     # > 0: `out` feeds a GroupNorm -- the epilogue also publishes its column statistics (engine.py)
-        args = ops.gemm(a0, w, out, launch=False, **kw)
-        if rb is not None:
-            args.rowbias, args.ldrb, args.rows_per_image = rb
-        if gn_hw > 0 and self.gn_from_gemm:
-            parts = ops.gemm_attach_gn_parts(args, gn_hw, self.device)
-            if parts is not None:
-                self._gn_parts[id(out)] = parts      # forward buffers are never recycled here: the entry stays valid
-                self._keep.append(parts)
-        self._keep.append((a0, w, out, kw))
-        plan.append(lambda a=args: ops.gemm_run(a))
-
-    def _groupnorm(self, x, skip, g, b, out, hw, eps, silu, raw_out=None, stats_out=None):
-        """forward GroupNorm(+SiLU, +concat): apply-only from the producers' epilogue statistics when every source has them
-        (the forward keeps (mean, rstd) in stats_out for the backward either way)"""
-        N = self.N
-        p0 = self._gn_parts.get(id(x))
-        p1 = self._gn_parts.get(id(skip)) if skip is not None else None
-        C = x.shape[-1] + (skip.shape[-1] if skip is not None else 0)
-        if p0 is not None and (skip is None or p1 is not None) and ops.gn_parts_supported(C, 32):
-            self.fwd.append(lambda: ops.groupnorm_silu_parts(x, skip, p0, p1, g, b, out, N, hw, 32, eps, silu, raw_out=raw_out,
-                                                             stats_out=stats_out))
-        else:
-            self.fwd.append(lambda: ops.groupnorm_silu(x, skip, g, b, out, N, hw, 32, eps, silu, raw_out=raw_out, stats_out=stats_out))
-
-    def _dgrad(self, dy, w, out, **kw):
-        args = ops.gemm_dgrad(dy, w, out, launch=False, **kw)
-        self._keep.append((dy, w, out, kw))
-        self.bwd.append(lambda a=args: ops.check(ops.lib().b200sd_gemm_dgrad(ops.C.byref(a), ops._stream()), "gemm_dgrad"))
-
-    def _wgrad(self, dy, x, dw, **kw):
-        if not self.train_weights:
-            return
-        args = ops.gemm_wgrad(dy, x, dw, launch=False, **kw)
-        self._keep.append((dy, x, dw, kw))
-        self.bwd.append(lambda a=args: ops.check(ops.lib().b200sd_gemm_wgrad(ops.C.byref(a), ops._stream()), "gemm_wgrad"))
 
     def _grad_of(self, t):
         """(grad buffer of residual-stream activation t, accumulate?) -- first writer overwrites, later ones add"""
@@ -371,11 +312,7 @@ class TrainEngine:
         resnets = list(m._iter_resnets())
         tp_w = flat.span([r.time_emb_proj.weight for _, r in resnets], "wb")
         tp_b = flat.span([r.time_emb_proj.bias for _, r in resnets], "master")
-        n_tp = tp_w.shape[0]
-        tp_off, o = {}, 0
-        for prefix, r in resnets:
-            tp_off[prefix] = o
-            o += r.cout
+        tp_off, n_tp = m._tproj_offsets()
         t_sin = torch.empty(N, boc[0], **f32)
         t_h1 = torch.empty(N, temb_dim, **f32)      # linear_1 output, pre-SiLU
         t_emb = torch.empty(N, temb_dim, **f32)     # linear_2 output (the SiLU lives in each time_emb_proj)
@@ -388,7 +325,7 @@ class TrainEngine:
 
         self.attn_ws = torch.empty(ops.attention_workspace_bytes(N, heads, self.H * self.W, max(boc[0] // heads, 8)) + 256,
                                    dtype=torch.uint8, device=dev)
-        self.attn_bwd_ws = torch.empty(int(ops.lib().b200sd_attention_bwd_workspace_bytes(N, heads, self.H * self.W)) + 256,
+        self.attn_bwd_ws = torch.empty(ops.attention_bwd_workspace_bytes(N, heads, self.H * self.W) + 256,
                                        dtype=torch.uint8, device=dev)
 
         blocks = []   # backward builders, run in reverse
@@ -401,27 +338,27 @@ class TrainEngine:
             t1 = self._new(M, cin)
             raw = self._new(M, cin) if has_sc else None
             st1, st2 = torch.empty(N, 32, 2, **f32), torch.empty(N, 32, 2, **f32)   # GroupNorm (mean, rstd), kept for the backward
-            self._groupnorm(x, skip, self.P(r.norm1.weight), self.P(r.norm1.bias), t1, hw, eps, True, raw_out=raw, stats_out=st1)
+            self.groupnorm(Fp, x, skip, self.P(r.norm1.weight), self.P(r.norm1.bias), t1, N, hw, eps, True, raw_out=raw, stats_out=st1)
             hbuf = self._new(M, cout, F32)
             rb = (self.tproj.data_ptr() + tp_off[prefix] * 4, n_tp, hw)
-            self._gemm(Fp, t1, self.Wb(r.conv1.weight), hbuf, bias=self.P(r.conv1.bias), conv=(N, h, w), rowbias_ptr=rb, gn_hw=hw)
+            self.gemm(Fp, t1, self.Wb(r.conv1.weight), hbuf, bias=self.P(r.conv1.bias), conv=(N, h, w), rowbias_ptr=rb, gn_hw=hw)
             t2 = self._new(M, cout)
-            self._groupnorm(hbuf, None, self.P(r.norm2.weight), self.P(r.norm2.bias), t2, hw, eps, True, stats_out=st2)
+            self.groupnorm(Fp, hbuf, None, self.P(r.norm2.weight), self.P(r.norm2.bias), t2, N, hw, eps, True, stats_out=st2)
             if has_sc:
                 sc = self._new(M, cout, F32)
-                self._gemm(Fp, raw, self.Wb(r.conv_shortcut.weight), sc, bias=self.P(r.conv_shortcut.bias))
+                self.gemm(Fp, raw, self.Wb(r.conv_shortcut.weight), sc, bias=self.P(r.conv_shortcut.bias))
             else:
                 sc = x
             y = self._new(M, cout, F32)
-            self._gemm(Fp, t2, self.Wb(r.conv2.weight), y, bias=self.P(r.conv2.bias), residual=sc, conv=(N, h, w), gn_hw=hw)
+            self.gemm(Fp, t2, self.Wb(r.conv2.weight), y, bias=self.P(r.conv2.bias), residual=sc, conv=(N, h, w), gn_hw=hw)
 
             def backward():
                 pool = self.pool
                 dy = self._grad_ready(y)
                 dy16 = self._prep(dy, bias_param=r.conv2.bias if tw else None)
-                self._wgrad(dy16, t2, self.G(r.conv2.weight), conv=(N, h, w))
+                self.wgrad(Bp, dy16, t2, self.G(r.conv2.weight), conv=(N, h, w))
                 dt2 = pool.get(M, cout)
-                self._dgrad(dy16, self.Wb(r.conv2.weight), dt2, conv=(N, h, w))
+                self.dgrad(Bp, dy16, self.Wb(r.conv2.weight), dt2, conv=(N, h, w))
                 dh16 = pool.get(M, cout)
                 Bp.append(lambda: ops.groupnorm_silu_bwd(hbuf, None, self.P(r.norm2.weight), self.P(r.norm2.bias), dt2, dh16, None, N, hw,
                                                          dgamma=self.G(r.norm2.weight), dbeta=self.G(r.norm2.bias), eps=eps, silu=True,
@@ -432,16 +369,16 @@ class TrainEngine:
                 Bp.append(lambda: ops.grad_prep(dh16, None, dtp, rows_per_image=hw, ldcs=n_tp))
                 if tw:   # conv1.bias is added at the same place as the time embedding: its gradient is the sum over images
                     Bp.append(lambda: ops.grad_prep(dtp, None, self.G(r.conv1.bias), rows=N, N=cout, ld=n_tp))
-                self._wgrad(dh16, t1, self.G(r.conv1.weight), conv=(N, h, w))
+                self.wgrad(Bp, dh16, t1, self.G(r.conv1.weight), conv=(N, h, w))
                 dt1 = pool.get(M, cin)
-                self._dgrad(dh16, self.Wb(r.conv1.weight), dt1, conv=(N, h, w))
+                self.dgrad(Bp, dh16, self.Wb(r.conv1.weight), dt1, conv=(N, h, w))
                 pool.put(dh16)
                 if has_sc:
                     if tw:
                         Bp.append(lambda: ops.grad_prep(dy, None, self.G(r.conv_shortcut.bias)))
-                    self._wgrad(dy16, raw, self.G(r.conv_shortcut.weight))
+                    self.wgrad(Bp, dy16, raw, self.G(r.conv_shortcut.weight))
                     add = pool.get(M, cin, F32)
-                    self._dgrad(dy16, self.Wb(r.conv_shortcut.weight), add)
+                    self.dgrad(Bp, dy16, self.Wb(r.conv_shortcut.weight), add)
                 else:
                     add = dy
                 gx, accx = self._grad_of(x)
@@ -466,93 +403,93 @@ class TrainEngine:
             w_kv2 = flat.span([a2m.to_k.weight, a2m.to_v.weight], "wb")
             t = self._new(M, Cc)
             st = torch.empty(N, 32, 2, **f32)
-            self._groupnorm(x, None, self.P(a.norm.weight), self.P(a.norm.bias), t, hw, 1e-6, False, stats_out=st)
+            self.groupnorm(Fp, x, None, self.P(a.norm.weight), self.P(a.norm.bias), t, N, hw, 1e-6, False, stats_out=st)
             hs0 = self._new(M, Cc, F32)
-            self._gemm(Fp, t, self.Wb(a.proj_in.weight), hs0, bias=self.P(a.proj_in.bias))
+            self.gemm(Fp, t, self.Wb(a.proj_in.weight), hs0, bias=self.P(a.proj_in.bias))
             # self attention
             n1 = self._new(M, Cc)
             Fp.append(lambda: ops.layernorm(hs0, self.P(blk.norm1.weight), self.P(blk.norm1.bias), n1))
             qkv = self._new(M, 3 * Cc)
-            self._gemm(Fp, n1, w_qkv, qkv)
+            self.gemm(Fp, n1, w_qkv, qkv)
             at1 = self._new(M, Cc)
             lse1 = torch.empty(N, heads, hw, **f32)
             Fp.append(lambda: ops.attention_lse(qkv, qkv, qkv, at1, lse1, N, heads, hw, hw, d, scale, ldq=3 * Cc, ldk=3 * Cc,
                                                 ldv=3 * Cc, ldo=Cc, k_off=Cc, v_off=2 * Cc, ws=self.attn_ws))
             hs1 = self._new(M, Cc, F32)
-            self._gemm(Fp, at1, self.Wb(a1m.to_out[0].weight), hs1, bias=self.P(a1m.to_out[0].bias), residual=hs0)
+            self.gemm(Fp, at1, self.Wb(a1m.to_out[0].weight), hs1, bias=self.P(a1m.to_out[0].bias), residual=hs0)
             # cross attention
             n2 = self._new(M, Cc)
             Fp.append(lambda: ops.layernorm(hs1, self.P(blk.norm2.weight), self.P(blk.norm2.bias), n2))
             q2 = self._new(M, Cc)
-            self._gemm(Fp, n2, self.Wb(a2m.to_q.weight), q2)
+            self.gemm(Fp, n2, self.Wb(a2m.to_q.weight), q2)
             kv = self._new(N * S, 2 * Cc)
-            self._gemm(Fp, self.in_ctx, w_kv2, kv)
+            self.gemm(Fp, self.in_ctx, w_kv2, kv)
             at2 = self._new(M, Cc)
             lse2 = torch.empty(N, heads, hw, **f32)
             Fp.append(lambda: ops.attention_lse(q2, kv, kv, at2, lse2, N, heads, hw, S, d, scale, ldq=Cc, ldk=2 * Cc, ldv=2 * Cc,
                                                 ldo=Cc, v_off=Cc, ws=self.attn_ws))
             hs2 = self._new(M, Cc, F32)
-            self._gemm(Fp, at2, self.Wb(a2m.to_out[0].weight), hs2, bias=self.P(a2m.to_out[0].bias), residual=hs1)
+            self.gemm(Fp, at2, self.Wb(a2m.to_out[0].weight), hs2, bias=self.P(a2m.to_out[0].bias), residual=hs1)
             # GEGLU feed-forward (pre-activation kept)
             n3 = self._new(M, Cc)
             Fp.append(lambda: ops.layernorm(hs2, self.P(blk.norm3.weight), self.P(blk.norm3.bias), n3))
             u = self._new(M, 8 * Cc)
-            self._gemm(Fp, n3, self.Wb(ff.net[0].proj.weight), u, bias=self.P(ff.net[0].proj.bias))
+            self.gemm(Fp, n3, self.Wb(ff.net[0].proj.weight), u, bias=self.P(ff.net[0].proj.bias))
             f = self._new(M, 4 * Cc)
             Fp.append(lambda: ops.geglu_fwd(u, f))
             hs3 = self._new(M, Cc)
-            self._gemm(Fp, f, self.Wb(ff.net[2].weight), hs3, bias=self.P(ff.net[2].bias), residual=hs2)
+            self.gemm(Fp, f, self.Wb(ff.net[2].weight), hs3, bias=self.P(ff.net[2].bias), residual=hs2)
             y = self._new(M, Cc, F32)
-            self._gemm(Fp, hs3, self.Wb(a.proj_out.weight), y, bias=self.P(a.proj_out.bias), residual=x, gn_hw=hw)
+            self.gemm(Fp, hs3, self.Wb(a.proj_out.weight), y, bias=self.P(a.proj_out.bias), residual=x, gn_hw=hw)
 
             def backward():
                 pool = self.pool
                 dy = self._grad_ready(y)
                 dy16 = self._prep(dy, bias_param=a.proj_out.bias if tw else None)
-                self._wgrad(dy16, hs3, self.G(a.proj_out.weight))
+                self.wgrad(Bp, dy16, hs3, self.G(a.proj_out.weight))
                 dhs = pool.get(M, Cc, F32)
-                self._dgrad(dy16, self.Wb(a.proj_out.weight), dhs)
+                self.dgrad(Bp, dy16, self.Wb(a.proj_out.weight), dhs)
                 pool.put(dy16)
                 # feed-forward
                 g16 = self._prep(dhs, bias_param=ff.net[2].bias if tw else None)
-                self._wgrad(g16, f, self.G(ff.net[2].weight))
+                self.wgrad(Bp, g16, f, self.G(ff.net[2].weight))
                 dff = pool.get(M, 4 * Cc)
-                self._dgrad(g16, self.Wb(ff.net[2].weight), dff)
+                self.dgrad(Bp, g16, self.Wb(ff.net[2].weight), dff)
                 pool.put(g16)
                 du = pool.get(M, 8 * Cc)
                 Bp.append(lambda: ops.geglu_bwd(u, dff, du))
                 pool.put(dff)
                 if tw:
                     Bp.append(lambda: ops.grad_prep(du, None, self.G(ff.net[0].proj.bias)))
-                self._wgrad(du, n3, self.G(ff.net[0].proj.weight))
+                self.wgrad(Bp, du, n3, self.G(ff.net[0].proj.weight))
                 dn = pool.get(M, Cc)
-                self._dgrad(du, self.Wb(ff.net[0].proj.weight), dn)
+                self.dgrad(Bp, du, self.Wb(ff.net[0].proj.weight), dn)
                 pool.put(du)
                 Bp.append(lambda: ops.layernorm_bwd(hs2, self.P(blk.norm3.weight), dn, dhs, self.G(blk.norm3.weight), self.G(blk.norm3.bias)))
                 # cross attention
                 g16 = self._prep(dhs, bias_param=a2m.to_out[0].bias if tw else None)
-                self._wgrad(g16, at2, self.G(a2m.to_out[0].weight))
+                self.wgrad(Bp, g16, at2, self.G(a2m.to_out[0].weight))
                 da = pool.get(M, Cc)
-                self._dgrad(g16, self.Wb(a2m.to_out[0].weight), da)
+                self.dgrad(Bp, g16, self.Wb(a2m.to_out[0].weight), da)
                 pool.put(g16)
                 dq2 = pool.get(M, Cc)
                 dkv = pool.get(N * S, 2 * Cc)
                 Bp.append(lambda: ops.attention_bwd(q2, kv, kv, at2, da, lse2, dq2, dkv, dkv, N, heads, hw, S, d, scale, ldq=Cc,
                                                     ldk=2 * Cc, ldv=2 * Cc, lddq=Cc, lddk=2 * Cc, lddv=2 * Cc, v_off=Cc, dv_off=Cc,
                                                     ws=self.attn_bwd_ws))
-                self._wgrad(dq2, n2, self.G(a2m.to_q.weight))
-                self._dgrad(dq2, self.Wb(a2m.to_q.weight), dn)
+                self.wgrad(Bp, dq2, n2, self.G(a2m.to_q.weight))
+                self.dgrad(Bp, dq2, self.Wb(a2m.to_q.weight), dn)
                 if tw:
-                    self._wgrad(dkv, self.in_ctx, flat.span([a2m.to_k.weight, a2m.to_v.weight], "grad"))
+                    self.wgrad(Bp, dkv, self.in_ctx, flat.span([a2m.to_k.weight, a2m.to_v.weight], "grad"))
                 if self.ctx_grad:
-                    self._dgrad(dkv, w_kv2, self.d_ctx, residual=self.d_ctx if ctx_state["init"] else None)
+                    self.dgrad(Bp, dkv, w_kv2, self.d_ctx, residual=self.d_ctx if ctx_state["init"] else None)
                     ctx_state["init"] = True
                 pool.put(dq2, dkv)
                 Bp.append(lambda: ops.layernorm_bwd(hs1, self.P(blk.norm2.weight), dn, dhs, self.G(blk.norm2.weight), self.G(blk.norm2.bias)))
                 # self attention
                 g16 = self._prep(dhs, bias_param=a1m.to_out[0].bias if tw else None)
-                self._wgrad(g16, at1, self.G(a1m.to_out[0].weight))
-                self._dgrad(g16, self.Wb(a1m.to_out[0].weight), da)
+                self.wgrad(Bp, g16, at1, self.G(a1m.to_out[0].weight))
+                self.dgrad(Bp, g16, self.Wb(a1m.to_out[0].weight), da)
                 pool.put(g16)
                 dqkv = pool.get(M, 3 * Cc)
                 Bp.append(lambda: ops.attention_bwd(qkv, qkv, qkv, at1, da, lse1, dqkv, dqkv, dqkv, N, heads, hw, hw, d, scale,
@@ -560,14 +497,14 @@ class TrainEngine:
                                                     k_off=Cc, v_off=2 * Cc, dk_off=Cc, dv_off=2 * Cc, ws=self.attn_bwd_ws))
                 pool.put(da)
                 if tw:
-                    self._wgrad(dqkv, n1, flat.span([a1m.to_q.weight, a1m.to_k.weight, a1m.to_v.weight], "grad"))
-                self._dgrad(dqkv, w_qkv, dn)
+                    self.wgrad(Bp, dqkv, n1, flat.span([a1m.to_q.weight, a1m.to_k.weight, a1m.to_v.weight], "grad"))
+                self.dgrad(Bp, dqkv, w_qkv, dn)
                 pool.put(dqkv)
                 Bp.append(lambda: ops.layernorm_bwd(hs0, self.P(blk.norm1.weight), dn, dhs, self.G(blk.norm1.weight), self.G(blk.norm1.bias)))
                 # proj_in + GroupNorm
                 g16 = self._prep(dhs, bias_param=a.proj_in.bias if tw else None)
-                self._wgrad(g16, t, self.G(a.proj_in.weight))
-                self._dgrad(g16, self.Wb(a.proj_in.weight), dn)
+                self.wgrad(Bp, g16, t, self.G(a.proj_in.weight))
+                self.dgrad(Bp, g16, self.Wb(a.proj_in.weight), dn)
                 pool.put(g16, dhs)
                 gx, accx = self._grad_of(x)
                 Bp.append(lambda: ops.groupnorm_silu_bwd(x, None, self.P(a.norm.weight), self.P(a.norm.bias), dn, gx, None, N, hw, add_src=dy,
@@ -578,19 +515,19 @@ class TrainEngine:
             blocks.append((backward, a.norm.weight))
             return y
 
-        def downsample(ds, x, h, w):
+        def downsample(_prefix, ds, x, h, w):
             Cc = x.shape[1]
             col = self._new(N * (h // 2) * (w // 2), 9 * Cc)
             Fp.append(lambda: ops.im2col_s2(x, col, N, h, w))
             y = self._new(N * (h // 2) * (w // 2), Cc, F32)
-            self._gemm(Fp, col, self.Wb(ds.conv.weight), y, bias=self.P(ds.conv.bias), gn_hw=(h // 2) * (w // 2))
+            self.gemm(Fp, col, self.Wb(ds.conv.weight), y, bias=self.P(ds.conv.bias), gn_hw=(h // 2) * (w // 2))
 
             def backward():
                 dy = self._grad_ready(y)
                 dy16 = self._prep(dy, bias_param=ds.conv.bias if tw else None)
-                self._wgrad(dy16, col, self.G(ds.conv.weight))
+                self.wgrad(Bp, dy16, col, self.G(ds.conv.weight))
                 dcol = self.pool.get(col.shape[0], col.shape[1])
-                self._dgrad(dy16, self.Wb(ds.conv.weight), dcol)
+                self.dgrad(Bp, dy16, self.Wb(ds.conv.weight), dcol)
                 gx, accx = self._grad_of(x)
                 Bp.append(lambda: ops.col2im_s2(dcol, gx, N, h, w, accumulate=accx))
                 self.pool.put(dcol, dy16)
@@ -598,19 +535,19 @@ class TrainEngine:
             blocks.append((backward, ds.conv.weight))
             return y
 
-        def upsample(us, x, h, w):
+        def upsample(_prefix, us, x, h, w):
             Cc = x.shape[1]
             up = self._new(N * 4 * h * w, Cc)
             Fp.append(lambda: ops.upsample2x(x, up, N, h, w))
             y = self._new(N * 4 * h * w, Cc, F32)
-            self._gemm(Fp, up, self.Wb(us.conv.weight), y, bias=self.P(us.conv.bias), conv=(N, 2 * h, 2 * w), gn_hw=4 * h * w)
+            self.gemm(Fp, up, self.Wb(us.conv.weight), y, bias=self.P(us.conv.bias), conv=(N, 2 * h, 2 * w), gn_hw=4 * h * w)
 
             def backward():
                 dy = self._grad_ready(y)
                 dy16 = self._prep(dy, bias_param=us.conv.bias if tw else None)
-                self._wgrad(dy16, up, self.G(us.conv.weight), conv=(N, 2 * h, 2 * w))
+                self.wgrad(Bp, dy16, up, self.G(us.conv.weight), conv=(N, 2 * h, 2 * w))
                 dup = self.pool.get(up.shape[0], Cc)
-                self._dgrad(dy16, self.Wb(us.conv.weight), dup, conv=(N, 2 * h, 2 * w))
+                self.dgrad(Bp, dy16, self.Wb(us.conv.weight), dup, conv=(N, 2 * h, 2 * w))
                 gx, accx = self._grad_of(x)
                 Bp.append(lambda: ops.upsample2x_bwd(dup, gx, N, h, w, accumulate=accx))
                 self.pool.put(dup, dy16)
@@ -638,7 +575,7 @@ class TrainEngine:
                 Bp.append(lambda: ops.grad_prep(g, g16, self.G(m.conv_in.bias)))
                 Bp.append(lambda: x8.view(N, self.H, self.W, 8)[..., :cin].copy_(self.in_sample.permute(0, 2, 3, 1)))
                 Bp.append(lambda: dw8.zero_())
-                self._wgrad(g16, x8, dw8, conv=(N, self.H, self.W))
+                self.wgrad(Bp, g16, x8, dw8, conv=(N, self.H, self.W))
                 Bp.append(lambda: ci_w.g.view(boc[0], 9, cin).add_(dw8.view(boc[0], 9, 8)[..., :cin]))
                 self.pool.put(g16)
             else:
@@ -646,34 +583,14 @@ class TrainEngine:
                 Bp.append(lambda: ops.grad_prep(g, None, self.G(m.conv_in.bias)))
 
         blocks.append((conv_in_backward, m.conv_in.weight))
-        x = x0
-        skips = [x]
-        for i, b in enumerate(m.down_blocks):
-            for j, r in enumerate(b.resnets):
-                x = resnet(f"down{i}.res{j}", r, x, None, h, w)
-                if hasattr(b, "attentions"):
-                    x = xformer(f"down{i}.attn{j}", b.attentions[j], x, h, w)
-                skips.append(x)
-            if hasattr(b, "downsamplers"):
-                x = downsample(b.downsamplers[0], x, h, w)
-                h, w = h // 2, w // 2
-                skips.append(x)
-        x = resnet("mid.res0", m.mid_block.resnets[0], x, None, h, w)
-        x = xformer("mid.attn0", m.mid_block.attentions[0], x, h, w)
-        x = resnet("mid.res1", m.mid_block.resnets[1], x, None, h, w)
-        for i, b in enumerate(m.up_blocks):
-            for j, r in enumerate(b.resnets):
-                x = resnet(f"up{i}.res{j}", r, x, skips.pop(), h, w)
-                if hasattr(b, "attentions"):
-                    x = xformer(f"up{i}.attn{j}", b.attentions[j], x, h, w)
-            if hasattr(b, "upsamplers"):
-                x = upsample(b.upsamplers[0], x, h, w)
-                h, w = 2 * h, 2 * w
+        # every forward activation is saved for the backward: nothing is released
+        x, h, w = m._walk(x0, h, w, resnet=resnet, xformer=xformer, downsample=downsample, upsample=upsample, release=lambda t: None)
         co_w = flat.reg(m.conv_out.weight)
         x_last = x
         t_out = self._new(N * h * w, boc[0])
         st_out = torch.empty(N, 32, 2, **f32)
-        self._groupnorm(x_last, None, self.P(m.conv_norm_out.weight), self.P(m.conv_norm_out.bias), t_out, h * w, eps, True, stats_out=st_out)
+        self.groupnorm(Fp, x_last, None, self.P(m.conv_norm_out.weight), self.P(m.conv_norm_out.bias), t_out, N, h * w, eps, True,
+                       stats_out=st_out)
         Fp.append(lambda: ops.conv_out(t_out, co_w.wf, self.P(m.conv_out.bias), self.out))
 
         # ---- backward graph: head, then the blocks in reverse, then the time MLP ----
@@ -688,7 +605,7 @@ class TrainEngine:
             dwo = torch.zeros(8, 9 * boc[0], dtype=F32, device=dev)
             Bp.append(lambda: dy8.view(N, h, w, 8)[..., :cout].copy_(self.d_out.permute(0, 2, 3, 1)))
             Bp.append(lambda: dwo.zero_())
-            self._wgrad(dy8, t_out, dwo, conv=(N, h, w))
+            self.wgrad(Bp, dy8, t_out, dwo, conv=(N, h, w))
             Bp.append(lambda: co_w.g.add_(dwo[:cout]))
             Bp.append(lambda: self.G(m.conv_out.bias).add_(self.d_out.sum(dim=(0, 2, 3))))
         Bp.append(lambda: ops.conv_out_bwd(self.d_out, t_out, co_w.wf, dt_out, co_w.g if (tw and not tc_wgrad) else None,
@@ -720,23 +637,23 @@ class TrainEngine:
         Bp.append(lambda: ops.grad_prep(self.d_tproj, dtp16, g_tpb))
         a_emb = torch.empty(N, temb_dim, dtype=BF16, device=dev)
         Bp.append(lambda: ops.cast_act(t_emb, a_emb, silu=True))
-        self._wgrad(dtp16, a_emb, g_tpw)
+        self.wgrad(Bp, dtp16, a_emb, g_tpw)
         d_emb = torch.empty(N, temb_dim, dtype=F32, device=dev)
-        self._dgrad(dtp16, tp_w, d_emb)
+        self.dgrad(Bp, dtp16, tp_w, d_emb)
         Bp.append(lambda: ops.silu_bwd_mul(t_emb, d_emb))
         d_emb16 = torch.empty(N, temb_dim, dtype=BF16, device=dev)
         Bp.append(lambda: ops.grad_prep(d_emb, d_emb16, self.G(te.linear_2.bias)))
         a_h1 = torch.empty(N, temb_dim, dtype=BF16, device=dev)
         Bp.append(lambda: ops.cast_act(t_h1, a_h1, silu=True))
-        self._wgrad(d_emb16, a_h1, self.G(te.linear_2.weight))
+        self.wgrad(Bp, d_emb16, a_h1, self.G(te.linear_2.weight))
         d_h1 = torch.empty(N, temb_dim, dtype=F32, device=dev)
-        self._dgrad(d_emb16, self.Wb(te.linear_2.weight), d_h1)
+        self.dgrad(Bp, d_emb16, self.Wb(te.linear_2.weight), d_h1)
         Bp.append(lambda: ops.silu_bwd_mul(t_h1, d_h1))
         d_h116 = torch.empty(N, temb_dim, dtype=BF16, device=dev)
         Bp.append(lambda: ops.grad_prep(d_h1, d_h116, self.G(te.linear_1.bias)))
         a_sin = torch.empty(N, t_sin.shape[1], dtype=BF16, device=dev)
         Bp.append(lambda: ops.cast_act(t_sin, a_sin, silu=False))
-        self._wgrad(d_h116, a_sin, self.G(te.linear_1.weight))
+        self.wgrad(Bp, d_h116, a_sin, self.G(te.linear_1.weight))
 
     # -- execution --------------------------------------------------------------------------------
     def run_forward(self, sample, timestep, ctx):

@@ -357,15 +357,12 @@ class UNet2DConditionModel(nn.Module):
         te = self.time_embedding
         W["temb"] = dict(w1=packing.pack_linear(te.linear_1.weight.detach()), b1=f32(te.linear_1.bias),
                          w2=packing.pack_linear(te.linear_2.weight.detach()), b2=f32(te.linear_2.bias))
-        tp_w, tp_b, off = [], [], 0
-        self._tproj_off = {}
+        tp_w, tp_b = [], []
         for prefix, r in self._iter_resnets():
             res(prefix, r)
             tp_w.append(r.time_emb_proj.weight.detach())
             tp_b.append(r.time_emb_proj.bias.detach())
-            self._tproj_off[prefix] = off
-            off += r.cout
-        W["tproj"] = dict(w=packing.pack_linear(torch.cat(tp_w, 0)), b=f32(torch.cat(tp_b, 0)), n=off)
+        W["tproj"] = dict(w=packing.pack_linear(torch.cat(tp_w, 0)), b=f32(torch.cat(tp_b, 0)))
         for prefix, a in self._iter_xformers():
             xf(prefix, a)
         for i, b in enumerate(self.down_blocks):
@@ -430,6 +427,59 @@ class UNet2DConditionModel(nn.Module):
             if hasattr(b, "attentions"):
                 for j, a in enumerate(b.attentions):
                     yield f"up{i}.attn{j}", a
+
+    def _tproj_offsets(self):
+        """All time_emb_proj heads run as ONE linear over their row-concatenation (in _iter_resnets order): ({resnet prefix:
+        first output column of its head}, total columns)."""
+        off, o = {}, 0
+        for prefix, r in self._iter_resnets():
+            off[prefix] = o
+            o += r.cout
+        return off, o
+
+    def _walk(self, x, h, w, *, resnet, xformer, downsample, upsample, release):
+        """Drive the down / mid / up blocks from conv_in's output x (h x w); returns (x, h, w) of the last up block.
+            resnet(prefix, r, x, skip, h, w) -> y          skip: the down-path activation concatenated to x (None outside up)
+            xformer(prefix, a, x, h, w) -> y
+            downsample(prefix, s, x, h, w) -> y at h/2     s: the block's downsamplers[0]
+            upsample(prefix, s, x, h, w) -> y at 2h        s: the block's upsamplers[0]
+        The walk owns the skip stack and the liveness of activations: release(t) is called exactly once per activation, as
+        soon as it is neither the running activation nor a pending skip (never for the returned one)."""
+        skips = [x]
+
+        def advance(y):         # y replaces x as the running activation
+            nonlocal x
+            if all(s is not x for s in skips):
+                release(x)
+            x = y
+
+        for i, b in enumerate(self.down_blocks):
+            for j, r in enumerate(b.resnets):
+                advance(resnet(f"down{i}.res{j}", r, x, None, h, w))
+                if hasattr(b, "attentions"):
+                    advance(xformer(f"down{i}.attn{j}", b.attentions[j], x, h, w))
+                skips.append(x)
+            if hasattr(b, "downsamplers"):
+                advance(downsample(f"down{i}.ds", b.downsamplers[0], x, h, w))
+                h, w = h // 2, w // 2
+                skips.append(x)
+        mid = self.mid_block
+        advance(resnet("mid.res0", mid.resnets[0], x, None, h, w))
+        advance(xformer("mid.attn0", mid.attentions[0], x, h, w))
+        advance(resnet("mid.res1", mid.resnets[1], x, None, h, w))
+        for i, b in enumerate(self.up_blocks):
+            for j, r in enumerate(b.resnets):
+                skip = skips.pop()
+                y = resnet(f"up{i}.res{j}", r, x, skip, h, w)
+                if skip is not x and all(s is not skip for s in skips):
+                    release(skip)
+                advance(y)
+                if hasattr(b, "attentions"):
+                    advance(xformer(f"up{i}.attn{j}", b.attentions[j], x, h, w))
+            if hasattr(b, "upsamplers"):
+                advance(upsample(f"up{i}.us", b.upsamplers[0], x, h, w))
+                h, w = 2 * h, 2 * w
+        return x, h, w
 
     # -- forward --------------------------------------------------------------------------------
     def forward(self, sample, timestep, encoder_hidden_states, return_dict: bool = True):

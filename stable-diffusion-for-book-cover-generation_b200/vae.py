@@ -26,7 +26,7 @@ import torch.nn as nn
 
 from . import ops, packing
 from ._lib import B200SDError
-from .engine import _Plan, _Pool
+from .plan import Builder, Plan, Pool, capture, profile_plan, run_plan
 from .unet import _Config, _P, _conv, _lin
 
 SD15_VAE_CONFIG = dict(in_channels=3, out_channels=3, latent_channels=4, block_out_channels=(128, 256, 512, 512),
@@ -142,29 +142,22 @@ class _Decoder(nn.Module):
 
 
 # ---- launch plans ----------------------------------------------------------------------------------------
-class _VaeEngine:
-    """Shared plan-building blocks of the encoder / decoder plans (mirrors engine.Engine's helpers)."""
+class _VaeEngine(Builder):
+    """Plan-building blocks shared by the encoder / decoder plans."""
 
     def __init__(self, model, B, H, W, device):
-        self.model, self.B, self.H, self.W, self.device = model, B, H, W, device
-        self.plan = _Plan()
-        self.pool = _Pool(device)
-        self._keep = []
+        super().__init__(device)
+        self.model, self.B, self.H, self.W = model, B, H, W
+        self.plan = Plan()
+        self.pool = Pool(device)
         self.graph = None
         self.groups = model.config.norm_num_groups
         with torch.cuda.device(device):
             self._build()
         self.activation_bytes = self.pool.total
 
-    def _gemm(self, a0, w, out, **kw):
-        args = ops.gemm(a0, w, out, launch=False, **kw)
-        self._keep.append((a0, w, out, kw))
-        kind = "conv3x3" if args.conv_taps == 9 else "gemm"
-        self.plan.append(lambda a=args: ops.gemm_run(a), kind, 2.0 * args.M * args.N * args.K, f"{kind} M{args.M} N{args.N} K{args.K}")
-
     def _gn(self, x, g, b, out, hw, silu, raw_out=None):
-        B = self.B
-        self.plan.append(lambda: ops.groupnorm_silu(x, None, g, b, out, B, hw, self.groups, 1e-6, silu, raw_out=raw_out), "groupnorm")
+        self.groupnorm(self.plan, x, None, g, b, out, self.B, hw, 1e-6, silu, groups=self.groups, raw_out=raw_out)
 
     def _resnet(self, w, x, h, wd):
         B, pool = self.B, self.pool
@@ -174,19 +167,19 @@ class _VaeEngine:
         raw = pool.get(M, cin) if "wsc" in w else None
         self._gn(x, w["g1"], w["b1"], t1, h * wd, True, raw_out=raw)
         hb = pool.get(M, cout, F32)
-        self._gemm(t1, w["w1"], hb, bias=w["cb1"], conv=(B, h, wd))
+        self.gemm(self.plan, t1, w["w1"], hb, bias=w["cb1"], conv=(B, h, wd))
         pool.put(t1)
         t2 = pool.get(M, cout)
         self._gn(hb, w["g2"], w["b2"], t2, h * wd, True)
         pool.put(hb)
         if raw is not None:
             sc = pool.get(M, cout, F32)
-            self._gemm(raw, w["wsc"], sc, bias=w["bsc"])
+            self.gemm(self.plan, raw, w["wsc"], sc, bias=w["bsc"])
             pool.put(raw)
         else:
             sc = x
         y = pool.get(M, cout, F32)
-        self._gemm(t2, w["w2"], y, bias=w["cb2"], residual=sc, conv=(B, h, wd))
+        self.gemm(self.plan, t2, w["w2"], y, bias=w["cb2"], residual=sc, conv=(B, h, wd))
         pool.put(t2)
         if sc is not x:
             pool.put(sc)
@@ -201,23 +194,20 @@ class _VaeEngine:
         t = pool.get(M, C)
         self._gn(x, w["g"], w["b"], t, S, False)
         q, k, v = pool.get(M, C), pool.get(M, C), pool.get(M, C)
-        self._gemm(t, w["wq"], q, bias=w["bq"])
-        self._gemm(t, w["wk"], k, bias=w["bk"])
-        self._gemm(t, w["wv"], v, bias=w["bv"])
+        self.gemm(self.plan, t, w["wq"], q, bias=w["bq"])
+        self.gemm(self.plan, t, w["wk"], k, bias=w["bk"])
+        self.gemm(self.plan, t, w["wv"], v, bias=w["bv"])
         scores = pool.get(S, S, F32)
         probs = pool.get(S, S)
         o = t                                          # the normalised input is dead once q, k, v exist
         scale = float(C) ** -0.5                       # (q C^-1/4) . (k C^-1/4)
         for b in range(B):
             qb, kb, vb, ob = (z[b * S:(b + 1) * S] for z in (q, k, v, o))
-            self._gemm(qb, kb, scores)                                           # scores = q k^T  (k is the "weight" operand)
+            self.gemm(self.plan, qb, kb, scores)                                           # scores = q k^T  (k is the "weight" operand)
             self.plan.append(lambda: ops.softmax_rows(scores, probs, scale), "attention", 0, "softmax rows")
-            args = ops.gemm_dgrad(probs, vb, ob, launch=False)                   # out = P v  (v read MN-major: no transpose)
-            self._keep.append((probs, vb, ob))
-            self.plan.append(lambda a=args: ops.check(ops.lib().b200sd_gemm_dgrad(ops.C.byref(a), ops._stream()), "gemm_dgrad"),
-                             "gemm", 2.0 * S * S * C, f"attention P.v S{S} C{C}")
+            self.dgrad(self.plan, probs, vb, ob, name=f"attention P.v S{S} C{C}")   # out = P v  (v read MN-major: no transpose)
         y = pool.get(M, C, F32)
-        self._gemm(o, w["wo"], y, bias=w["bo"], residual=x)
+        self.gemm(self.plan, o, w["wo"], y, bias=w["bo"], residual=x)
         for z in (q, k, v, scores, probs, t, x):
             pool.put(z)
         return y
@@ -229,7 +219,6 @@ class _VaeEngine:
         return self._resnet(W[prefix + ".res1"], x, h, wd)
 
     def profile(self, iters=3):
-        from .engine import profile_plan
         return profile_plan(self.plan, self.device, iters)
 
     def _replay(self, set_inputs):
@@ -237,16 +226,10 @@ class _VaeEngine:
             set_inputs()
             if self.graph is not None:
                 self.graph.replay()
+            elif self.model.use_cuda_graph:
+                self.graph, _ = capture(self.plan)
             else:
-                for op in self.plan:             # first call: eager (lazy one-time setup happens outside any capture)
-                    op()
-                if self.model.use_cuda_graph:
-                    torch.cuda.current_stream().synchronize()
-                    g = torch.cuda.CUDAGraph()
-                    with torch.cuda.graph(g):
-                        for op in self.plan:
-                            op()
-                    self.graph = g
+                run_plan(self.plan)
             return self.out.clone()
 
 
@@ -276,7 +259,7 @@ class VaeDecodeEngine(_VaeEngine):
                 pool.put(x)
                 h, w = 2 * h, 2 * w
                 x = pool.get(B * h * w, C, F32)
-                self._gemm(up, wu["w"], x, bias=wu["b"], conv=(B, h, w))
+                self.gemm(self.plan, up, wu["w"], x, bias=wu["b"], conv=(B, h, w))
                 pool.put(up)
         wo = Wp["dec.conv_out"]
         t = pool.get(B * h * w, rev[-1])
@@ -285,8 +268,7 @@ class VaeDecodeEngine(_VaeEngine):
         # conv_out (128 -> 3) on the tensor cores: [x | x] . [w_hi | w_lo] per tap (fp32-accurate weights), the 3 channels padded
         # to a 32-wide tile, then bias + NHWC -> NCHW (the CUDA-core kernel took 0.5 ms of an 11 ms decode at 512 x 512)
         tmp = pool.get(B * h * w, 32, F32)
-        self._gemm(t, wo["w_tc"], tmp, a1=t, conv=(B, h, w), block_n=32)
-        self.plan.meta[-1] = ("conv_io", self.plan.meta[-1][1], "decoder conv_out (tensor cores)")
+        self.gemm(P, t, wo["w_tc"], tmp, a1=t, conv=(B, h, w), block_n=32, kind="conv_io", name="decoder conv_out (tensor cores)")
         P.append(lambda tmp=tmp: ops.nhwc_bias_to_nchw(tmp, wo["b"], self.out), "conv_io", 0, "decoder conv_out: bias + NCHW")
 
     def run(self, z):
@@ -315,14 +297,14 @@ class VaeEncodeEngine(_VaeEngine):
                 pool.put(x)
                 h, w = h // 2, w // 2
                 x = pool.get(B * h * w, C, F32)
-                self._gemm(col, wd_["w"], x, bias=wd_["b"])
+                self.gemm(self.plan, col, wd_["w"], x, bias=wd_["b"])
                 pool.put(col)
         x = self._mid("enc.mid", x, h, w)
         wo = Wp["enc.conv_out"]
         t = pool.get(B * h * w, boc[-1])
         self._gn(x, wo["g"], wo["beta"], t, h * w, True)
         tmp = pool.get(B * h * w, 32, F32)
-        self._gemm(t, wo["w_tc"], tmp, a1=t, conv=(B, h, w), block_n=32)
+        self.gemm(self.plan, t, wo["w_tc"], tmp, a1=t, conv=(B, h, w), block_n=32)
         self.out = torch.zeros(B, 2 * cfg.latent_channels, h, w, dtype=F32, device=dev)
         P.append(lambda tmp=tmp: ops.nhwc_bias_to_nchw(tmp, wo["b"], self.out), "conv_io", 0, "conv_out + quant_conv: bias + NCHW")
 

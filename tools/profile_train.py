@@ -13,9 +13,9 @@ from b200sd.unet import UNet2DConditionModel
 
 def kind_of(fn):
     names = fn.__code__.co_names
-    for n in ("b200sd_gemm_dgrad", "b200sd_gemm_wgrad", "gemm_run"):
+    for n in ("gemm_dgrad_run", "gemm_wgrad_run", "gemm_run"):
         if n in names:
-            return n.replace("b200sd_", "")
+            return n
     for n in names:
         if hasattr(ops, n) and n not in ("check", "lib", "C"):
             return n

@@ -1,4 +1,4 @@
-"""In-step per-launch times of the VAE decode / encode plans (engine.profile_plan) on random-init SD v1.x weights."""
+"""In-step per-launch times of the VAE decode / encode plans (plan.profile_plan) on random-init SD v1.x weights."""
 import sys, torch
 sys.path.insert(0, '.')
 from b200sd.vae import AutoencoderKL
