@@ -44,10 +44,7 @@ int64_t b200sd_launch_count(void);
 /* In-graph timers (measurement plumbing, SURVEY.md 8d): process-wide CUDA events.  b200sd_timer_record(i) records event i on
  * `stream`; while the stream is being captured the record becomes an external event-record node, so a replay of the captured
  * plan timestamps the gaps between its kernels and b200sd_timer_elapsed_ms(i, j) gives per-kernel times inside the real step. */
-/* debug: every CTA of the GEMM kernels stamps %globaltimer at 8 phase boundaries into buf[cta][8] (NULL switches it off) */
-void b200sd_debug_gemm_trace(void* buf);
-/* debug / tuning overrides of the GEMM launch policy: key 0 = persistent kernel (-1 default, 0 off, 1 on), 1 = smem ring depth cap
- * (0 = auto), 2 = cap on the persistent grid (0 = one CTA per SM) */
+/* debug override of the GEMM launch policy: key 0 = persistent kernel (-1 default, 0 off, 1 on); other keys are ignored */
 void b200sd_debug_set(int key, int value);
 int b200sd_timer_reserve(int n);
 int b200sd_timer_record(int i, b200sd_stream_t stream);
@@ -146,8 +143,6 @@ int b200sd_small_linear(const float* in, const void* w_bf16, const float* bias, 
  */
 #define B200SD_EPI_LINEAR 0
 #define B200SD_EPI_GEGLU 1
-#define B200SD_W_ROW_MAJOR 0
-#define B200SD_W_KBLOCK_MAJOR 1
 
 typedef struct b200sd_gemm_args {
     const void* a0;        /* bf16 */
@@ -175,12 +170,6 @@ typedef struct b200sd_gemm_args {
     int pair;              /* CTA pairs (tcgen05 cta_group::2, 256-row MMA tiles): 0 = auto, 1 = on, -1 = off */
     float* gn_part;        /* optional: per-CTA column statistics [parts][2][N] of the fp32 output (sum | sum of squares over the
                               rows each CTA stores), consumed by b200sd_groupnorm_silu_parts; layout from b200sd_gemm_gn_layout */
-    const void* prefetch;  /* optional: memory the NEXT kernels of the stream will stream from HBM (the next layer's weights): this
-                              launch pulls prefetch_bytes of it into L2 while it runs (cp.async.bulk.prefetch.L2, spread over its CTAs) */
-    size_t prefetch_bytes;
-    int w_layout;          /* B200SD_W_ROW_MAJOR: w is [N][K]; B200SD_W_KBLOCK_MAJOR: w is [K/64][N][64] (the 64-wide k-blocks of
-                              all N rows stored together), so the weight tile of one k-block is one contiguous run of DRAM --
-                              the layout for weights that are streamed from HBM once per step (small-M / deep-K layers) */
 } b200sd_gemm_args;
 
 size_t b200sd_gemm_workspace_bytes(void);

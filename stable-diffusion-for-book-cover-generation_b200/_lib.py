@@ -23,7 +23,7 @@ class GemmArgs(C.Structure):
         ("lda0", C.c_int), ("lda1", C.c_int), ("ldc", C.c_int), ("ldr", C.c_int), ("ldrb", C.c_int), ("conv_taps", C.c_int),
         ("batch", C.c_int), ("H", C.c_int), ("W", C.c_int), ("rows_per_image", C.c_int), ("epilogue", C.c_int),
         ("out_dtype", C.c_int), ("residual_dtype", C.c_int), ("block_n", C.c_int), ("split_k", C.c_int),
-        ("workspace", C.c_void_p), ("workspace_bytes", C.c_size_t), ("pair", C.c_int), ("gn_part", C.c_void_p), ("prefetch", C.c_void_p), ("prefetch_bytes", C.c_size_t), ("w_layout", C.c_int),
+        ("workspace", C.c_void_p), ("workspace_bytes", C.c_size_t), ("pair", C.c_int), ("gn_part", C.c_void_p),
     ]
 
 
@@ -52,7 +52,6 @@ SIGNATURES = {
     "b200sd_last_error": (C.c_char_p, []),
     "b200sd_version": (_i, []),
     "b200sd_launch_count": (_i64, []),
-    "b200sd_debug_gemm_trace": (None, [_vp]),
     "b200sd_debug_set": (None, [_i, _i]),
     "b200sd_timer_reserve": (_i, [_i]),
     "b200sd_timer_record": (_i, [_i, _vp]),

@@ -2,7 +2,6 @@
 #include <atomic>
 #include <cstdarg>
 #include <cstdio>
-#include <cstdlib>
 #include <mutex>
 
 #include "common.cuh"
@@ -42,7 +41,7 @@ cudaError_t b200sd_opt_in_smem_impl(const void* kernel, int bytes, bool max_carv
     configured[key] = bytes;
     return cudaSuccess;
 }
-extern "C" int b200sd_version(void) { return 100; }
+extern "C" int b200sd_version(void) { return 101; }
 extern "C" int64_t b200sd_launch_count(void) { return g_b200sd_launches.load(); }
 
 // ---- in-graph timers: events recorded with cudaEventRecordExternal, so that a captured plan can carry a timestamp between
@@ -71,15 +70,6 @@ extern "C" int b200sd_timer_elapsed_ms(int i, int j, float* ms) {
     B200SD_REQUIRE(ms && i >= 0 && j >= 0 && i < (int)g_timers.size() && j < (int)g_timers.size(), "timer_elapsed: bad index");
     B200SD_CUDA(cudaEventElapsedTime(ms, g_timers[i], g_timers[j]));
     return B200SD_OK;
-}
-
-bool b200sd_pdl_enabled() {
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("B200SD_PDL");
-        v = (e && e[0] == '1') ? 1 : 0;  // measured on B200: no gain for this dependent chain of short kernels -> opt-in
-    }
-    return v != 0;
 }
 
 int b200sd_num_sms() {

@@ -7,7 +7,6 @@
 // shared memory (zero-filled), key tails (S_kv = 77) are masked to -inf.  The tcgen05/TMEM version
 // of this kernel is the next step for this row (DESIGN.md).
 #include <atomic>
-#include <cstdlib>
 
 #include "common.cuh"
 
@@ -73,7 +72,6 @@ __global__ void __launch_bounds__(kThreads, (DP <= 80) ? 2 : 1)
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int chunks = D / 8;
 
-    ptx::pdl_trigger();
     // zero the head-dim padding once (cp.async never touches it)
     {
         constexpr int PAD16 = PITCH / 16;  // 16-byte slots per row incl. the bank-skew slot
@@ -84,7 +82,6 @@ __global__ void __launch_bounds__(kThreads, (DP <= 80) ? 2 : 1)
         }
     }
 
-    ptx::pdl_wait();
     const bf16* qg = q + ((size_t)b * Sq + q0) * ldq + h * D;
     const bf16* kg = k + (size_t)b * Skv * ldk + h * D;
     const bf16* vg = v + (size_t)b * Skv * ldv + h * D;
@@ -229,8 +226,8 @@ int launch_attention(const bf16* q, const bf16* k, const bf16* v, bf16* out, flo
     const size_t smem = (size_t)(kBM + 4 * kBN) * PITCH;
     B200SD_CUDA(b200sd_opt_in_smem(attention_kernel<DP>, (int)smem));
     dim3 grid(ceil_div(Sq, kBM), heads, batch);
-    B200SD_CUDA(b200sd_launch(attention_kernel<DP>, dim3(grid), dim3(kThreads), smem, s, q, k, v, out, lse, Sq, Skv, D, ldq, ldk, ldv, ldo,
-                                                      scale * 1.4426950408889634f));
+    attention_kernel<DP><<<dim3(grid), dim3(kThreads), smem, s>>>(q, k, v, out, lse, Sq, Skv, D, ldq, ldk, ldv, ldo,
+                                                      scale * 1.4426950408889634f);
     g_b200sd_launches.fetch_add(1, std::memory_order_relaxed);
     B200SD_LAUNCH_CHECK();
     return B200SD_OK;
@@ -263,12 +260,9 @@ extern "C" int b200sd_attention_lse(const void* q, const void* k, const void* v,
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     {
         // tensor-core (tcgen05/TMEM) path for the self-attention-sized shapes
-        static const bool no_tc = getenv("B200SD_ATTN_TC") && getenv("B200SD_ATTN_TC")[0] == '0';
-        if (!no_tc) {
-            const int rc = b200sd_attention_tc(q, k, v, out, lse, batch, heads, Sq, Skv, d, ldq, ldk, ldv, ldo, scale, workspace,
-                                               workspace_bytes, s);
-            if (rc != B200SD_ERR_UNSUPPORTED) return rc;
-        }
+        const int rc = b200sd_attention_tc(q, k, v, out, lse, batch, heads, Sq, Skv, d, ldq, ldk, ldv, ldo, scale, workspace,
+                                           workspace_bytes, s);
+        if (rc != B200SD_ERR_UNSUPPORTED) return rc;
     }
     const bf16* qq = static_cast<const bf16*>(q);
     const bf16* kk = static_cast<const bf16*>(k);

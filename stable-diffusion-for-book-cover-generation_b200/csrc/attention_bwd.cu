@@ -10,7 +10,6 @@
 // forward kernel in attention.cu; head dims 40 / 80 / 160 are zero-padded to a multiple of 16 in shared memory.
 // For head dims > 96 the dK/dV accumulators are split in two halves of d across CTAs (register budget).
 #include <atomic>
-#include <cstdlib>
 
 #include "common.cuh"
 
@@ -120,8 +119,6 @@ struct BwdParams {
 // ---- delta[b, h, row] = sum_d dO o O -------------------------------------------------------------------------
 __global__ void attn_delta_kernel(const bf16* __restrict__ o, const bf16* __restrict__ dout, float* __restrict__ delta,
                                   int batch, int heads, int Sq, int D, int ldo, int lddo) {
-    ptx::pdl_trigger();
-    ptx::pdl_wait();
     const int64_t total = (int64_t)batch * Sq * heads;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
         const int h = (int)(i % heads);
@@ -152,9 +149,7 @@ __global__ void __launch_bounds__(kThreads) attn_bwd_dq_kernel(const BwdParams p
     const int b = blockIdx.z, h = blockIdx.y, q0 = blockIdx.x * kT;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int D = p.D, chunks = D / 8;
-    ptx::pdl_trigger();
     zero_pad<PITCH>(smem, 6 * kT, chunks);
-    ptx::pdl_wait();
     const bf16* qg = p.q + ((size_t)b * p.Sq + q0) * p.ldq + h * D;
     const bf16* dog = p.dout + ((size_t)b * p.Sq + q0) * p.ldo + h * D;
     const bf16* kg = p.k + (size_t)b * p.Skv * p.ldk + h * D;
@@ -234,9 +229,7 @@ __global__ void __launch_bounds__(kThreads) attn_bwd_dkv_kernel(const BwdParams 
     const int k0 = kt * kT, d0 = dh * NKS * 16;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int D = p.D, chunks = D / 8;
-    ptx::pdl_trigger();
     zero_pad<PITCH>(smem, 6 * kT, chunks);
-    ptx::pdl_wait();
     const bf16* kg = p.k + ((size_t)b * p.Skv + k0) * p.ldk + h * D;
     const bf16* vg = p.v + ((size_t)b * p.Skv + k0) * p.ldv + h * D;
     const bf16* qg = p.q + (size_t)b * p.Sq * p.ldq + h * D;
@@ -329,9 +322,10 @@ int launch_bwd(const BwdParams& p, int batch, cudaStream_t s) {
     const size_t smem_dkv = (size_t)6 * kT * PITCH + 4 * kT * sizeof(float);
     B200SD_CUDA(b200sd_opt_in_smem(attn_bwd_dq_kernel<DP>, (int)smem_dq));
     B200SD_CUDA(b200sd_opt_in_smem(attn_bwd_dkv_kernel<DP, DSPLIT>, (int)smem_dkv));
-    B200SD_CUDA(b200sd_launch(attn_bwd_dq_kernel<DP>, dim3(ceil_div(p.Sq, kT), p.heads, batch), dim3(kThreads), smem_dq, s, p));
+    attn_bwd_dq_kernel<DP><<<dim3(ceil_div(p.Sq, kT), p.heads, batch), dim3(kThreads), smem_dq, s>>>(p);
     COUNT_LAUNCH();
-    B200SD_CUDA(b200sd_launch(attn_bwd_dkv_kernel<DP, DSPLIT>, dim3(ceil_div(p.Skv, kT) * DSPLIT, p.heads, batch), dim3(kThreads), smem_dkv, s, p));
+    B200SD_LAUNCH_CHECK();
+    attn_bwd_dkv_kernel<DP, DSPLIT><<<dim3(ceil_div(p.Skv, kT) * DSPLIT, p.heads, batch), dim3(kThreads), smem_dkv, s>>>(p);
     COUNT_LAUNCH();
     B200SD_LAUNCH_CHECK();
     return B200SD_OK;
@@ -368,20 +362,18 @@ extern "C" int b200sd_attention_bwd(const void* q, const void* k, const void* v,
         int blocks = (int)((total + 255) / 256);
         const int cap = b200sd_num_sms() * 8;
         if (blocks > cap) blocks = cap;
-        B200SD_CUDA(b200sd_launch(attn_delta_kernel, dim3(blocks), dim3(256), 0, s, static_cast<const bf16*>(out), static_cast<const bf16*>(dout),
-                                  delta, batch, heads, Sq, d, ldo, lddo));
+        attn_delta_kernel<<<dim3(blocks), dim3(256), 0, s>>>(static_cast<const bf16*>(out), static_cast<const bf16*>(dout),
+                                  delta, batch, heads, Sq, d, ldo, lddo);
         COUNT_LAUNCH();
+        B200SD_LAUNCH_CHECK();
     }
     {
         // tensor-core (tcgen05 / TMEM) kernels for the self-attention-sized shapes
-        static const bool no_tc = getenv("B200SD_ATTN_BWD_TC") && getenv("B200SD_ATTN_BWD_TC")[0] == '0';
-        if (!no_tc) {
-            const int rc = b200sd_attention_bwd_tc(static_cast<const bf16*>(q), static_cast<const bf16*>(k), static_cast<const bf16*>(v),
-                                                   static_cast<const bf16*>(dout), lse, delta, static_cast<bf16*>(dq), static_cast<bf16*>(dk),
-                                                   static_cast<bf16*>(dv), batch, heads, Sq, Skv, d, ldq, ldk, ldv, lddo, lddq, lddk, lddv,
-                                                   scale, s);
-            if (rc != B200SD_ERR_UNSUPPORTED) return rc;
-        }
+        const int rc = b200sd_attention_bwd_tc(static_cast<const bf16*>(q), static_cast<const bf16*>(k), static_cast<const bf16*>(v),
+                                               static_cast<const bf16*>(dout), lse, delta, static_cast<bf16*>(dq), static_cast<bf16*>(dk),
+                                               static_cast<bf16*>(dv), batch, heads, Sq, Skv, d, ldq, ldk, ldv, lddo, lddq, lddk, lddv,
+                                               scale, s);
+        if (rc != B200SD_ERR_UNSUPPORTED) return rc;
     }
     BwdParams p;
     p.q = static_cast<const bf16*>(q); p.k = static_cast<const bf16*>(k); p.v = static_cast<const bf16*>(v);

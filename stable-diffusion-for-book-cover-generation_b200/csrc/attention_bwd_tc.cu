@@ -17,7 +17,6 @@
 //               tcgen05.ld, exp2 / FMA in fp32, bf16 P^T / dS^T written into 128B-swizzled smem tiles (the A operands
 //               of the accumulating MMAs); at the end the accumulators are scaled and stored as bf16.
 #include <atomic>
-#include <cstdlib>
 #include <cstring>
 
 #include "common.cuh"
@@ -119,7 +118,6 @@ __global__ void __launch_bounds__(kThreads, 1) attn_bwd_tc_kernel(const __grid_c
     const int num_tiles = p.Sy / kT;
     const int Sq = DKV ? p.Sy : p.Sx;
 
-    ptx::pdl_trigger();
     if (warp == 0 && lane == 0) {
         ptx::prefetch_tmap(&p.tmX1);
         ptx::prefetch_tmap(&p.tmX2);
@@ -150,7 +148,6 @@ __global__ void __launch_bounds__(kThreads, 1) attn_bwd_tc_kernel(const __grid_c
     // ATMEM: P^T operand [384,448), dS^T operand [448,512): 64 bf16 (= 32 columns) per 64-row half of the streamed tile
     const uint32_t tT1 = tmem_base, tT2 = tmem_base + 128, tA1 = tmem_base + 256, tA2 = tmem_base + (ATMEM ? 320 : 384);
     const uint32_t tP = tmem_base + 384, tdS = tmem_base + 448;
-    ptx::pdl_wait();
 
     if (warp == 0) {
         // ================= TMA producer =================
@@ -362,7 +359,7 @@ template <int D, int DKB, int STAGES, bool DKV, bool ATMEM>
 int launch_one(const BwdTcParams& p, int batch, cudaStream_t s) {
     const size_t smem = (size_t)(2 * DKB + 2 * STAGES * DKB + 4) * kBlk + STAGES * 2 * kT * 4 + 256 + 1024;
     B200SD_CUDA(b200sd_opt_in_smem(attn_bwd_tc_kernel<D, DKB, STAGES, DKV, ATMEM>, (int)smem));
-    B200SD_CUDA(b200sd_launch(attn_bwd_tc_kernel<D, DKB, STAGES, DKV, ATMEM>, dim3(p.Sx / kT, p.heads, batch), dim3(kThreads), smem, s, p));
+    attn_bwd_tc_kernel<D, DKB, STAGES, DKV, ATMEM><<<dim3(p.Sx / kT, p.heads, batch), dim3(kThreads), smem, s>>>(p);
     g_b200sd_launches.fetch_add(1, std::memory_order_relaxed);
     B200SD_LAUNCH_CHECK();
     return B200SD_OK;
@@ -398,12 +395,7 @@ int b200sd_attention_bwd_tc(const bf16* q, const bf16* k, const bf16* v, const b
     if ((rc = make_map(&pq.tmY2, v, d, heads, (int64_t)batch * Skv, ldv))) return rc;
     pq.lse = lse; pq.delta = delta; pq.out1 = nullptr; pq.out2 = dq; pq.Sx = Sq; pq.Sy = Skv; pq.heads = heads; pq.ld1 = 0; pq.ld2 = lddq;
     pq.scale = scale; pq.scale_log2 = scale * 1.4426950408889634f;
-    static const bool a_smem = getenv("B200SD_ATTN_BWD_ATMEM") && getenv("B200SD_ATTN_BWD_ATMEM")[0] == '0';
     if (d == 40) {
-        if (a_smem) {
-            if ((rc = launch_one<40, 1, 2, false, false>(pq, batch, s))) return rc;
-            return launch_one<40, 1, 2, true, false>(pk, batch, s);
-        }
         if ((rc = launch_one<40, 1, 2, false, true>(pq, batch, s))) return rc;
         return launch_one<40, 1, 2, true, true>(pk, batch, s);
     }

@@ -23,7 +23,6 @@
 // Measured (B200, d=40, S=4096): batch 2 145 -> 117 us, batch 8 480 -> 372 us against the first version (128-key
 // tiles, S single-buffered, P through shared memory, O folded in registers every tile, two-pass softmax).
 #include <atomic>
-#include <cstdlib>
 #include <cstring>
 #include <mutex>
 
@@ -42,7 +41,6 @@ struct AttnParams {
     float* lse;   // optional [batch][heads][Sq]: log2-domain log-sum-exp of the scaled scores (for the backward)
     int Sq, Skv, heads, ldo;
     float scale_log2;
-    float lazy_thr;   // log2 units a row may outgrow the lagging reference max before its tile is redone
 };
 
 __device__ __forceinline__ void tma_load_3d(void* dst, const CUtensorMap* m, uint64_t* bar, int c0, int c1, int c2) {
@@ -89,29 +87,14 @@ __device__ __forceinline__ void tmem_ld_32x32b_x32(uint32_t taddr, uint32_t (&r)
 // log2 units a row may outgrow the lagging reference max before its tile is redone (P <= 2^6 is harmless in bf16/fp32)
 constexpr float kLazyThr = 6.0f;
 constexpr int kKV = 64;
+constexpr int kThreads = 64 + 4 * 32;   // producer warp, MMA warp, 4 softmax warps
+constexpr int kPoly = 4;                // every kPoly-th score pair is exponentiated by poly_exp2x2 instead of MUFU.EX2
 __device__ __forceinline__ void tmem_st_32x32b_x16(uint32_t taddr, const uint32_t* r) {
     asm volatile(
         "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16};" ::"r"(taddr),
         "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]), "r"(r[8]), "r"(r[9]), "r"(r[10]), "r"(r[11]),
         "r"(r[12]), "r"(r[13]), "r"(r[14]), "r"(r[15])
         : "memory");
-}
-
-__device__ __forceinline__ void tmem_st_32x32b_x8(uint32_t taddr, const uint32_t* r) {
-    asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]),
-                 "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7])
-                 : "memory");
-}
-
-// 64-thread named barrier of the two softmax warps that share TMEM lane quadrant qd (ids 1..4 as immediates: a register id makes
-// ptxas reserve all 16 barriers of the CTA)
-__device__ __forceinline__ void quad_pair_sync(int qd) {
-    switch (qd) {
-        case 0: asm volatile("bar.sync 1, 64;" ::: "memory"); break;
-        case 1: asm volatile("bar.sync 2, 64;" ::: "memory"); break;
-        case 2: asm volatile("bar.sync 3, 64;" ::: "memory"); break;
-        default: asm volatile("bar.sync 4, 64;" ::: "memory"); break;
-    }
 }
 
 // 2^t for a pair of scores on the FMA pipe (Cody-Waite split + degree-3 minimax polynomial, 7.5e-5 max relative error --
@@ -133,19 +116,11 @@ __device__ __forceinline__ float2 poly_exp2x2(float2 t) {
     return e;
 }
 
-// POLY: every POLY-th score pair takes the polynomial instead of MUFU.EX2 (0 = none)
 // kStages: depth of the K / V smem ring (4; 2 at d = 160, whose three 64-wide d blocks per tile would not fit otherwise)
-// SW: softmax warps per CTA.  4 = one thread per query row (default).  8 = TWO warps per TMEM lane quadrant, each taking 32 of a
-// tile's 64 key columns of the same 32 rows; the two agree on the reference max per tile through a 64-thread named barrier (redo
-// vote; row maxima only when a redo happens), add their partial row sums once at the end, and each rescales / normalises / stores
-// its half of the O columns.  Built in r02b to test whether the softmax is bound by latency hiding (two softmax warps per
-// scheduler at 4 warps x 2 CTAs): it is NOT -- same results bit for bit, B2 S4096 d40 120.9 (4 warps) vs 129.0 us (8), B8 438.5 vs
-// 436.2, S1024 d80 20.3 vs 20.0.  Neither is it bound by MUFU (moving 0 / 25 / 33 / 50 % of the exponentials to the FMA pipe:
-// 123.5 / 121.4 / 122.1 / 128.6 us), nor by occupancy alone (one CTA per SM: +26 %), nor by TMEM read bandwidth (reading the scores
-// twice per tile: 124.0 us).  ncu: XU 47 % (busiest SM 55 %), issue 51 % (61 %), FMA 36 %, tensor 24 % -- two co-limiting pipes fed by
-// mutually dependent work, plus a 2-wave imbalance at batch 2 (DESIGN.md section 5).  Kept behind B200SD_ATTN_WARPS=8.
-template <int D, int DKB, int POLY, int kStages, int SW>
-__global__ void __launch_bounds__(64 + SW * 32, (D <= 40) ? 2 : 1) attention_tc_kernel(const __grid_constant__ AttnParams p) {
+// Two softmax warps per TMEM lane quadrant (B2 S4096 d40: 129.0 vs 120.9 us) and every exponential on MUFU.EX2 (123.5 vs
+// 121.4 us) were measured on B200 and were not faster (DESIGN.md section 5).
+template <int D, int DKB, int kStages>
+__global__ void __launch_bounds__(kThreads, (D <= 40) ? 2 : 1) attention_tc_kernel(const __grid_constant__ AttnParams p) {
     constexpr int DN = (D + 15) / 16 * 16;    // MMA N of the PV product (48 / 80)
     constexpr int KSTEPS = (D + 15) / 16;     // UMMA K steps of the QK^T product
     constexpr int KBLK = kKV * 128;          // bytes of one K block [64 keys x 64 d]
@@ -168,16 +143,11 @@ __global__ void __launch_bounds__(64 + SW * 32, (D <= 40) ? 2 : 1) attention_tc_
                                                   // phase BEFORE the one it waits for still open, which a parity wait cannot tell
                                                   // from "already complete"
     uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(o_full + 2);
-    float* xch = reinterpret_cast<float*>(tmem_slot + 4);          // SW == 8: [2 halves][128 rows] row maxima / row sums
-    float* xl = xch + 2 * kQ;                                      // SW == 8: [2 halves][128 rows] final row sums (own region: no
-                                                                   //          barrier separates it from the last tile's maxima)
-    int* xflag = reinterpret_cast<int*>(xl + 2 * kQ);              // SW == 8: [2 tile parities][4 quadrants][2 halves] redo votes
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int q0 = blockIdx.x * kQ, h = blockIdx.y, b = blockIdx.z;
     const int num_tiles = (p.Skv + kKV - 1) / kKV;   // the last tile may be partial (cross-attention: 77 = 64 + 13 keys)
 
-    ptx::pdl_trigger();
     if (warp == 0 && lane == 0) {
         ptx::prefetch_tmap(&p.tmQ);
         ptx::prefetch_tmap(&p.tmK);
@@ -191,7 +161,7 @@ __global__ void __launch_bounds__(64 + SW * 32, (D <= 40) ? 2 : 1) attention_tc_
         }
         for (int i = 0; i < 2; ++i) {
             ptx::mbar_init(&s_full[i], 1);
-            ptx::mbar_init(&p_full[i], SW);   // one (warp-aggregated) arrival per softmax warp
+            ptx::mbar_init(&p_full[i], 4);    // one (warp-aggregated) arrival per softmax warp
             ptx::mbar_init(&o_full[i], 1);
         }
         ptx::fence_barrier_init();
@@ -207,7 +177,6 @@ __global__ void __launch_bounds__(64 + SW * 32, (D <= 40) ? 2 : 1) attention_tc_
     // P has its own columns: were it written over S (as a first version did), the QK^T of tile j+2 would overwrite columns the
     // PV product of tile j is still reading, ordered by nothing but the tensor pipe's issue order
     const uint32_t tmem_S = tmem_base, tmem_O = tmem_base + 128, tmem_P = tmem_base + 128 + DN;
-    ptx::pdl_wait();
 
     if (warp == 0) {
         // ================= TMA producer =================
@@ -266,112 +235,6 @@ __global__ void __launch_bounds__(64 + SW * 32, (D <= 40) ? 2 : 1) attention_tc_
                 ptx::umma_commit(&o_full[j & 1]);
             }
         }
-    } else if constexpr (SW == 8) {
-        // ================= softmax warps, two per TMEM lane quadrant: one thread per (query row, 32-key half tile) ==========
-        const int qd = warp & 3;                              // TMEM lane quadrant this warp may address
-        const int half = (warp - 2) >> 2;                     // which 32 of the tile's 64 key columns (and which half of O's columns)
-        const int row = qd * 32 + lane;
-        const uint32_t lane_addr = (uint32_t)(qd * 32) << 16;
-        constexpr int OH = DN / 2;                            // O columns owned by this half (24 / 40 / 80)
-        const uint32_t tO = tmem_O + lane_addr + half * OH;
-        const float2 sc2 = make_float2(p.scale_log2, p.scale_log2);
-        float m = -INFINITY, l = 0.f;
-        for (int j = 0; j < num_tiles; ++j) {
-            const uint32_t tS = tmem_S + lane_addr + (j & 1) * kKV + half * 32;
-            ptx::mbar_wait(&s_full[j & 1], (j >> 1) & 1);
-            ptx::tc_fence_after();
-            uint32_t r[32], pk[16];
-            tmem_ld_32x32b_x32(tS, r);
-            ptx::tmem_ld_wait();
-            if ((j + 1) * kKV > p.Skv) {
-                const int valid = p.Skv - j * kKV - half * 32;   // key columns of this half that exist
-#pragma unroll
-                for (int i = 0; i < 32; ++i)
-                    if (i >= valid) r[i] = 0xff800000u;
-            }
-            auto exps = [&](float off, bool track, float& mx) -> float {
-                const float2 noff2 = make_float2(-off, -off);
-                float2 rs2 = make_float2(0.f, 0.f);
-#pragma unroll
-                for (int i = 0; i < 16; ++i) {
-                    const float2 t = ffma2(make_float2(__uint_as_float(r[2 * i]), __uint_as_float(r[2 * i + 1])), sc2, noff2);
-                    const float2 e = (POLY > 0 && i % (POLY > 0 ? POLY : 1) == POLY - 1) ? poly_exp2x2(t)
-                                                                                        : make_float2(fast_exp2(t.x), fast_exp2(t.y));
-                    rs2 = fadd2(rs2, e);
-                    pk[i] = pack_bf16x2(e.x, e.y);
-                    if (track) mx = fmax3(mx, __uint_as_float(r[2 * i]), __uint_as_float(r[2 * i + 1]));
-                }
-                return rs2.x + rs2.y;
-            };
-            float mx = -INFINITY, rs = 0.f;
-            bool redo = true;
-            if (j > 0) {
-                rs = exps(m * p.scale_log2, true, mx);
-                const bool mine = __any_sync(0xffffffffu, (mx - m) * p.scale_log2 > p.lazy_thr);
-                int* fl = xflag + ((j & 1) * 4 + qd) * 2;
-                if (lane == 0) fl[half] = mine ? 1 : 0;
-                quad_pair_sync(qd);
-                redo = mine || (fl[half ^ 1] != 0);           // both warps of the quadrant take the same branch
-            } else {
-#pragma unroll
-                for (int i = 0; i < 16; ++i) mx = fmax3(mx, __uint_as_float(r[2 * i]), __uint_as_float(r[2 * i + 1]));
-            }
-            if (redo) {   // uniform over the quadrant's 64 threads: move every row to its true running max over BOTH halves
-                xch[half * kQ + row] = mx;
-                quad_pair_sync(qd);
-                const float mn = fmaxf(m, fmaxf(mx, xch[(half ^ 1) * kQ + row]));
-                // a row whose keys are all masked so far (cross-attention tail) keeps m = -inf: exp2(-inf - -inf) must not be NaN
-                const float corr = (m == -INFINITY) ? 0.f : fast_exp2((m - mn) * p.scale_log2);
-                m = mn;
-                float unused = 0.f;
-                rs = exps(mn * p.scale_log2, false, unused);
-                l *= corr;
-                if (j > 0) {   // rescale this half's O columns (PV_{j-1} must have landed; PV_j waits for p_full)
-                    ptx::mbar_wait(&o_full[(j - 1) & 1], ((j - 1) >> 1) & 1);
-                    ptx::tc_fence_after();
-#pragma unroll
-                    for (int c0 = 0; c0 < OH; c0 += 8) {
-                        uint32_t ob[8];
-                        ptx::tmem_ld_32x32b_x8(tO + c0, ob);
-                        ptx::tmem_ld_wait();
-#pragma unroll
-                        for (int i = 0; i < 8; ++i) ob[i] = __float_as_uint(__uint_as_float(ob[i]) * corr);
-                        tmem_st_32x32b_x8(tO + c0, ob);
-                    }
-                }
-            }
-            l += rs;
-            const uint32_t tP = tmem_P + lane_addr + (j & 1) * 32 + half * 16;
-            tmem_st_32x32b_x16(tP, &pk[0]);
-            ptx::tmem_st_wait();
-            ptx::tc_fence_before();
-            __syncwarp();
-            if (lane == 0) ptx::mbar_arrive(&p_full[j & 1]);
-        }
-        // ---- add the two halves' row sums, normalise and store this half's O columns ----
-        ptx::mbar_wait(&o_full[(num_tiles - 1) & 1], ((num_tiles - 1) >> 1) & 1);
-        ptx::tc_fence_after();
-        xl[half * kQ + row] = l;
-        quad_pair_sync(qd);
-        l += xl[(half ^ 1) * kQ + row];
-        const float inv = 1.0f / l;
-        const bool live = q0 + row < p.Sq;
-        if (p.lse != nullptr && live && half == 0) p.lse[((size_t)b * p.heads + h) * p.Sq + q0 + row] = m * p.scale_log2 + log2f(l);
-        bf16* dst = p.out + ((size_t)b * p.Sq + q0 + row) * p.ldo + h * D + half * OH;
-#pragma unroll
-        for (int c0 = 0; c0 < OH; c0 += 8) {
-            uint32_t ob[8];
-            ptx::tmem_ld_32x32b_x8(tO + c0, ob);
-            ptx::tmem_ld_wait();
-            if (half * OH + c0 < D && live) {
-                uint4 u;
-                u.x = pack_bf16x2(__uint_as_float(ob[0]) * inv, __uint_as_float(ob[1]) * inv);
-                u.y = pack_bf16x2(__uint_as_float(ob[2]) * inv, __uint_as_float(ob[3]) * inv);
-                u.z = pack_bf16x2(__uint_as_float(ob[4]) * inv, __uint_as_float(ob[5]) * inv);
-                u.w = pack_bf16x2(__uint_as_float(ob[6]) * inv, __uint_as_float(ob[7]) * inv);
-                *reinterpret_cast<uint4*>(dst + c0) = u;
-            }
-        }
     } else {
         // ================= softmax warps: one thread per query row =================
         const int qd = warp & 3;                              // TMEM lane quadrant this warp may address
@@ -403,8 +266,7 @@ __global__ void __launch_bounds__(64 + SW * 32, (D <= 40) ? 2 : 1) attention_tc_
 #pragma unroll
                 for (int i = 0; i < 32; ++i) {
                     const float2 t = ffma2(make_float2(__uint_as_float(r[2 * i]), __uint_as_float(r[2 * i + 1])), sc2, noff2);
-                    const float2 e = (POLY > 0 && i % (POLY > 0 ? POLY : 1) == POLY - 1) ? poly_exp2x2(t)
-                                                                                        : make_float2(fast_exp2(t.x), fast_exp2(t.y));
+                    const float2 e = (i % kPoly == kPoly - 1) ? poly_exp2x2(t) : make_float2(fast_exp2(t.x), fast_exp2(t.y));
                     rs2 = fadd2(rs2, e);
                     pk[i] = pack_bf16x2(e.x, e.y);
                     if (track) mx = fmax3(mx, __uint_as_float(r[2 * i]), __uint_as_float(r[2 * i + 1]));
@@ -415,7 +277,7 @@ __global__ void __launch_bounds__(64 + SW * 32, (D <= 40) ? 2 : 1) attention_tc_
             bool redo = true;
             if (j > 0) {
                 rs = exps(m * p.scale_log2, true, mx);
-                redo = __any_sync(0xffffffffu, (mx - m) * p.scale_log2 > p.lazy_thr);
+                redo = __any_sync(0xffffffffu, (mx - m) * p.scale_log2 > kLazyThr);
             } else {
 #pragma unroll
                 for (int i = 0; i < 32; ++i) mx = fmax3(mx, __uint_as_float(r[2 * i]), __uint_as_float(r[2 * i + 1]));
@@ -491,7 +353,7 @@ __global__ void __launch_bounds__(64 + SW * 32, (D <= 40) ? 2 : 1) attention_tc_
     }
 }
 
-template <int D, int DKB, int POLY, int kStages, int SW>
+template <int D, int DKB, int kStages>
 int launch_tc(const bf16* q, const bf16* k, const bf16* v, bf16* out, float* lse, int batch, int heads, int Sq, int Skv, int ldq,
                int ldk, int ldv, int ldo, float scale, cudaStream_t s) {
     AttnParams p;
@@ -524,12 +386,9 @@ int launch_tc(const bf16* q, const bf16* k, const bf16* v, bf16* out, float* lse
     p.heads = heads;
     p.ldo = ldo;
     p.scale_log2 = scale * 1.4426950408889634f;
-    static const float thr = [] { const char* e = getenv("B200SD_ATTN_THR"); return e ? (float)atof(e) : kLazyThr; }();
-    p.lazy_thr = thr;
-    static const size_t smem_pad = [] { const char* e = getenv("B200SD_ATTN_SMEM_PAD"); return e ? (size_t)atol(e) : (size_t)0; }();   // occupancy experiment
-    const size_t smem = (size_t)DKB * kBlk + (size_t)2 * kStages * DKB * kKV * 128 + 256 + 4 * kQ * 4 + 64 + 1024 + smem_pad;
-    B200SD_CUDA(b200sd_opt_in_smem(attention_tc_kernel<D, DKB, POLY, kStages, SW>, (int)smem, /*max_carveout=*/true));
-    B200SD_CUDA(b200sd_launch(attention_tc_kernel<D, DKB, POLY, kStages, SW>, dim3((Sq + kQ - 1) / kQ, heads, batch), dim3(64 + SW * 32), smem, s, p));
+    const size_t smem = (size_t)DKB * kBlk + (size_t)2 * kStages * DKB * kKV * 128 + 256 + 1024;
+    B200SD_CUDA(b200sd_opt_in_smem(attention_tc_kernel<D, DKB, kStages>, (int)smem, /*max_carveout=*/true));
+    attention_tc_kernel<D, DKB, kStages><<<dim3((Sq + kQ - 1) / kQ, heads, batch), dim3(kThreads), smem, s>>>(p);
     g_b200sd_launches.fetch_add(1, std::memory_order_relaxed);
     B200SD_LAUNCH_CHECK();
     return B200SD_OK;
@@ -545,26 +404,9 @@ int b200sd_attention_tc(const void* q, const void* k, const void* v, void* out, 
     (void)workspace;   // no scratch any more: V is consumed in place (MN-major B operand), the V^T transpose kernel is gone
     (void)ws_bytes;
     if ((ldq * 2) % 16 != 0 || (ldk * 2) % 16 != 0 || (ldv * 2) % 16 != 0) return B200SD_ERR_UNSUPPORTED;
-    // B200SD_ATTN_POLY=0 keeps every exponential on MUFU.EX2 (A/B switch; default: every 4th pair on the FMA pipe)
-    static const int poly = [] { const char* e = getenv("B200SD_ATTN_POLY"); return e ? atoi(e) : 4; }();
-#define B200SD_ATTN_GO(DD, KB, PL, ST)                                                                                        \
-    do {                                                                                                                      \
-        if (sw == 8)                                                                                                          \
-            return launch_tc<DD, KB, PL, ST, 8>(static_cast<const bf16*>(q), static_cast<const bf16*>(k), static_cast<const bf16*>(v), \
-                                                static_cast<bf16*>(out), lse, batch, heads, Sq, Skv, ldq, ldk, ldv, ldo, scale, s);  \
-        return launch_tc<DD, KB, PL, ST, 4>(static_cast<const bf16*>(q), static_cast<const bf16*>(k), static_cast<const bf16*>(v),   \
-                                            static_cast<bf16*>(out), lse, batch, heads, Sq, Skv, ldq, ldk, ldv, ldo, scale, s);      \
-    } while (0)
-    // B200SD_ATTN_WARPS=8: two softmax warps per TMEM lane quadrant (A/B switch; measured not faster, default 4 = one thread per row)
-    static const int sw = [] { const char* e = getenv("B200SD_ATTN_WARPS"); return (e && atoi(e) == 8) ? 8 : 4; }();
-    if (d == 40) {
-        if (poly == 0) B200SD_ATTN_GO(40, 1, 0, 4);
-        B200SD_ATTN_GO(40, 1, 4, 4);
-    }
-    if (d == 80) {
-        if (poly == 0) B200SD_ATTN_GO(80, 2, 0, 4);
-        B200SD_ATTN_GO(80, 2, 4, 4);
-    }
-    B200SD_ATTN_GO(160, 3, 4, 2);
-#undef B200SD_ATTN_GO
+    const bf16 *qb = static_cast<const bf16*>(q), *kb = static_cast<const bf16*>(k), *vb = static_cast<const bf16*>(v);
+    bf16* ob = static_cast<bf16*>(out);
+    if (d == 40) return launch_tc<40, 1, 4>(qb, kb, vb, ob, lse, batch, heads, Sq, Skv, ldq, ldk, ldv, ldo, scale, s);
+    if (d == 80) return launch_tc<80, 2, 4>(qb, kb, vb, ob, lse, batch, heads, Sq, Skv, ldq, ldk, ldv, ldo, scale, s);
+    return launch_tc<160, 3, 2>(qb, kb, vb, ob, lse, batch, heads, Sq, Skv, ldq, ldk, ldv, ldo, scale, s);
 }

@@ -43,8 +43,6 @@ __global__ void __launch_bounds__(256) grad_prep_kernel(const void* __restrict__
                                                         float* __restrict__ colsum, int rows, int N, int ld,
                                                         int rows_per_block, int rows_per_image, int ldcs) {
     __shared__ float s_acc[32][65];
-    ptx::pdl_trigger();
-    ptx::pdl_wait();
     const int v = threadIdx.x & 7, r = threadIdx.x >> 3;
     const int c = blockIdx.x * 64 + v * 8;
     const int r0 = blockIdx.y * rows_per_block, r1 = min(rows, r0 + rows_per_block);
@@ -88,8 +86,6 @@ __global__ void __launch_bounds__(512) gn_bwd_stats_kernel(const void* __restric
                                                            int silu) {
     extern __shared__ float s_red[];   // [4][blockDim.x]
     __shared__ float s_ms[4];
-    ptx::pdl_trigger();
-    ptx::pdl_wait();
     const int C = C0 + C1, cpg = C / groups;
     const int g = blockIdx.x, b = blockIdx.y;
     const int rpp = blockDim.x / cpg;           // pixel rows per pass
@@ -181,8 +177,6 @@ __global__ void __launch_bounds__(256) gn_bwd_partial_kernel(const void* __restr
                                                              float* __restrict__ chan_ws, int hw, int groups, int silu, int VC,
                                                              int pix_per_slab) {
     extern __shared__ float s_fold[];   // [2][R][VC * 8]
-    ptx::pdl_trigger();
-    ptx::pdl_wait();
     const int C = C0 + C1, cpg = C / groups, C8 = C / 8;
     const int b = blockIdx.z, chunk = blockIdx.y;
     const int R = blockDim.x / VC;
@@ -249,8 +243,6 @@ __global__ void __launch_bounds__(256) gn_bwd_finalize_kernel(const float* __res
                                                               float* __restrict__ dgamma, float* __restrict__ dbeta, int C, int hw,
                                                               int groups, int slabs) {
     extern __shared__ float s_part[];   // [parts][2 * cpg] then [2 * cpg] folded
-    ptx::pdl_trigger();
-    ptx::pdl_wait();
     const int g = blockIdx.x, b = blockIdx.y, cpg = C / groups;
     const int nE = 2 * cpg;                               // (sum g, sum g xhat) per channel of the group, interleaved
     const int parts = max(1, (int)blockDim.x / nE);
@@ -296,8 +288,6 @@ __global__ void __launch_bounds__(256) gn_bwd_apply_kernel(const void* __restric
                                                            const float4* __restrict__ stats, int hw, int groups, int silu,
                                                            int pix_per_block) {
     __shared__ float4 s_st[32];
-    ptx::pdl_trigger();
-    ptx::pdl_wait();
     const int C = C0 + C1, cpg = C / groups, b = blockIdx.y;
     if (threadIdx.x < groups) s_st[threadIdx.x] = stats[(size_t)b * groups + threadIdx.x];
     __syncthreads();
@@ -350,8 +340,6 @@ __global__ void __launch_bounds__(256) layernorm_bwd_kernel(const void* __restri
                                                             float* __restrict__ dgamma, float* __restrict__ dbeta, int rows,
                                                             int C, float eps, int rows_per_block) {
     extern __shared__ float s_buf[];   // [8][C]
-    ptx::pdl_trigger();
-    ptx::pdl_wait();
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int r_begin = blockIdx.x * rows_per_block, r_end = min(rows, r_begin + rows_per_block);
     float2 dg[P], db[P], gm[P];
@@ -421,8 +409,6 @@ __global__ void __launch_bounds__(256) layernorm_bwd_kernel(const void* __restri
 
 // ---- GEGLU (training path: natural [values | gates] column order, pre-activation kept) ----------------------
 __global__ void geglu_fwd_kernel(const bf16* __restrict__ u, bf16* __restrict__ out, int64_t rows, int Ch8) {
-    ptx::pdl_trigger();
-    ptx::pdl_wait();
     const int64_t total = rows * Ch8, stride = (int64_t)gridDim.x * blockDim.x;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += stride) {
         const int64_t row = i / Ch8;
@@ -437,8 +423,6 @@ __global__ void geglu_fwd_kernel(const bf16* __restrict__ u, bf16* __restrict__ 
 }
 __global__ void geglu_bwd_kernel(const bf16* __restrict__ u, const bf16* __restrict__ dff, bf16* __restrict__ du,
                                  int64_t rows, int Ch8) {
-    ptx::pdl_trigger();
-    ptx::pdl_wait();
     const int64_t total = rows * Ch8, stride = (int64_t)gridDim.x * blockDim.x;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += stride) {
         const int64_t row = i / Ch8;
@@ -462,8 +446,6 @@ __global__ void geglu_bwd_kernel(const bf16* __restrict__ u, const bf16* __restr
 // nearest x2 upsample backward: dx[b,y,x,:] (+)= sum of the 2x2 block of dy
 __global__ void upsample2x_bwd_kernel(const bf16* __restrict__ dy, float* __restrict__ dx, int batch, int H, int W, int C8,
                                       int accumulate) {
-    ptx::pdl_trigger();
-    ptx::pdl_wait();
     const int64_t total = (int64_t)batch * H * W * C8, stride = (int64_t)gridDim.x * blockDim.x;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += stride) {
         const int c = (int)(i % C8);
@@ -492,8 +474,6 @@ __global__ void upsample2x_bwd_kernel(const bf16* __restrict__ dy, float* __rest
 // col2im of the stride-2 pad-1 3x3 im2col: dx[b,y,x,:] (+)= sum over taps (ky,kx) with y = 2 oy + ky - 1, x = 2 ox + kx - 1
 __global__ void col2im_s2_kernel(const bf16* __restrict__ dcol, float* __restrict__ dx, int batch, int H, int W, int C8,
                                  int accumulate) {
-    ptx::pdl_trigger();
-    ptx::pdl_wait();
     const int OH = H / 2, OW = W / 2;
     const int64_t total = (int64_t)batch * H * W * C8, stride = (int64_t)gridDim.x * blockDim.x;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += stride) {
@@ -530,8 +510,6 @@ __global__ void col2im_s2_kernel(const bf16* __restrict__ dcol, float* __restric
 // conv_out data gradient: dt[p, ci] = sum_tap sum_co dout[b, co, p - d(tap)] * w[co][tap][ci]   (bf16 NHWC out)
 __global__ void __launch_bounds__(256) conv_out_dgrad_kernel(const float* __restrict__ dout, const float* __restrict__ w,
                                                              bf16* __restrict__ dt, int batch, int Cin, int Cout, int H, int W) {
-    ptx::pdl_trigger();
-    ptx::pdl_wait();
     const int C8 = Cin / 8;
     const int64_t total = (int64_t)batch * H * W * C8, stride = (int64_t)gridDim.x * blockDim.x;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += stride) {
@@ -565,8 +543,6 @@ template <int DT>
 __global__ void __launch_bounds__(256) conv_small_wgrad_kernel(const void* __restrict__ wide, const float* __restrict__ narrow,
                                                                float* __restrict__ dw, int batch, int H, int W, int Cw, int Cn,
                                                                int sign, int out_mode, int pix_per_block) {
-    ptx::pdl_trigger();
-    ptx::pdl_wait();
     const int cw = blockIdx.y * blockDim.x + threadIdx.x;
     const int hw = H * W, total = batch * hw;
     const int q0 = blockIdx.x * pix_per_block, q1 = min(total, q0 + pix_per_block);
@@ -603,8 +579,6 @@ __global__ void __launch_bounds__(256) conv_small_wgrad_kernel(const void* __res
 __global__ void __launch_bounds__(256) nchw_channel_sum_kernel(const float* __restrict__ x, float* __restrict__ out, int batch,
                                                                int C, int hw) {
     __shared__ float s_w[8];
-    ptx::pdl_trigger();
-    ptx::pdl_wait();
     const int c = blockIdx.x;
     float a = 0.f;
     for (int i = threadIdx.x; i < batch * hw; i += blockDim.x) a += x[((size_t)(i / hw) * C + c) * hw + i % hw];
@@ -620,8 +594,6 @@ __global__ void __launch_bounds__(256) nchw_channel_sum_kernel(const float* __re
 
 // ---- small elementwise helpers of the time-embedding backward -----------------------------------------------
 __global__ void cast_act_kernel(const float* __restrict__ in, bf16* __restrict__ out, int64_t n, int silu) {
-    ptx::pdl_trigger();
-    ptx::pdl_wait();
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
         float v = in[i];
         if (silu) v = v * sigmoid_f(v);
@@ -629,8 +601,6 @@ __global__ void cast_act_kernel(const float* __restrict__ in, bf16* __restrict__
     }
 }
 __global__ void silu_bwd_mul_kernel(const float* __restrict__ pre, float* __restrict__ g, int64_t n) {
-    ptx::pdl_trigger();
-    ptx::pdl_wait();
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
         g[i] *= silu_grad_f(pre[i]);
 }
@@ -638,8 +608,6 @@ __global__ void silu_bwd_mul_kernel(const float* __restrict__ pre, float* __rest
 // ---- flat-buffer kernels of the optimizer step ----------------------------------------------------------------
 // fp32 master -> bf16 tensor-core copy, 8 elements per thread
 __global__ void cast_flat_kernel(const float* __restrict__ in, bf16* __restrict__ out, int64_t n8) {
-    ptx::pdl_trigger();
-    ptx::pdl_wait();
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n8; i += (int64_t)gridDim.x * blockDim.x) {
         float v[8];
         ld8<B200SD_F32>(in, (size_t)i * 8, v);
@@ -654,8 +622,6 @@ __global__ void __launch_bounds__(256) adamw_flat_kernel(float* __restrict__ p, 
                                                          float* __restrict__ v, bf16* __restrict__ wb, int64_t n4, float lr,
                                                          float beta1, float beta2, float eps, float wd, float bc1, float rsqrt_bc2,
                                                          float grad_scale, int zero_grad) {
-    ptx::pdl_trigger();
-    ptx::pdl_wait();
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (int64_t)gridDim.x * blockDim.x) {
         float4 P = reinterpret_cast<float4*>(p)[i], G = reinterpret_cast<float4*>(g)[i];
         float4 M = reinterpret_cast<float4*>(m)[i], V = reinterpret_cast<float4*>(v)[i];
@@ -703,11 +669,11 @@ extern "C" int b200sd_grad_prep(const void* in, int in_dtype, void* out_bf16, fl
     dim3 grid(col_blocks, ceil_div(rows, rpb));
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     if (in_dtype == B200SD_F32)
-        B200SD_CUDA(b200sd_launch(grad_prep_kernel<B200SD_F32>, grid, dim3(256), 0, s, in, static_cast<bf16*>(out_bf16), colsum, rows, N,
-                                  ld, rpb, rows_per_image, ldcs));
+        grad_prep_kernel<B200SD_F32><<<grid, dim3(256), 0, s>>>(in, static_cast<bf16*>(out_bf16), colsum, rows, N,
+                                  ld, rpb, rows_per_image, ldcs);
     else
-        B200SD_CUDA(b200sd_launch(grad_prep_kernel<B200SD_BF16>, grid, dim3(256), 0, s, in, static_cast<bf16*>(out_bf16), colsum, rows, N,
-                                  ld, rpb, rows_per_image, ldcs));
+        grad_prep_kernel<B200SD_BF16><<<grid, dim3(256), 0, s>>>(in, static_cast<bf16*>(out_bf16), colsum, rows, N,
+                                  ld, rpb, rows_per_image, ldcs);
     COUNT_LAUNCH();
     B200SD_LAUNCH_CHECK();
     return B200SD_OK;
@@ -753,17 +719,18 @@ extern "C" int b200sd_groupnorm_silu_bwd(const void* x0, const void* x1, int C0,
         slabs = ceil_div(hw, pps);
         const size_t smem = (size_t)2 * R * VC * 8 * sizeof(float);
         if (in_dtype == B200SD_F32)
-            B200SD_CUDA(b200sd_launch(gn_bwd_partial_kernel<B200SD_F32>, dim3(slabs, chunks, batch), dim3(threads), smem, s, x0, x1, C0, C1, gamma,
-                                      beta, static_cast<const bf16*>(dy), mean_rstd, chan_ws, hw, groups, silu, VC, pps));
+            gn_bwd_partial_kernel<B200SD_F32><<<dim3(slabs, chunks, batch), dim3(threads), smem, s>>>(x0, x1, C0, C1, gamma,
+                                      beta, static_cast<const bf16*>(dy), mean_rstd, chan_ws, hw, groups, silu, VC, pps);
         else
-            B200SD_CUDA(b200sd_launch(gn_bwd_partial_kernel<B200SD_BF16>, dim3(slabs, chunks, batch), dim3(threads), smem, s, x0, x1, C0, C1, gamma,
-                                      beta, static_cast<const bf16*>(dy), mean_rstd, chan_ws, hw, groups, silu, VC, pps));
+            gn_bwd_partial_kernel<B200SD_BF16><<<dim3(slabs, chunks, batch), dim3(threads), smem, s>>>(x0, x1, C0, C1, gamma,
+                                      beta, static_cast<const bf16*>(dy), mean_rstd, chan_ws, hw, groups, silu, VC, pps);
         COUNT_LAUNCH();
+        B200SD_LAUNCH_CHECK();
         {
             const int nE = 2 * cpg;
             const int parts = 256 / nE > 0 ? 256 / nE : 1;
-            B200SD_CUDA(b200sd_launch(gn_bwd_finalize_kernel, dim3(groups, batch), dim3(256), (size_t)(parts + 1) * nE * sizeof(float), s, gamma,
-                                      mean_rstd, chan_ws, stats, dgamma, dbeta, C, hw, groups, slabs));
+            gn_bwd_finalize_kernel<<<dim3(groups, batch), dim3(256), (size_t)(parts + 1) * nE * sizeof(float), s>>>(gamma,
+                                      mean_rstd, chan_ws, stats, dgamma, dbeta, C, hw, groups, slabs);
         }
         COUNT_LAUNCH();
         B200SD_LAUNCH_CHECK();
@@ -774,11 +741,11 @@ extern "C" int b200sd_groupnorm_silu_bwd(const void* x0, const void* x1, int C0,
         if (threads < 128) threads = 128;
         const size_t smem = (size_t)4 * threads * sizeof(float);
         if (in_dtype == B200SD_F32)
-            B200SD_CUDA(b200sd_launch(gn_bwd_stats_kernel<B200SD_F32>, dim3(groups, batch), dim3(threads), smem, s, x0, x1, C0, C1, gamma, beta,
-                                      static_cast<const bf16*>(dy), dgamma, dbeta, stats, hw, groups, eps, silu));
+            gn_bwd_stats_kernel<B200SD_F32><<<dim3(groups, batch), dim3(threads), smem, s>>>(x0, x1, C0, C1, gamma, beta,
+                                      static_cast<const bf16*>(dy), dgamma, dbeta, stats, hw, groups, eps, silu);
         else
-            B200SD_CUDA(b200sd_launch(gn_bwd_stats_kernel<B200SD_BF16>, dim3(groups, batch), dim3(threads), smem, s, x0, x1, C0, C1, gamma, beta,
-                                      static_cast<const bf16*>(dy), dgamma, dbeta, stats, hw, groups, eps, silu));
+            gn_bwd_stats_kernel<B200SD_BF16><<<dim3(groups, batch), dim3(threads), smem, s>>>(x0, x1, C0, C1, gamma, beta,
+                                      static_cast<const bf16*>(dy), dgamma, dbeta, stats, hw, groups, eps, silu);
         COUNT_LAUNCH();
         B200SD_LAUNCH_CHECK();
     }
@@ -790,9 +757,9 @@ extern "C" int b200sd_groupnorm_silu_bwd(const void* x0, const void* x1, int C0,
         blocks = ceil_div(hw, ppb);
         const dim3 grid(blocks, batch);
 #define GN_BWD_APPLY(DT, ODT)                                                                                                   \
-    B200SD_CUDA(b200sd_launch(gn_bwd_apply_kernel<DT, ODT>, grid, dim3(256), 0, s, x0, x1, C0, C1, gamma, beta,                    \
+    gn_bwd_apply_kernel<DT, ODT><<<grid, dim3(256), 0, s>>>(x0, x1, C0, C1, gamma, beta,                    \
                               static_cast<const bf16*>(dy), add_src, out0, out1, accumulate0, accumulate1,                       \
-                              static_cast<const float4*>(stats), hw, groups, silu, ppb))
+                              static_cast<const float4*>(stats), hw, groups, silu, ppb)
         if (in_dtype == B200SD_F32 && out_dtype == B200SD_F32) GN_BWD_APPLY(B200SD_F32, B200SD_F32);
         else if (in_dtype == B200SD_F32) GN_BWD_APPLY(B200SD_F32, B200SD_BF16);
         else if (out_dtype == B200SD_F32) GN_BWD_APPLY(B200SD_BF16, B200SD_F32);
@@ -820,9 +787,9 @@ extern "C" int b200sd_layernorm_bwd(const void* x, int in_dtype, const float* ga
 #define LNB_CASE(P)                                                                                                              \
     case P:                                                                                                                      \
         if (in_dtype == B200SD_F32)                                                                                              \
-            B200SD_CUDA(b200sd_launch(layernorm_bwd_kernel<P, B200SD_F32>, dim3(blocks), dim3(256), smem, s, x, gamma, dyb, dres, dgamma, dbeta, rows, C, eps, rpb)); \
+            layernorm_bwd_kernel<P, B200SD_F32><<<dim3(blocks), dim3(256), smem, s>>>(x, gamma, dyb, dres, dgamma, dbeta, rows, C, eps, rpb); \
         else                                                                                                                     \
-            B200SD_CUDA(b200sd_launch(layernorm_bwd_kernel<P, B200SD_BF16>, dim3(blocks), dim3(256), smem, s, x, gamma, dyb, dres, dgamma, dbeta, rows, C, eps, rpb)); \
+            layernorm_bwd_kernel<P, B200SD_BF16><<<dim3(blocks), dim3(256), smem, s>>>(x, gamma, dyb, dres, dgamma, dbeta, rows, C, eps, rpb); \
         break;
     switch (C / 64) {
         LNB_CASE(1) LNB_CASE(2) LNB_CASE(3) LNB_CASE(4) LNB_CASE(5) LNB_CASE(6) LNB_CASE(7) LNB_CASE(8) LNB_CASE(9) LNB_CASE(10)
@@ -838,8 +805,8 @@ extern "C" int b200sd_layernorm_bwd(const void* x, int in_dtype, const float* ga
 
 extern "C" int b200sd_geglu_fwd(const void* u, void* out, int64_t rows, int C_half, b200sd_stream_t stream) {
     B200SD_REQUIRE(u && out && rows > 0 && C_half > 0 && C_half % 8 == 0, "geglu_fwd: bad arguments");
-    B200SD_CUDA(b200sd_launch(geglu_fwd_kernel, dim3(ew_grid(rows * (C_half / 8), 256)), dim3(256), 0, static_cast<cudaStream_t>(stream),
-                              static_cast<const bf16*>(u), static_cast<bf16*>(out), rows, C_half / 8));
+    geglu_fwd_kernel<<<dim3(ew_grid(rows * (C_half / 8), 256)), dim3(256), 0, static_cast<cudaStream_t>(stream)>>>(
+                              static_cast<const bf16*>(u), static_cast<bf16*>(out), rows, C_half / 8);
     COUNT_LAUNCH();
     B200SD_LAUNCH_CHECK();
     return B200SD_OK;
@@ -847,8 +814,8 @@ extern "C" int b200sd_geglu_fwd(const void* u, void* out, int64_t rows, int C_ha
 
 extern "C" int b200sd_geglu_bwd(const void* u, const void* dff, void* du, int64_t rows, int C_half, b200sd_stream_t stream) {
     B200SD_REQUIRE(u && dff && du && rows > 0 && C_half > 0 && C_half % 8 == 0, "geglu_bwd: bad arguments");
-    B200SD_CUDA(b200sd_launch(geglu_bwd_kernel, dim3(ew_grid(rows * (C_half / 8), 256)), dim3(256), 0, static_cast<cudaStream_t>(stream),
-                              static_cast<const bf16*>(u), static_cast<const bf16*>(dff), static_cast<bf16*>(du), rows, C_half / 8));
+    geglu_bwd_kernel<<<dim3(ew_grid(rows * (C_half / 8), 256)), dim3(256), 0, static_cast<cudaStream_t>(stream)>>>(
+                              static_cast<const bf16*>(u), static_cast<const bf16*>(dff), static_cast<bf16*>(du), rows, C_half / 8);
     COUNT_LAUNCH();
     B200SD_LAUNCH_CHECK();
     return B200SD_OK;
@@ -858,8 +825,8 @@ extern "C" int b200sd_upsample2x_bwd(const void* dy, float* dx, int batch, int H
                                      b200sd_stream_t stream) {
     B200SD_REQUIRE(dy && dx && C % 8 == 0 && batch > 0 && H > 0 && W > 0, "upsample2x_bwd: bad arguments");
     const int64_t total = (int64_t)batch * H * W * (C / 8);
-    B200SD_CUDA(b200sd_launch(upsample2x_bwd_kernel, dim3(ew_grid(total, 256)), dim3(256), 0, static_cast<cudaStream_t>(stream),
-                              static_cast<const bf16*>(dy), dx, batch, H, W, C / 8, accumulate));
+    upsample2x_bwd_kernel<<<dim3(ew_grid(total, 256)), dim3(256), 0, static_cast<cudaStream_t>(stream)>>>(
+                              static_cast<const bf16*>(dy), dx, batch, H, W, C / 8, accumulate);
     COUNT_LAUNCH();
     B200SD_LAUNCH_CHECK();
     return B200SD_OK;
@@ -869,8 +836,8 @@ extern "C" int b200sd_col2im_s2(const void* dcol, float* dx, int batch, int H, i
                                 b200sd_stream_t stream) {
     B200SD_REQUIRE(dcol && dx && C % 8 == 0 && batch > 0 && H % 2 == 0 && W % 2 == 0, "col2im_s2: bad arguments");
     const int64_t total = (int64_t)batch * H * W * (C / 8);
-    B200SD_CUDA(b200sd_launch(col2im_s2_kernel, dim3(ew_grid(total, 256)), dim3(256), 0, static_cast<cudaStream_t>(stream),
-                              static_cast<const bf16*>(dcol), dx, batch, H, W, C / 8, accumulate));
+    col2im_s2_kernel<<<dim3(ew_grid(total, 256)), dim3(256), 0, static_cast<cudaStream_t>(stream)>>>(
+                              static_cast<const bf16*>(dcol), dx, batch, H, W, C / 8, accumulate);
     COUNT_LAUNCH();
     B200SD_LAUNCH_CHECK();
     return B200SD_OK;
@@ -882,18 +849,20 @@ extern "C" int b200sd_conv_out_bwd(const float* dout_nchw, const void* x_nhwc, c
     B200SD_REQUIRE(Cout >= 1 && Cout <= 4 && Cin % 8 == 0 && batch > 0 && H > 0 && W > 0, "conv_out_bwd: bad sizes");
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     const int64_t total = (int64_t)batch * H * W * (Cin / 8);
-    B200SD_CUDA(b200sd_launch(conv_out_dgrad_kernel, dim3(ew_grid(total, 256)), dim3(256), 0, s, dout_nchw, w,
-                              static_cast<bf16*>(dx_nhwc), batch, Cin, Cout, H, W));
+    conv_out_dgrad_kernel<<<dim3(ew_grid(total, 256)), dim3(256), 0, s>>>(dout_nchw, w,
+                              static_cast<bf16*>(dx_nhwc), batch, Cin, Cout, H, W);
     COUNT_LAUNCH();
+    B200SD_LAUNCH_CHECK();
     if (dw != nullptr) {
         B200SD_REQUIRE(x_nhwc != nullptr && dbias != nullptr, "conv_out_bwd: x / dbias missing");
         const int pix = batch * H * W;
         int ppb = ceil_div(pix, b200sd_num_sms() * 2);
         if (ppb < 16) ppb = 16;
-        B200SD_CUDA(b200sd_launch(conv_small_wgrad_kernel<B200SD_BF16>, dim3(ceil_div(pix, ppb), ceil_div(Cin, 256)), dim3(256), 0, s, x_nhwc,
-                                  dout_nchw, dw, batch, H, W, Cin, Cout, -1, 1, ppb));
+        conv_small_wgrad_kernel<B200SD_BF16><<<dim3(ceil_div(pix, ppb), ceil_div(Cin, 256)), dim3(256), 0, s>>>(x_nhwc,
+                                  dout_nchw, dw, batch, H, W, Cin, Cout, -1, 1, ppb);
         COUNT_LAUNCH();
-        B200SD_CUDA(b200sd_launch(nchw_channel_sum_kernel, dim3(Cout), dim3(256), 0, s, dout_nchw, dbias, batch, Cout, H * W));
+        B200SD_LAUNCH_CHECK();
+        nchw_channel_sum_kernel<<<dim3(Cout), dim3(256), 0, s>>>(dout_nchw, dbias, batch, Cout, H * W);
         COUNT_LAUNCH();
     }
     B200SD_LAUNCH_CHECK();
@@ -911,9 +880,9 @@ extern "C" int b200sd_conv_in_wgrad(const void* dy_nhwc, int dy_dtype, const flo
     const dim3 grid(ceil_div(pix, ppb), ceil_div(Cout, 256));
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     if (dy_dtype == B200SD_F32)
-        B200SD_CUDA(b200sd_launch(conv_small_wgrad_kernel<B200SD_F32>, grid, dim3(256), 0, s, dy_nhwc, x_nchw, dw, batch, H, W, Cout, Cin, 1, 0, ppb));
+        conv_small_wgrad_kernel<B200SD_F32><<<grid, dim3(256), 0, s>>>(dy_nhwc, x_nchw, dw, batch, H, W, Cout, Cin, 1, 0, ppb);
     else
-        B200SD_CUDA(b200sd_launch(conv_small_wgrad_kernel<B200SD_BF16>, grid, dim3(256), 0, s, dy_nhwc, x_nchw, dw, batch, H, W, Cout, Cin, 1, 0, ppb));
+        conv_small_wgrad_kernel<B200SD_BF16><<<grid, dim3(256), 0, s>>>(dy_nhwc, x_nchw, dw, batch, H, W, Cout, Cin, 1, 0, ppb);
     COUNT_LAUNCH();
     B200SD_LAUNCH_CHECK();
     return B200SD_OK;
@@ -921,8 +890,8 @@ extern "C" int b200sd_conv_in_wgrad(const void* dy_nhwc, int dy_dtype, const flo
 
 extern "C" int b200sd_cast_act(const float* in, void* out_bf16, int64_t n, int silu, b200sd_stream_t stream) {
     B200SD_REQUIRE(in && out_bf16 && n > 0, "cast_act: bad arguments");
-    B200SD_CUDA(b200sd_launch(cast_act_kernel, dim3(ew_grid(n, 256)), dim3(256), 0, static_cast<cudaStream_t>(stream), in,
-                              static_cast<bf16*>(out_bf16), n, silu));
+    cast_act_kernel<<<dim3(ew_grid(n, 256)), dim3(256), 0, static_cast<cudaStream_t>(stream)>>>(in,
+                              static_cast<bf16*>(out_bf16), n, silu);
     COUNT_LAUNCH();
     B200SD_LAUNCH_CHECK();
     return B200SD_OK;
@@ -930,7 +899,7 @@ extern "C" int b200sd_cast_act(const float* in, void* out_bf16, int64_t n, int s
 
 extern "C" int b200sd_silu_bwd_mul(const float* pre, float* grad, int64_t n, b200sd_stream_t stream) {
     B200SD_REQUIRE(pre && grad && n > 0, "silu_bwd_mul: bad arguments");
-    B200SD_CUDA(b200sd_launch(silu_bwd_mul_kernel, dim3(ew_grid(n, 256)), dim3(256), 0, static_cast<cudaStream_t>(stream), pre, grad, n));
+    silu_bwd_mul_kernel<<<dim3(ew_grid(n, 256)), dim3(256), 0, static_cast<cudaStream_t>(stream)>>>(pre, grad, n);
     COUNT_LAUNCH();
     B200SD_LAUNCH_CHECK();
     return B200SD_OK;
@@ -939,8 +908,8 @@ extern "C" int b200sd_silu_bwd_mul(const float* pre, float* grad, int64_t n, b20
 extern "C" int b200sd_cast_flat(const float* in, void* out_bf16, int64_t n, b200sd_stream_t stream) {
     B200SD_REQUIRE(in && out_bf16 && n > 0 && n % 8 == 0, "cast_flat: n must be a positive multiple of 8");
     B200SD_REQUIRE(((reinterpret_cast<uintptr_t>(in) | reinterpret_cast<uintptr_t>(out_bf16)) & 15) == 0, "cast_flat: pointers must be 16-byte aligned");
-    B200SD_CUDA(b200sd_launch(cast_flat_kernel, dim3(ew_grid(n / 8, 256)), dim3(256), 0, static_cast<cudaStream_t>(stream), in,
-                              static_cast<bf16*>(out_bf16), n / 8));
+    cast_flat_kernel<<<dim3(ew_grid(n / 8, 256)), dim3(256), 0, static_cast<cudaStream_t>(stream)>>>(in,
+                              static_cast<bf16*>(out_bf16), n / 8);
     COUNT_LAUNCH();
     B200SD_LAUNCH_CHECK();
     return B200SD_OK;
@@ -956,9 +925,9 @@ extern "C" int b200sd_adamw_step(float* param, float* grad, float* exp_avg, floa
                    "adamw_step: pointers must be 16-byte aligned");
     const double bc1 = 1.0 - pow((double)beta1, (double)step);
     const double bc2 = 1.0 - pow((double)beta2, (double)step);
-    B200SD_CUDA(b200sd_launch(adamw_flat_kernel, dim3(ew_grid(n / 4, 256)), dim3(256), 0, static_cast<cudaStream_t>(stream), param, grad,
+    adamw_flat_kernel<<<dim3(ew_grid(n / 4, 256)), dim3(256), 0, static_cast<cudaStream_t>(stream)>>>(param, grad,
                               exp_avg, exp_avg_sq, static_cast<bf16*>(weights_bf16), n / 4, lr, beta1, beta2, eps, weight_decay,
-                              (float)bc1, (float)(1.0 / sqrt(bc2)), grad_scale, zero_grad));
+                              (float)bc1, (float)(1.0 / sqrt(bc2)), grad_scale, zero_grad);
     COUNT_LAUNCH();
     B200SD_LAUNCH_CHECK();
     return B200SD_OK;

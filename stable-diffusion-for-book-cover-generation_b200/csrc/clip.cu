@@ -32,8 +32,6 @@ __device__ __forceinline__ float warp_max_f(float v) {
 // ---- embeddings: x[b*S + s][:] = tok[ids[b][s]][:] + pos[s][:]  (fp32) ------------------------------------------------
 __global__ void clip_embed_kernel(const int64_t* __restrict__ ids, const float* __restrict__ tok, const float* __restrict__ pos,
                                   float* __restrict__ out, int rows, int S, int C4, int vocab) {
-    ptx::pdl_trigger();
-    ptx::pdl_wait();
     const int64_t total = (int64_t)rows * C4, stride = (int64_t)gridDim.x * blockDim.x;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += stride) {
         const int row = (int)(i / C4), c = (int)(i % C4);
@@ -48,8 +46,6 @@ __global__ void clip_embed_kernel(const int64_t* __restrict__ ids, const float* 
 // backward: dpos[s] += sum_b dx[b][s] (fixed order over b), dtok[ids[b][s]] += dx[b][s] (fp32 atomics: a token may repeat)
 __global__ void clip_embed_bwd_kernel(const int64_t* __restrict__ ids, const float* __restrict__ dx, float* __restrict__ dtok,
                                       float* __restrict__ dpos, int batch, int S, int C, int vocab) {
-    ptx::pdl_trigger();
-    ptx::pdl_wait();
     const int s = blockIdx.x;
     for (int c = threadIdx.x; c < C; c += blockDim.x) {
         float acc = 0.f;
@@ -68,8 +64,6 @@ __global__ void clip_embed_bwd_kernel(const int64_t* __restrict__ ids, const flo
 __device__ __forceinline__ float sigmoid_f(float x) { return 1.f / (1.f + __expf(-x)); }
 
 __global__ void quick_gelu_fwd_kernel(const bf16* __restrict__ u, bf16* __restrict__ out, int64_t n8) {
-    ptx::pdl_trigger();
-    ptx::pdl_wait();
     const int64_t stride = (int64_t)gridDim.x * blockDim.x;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n8; i += stride) {
         uint4 raw = __ldg(reinterpret_cast<const uint4*>(u) + i);
@@ -86,8 +80,6 @@ __global__ void quick_gelu_fwd_kernel(const bf16* __restrict__ u, bf16* __restri
 }
 
 __global__ void quick_gelu_bwd_kernel(const bf16* __restrict__ u, const bf16* __restrict__ dg, bf16* __restrict__ du, int64_t n8) {
-    ptx::pdl_trigger();
-    ptx::pdl_wait();
     const int64_t stride = (int64_t)gridDim.x * blockDim.x;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n8; i += stride) {
         uint4 ru = __ldg(reinterpret_cast<const uint4*>(u) + i), rg = __ldg(reinterpret_cast<const uint4*>(dg) + i);
@@ -109,8 +101,6 @@ __global__ void quick_gelu_bwd_kernel(const bf16* __restrict__ u, const bf16* __
 __global__ void __launch_bounds__(256) layernorm_f32out_kernel(const float* __restrict__ x, const float* __restrict__ gamma,
                                                                const float* __restrict__ beta, float* __restrict__ out, int rows,
                                                                int C, float eps) {
-    ptx::pdl_trigger();
-    ptx::pdl_wait();
     const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
     if (warp >= rows) return;
     const float* xr = x + (size_t)warp * C;
@@ -174,8 +164,6 @@ __device__ __forceinline__ void causal_probs(const float* __restrict__ q, const 
 __global__ void __launch_bounds__(256) clip_attention_fwd_kernel(const bf16* __restrict__ qkv, bf16* __restrict__ out, int S, int D,
                                                                  int ld, int ldo, int q_off, int k_off, int v_off, float scale) {
     extern __shared__ float sm[];
-    ptx::pdl_trigger();
-    ptx::pdl_wait();
     float* q = sm;
     float* k = q + kMaxS * (kMaxD + 1);
     float* v = k + kMaxS * (kMaxD + 1);
@@ -201,8 +189,6 @@ __global__ void __launch_bounds__(256) clip_attention_bwd_kernel(const bf16* __r
                                                                  bf16* __restrict__ dqkv, int S, int D, int ld, int lddo, int ldd,
                                                                  int q_off, int k_off, int v_off, float scale) {
     extern __shared__ float sm[];
-    ptx::pdl_trigger();
-    ptx::pdl_wait();
     float* q = sm;
     float* k = q + kMaxS * (kMaxD + 1);
     float* v = k + kMaxS * (kMaxD + 1);
@@ -263,8 +249,8 @@ extern "C" int b200sd_clip_embed(const int64_t* ids, const float* tok, const flo
     B200SD_REQUIRE(ids && tok && pos && out, "clip_embed: null pointer");
     B200SD_REQUIRE(batch > 0 && S > 0 && C > 0 && C % 4 == 0 && vocab > 0, "clip_embed: bad sizes");
     const int64_t total = (int64_t)batch * S * (C / 4);
-    B200SD_CUDA(b200sd_launch(clip_embed_kernel, dim3(ew_grid(total, 256)), dim3(256), 0, static_cast<cudaStream_t>(stream), ids, tok,
-                              pos, out, batch * S, S, C / 4, vocab));
+    clip_embed_kernel<<<dim3(ew_grid(total, 256)), dim3(256), 0, static_cast<cudaStream_t>(stream)>>>(ids, tok,
+                              pos, out, batch * S, S, C / 4, vocab);
     COUNT_LAUNCH();
     B200SD_LAUNCH_CHECK();
     return B200SD_OK;
@@ -274,8 +260,8 @@ extern "C" int b200sd_clip_embed_bwd(const int64_t* ids, const float* dx, float*
                                      int vocab, b200sd_stream_t stream) {
     B200SD_REQUIRE(ids && dx && dtok && dpos, "clip_embed_bwd: null pointer");
     B200SD_REQUIRE(batch > 0 && S > 0 && C > 0 && vocab > 0, "clip_embed_bwd: bad sizes");
-    B200SD_CUDA(b200sd_launch(clip_embed_bwd_kernel, dim3(S), dim3(256), 0, static_cast<cudaStream_t>(stream), ids, dx, dtok, dpos,
-                              batch, S, C, vocab));
+    clip_embed_bwd_kernel<<<dim3(S), dim3(256), 0, static_cast<cudaStream_t>(stream)>>>(ids, dx, dtok, dpos,
+                              batch, S, C, vocab);
     COUNT_LAUNCH();
     B200SD_LAUNCH_CHECK();
     return B200SD_OK;
@@ -283,8 +269,8 @@ extern "C" int b200sd_clip_embed_bwd(const int64_t* ids, const float* dx, float*
 
 extern "C" int b200sd_quick_gelu_fwd(const void* u, void* out, int64_t n, b200sd_stream_t stream) {
     B200SD_REQUIRE(u && out && n > 0 && n % 8 == 0, "quick_gelu_fwd: bad arguments (n must be a multiple of 8)");
-    B200SD_CUDA(b200sd_launch(quick_gelu_fwd_kernel, dim3(ew_grid(n / 8, 256)), dim3(256), 0, static_cast<cudaStream_t>(stream),
-                              static_cast<const bf16*>(u), static_cast<bf16*>(out), n / 8));
+    quick_gelu_fwd_kernel<<<dim3(ew_grid(n / 8, 256)), dim3(256), 0, static_cast<cudaStream_t>(stream)>>>(
+                              static_cast<const bf16*>(u), static_cast<bf16*>(out), n / 8);
     COUNT_LAUNCH();
     B200SD_LAUNCH_CHECK();
     return B200SD_OK;
@@ -292,8 +278,8 @@ extern "C" int b200sd_quick_gelu_fwd(const void* u, void* out, int64_t n, b200sd
 
 extern "C" int b200sd_quick_gelu_bwd(const void* u, const void* dg, void* du, int64_t n, b200sd_stream_t stream) {
     B200SD_REQUIRE(u && dg && du && n > 0 && n % 8 == 0, "quick_gelu_bwd: bad arguments (n must be a multiple of 8)");
-    B200SD_CUDA(b200sd_launch(quick_gelu_bwd_kernel, dim3(ew_grid(n / 8, 256)), dim3(256), 0, static_cast<cudaStream_t>(stream),
-                              static_cast<const bf16*>(u), static_cast<const bf16*>(dg), static_cast<bf16*>(du), n / 8));
+    quick_gelu_bwd_kernel<<<dim3(ew_grid(n / 8, 256)), dim3(256), 0, static_cast<cudaStream_t>(stream)>>>(
+                              static_cast<const bf16*>(u), static_cast<const bf16*>(dg), static_cast<bf16*>(du), n / 8);
     COUNT_LAUNCH();
     B200SD_LAUNCH_CHECK();
     return B200SD_OK;
@@ -302,8 +288,8 @@ extern "C" int b200sd_quick_gelu_bwd(const void* u, const void* dg, void* du, in
 extern "C" int b200sd_layernorm_f32out(const float* x, const float* gamma, const float* beta, float* out, int rows, int C, float eps,
                                        b200sd_stream_t stream) {
     B200SD_REQUIRE(x && gamma && beta && out && rows > 0 && C > 0, "layernorm_f32out: bad arguments");
-    B200SD_CUDA(b200sd_launch(layernorm_f32out_kernel, dim3(ceil_div(rows, 8)), dim3(256), 0, static_cast<cudaStream_t>(stream), x,
-                              gamma, beta, out, rows, C, eps));
+    layernorm_f32out_kernel<<<dim3(ceil_div(rows, 8)), dim3(256), 0, static_cast<cudaStream_t>(stream)>>>(x,
+                              gamma, beta, out, rows, C, eps);
     COUNT_LAUNCH();
     B200SD_LAUNCH_CHECK();
     return B200SD_OK;
@@ -324,8 +310,8 @@ extern "C" int b200sd_causal_attention(const void* qkv, void* out, int batch, in
     B200SD_REQUIRE(q_off % 8 == 0 && k_off % 8 == 0 && v_off % 8 == 0, "causal_attention: offsets must be multiples of 8 elements");
     const size_t smem = (size_t)(3 * kMaxS * (kMaxD + 1) + kMaxS * (kMaxS + 1)) * sizeof(float);
     B200SD_CUDA(b200sd_opt_in_smem(clip_attention_fwd_kernel, (int)smem));
-    B200SD_CUDA(b200sd_launch(clip_attention_fwd_kernel, dim3(heads, batch), dim3(256), smem, static_cast<cudaStream_t>(stream),
-                              static_cast<const bf16*>(qkv), static_cast<bf16*>(out), S, d, ld, ldo, q_off, k_off, v_off, scale));
+    clip_attention_fwd_kernel<<<dim3(heads, batch), dim3(256), smem, static_cast<cudaStream_t>(stream)>>>(
+                              static_cast<const bf16*>(qkv), static_cast<bf16*>(out), S, d, ld, ldo, q_off, k_off, v_off, scale);
     COUNT_LAUNCH();
     B200SD_LAUNCH_CHECK();
     return B200SD_OK;
@@ -338,9 +324,9 @@ extern "C" int b200sd_causal_attention_bwd(const void* qkv, const void* dout, vo
     B200SD_REQUIRE(lddo % 8 == 0, "causal_attention_bwd: lddo must be a multiple of 8 elements");
     const size_t smem = (size_t)(4 * kMaxS * (kMaxD + 1) + 2 * kMaxS * (kMaxS + 1)) * sizeof(float);
     B200SD_CUDA(b200sd_opt_in_smem(clip_attention_bwd_kernel, (int)smem));
-    B200SD_CUDA(b200sd_launch(clip_attention_bwd_kernel, dim3(heads, batch), dim3(256), smem, static_cast<cudaStream_t>(stream),
+    clip_attention_bwd_kernel<<<dim3(heads, batch), dim3(256), smem, static_cast<cudaStream_t>(stream)>>>(
                               static_cast<const bf16*>(qkv), static_cast<const bf16*>(dout), static_cast<bf16*>(dqkv), S, d, ld, lddo,
-                              ldd, q_off, k_off, v_off, scale));
+                              ldd, q_off, k_off, v_off, scale);
     COUNT_LAUNCH();
     B200SD_LAUNCH_CHECK();
     return B200SD_OK;

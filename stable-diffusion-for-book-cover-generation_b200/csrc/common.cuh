@@ -8,7 +8,6 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
-#include <utility>
 
 #include "../../include/b200sd.h"
 
@@ -42,8 +41,6 @@ static inline int ceil_div(int a, int b) { return (a + b - 1) / b; }
 
 // number of SMs of the current device (cached)
 int b200sd_num_sms();
-// programmatic dependent launch (PDL) between consecutive kernels of a stream (opt-in: B200SD_PDL=1)
-bool b200sd_pdl_enabled();
 
 // Encode a tiled TMA descriptor (driver entry point fetched through the runtime; no -lcuda needed).
 // dims/strides are innermost-first; strides are in bytes for dims 1..rank-1.
@@ -61,35 +58,10 @@ static inline cudaError_t b200sd_opt_in_smem(K kernel, int bytes, bool max_carve
     return b200sd_opt_in_smem_impl(reinterpret_cast<const void*>(kernel), bytes, max_carveout);
 }
 
-// Launch with the programmatic-stream-serialization attribute: the next kernel's CTAs may become
-// resident (and run their prologue up to ptx::pdl_wait()) while this kernel drains.  Every kernel of
-// the library calls ptx::pdl_wait() before its first dependent global access, which keeps the
-// stream's transitive ordering intact.
-template <typename... KArgs, typename... Args>
-static inline cudaError_t b200sd_launch(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem,
-                                        cudaStream_t stream, Args&&... args) {
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = grid;
-    cfg.blockDim = block;
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = b200sd_pdl_enabled() ? 1 : 0;
-    return cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...);
-}
-
 // ----------------------------------------------------------------------------------------------
 // device helpers
 // ----------------------------------------------------------------------------------------------
 namespace ptx {
-
-// PDL: wait until the preceding kernel of the stream has completed and its writes are visible
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-// PDL: allow the next kernel of the stream to start launching
-__device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) {
     return static_cast<uint32_t>(__cvta_generic_to_shared(p));
@@ -173,35 +145,6 @@ __device__ __forceinline__ void tma_load_4d(void* dst, const CUtensorMap* m, uin
         "[%2];" ::"r"(smem_u32(dst)),
         "l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
         : "memory");
-}
-
-// L2 prefetch of a tensor-map box (no smem destination, no barrier): pulls weights from HBM into L2 ahead of the smem ring
-__device__ __forceinline__ void tma_prefetch_2d(const CUtensorMap* m, int c0, int c1) {
-    asm volatile("cp.async.bulk.prefetch.tensor.2d.L2.global.tile [%0, {%1, %2}];" ::"l"(reinterpret_cast<uint64_t>(m)), "r"(c0), "r"(c1)
-                 : "memory");
-}
-__device__ __forceinline__ void tma_prefetch_3d(const CUtensorMap* m, int c0, int c1, int c2) {
-    asm volatile("cp.async.bulk.prefetch.tensor.3d.L2.global.tile [%0, {%1, %2, %3}];" ::"l"(reinterpret_cast<uint64_t>(m)), "r"(c0), "r"(c1),
-                 "r"(c2)
-                 : "memory");
-}
-
-// pull `bytes` (multiple of 16, 16-byte aligned) of global memory into L2; fire and forget
-__device__ __forceinline__ void bulk_prefetch_l2(const void* p, uint32_t bytes) {
-    asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(p), "r"(bytes) : "memory");
-}
-// this CTA's share of a [ptr, ptr + bytes) prefetch spread over `nctas` CTAs (called by ONE thread)
-__device__ __forceinline__ void prefetch_share_l2(const void* ptr, size_t bytes, int cta, int nctas) {
-    if (ptr == nullptr || bytes == 0) return;
-    const size_t per = ((bytes + nctas - 1) / nctas + 4095) & ~size_t(4095);
-    size_t off = (size_t)cta * per;
-    const size_t end = off + per < bytes ? off + per : (bytes & ~size_t(15));
-    const char* base = static_cast<const char*>(ptr);
-    while (off < end) {
-        const size_t n = end - off < 65536 ? end - off : 65536;
-        bulk_prefetch_l2(base + off, (uint32_t)n);
-        off += n;
-    }
 }
 
 // ---- TMA store: smem tile -> global through a tensor map (bulk async-group completion) ----

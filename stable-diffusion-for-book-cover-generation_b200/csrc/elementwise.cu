@@ -92,8 +92,6 @@ __global__ void __launch_bounds__(kThreads) cfg_ddim_kernel(const void* __restri
                                                             const void* __restrict__ x, void* __restrict__ out,
                                                             void* __restrict__ eps_out, int64_t n, int64_t nvec, DdimCoef c,
                                                             const float4* __restrict__ coef_table, const int* __restrict__ cursor) {
-    ptx::pdl_trigger();
-    ptx::pdl_wait();
     if (coef_table != nullptr) {     // captured sampler: this step's coefficients come from a device table (b200sd_sampler_advance)
         const float4 v = coef_table[cursor[1]];
         c.sa_t = v.x, c.sb_t = v.y, c.sa_p = v.z, c.sb_p = v.w;
@@ -138,8 +136,6 @@ __global__ void __launch_bounds__(kThreads) cfg_plms_kernel(const void* __restri
                                                             const void* __restrict__ eps_c,
                                                             const void* __restrict__ x, void* __restrict__ out,
                                                             void* __restrict__ eps_out, int64_t n, int64_t nvec, PlmsArgs a) {
-    ptx::pdl_trigger();
-    ptx::pdl_wait();
     const bool cfg = eps_c != nullptr;
     const int64_t stride = (int64_t)gridDim.x * blockDim.x;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < nvec; i += stride) {
@@ -185,8 +181,6 @@ __global__ void __launch_bounds__(kThreads) add_noise_kernel(const void* __restr
                                                              const float* __restrict__ sa_table,
                                                              const float* __restrict__ sb_table,
                                                              void* __restrict__ out, int64_t per_sample, int64_t nvec, int T) {
-    ptx::pdl_trigger();
-    ptx::pdl_wait();
     const int b = blockIdx.y;
     int64_t t = timesteps[b];
     t = t < 0 ? 0 : (t >= T ? T - 1 : t);
@@ -232,8 +226,6 @@ __global__ void __launch_bounds__(kThreads) mse_fwd_kernel(const void* __restric
                                                            int64_t n, int64_t nvec) {
     __shared__ float sm[32];
     __shared__ bool is_last;
-    ptx::pdl_trigger();
-    ptx::pdl_wait();
     float acc = 0.f;
     const int64_t stride = (int64_t)gridDim.x * blockDim.x;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < nvec; i += stride) {
@@ -285,8 +277,6 @@ __global__ void __launch_bounds__(kThreads) mse_bwd_kernel(const void* __restric
                                                            const void* __restrict__ target,
                                                            const float* __restrict__ grad_loss,
                                                            void* __restrict__ grad_pred, int64_t n, int64_t nvec) {
-    ptx::pdl_trigger();
-    ptx::pdl_wait();
     const float s = __ldg(grad_loss) * 2.0f / (float)n;
     const int64_t stride = (int64_t)gridDim.x * blockDim.x;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < nvec; i += stride) {
@@ -307,16 +297,16 @@ bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 
 
 }  // namespace
 
-#define DISPATCH2(E, X, KERNEL, GRID, STREAM, ...)                                                                   \
-    do {                                                                                                              \
-        if ((E) == B200SD_F32 && (X) == B200SD_F32)                                                                   \
-            B200SD_CUDA(b200sd_launch(KERNEL<B200SD_F32, B200SD_F32>, dim3(GRID), dim3(kThreads), 0, STREAM, __VA_ARGS__));  \
-        else if ((E) == B200SD_BF16 && (X) == B200SD_F32)                                                             \
-            B200SD_CUDA(b200sd_launch(KERNEL<B200SD_BF16, B200SD_F32>, dim3(GRID), dim3(kThreads), 0, STREAM, __VA_ARGS__)); \
-        else if ((E) == B200SD_F32 && (X) == B200SD_BF16)                                                             \
-            B200SD_CUDA(b200sd_launch(KERNEL<B200SD_F32, B200SD_BF16>, dim3(GRID), dim3(kThreads), 0, STREAM, __VA_ARGS__)); \
-        else                                                                                                          \
-            B200SD_CUDA(b200sd_launch(KERNEL<B200SD_BF16, B200SD_BF16>, dim3(GRID), dim3(kThreads), 0, STREAM, __VA_ARGS__)); \
+#define DISPATCH2(E, X, KERNEL, GRID, STREAM, ...)                                                    \
+    do {                                                                                              \
+        if ((E) == B200SD_F32 && (X) == B200SD_F32)                                                   \
+            KERNEL<B200SD_F32, B200SD_F32><<<dim3(GRID), dim3(kThreads), 0, STREAM>>>(__VA_ARGS__);   \
+        else if ((E) == B200SD_BF16 && (X) == B200SD_F32)                                             \
+            KERNEL<B200SD_BF16, B200SD_F32><<<dim3(GRID), dim3(kThreads), 0, STREAM>>>(__VA_ARGS__);  \
+        else if ((E) == B200SD_F32 && (X) == B200SD_BF16)                                             \
+            KERNEL<B200SD_F32, B200SD_BF16><<<dim3(GRID), dim3(kThreads), 0, STREAM>>>(__VA_ARGS__);  \
+        else                                                                                          \
+            KERNEL<B200SD_BF16, B200SD_BF16><<<dim3(GRID), dim3(kThreads), 0, STREAM>>>(__VA_ARGS__); \
     } while (0)
 
 static bool dtype_ok(int d) { return d == B200SD_F32 || d == B200SD_BF16; }
@@ -361,7 +351,7 @@ extern "C" int b200sd_sampler_advance(const float* timesteps, int n_steps, int* 
     B200SD_REQUIRE(timesteps && cursor && in_t, "sampler_advance: null pointer");
     B200SD_REQUIRE(n_steps > 0 && n_t > 0, "sampler_advance: empty table");
     cudaStream_t s = static_cast<cudaStream_t>(stream);
-    B200SD_CUDA(b200sd_launch(sampler_advance_kernel, dim3(1), dim3(64), 0, s, timesteps, n_steps, cursor, in_t, n_t));
+    sampler_advance_kernel<<<dim3(1), dim3(64), 0, s>>>(timesteps, n_steps, cursor, in_t, n_t);
     COUNT_LAUNCH();
     B200SD_LAUNCH_CHECK();
     return B200SD_OK;
@@ -378,8 +368,6 @@ __global__ void __launch_bounds__(kThreads) cfg_plms_table_kernel(const float* _
                                                                   float* __restrict__ x, float* __restrict__ saved,
                                                                   float* __restrict__ ring, int64_t n, float g,
                                                                   const float* __restrict__ table, const int* __restrict__ cursor) {
-    ptx::pdl_trigger();
-    ptx::pdl_wait();
     const float* row = table + (size_t)cursor[1] * kPlmsRow;
     const float w0 = row[0], w1 = row[1], w2 = row[2], w3 = row[3], cx = row[4], ce = row[5];
     const int h1 = (int)row[6], h2 = (int)row[7], h3 = (int)row[8], slot = (int)row[9];
@@ -408,8 +396,8 @@ extern "C" int b200sd_cfg_plms_step_table(const float* eps_u, const float* eps_c
     B200SD_REQUIRE(n >= 0, "cfg_plms_step_table: negative n");
     if (n == 0) return B200SD_OK;
     cudaStream_t s = static_cast<cudaStream_t>(stream);
-    B200SD_CUDA(b200sd_launch(cfg_plms_table_kernel, dim3(grid_for(n)), dim3(kThreads), 0, s, eps_u, eps_c, x, saved, ring, n, guidance,
-                              table, cursor));
+    cfg_plms_table_kernel<<<dim3(grid_for(n)), dim3(kThreads), 0, s>>>(eps_u, eps_c, x, saved, ring, n, guidance,
+                              table, cursor);
     COUNT_LAUNCH();
     B200SD_LAUNCH_CHECK();
     return B200SD_OK;
@@ -475,9 +463,9 @@ extern "C" int b200sd_add_noise(const void* x0, const void* noise, const int64_t
     if (gx > cap) gx = cap;
     dim3 grid(gx, batch);
     if (dtype == B200SD_F32)
-        B200SD_CUDA(b200sd_launch(add_noise_kernel<B200SD_F32>, dim3(grid), dim3(kThreads), 0, s, x0, noise, timesteps, sa_table, sb_table, out, per_sample, nvec, num_train_timesteps));
+        add_noise_kernel<B200SD_F32><<<dim3(grid), dim3(kThreads), 0, s>>>(x0, noise, timesteps, sa_table, sb_table, out, per_sample, nvec, num_train_timesteps);
     else
-        B200SD_CUDA(b200sd_launch(add_noise_kernel<B200SD_BF16>, dim3(grid), dim3(kThreads), 0, s, x0, noise, timesteps, sa_table, sb_table, out, per_sample, nvec, num_train_timesteps));
+        add_noise_kernel<B200SD_BF16><<<dim3(grid), dim3(kThreads), 0, s>>>(x0, noise, timesteps, sa_table, sb_table, out, per_sample, nvec, num_train_timesteps);
     COUNT_LAUNCH();
     B200SD_LAUNCH_CHECK();
     return B200SD_OK;

@@ -32,8 +32,6 @@ __device__ __forceinline__ void split8(const float (&y)[8], float (&hi)[8], floa
 
 // x fp32 [n] -> hi, lo bf16 [n]
 __global__ void split_hi_lo_kernel(const float* __restrict__ x, bf16* __restrict__ hi, bf16* __restrict__ lo, int64_t n8) {
-    ptx::pdl_trigger();
-    ptx::pdl_wait();
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n8; i += (int64_t)gridDim.x * blockDim.x) {
         float v[8], h[8], l[8];
         ld8<B200SD_F32>(x, (size_t)i * 8, v);
@@ -45,8 +43,6 @@ __global__ void split_hi_lo_kernel(const float* __restrict__ x, bf16* __restrict
 
 // u fp32 [rows, 2*Ch] = [values | gates] -> (hi, lo) of values * gelu_erf(gates), [rows, Ch]
 __global__ void geglu_f32_kernel(const float* __restrict__ u, bf16* __restrict__ hi, bf16* __restrict__ lo, int64_t rows, int Ch8) {
-    ptx::pdl_trigger();
-    ptx::pdl_wait();
     const int64_t total = rows * Ch8;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
         const int64_t row = i / Ch8;
@@ -77,8 +73,6 @@ __global__ void __launch_bounds__(kFThreads) attention_f32_kernel(const float* _
     float* sK = sQ + kFQ * (D + 1);       // [64][D + 1]
     float* sV = sK + kFK * (D + 1);       // [64][D + 1]
     float* sP = sV + kFK * (D + 1);       // [64][65]
-    ptx::pdl_trigger();
-    ptx::pdl_wait();
     const int b = blockIdx.z, h = blockIdx.y, q0 = blockIdx.x * kFQ;
     const int qi = threadIdx.x >> 2, part = threadIdx.x & 3;
     const float* qg = q + ((size_t)b * Sq + q0) * ldq + h * D;
@@ -156,8 +150,8 @@ int launch_attn_f32(const float* q, const float* k, const float* v, float* out, 
     constexpr int D = DQ * 4;
     const size_t smem = ((size_t)3 * 64 * (D + 1) + 64 * 65) * sizeof(float);
     B200SD_CUDA(b200sd_opt_in_smem(attention_f32_kernel<DQ>, (int)smem));
-    B200SD_CUDA(b200sd_launch(attention_f32_kernel<DQ>, dim3(ceil_div(Sq, kFQ), heads, batch), dim3(kFThreads), smem, s, q, k, v, out, Sq, Skv,
-                              ldq, ldk, ldv, ldo, scale));
+    attention_f32_kernel<DQ><<<dim3(ceil_div(Sq, kFQ), heads, batch), dim3(kFThreads), smem, s>>>(q, k, v, out, Sq, Skv,
+                              ldq, ldk, ldv, ldo, scale);
     COUNT_LAUNCH();
     B200SD_LAUNCH_CHECK();
     return B200SD_OK;
@@ -167,8 +161,6 @@ int launch_attn_f32(const float* q, const float* k, const float* v, float* out, 
 __global__ void __launch_bounds__(256) small_linear_f32_kernel(const float* __restrict__ in, const float* __restrict__ w,
                                                                const float* __restrict__ bias, float* __restrict__ out, int batch,
                                                                int N, int K, int silu_in, int silu_out) {
-    ptx::pdl_trigger();
-    ptx::pdl_wait();
     const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
     if (warp >= N) return;
     for (int b = 0; b < batch; ++b) {
@@ -191,8 +183,8 @@ __global__ void __launch_bounds__(256) small_linear_f32_kernel(const float* __re
 
 extern "C" int b200sd_split_hi_lo(const float* x, void* hi, void* lo, int64_t n, b200sd_stream_t stream) {
     B200SD_REQUIRE(x && hi && lo && n > 0 && n % 8 == 0, "split_hi_lo: n must be a positive multiple of 8");
-    B200SD_CUDA(b200sd_launch(split_hi_lo_kernel, dim3(ew_grid(n / 8, 256)), dim3(256), 0, static_cast<cudaStream_t>(stream), x,
-                              static_cast<bf16*>(hi), static_cast<bf16*>(lo), n / 8));
+    split_hi_lo_kernel<<<dim3(ew_grid(n / 8, 256)), dim3(256), 0, static_cast<cudaStream_t>(stream)>>>(x,
+                              static_cast<bf16*>(hi), static_cast<bf16*>(lo), n / 8);
     COUNT_LAUNCH();
     B200SD_LAUNCH_CHECK();
     return B200SD_OK;
@@ -200,8 +192,8 @@ extern "C" int b200sd_split_hi_lo(const float* x, void* hi, void* lo, int64_t n,
 
 extern "C" int b200sd_geglu_f32(const float* u, void* hi, void* lo, int64_t rows, int C_half, b200sd_stream_t stream) {
     B200SD_REQUIRE(u && hi && lo && rows > 0 && C_half > 0 && C_half % 8 == 0, "geglu_f32: bad arguments");
-    B200SD_CUDA(b200sd_launch(geglu_f32_kernel, dim3(ew_grid(rows * (C_half / 8), 256)), dim3(256), 0, static_cast<cudaStream_t>(stream), u,
-                              static_cast<bf16*>(hi), static_cast<bf16*>(lo), rows, C_half / 8));
+    geglu_f32_kernel<<<dim3(ew_grid(rows * (C_half / 8), 256)), dim3(256), 0, static_cast<cudaStream_t>(stream)>>>(u,
+                              static_cast<bf16*>(hi), static_cast<bf16*>(lo), rows, C_half / 8);
     COUNT_LAUNCH();
     B200SD_LAUNCH_CHECK();
     return B200SD_OK;
@@ -223,8 +215,8 @@ extern "C" int b200sd_attention_f32(const float* q, const float* k, const float*
 extern "C" int b200sd_small_linear_f32(const float* in, const float* w, const float* bias, float* out, int batch, int N, int K,
                                        int silu_in, int silu_out, b200sd_stream_t stream) {
     B200SD_REQUIRE(in && w && out && batch > 0 && N > 0 && K > 0, "small_linear_f32: bad arguments");
-    B200SD_CUDA(b200sd_launch(small_linear_f32_kernel, dim3(ceil_div(N * 32, 256)), dim3(256), 0, static_cast<cudaStream_t>(stream), in, w, bias,
-                              out, batch, N, K, silu_in, silu_out));
+    small_linear_f32_kernel<<<dim3(ceil_div(N * 32, 256)), dim3(256), 0, static_cast<cudaStream_t>(stream)>>>(in, w, bias,
+                              out, batch, N, K, silu_in, silu_out);
     COUNT_LAUNCH();
     B200SD_LAUNCH_CHECK();
     return B200SD_OK;

@@ -18,35 +18,16 @@
 #include <cstring>
 #include <mutex>
 #include <cstdio>
-#include <cstdlib>
 
 #include "common.cuh"
 
 extern std::atomic<long long> g_b200sd_launches;
 
-static unsigned long long* g_gemm_trace = nullptr;
-// debug / tuning overrides (tools/conv_probe.py): key 0 = persistent kernel (-1 default, 0 off, 1 on), key 1 = smem ring depth
-// (0 = auto), key 2 = cap on the persistent grid (0 = one CTA per SM)
-static int g_dbg[4] = {-1, 0, 0, 0};   // [3] = residual prefetch depth (2 / 3)
-static const int g_dbg_env = [] {
-    const char* e = getenv("B200SD_EPI_DEPTH");
-    if (e) g_dbg[3] = atoi(e);
-    return 0;
-}();
-extern "C" void b200sd_debug_set(int key, int value) { if (key >= 0 && key < 4) g_dbg[key] = value; }
-extern "C" void b200sd_debug_gemm_trace(void* buf) { g_gemm_trace = static_cast<unsigned long long*>(buf); }
+// debug override (tools/cold_probe.py): key 0 = persistent kernel (-1 default, 0 off, 1 on)
+static int g_persist = -1;
+extern "C" void b200sd_debug_set(int key, int value) { if (key == 0) g_persist = value; }
 
 namespace {
-
-__device__ __forceinline__ unsigned long long gtimer() {
-    unsigned long long t;
-    asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t));
-    return t;
-}
-#define TRACE(slot)                                                                                   \
-    do {                                                                                              \
-        if (p.trace) p.trace[((size_t)(blockIdx.z * gridDim.y + blockIdx.y) * gridDim.x + blockIdx.x) * 16 + (slot)] = gtimer(); \
-    } while (0)
 
 constexpr int BLOCK_M = 128;
 constexpr size_t kWsPartialBytes = (size_t)160 * 128 * 256 * sizeof(float);   // split-K partial tiles (<= one per SM), see b200sd_gemm_workspace_bytes
@@ -96,13 +77,8 @@ struct KParams {
                          // 128 A rows and HALF of the B tile, so the L2 -> smem traffic per FLOP drops by ~1/3
     int persist;         // host only: this launch goes to gemm_persist_kernel (set by gemm_tiling)
     int psplit;          // host only: ... in its split-K mode with this many K slices per tile (0 = no)
-    int w_kmajor;        // forward B operand stored k-block-major [K/64][N][64]: one tile k-block = ONE contiguous bn x 128 B run of
-                         // DRAM instead of bn 128-byte pieces a whole weight row (K * 2 B) apart
-    const void* prefetch;       // next layer's weights: pulled into L2 while this kernel runs (see b200sd_gemm_args::prefetch)
-    size_t prefetch_bytes;
     float* gn_part;      // optional [m_tiles * split_k][2][N]: per-column (sum, sum of squares) of the rows each CTA stores --
                          // the GroupNorm that consumes this output gets its statistics from here instead of re-reading it
-    unsigned long long* trace;  // optional [ctas][8] globaltimer stamps (debug)
 };
 
 // cluster helpers (split-K reduction over distributed shared memory)
@@ -244,8 +220,6 @@ __global__ void __launch_bounds__(kNumThreads, 1) gemm_tcgen05_kernel(const __gr
     const int col_valid = min(p.block_n, p.n_valid - n0);
     const int m0 = m_tile * p.rows_valid;
 
-    ptx::pdl_trigger();
-    if (threadIdx.x == 0) TRACE(0);
     if (warp == 0 && lane == 0) {
         ptx::prefetch_tmap(&p.tmA0);
         ptx::prefetch_tmap(&p.tmB);
@@ -266,8 +240,6 @@ __global__ void __launch_bounds__(kNumThreads, 1) gemm_tcgen05_kernel(const __gr
     if constexpr (pair) cluster_sync_all();   // the peer's barriers must be initialised before anything is signalled on them
     ptx::tc_fence_after();
     const uint32_t tmem_base = *tmem_slot;
-    ptx::pdl_wait();  // everything above overlapped the previous kernel's tail
-    if (threadIdx.x == 0) TRACE(1);
 
     // epilogue-side shared state (also visible to part 2 after the role dispatch)
     const int epi_tid = threadIdx.x - 64;  // 0..127 for the epilogue warps
@@ -331,8 +303,7 @@ __global__ void __launch_bounds__(kNumThreads, 1) gemm_tcgen05_kernel(const __gr
                 }
                 // ---- B ----
                 if (b_mode == 0) {
-                    if (p.w_kmajor) LD3(dst_b, &p.tmB, 0, nb0, kb);
-                    else LD2(dst_b, &p.tmB, kb * BLOCK_K, nb0);
+                    LD2(dst_b, &p.tmB, kb * BLOCK_K, nb0);
                 } else if (b_mode == 1) {
                     if (!p.conv) {
                         for (int j = 0; j < nboxb; ++j) LD2(dst_b + j * 8192, &p.tmB, nb0 + j * 64, kb * BLOCK_K);
@@ -370,7 +341,6 @@ __global__ void __launch_bounds__(kNumThreads, 1) gemm_tcgen05_kernel(const __gr
             for (int kb = kb_begin; kb < kb_end; ++kb) {
                 ptx::mbar_wait(&full_bar[stage], phase);
                 ptx::tc_fence_after();
-                if (kb == kb_begin) TRACE(2);
                 const uint32_t sa = ptx::smem_u32(smem_a + (size_t)stage * kABytes), sb = ptx::smem_u32(smem_b + (size_t)stage * b_bytes);
                 const uint64_t da = a_mn ? ptx::umma_desc_mn_sw128(sa, 8192) : ptx::umma_desc_k_sw128(sa);
                 const uint64_t db = b_mn ? ptx::umma_desc_mn_sw128(sb, 8192) : ptx::umma_desc_k_sw128(sb);
@@ -385,7 +355,6 @@ __global__ void __launch_bounds__(kNumThreads, 1) gemm_tcgen05_kernel(const __gr
                 if (++stage == p.stages) { stage = 0; phase ^= 1; }
             }
             if constexpr (pair) ptx::umma_commit_cg2(tmem_full_bar, 3); else ptx::umma_commit(tmem_full_bar);
-            TRACE(3);
         }
     } else {
         // ================= epilogue warps, part 1 =================
@@ -401,12 +370,8 @@ __global__ void __launch_bounds__(kNumThreads, 1) gemm_tcgen05_kernel(const __gr
                 s_rb[256 + c] = __ldg(p.rowbias + (size_t)img1 * p.ldrb + n0 + c);
             }
         }
-        if (epi_tid == 0 && p.prefetch_bytes)   // idle until the accumulator is ready: stage the NEXT layer's weights in L2
-            ptx::prefetch_share_l2(p.prefetch, p.prefetch_bytes, (blockIdx.z * gridDim.y + blockIdx.y) * gridDim.x + blockIdx.x,
-                              gridDim.x * gridDim.y * gridDim.z);
         ptx::mbar_wait(tmem_full_bar, 0);
         ptx::tc_fence_after();
-        if (epi_tid == 0) TRACE(4);
         {
             float4* my_row = reinterpret_cast<float4*>(stage + (size_t)r_in_tile * pitch_f);
             for (int c = 0; c < p.block_n; c += 32) {
@@ -429,7 +394,6 @@ __global__ void __launch_bounds__(kNumThreads, 1) gemm_tcgen05_kernel(const __gr
         }
         ptx::tc_fence_before();
         ptx::named_bar_sync(1, 128);  // whole staging tile (and the bias tiles) written
-        if (epi_tid == 0) TRACE(5);
     }
 
     // Split-K: the `split_k` CTAs of a tile form one thread-block cluster; after this barrier every CTA can
@@ -505,7 +469,6 @@ __global__ void __launch_bounds__(kNumThreads, 1) gemm_tcgen05_kernel(const __gr
                 if (col < col_valid) dst[(size_t)(k >> 3) * p.N + n0 + col] = a;
             }
         }
-        if (epi_tid == 0) TRACE(6);
     }
     // peers may still be reading this CTA's staging tile (with gn_part the cluster has already synchronised above)
     if (p.split_k > 1 && p.gn_part == nullptr) cluster_sync_all();
@@ -517,7 +480,6 @@ __global__ void __launch_bounds__(kNumThreads, 1) gemm_tcgen05_kernel(const __gr
         ptx::tc_fence_after();
         if constexpr (pair) ptx::tmem_dealloc_cg2(tmem_base, p.tmem_cols); else ptx::tmem_dealloc(tmem_base, p.tmem_cols);
     }
-    if (threadIdx.x == 0) TRACE(7);
 }
 
 // =================================================================================================================
@@ -546,12 +508,11 @@ struct PParams {
     float* gn_part;
     int M, N;
     int num_k_blocks, block_n, stages;
-    int conv, cblocks0, cblocks, tile_h, tile_n, tiles_y, w_kmajor;
+    int conv, cblocks0, cblocks, tile_h, tile_n, tiles_y;
     int tile_w, tiles_x;            // image rows wider than a tile (see KParams::tiles_x)
     int n_tiles, num_tiles;
     int ldrb, rows_per_image;
     int geglu, out_f32, res_kind;   // res_kind: 0 none, 1 bf16, 2 fp32
-    int pf_share;                   // CTAs that stream the same weight tile concurrently: they split its L2 prefetch k-block by k-block
     int depth;                      // smem chunks per epilogue warp (3 with a residual, 2 without)
     int chunk_bytes;                // 4096: 32 rows x 128 B (an fp32 chunk is involved); 2048: 32 rows x 64 B (bf16 only)
     uint32_t tmem_cols, acc_stride;
@@ -561,21 +522,10 @@ struct PParams {
     CUtensorMap tmWs;               // fp32 partial tiles in the workspace: [units * 128][block_n]
     float* ws;                      // the same buffer, for the reduction's plain loads
     int* cnt;                       // [2][num_tiles] arrival / departure counters (zero between launches: self-resetting)
-    const void* prefetch;           // next layer's weights -> L2 (b200sd_gemm_args::prefetch)
-    size_t prefetch_bytes;
     const void* residual;           // raw pointers for the reduction phase
     void* out;
     int ldc, ldr;
-    unsigned long long* trace;      // optional [ctas][8] globaltimer stamps (debug)
 };
-#define PTRACE(slot) do { if (p.trace) p.trace[(size_t)blockIdx.x * 16 + (slot)] = gtimer(); } while (0)
-// epilogue phase accounting of warp 2, lane 0 (clock64 ticks summed over its chunks) -> trace slots 8..13
-#ifdef B200SD_TRACE_EPILOGUE
-#define PACC(i) do { if (p.trace && ew == 0) { const long long t__ = clock64(); pacc[i] += t__ - pt0; pt0 = t__; } } while (0)
-#else
-#define PACC(i) do { } while (0)
-#endif
-
 
 // one 32-column chunk of this warp's 32 accumulator rows; cb = the warp's smem chunk (holds the residual when RES != 0)
 template <bool OUT_F32, int RES, bool GEGLU, bool STATS>
@@ -714,15 +664,11 @@ __device__ __forceinline__ void persist_epilogue(const PParams& p, uint8_t* smem
     }
 
     int g = 0;
-#ifdef B200SD_TRACE_EPILOGUE
-    long long pacc[6] = {0, 0, 0, 0, 0, 0}, pt0 = clock64();
-#endif
     for (int it = 0; it < my_tiles; ++it) {
         const int tile = (int)blockIdx.x + it * (int)gridDim.x;
         const int m_tile = tile / p.n_tiles, n_tile = tile - m_tile * p.n_tiles;
         const int n0 = n_tile * p.block_n;
         const int row0 = m_tile * BLOCK_M + q * 32;
-        PACC(5);
         // the biases of this warp's chunks (+ the time-embedding row of this warp's image) -> the warp's smem copy
         __syncwarp();
         {
@@ -736,12 +682,9 @@ __device__ __forceinline__ void persist_epilogue(const PParams& p, uint8_t* smem
             }
         }
         __syncwarp();
-        PACC(0);   // bias staging
         const int acc = it & 1;
         ptx::mbar_wait(&tfull[acc], (uint32_t)(it >> 1) & 1u);
         ptx::tc_fence_after();
-        PACC(1);   // waiting for the accumulator
-        if (it == 0 && ew == 0 && lane == 0) PTRACE(4);
         const uint32_t taddr = tmem_base + (uint32_t)acc * p.acc_stride + ((uint32_t)(q * 32) << 16);
         const int nrows = max(0, min(32, p.M - row0));
         float* sstat = reinterpret_cast<float*>(smem + p.off_stat);   // [4 quarters][2][256]
@@ -760,10 +703,8 @@ __device__ __forceinline__ void persist_epilogue(const PParams& p, uint8_t* smem
                 if (lane == 0) ptx::tma_store_wait_read<1>();
                 __syncwarp();
             }
-            PACC(2);   // waiting for the smem chunk to be free
             persist_chunk<OUT_F32, RES, GEGLU, STATS>(p, taddr, ch, sb + l * 32, sb + 128 + l * 32, cb, lane, l == nl - 1, &tempty[acc],
                                                      &rfull[buf], (uint32_t)(g / D) & 1u, gn_dst, nrows);
-            PACC(3);   // TMEM -> registers -> epilogue math -> smem
             ptx::fence_proxy_async();   // generic-proxy smem writes -> visible to the TMA (async proxy)
             __syncwarp();
             if (lane == 0) {
@@ -777,7 +718,6 @@ __device__ __forceinline__ void persist_epilogue(const PParams& p, uint8_t* smem
                     }
                 }
             }
-            PACC(4);   // proxy fence + TMA store issue (+ residual refill)
         }
         if constexpr (STATS) {
             // GroupNorm statistics of the tile: the four quarters' column sums folded in a fixed order (bit-reproducible) into
@@ -795,14 +735,8 @@ __device__ __forceinline__ void persist_epilogue(const PParams& p, uint8_t* smem
             ptx::named_bar_sync(1, kEpiWarps * 32);   // the scratch is rewritten by the next tile
         }
     }
-    if (ew == 0 && lane == 0) PTRACE(5);
-#ifdef B200SD_TRACE_EPILOGUE
-    if (p.trace && ew == 0 && lane == 0)
-        for (int i = 0; i < 6; ++i) p.trace[(size_t)blockIdx.x * 16 + 8 + i] = (unsigned long long)pacc[i];
-#endif
     if (lane == 0) ptx::tma_store_wait<0>();   // all output writes performed before the CTA may exit
     __syncwarp();
-    if (ew == 0 && lane == 0) PTRACE(6);
 }
 
 // ---- split-K epilogue: K slice s of a tile.  Phase 1: the fp32 partial accumulator goes to the workspace (TMA stores, same
@@ -981,22 +915,9 @@ __global__ void __launch_bounds__(kPersistThreads, 1) gemm_persist_kernel(const 
     const int sk_kb0 = splitk ? (sk_s * p.num_k_blocks) / p.split : 0;
     const int sk_kb1 = splitk ? ((sk_s + 1) * p.num_k_blocks) / p.split : p.num_k_blocks;
     int pr_stage = 0, pr_tile = splitk ? sk_tile : (int)blockIdx.x, pr_kb = sk_kb0, pr_m0 = 0, pr_n0 = 0, pr_img = 0, pr_y0 = 0, pr_x0 = 0, pr_tap = 0,
-        pr_cb = 0, pr_me = 0;
+        pr_cb = 0;
     bool pr_new = true;
     uint32_t pr_phase = 0;
-    // The weights are cold in HBM at every kernel of the step (1.7 GB stream through a 126 MB L2), and the smem ring is only 3-4
-    // k-blocks deep: the weight tiles beyond the ring are pulled into L2 by prefetch boxes, kPrefetch k-blocks ahead of the loads.
-    // CTAs that work on the same n-tile at the same time (different m-tiles) share that duty: k-block k is prefetched by the
-    // CTA with m_tile % pf_share == k % pf_share.
-    // Measured inside the step: 5.126 ms without, 5.203 ms with the prefetch boxes -- every cp.async.bulk.* instruction costs the
-    // issuing producer thread a few hundred cycles, which is what paces the main loop; kept behind kPrefetch for a third thread.
-    constexpr int kPrefetch = 0;
-    auto prefetch_b = [&](int k) {
-        if (k < p.num_k_blocks && k % p.pf_share == pr_me) {
-            if (p.w_kmajor) ptx::tma_prefetch_3d(&p.tmB, 0, pr_n0, k);
-            else ptx::tma_prefetch_2d(&p.tmB, k * BLOCK_K, pr_n0);
-        }
-    };
     // what: bit 0 = issue the A load, bit 1 = issue the B load, 0 = only advance the cursor (the B producer skips the first ring,
     // which thread 0 issued in full before the prologue sync)
     auto produce = [&](int limit, const int what) {
@@ -1017,9 +938,6 @@ __global__ void __launch_bounds__(kPersistThreads, 1) gemm_persist_kernel(const 
                 }
                 pr_tap = pr_kb / p.cblocks;           // 0 unless this is a K slice
                 pr_cb = pr_kb - pr_tap * p.cblocks;
-                pr_me = m_tile % p.pf_share;
-                if (load_b)
-                    for (int k = p.stages; k < kPrefetch; ++k) prefetch_b(k);   // k-blocks [0, stages) are loaded right away, [kPrefetch, ..) follow the loads
             }
             uint64_t* fb = &full_bar[pr_stage];
             if (what) ptx::mbar_wait(&empty_bar[pr_stage], pr_phase ^ 1);
@@ -1038,10 +956,7 @@ __global__ void __launch_bounds__(kPersistThreads, 1) gemm_persist_kernel(const 
             }
             if (load_b) {
                 ptx::mbar_expect_tx(fb, (uint32_t)b_bytes);
-                uint8_t* dst_b = smem_b + (size_t)pr_stage * b_bytes;
-                if (p.w_kmajor) ptx::tma_load_3d(dst_b, &p.tmB, fb, 0, pr_n0, pr_kb);
-                else ptx::tma_load_2d(dst_b, &p.tmB, fb, pr_kb * BLOCK_K, pr_n0);
-                if (kPrefetch > 0) prefetch_b(pr_kb + kPrefetch);
+                ptx::tma_load_2d(smem_b + (size_t)pr_stage * b_bytes, &p.tmB, fb, pr_kb * BLOCK_K, pr_n0);
             }
             if (++pr_stage == p.stages) { pr_stage = 0; pr_phase ^= 1; }
             if (++pr_cb == p.cblocks) { pr_cb = 0; ++pr_tap; }
@@ -1051,8 +966,6 @@ __global__ void __launch_bounds__(kPersistThreads, 1) gemm_persist_kernel(const 
     };
     const bool is_prod_a = threadIdx.x == 0, is_prod_b = threadIdx.x == kPersistThreads - 32;
 
-    ptx::pdl_trigger();
-    if (threadIdx.x == 0) PTRACE(0);
     if (warp == 0 && lane == 0) {
         ptx::prefetch_tmap(&p.tmA0);
         ptx::prefetch_tmap(&p.tmB);
@@ -1069,7 +982,6 @@ __global__ void __launch_bounds__(kPersistThreads, 1) gemm_persist_kernel(const 
         }
         for (int s = 0; s < kEpiWarps * kMaxDepth; ++s) ptx::mbar_init(&rfull[s], 1);
         ptx::fence_barrier_init();
-        ptx::pdl_wait();          // the operands may be the previous kernel's output
         produce(p.stages, 3);     // first ring, both operands; every ring slot is free: none of these waits blocks
     }
     if (warp == 1) {
@@ -1080,8 +992,6 @@ __global__ void __launch_bounds__(kPersistThreads, 1) gemm_persist_kernel(const 
     __syncthreads();
     ptx::tc_fence_after();
     const uint32_t tmem_base = *tmem_slot;
-    ptx::pdl_wait();   // everything above overlapped the previous kernel's tail
-    if (threadIdx.x == 0) PTRACE(1);
 
     if (warp == 0) {
         // ================= TMA producer of the A tiles (its first ring of loads went out before the CTA-wide sync above) =================
@@ -1108,7 +1018,6 @@ __global__ void __launch_bounds__(kPersistThreads, 1) gemm_persist_kernel(const 
                 for (int kb = 0; kb < nkb; ++kb) {
                     ptx::mbar_wait(&full_bar[stage], phase);
                     ptx::tc_fence_after();
-                    if (it == 0 && kb == 0) PTRACE(2);
                     const uint64_t da = ptx::umma_desc_k_sw128(ptx::smem_u32(smem_a + (size_t)stage * kABytes));
                     const uint64_t db = ptx::umma_desc_k_sw128(ptx::smem_u32(smem_b + (size_t)stage * b_bytes));
 #pragma unroll
@@ -1118,13 +1027,10 @@ __global__ void __launch_bounds__(kPersistThreads, 1) gemm_persist_kernel(const 
                     if (++stage == p.stages) { stage = 0; phase ^= 1; }
                 }
                 ptx::umma_commit(&tfull[acc]);
-                if (it == 0) PTRACE(3);
             }
         }
     } else {
         // ================= epilogue warps =================
-        if (warp == 2 && lane == 0 && p.prefetch_bytes)   // idle until the first accumulator: stage the NEXT layer's weights in L2
-            ptx::prefetch_share_l2(p.prefetch, p.prefetch_bytes, blockIdx.x, gridDim.x);
         const int variant = (p.geglu ? 100 : 0) + (p.out_f32 ? 10 : 0) + p.res_kind + (p.gn_part ? 1000 : 0);
         if (splitk) {
             switch (variant) {
@@ -1158,7 +1064,6 @@ __global__ void __launch_bounds__(kPersistThreads, 1) gemm_persist_kernel(const 
         ptx::tc_fence_after();
         ptx::tmem_dealloc(tmem_base, p.tmem_cols);
     }
-    if (threadIdx.x == 0) PTRACE(7);
 }
 
 uint32_t pow2_cols(int n) {
@@ -1228,11 +1133,7 @@ int configure_gemm_kernels() {
 }
 
 // ---- persistent path (gemm_persist_kernel): tile width, eligibility, launch ----
-bool persist_enabled() {
-    static const bool off = getenv("B200SD_PERSIST") && getenv("B200SD_PERSIST")[0] == '0';
-    if (g_dbg[0] >= 0) return g_dbg[0] != 0;
-    return !off;
-}
+bool persist_enabled() { return g_persist != 0; }
 // Tile width for the persistent kernel: a multiple of 32 (its epilogue chunk; 64 for GEGLU: values | gates) dividing N.
 // cost = rounds of tiles per SM x operand bytes a tile pulls per k-block (128 + bn rows): the smallest tile that still
 // fits one round wins on short grids (more CTAs, shorter epilogue), wide tiles win once several rounds are needed anyway.
@@ -1258,7 +1159,7 @@ int launch_persist(const b200sd_gemm_args* a, const KParams& k, int m_tiles, b20
     p.M = k.M; p.N = k.N;
     p.num_k_blocks = k.num_k_blocks; p.block_n = k.block_n;
     p.conv = k.conv; p.cblocks0 = k.cblocks0; p.cblocks = k.cblocks;
-    p.tile_h = k.tile_h; p.tile_n = k.tile_n; p.tiles_y = k.tiles_y; p.w_kmajor = k.w_kmajor;
+    p.tile_h = k.tile_h; p.tile_n = k.tile_n; p.tiles_y = k.tiles_y;
     p.tile_w = k.tile_w; p.tiles_x = k.tiles_x;
     p.n_tiles = k.N / k.block_n;
     p.num_tiles = m_tiles * p.n_tiles;
@@ -1266,19 +1167,10 @@ int launch_persist(const b200sd_gemm_args* a, const KParams& k, int m_tiles, b20
     p.geglu = k.epilogue == B200SD_EPI_GEGLU;
     p.out_f32 = k.out_f32;
     p.res_kind = k.residual ? (k.res_f32 ? 2 : 1) : 0;
-    {
-        const int sms_ = b200sd_num_sms();
-        const int grid_ = p.num_tiles < sms_ ? p.num_tiles : sms_;
-        int share = grid_ / p.n_tiles;
-        if (share > m_tiles) share = m_tiles;
-        p.pf_share = share < 1 ? 1 : share;
-    }
     p.depth = p.res_kind ? kMaxDepth : 2;
-    if (p.res_kind && g_dbg[3] >= 2 && g_dbg[3] <= kMaxDepth) p.depth = g_dbg[3];
     p.split = k.psplit > 1 ? k.psplit : 1;
     p.kb_per_split = ceil_div(k.num_k_blocks, p.split);
     p.residual = k.residual; p.out = k.out; p.ldc = k.ldc; p.ldr = k.ldr;
-    p.prefetch = k.prefetch; p.prefetch_bytes = k.prefetch_bytes;
     const int units = p.num_tiles * p.split;
     if (p.split > 1) {
         B200SD_REQUIRE(k.num_k_blocks >= p.split, "gemm(split-K): fewer K blocks (%d) than slices (%d)", k.num_k_blocks, p.split);
@@ -1325,7 +1217,6 @@ int launch_persist(const b200sd_gemm_args* a, const KParams& k, int m_tiles, b20
     const int budget = 227 * 1024 - 1024;
     int stages = (budget - epi_bytes - bias_bytes - stat_bytes - bars_bytes) / stage_bytes;
     if (stages > kMaxStages) stages = kMaxStages;
-    if (g_dbg[1] > 0 && g_dbg[1] < stages) stages = g_dbg[1];
     B200SD_REQUIRE(stages >= 2, "gemm(persistent): smem budget leaves %d stages for block_n %d", stages, bn);
     p.stages = stages;
     p.off_b = (uint32_t)stages * kABytes;
@@ -1334,34 +1225,23 @@ int launch_persist(const b200sd_gemm_args* a, const KParams& k, int m_tiles, b20
     p.off_stat = p.off_bias + bias_bytes;
     p.off_bars = p.off_stat + stat_bytes;
     const size_t smem_bytes = (size_t)p.off_bars + bars_bytes + 1024;
-    p.trace = g_gemm_trace;
     {
         const int rc = configure_gemm_kernels();
         if (rc) return rc;
     }
     const int sms = b200sd_num_sms();
     cudaLaunchConfig_t cfg = {};
-    int grid = p.num_tiles < sms ? p.num_tiles : sms;
-    if (g_dbg[2] > 0 && g_dbg[2] < grid) grid = g_dbg[2];
-    if (p.split > 1) grid = units;
-    cfg.gridDim = dim3(grid);
+    cfg.gridDim = dim3(p.split > 1 ? units : (p.num_tiles < sms ? p.num_tiles : sms));
     cfg.blockDim = dim3(kPersistThreads);
     cfg.dynamicSmemBytes = smem_bytes;
     cfg.stream = static_cast<cudaStream_t>(stream);
-    cudaLaunchAttribute attr[2];
-    int na = 0;
+    cudaLaunchAttribute attr[1];
     if (p.split > 1) {   // the K slices of a tile wait for one another: every CTA of the grid must be resident
-        attr[na].id = cudaLaunchAttributeCooperative;
-        attr[na].val.cooperative = 1;
-        ++na;
+        attr[0].id = cudaLaunchAttributeCooperative;
+        attr[0].val.cooperative = 1;
+        cfg.attrs = attr;
+        cfg.numAttrs = 1;
     }
-    if (b200sd_pdl_enabled()) {
-        attr[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        attr[na].val.programmaticStreamSerializationAllowed = 1;
-        ++na;
-    }
-    cfg.attrs = attr;
-    cfg.numAttrs = na;
     B200SD_CUDA(cudaLaunchKernelEx(&cfg, gemm_persist_kernel, p));
     g_b200sd_launches.fetch_add(1, std::memory_order_relaxed);
     B200SD_LAUNCH_CHECK();
@@ -1380,7 +1260,6 @@ int launch_gemm(KParams& p, int m_tiles, int n_tiles, int grid_z, bool cluster, 
     if (stages > kMaxStages) stages = kMaxStages;
     if (stages > p.kb_per_split && total_ctas <= sms) stages = p.kb_per_split;
     const int min_stages = ceil_div(BLOCK_M * (bn + 4) * (int)sizeof(float), stage_bytes);  // epilogue staging tile
-    if (g_dbg[1] > 0 && g_dbg[1] < stages) stages = g_dbg[1];
     if (stages < min_stages) stages = min_stages;
     if (stages < 2) stages = 2;
     p.stages = stages;
@@ -1392,42 +1271,33 @@ int launch_gemm(KParams& p, int m_tiles, int n_tiles, int grid_z, bool cluster, 
         const int rc = configure_gemm_kernels();
         if (rc) return rc;
     }
-    p.trace = g_gemm_trace;
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(m_tiles, n_tiles, grid_z);
     cfg.blockDim = dim3(kNumThreads);
     cfg.dynamicSmemBytes = smem_bytes;
     cfg.stream = static_cast<cudaStream_t>(stream);
-    cudaLaunchAttribute attr[2];
-    int na = 0;
+    cudaLaunchAttribute attr[1];
     if ((cluster && grid_z > 1) || p.pair) {
-        attr[na].id = cudaLaunchAttributeClusterDimension;
-        attr[na].val.clusterDim.x = p.pair ? 2 : 1;
-        attr[na].val.clusterDim.y = 1;
-        attr[na].val.clusterDim.z = p.pair ? 1 : grid_z;
-        ++na;
+        attr[0].id = cudaLaunchAttributeClusterDimension;
+        attr[0].val.clusterDim.x = p.pair ? 2 : 1;
+        attr[0].val.clusterDim.y = 1;
+        attr[0].val.clusterDim.z = p.pair ? 1 : grid_z;
+        cfg.attrs = attr;
+        cfg.numAttrs = 1;
     }
-    if (b200sd_pdl_enabled()) {
-        attr[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        attr[na].val.programmaticStreamSerializationAllowed = 1;
-        ++na;
-    }
-    cfg.attrs = attr;
-    cfg.numAttrs = na;
     B200SD_CUDA(cudaLaunchKernelEx(&cfg, gemm_entry(p.pair, p.b_mode), p));
     g_b200sd_launches.fetch_add(1, std::memory_order_relaxed);
     B200SD_LAUNCH_CHECK();
     return B200SD_OK;
 }
 
-// CTA pairs (cta_group::2): 0 = auto, 1 = force, -1 = off; env B200SD_PAIR=0 disables the auto choice
+// CTA pairs (cta_group::2): 0 = auto, 1 = force, -1 = off
 // Measured on B200 (tools/pair_check.py): pairs win 5-13 % on long-K tiles of grids that fill the machine
 // (conv3x3 at batch 8: 1171 -> 1325 TFLOP/s) and lose ~5 % on short-K GEMMs (one more cluster barrier per tile).
 bool want_pair(int request, int split, int m_tiles, int n_tiles, int k_blocks) {
-    static const bool env_off = getenv("B200SD_PAIR") && getenv("B200SD_PAIR")[0] == '0';
     if (request < 0 || split != 1) return false;
     if (request > 0) return true;
-    return !env_off && m_tiles >= 2 && k_blocks >= 32 && (long)m_tiles * n_tiles >= b200sd_num_sms();
+    return m_tiles >= 2 && k_blocks >= 32 && (long)m_tiles * n_tiles >= b200sd_num_sms();
 }
 
 // Tile width for MN-major B operands (64-column TMA boxes), from the sweep in tools/bwd_gemm_bench.py (B200, batch 8):
@@ -1522,8 +1392,7 @@ static int gemm_tiling(const b200sd_gemm_args* a, KParams& p, int* m_tiles_out, 
     const int m_tiles = *m_tiles_out;
 
     // ---- N tiling ----
-    static const bool no_split = getenv("B200SD_SPLITK") && getenv("B200SD_SPLITK")[0] == '0';
-    const bool can_split = !no_split && a->split_k <= 0 && a->epilogue == B200SD_EPI_LINEAR && p.num_k_blocks >= 16;
+    const bool can_split = a->split_k <= 0 && a->epilogue == B200SD_EPI_LINEAR && p.num_k_blocks >= 16;
     int bn = a->block_n > 0 ? a->block_n : pick_block_n(a->N, m_tiles, a->epilogue, can_split);
     B200SD_REQUIRE(bn >= 16 && bn <= 256 && bn % 16 == 0 && a->N % bn == 0, "gemm: bad block_n %d for N=%d", bn, a->N);
     B200SD_REQUIRE(a->epilogue != B200SD_EPI_GEGLU || bn % 32 == 0, "gemm: GEGLU needs block_n %% 32 == 0");
@@ -1537,7 +1406,7 @@ static int gemm_tiling(const b200sd_gemm_args* a, KParams& p, int* m_tiles_out, 
     if (split <= 0) {
         split = 1;
         const int tiles = m_tiles * n_tiles;
-        if (!no_split && a->epilogue == B200SD_EPI_LINEAR && tiles * 2 <= sms && p.num_k_blocks >= 16) {
+        if (a->epilogue == B200SD_EPI_LINEAR && tiles * 2 <= sms && p.num_k_blocks >= 16) {
             while (split < 8 && tiles * split * 2 <= sms && p.num_k_blocks / (split * 2) >= 8) split *= 2;
         }
     }
@@ -1567,8 +1436,7 @@ static int gemm_tiling(const b200sd_gemm_args* a, KParams& p, int* m_tiles_out, 
     const bool geglu = a->epilogue == B200SD_EPI_GEGLU;
     // ---- ... and its split-K mode for the few-tile / deep-K layers the policy above would hand to a split cluster: up to 16
     // K slices per tile, one CTA per slice, partials through an L2-resident workspace (persist_epilogue_split) ----
-    static const bool no_psplit = getenv("B200SD_PSPLIT") && getenv("B200SD_PSPLIT")[0] == '0';
-    if (persist_enabled() && !no_psplit && a->split_k <= 0 && a->block_n <= 0 && split > 1 && !geglu && p.rows_valid == BLOCK_M &&
+    if (persist_enabled() && a->split_k <= 0 && a->block_n <= 0 && split > 1 && !geglu && p.rows_valid == BLOCK_M &&
         a->N % 32 == 0 && a->workspace != nullptr && a->workspace_bytes >= kWsPartialBytes + kWsCounterBytes &&
         (reinterpret_cast<uintptr_t>(a->workspace) & 127) == 0 && a->ldc % 4 == 0 && (!a->residual || a->ldr % 4 == 0)) {
         int bnp = 0;
@@ -1603,14 +1471,11 @@ static int gemm_tiling(const b200sd_gemm_args* a, KParams& p, int* m_tiles_out, 
         // overlaps the main loop of tile i+1 and no CTA is launched / set up per tile.  On one-tile-per-CTA grids (<= 148
         // tiles) the critical path is load latency -> MMAs -> epilogue either way, the deeper ring of gemm_tcgen05_kernel
         // (5-6 stages: nothing of its smem is set aside for epilogue chunks) hides the HBM latency of the cold weights better,
-        // and the persistent kernel measured level or slower (M8192 N320 K1280 12.4 -> 14.1 us): those grids stay there.
-        // B200SD_PERSIST_MASK (A/B switch): 1 = GEGLU, 2 = multi-round plain GEMMs / convs, 4 = one-round grids
+        // and the persistent kernel measured level or slower (M8192 N320 K1280 12.4 -> 14.1 us): those grids stay there
+        // unless debug key 0 forces the persistent kernel.
         const long ptiles = bnp > 0 ? (long)m_tiles * (a->N / bnp) : 0;
-        const int sms_p = b200sd_num_sms();
-        static const int mask = [] { const char* e = getenv("B200SD_PERSIST_MASK"); return e ? atoi(e) : 3; }();
-        const bool multi = ptiles >= 2L * sms_p;
-        const int cls = !multi ? 4 : (geglu ? 1 : 2);
-        if (bnp > 0 && bnp <= 256 && bnp % (geglu ? 64 : 32) == 0 && a->N % bnp == 0 && ((mask & cls) || g_dbg[0] > 0)) {
+        const bool multi = ptiles >= 2L * b200sd_num_sms();
+        if (bnp > 0 && bnp <= 256 && bnp % (geglu ? 64 : 32) == 0 && a->N % bnp == 0 && (multi || g_persist > 0)) {
             p.persist = 1;
             p.block_n = bnp;
             *n_tiles_out = a->N / bnp;
@@ -1671,9 +1536,6 @@ extern "C" int b200sd_gemm(const b200sd_gemm_args* a, b200sd_stream_t stream) {
     }
     const int bn = p.block_n, split = p.split_k;
     p.gn_part = a->gn_part;
-    p.prefetch = a->prefetch;
-    p.prefetch_bytes = a->prefetch ? a->prefetch_bytes : 0;
-    B200SD_REQUIRE(!a->prefetch || (reinterpret_cast<uintptr_t>(a->prefetch) & 15) == 0, "gemm: prefetch pointer must be 16-byte aligned");
     B200SD_REQUIRE(!a->gn_part || (a->out_dtype == B200SD_F32 && a->epilogue == B200SD_EPI_LINEAR &&
                                    (!a->residual || a->residual_dtype == B200SD_F32)),
                    "gemm: gn_part needs fp32 output, the linear epilogue and no bf16 residual");
@@ -1704,15 +1566,7 @@ extern "C" int b200sd_gemm(const b200sd_gemm_args* a, b200sd_stream_t stream) {
             if (rc) return rc;
         }
     }
-    p.w_kmajor = a->w_layout == B200SD_W_KBLOCK_MAJOR;
-    B200SD_REQUIRE(a->w_layout == B200SD_W_ROW_MAJOR || a->w_layout == B200SD_W_KBLOCK_MAJOR, "gemm: bad w_layout %d", a->w_layout);
-    if (p.w_kmajor) {
-        const uint64_t dimsB[3] = {(uint64_t)BLOCK_K, (uint64_t)a->N, (uint64_t)(a->K / BLOCK_K)};
-        const uint64_t strB[3] = {0, (uint64_t)BLOCK_K * 2, (uint64_t)a->N * BLOCK_K * 2};
-        const uint32_t boxB[3] = {BLOCK_K, (uint32_t)(p.pair ? bn / 2 : bn), 1};
-        int rc = b200sd_make_tmap(&p.tmB, a->w, 3, dimsB, strB, boxB, CU_TENSOR_MAP_SWIZZLE_128B);
-        if (rc) return rc;
-    } else {
+    {
         const uint64_t dimsB[2] = {(uint64_t)a->K, (uint64_t)a->N};
         const uint64_t strB[2] = {0, (uint64_t)a->K * 2};
         const uint32_t boxB[2] = {BLOCK_K, (uint32_t)(p.pair ? bn / 2 : bn)};
@@ -1837,10 +1691,9 @@ extern "C" int b200sd_gemm_dgrad(const b200sd_dgrad_args* a, b200sd_stream_t str
     // split-K clusters for the few-tile / deep-K layers (the 8x8 and 16x16 levels), same policy as the forward GEMM
     int split = 1;
     {
-        static const bool no_split = getenv("B200SD_SPLITK") && getenv("B200SD_SPLITK")[0] == '0';
         const int sms = b200sd_num_sms();
         const int tiles = m_tiles * n_tiles;
-        if (!no_split && !p.pair && tiles * 2 <= sms && p.num_k_blocks >= 16) {
+        if (!p.pair && tiles * 2 <= sms && p.num_k_blocks >= 16) {
             while (split < 8 && tiles * split * 2 <= sms && p.num_k_blocks / (split * 2) >= 8) split *= 2;
             if (split == 8 && tiles > 8) split = 4;
         }

@@ -12,8 +12,6 @@ namespace {
 
 // ---- sinusoidal timestep embedding (fp32, accurate sin/cos: arguments reach ~1000 rad) -----------
 __global__ void temb_kernel(const float* __restrict__ t, float* __restrict__ out, int batch, int dim) {
-    ptx::pdl_trigger();
-    ptx::pdl_wait();
     const int half = dim / 2;
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= batch * half) return;
@@ -31,8 +29,6 @@ __global__ void __launch_bounds__(256) small_linear_kernel(const float* __restri
                                                            const float* __restrict__ bias, float* __restrict__ out,
                                                            int batch, int N, int K, int silu_in, int silu_out) {
     extern __shared__ float s_in[];  // [kSlRows][K]
-    ptx::pdl_trigger();
-    ptx::pdl_wait();
     const int b0 = blockIdx.y * kSlRows;
     const int nb = min(kSlRows, batch - b0);
     for (int i = threadIdx.x; i < kSlRows * K; i += blockDim.x) {
@@ -108,8 +104,6 @@ __global__ void conv_in_kernel(const float* __restrict__ x, const float* __restr
                                void* __restrict__ out, int batch, int Cout, int H, int W) {
     constexpr int Cin = 4;
     __shared__ float patch[kCinPix][9 * Cin];
-    ptx::pdl_trigger();
-    ptx::pdl_wait();
     const int hw = H * W;
     const int pix0 = blockIdx.x * kCinPix;
     const int total = batch * hw;
@@ -160,11 +154,9 @@ __global__ void __launch_bounds__(256) conv_out_kernel(const bf16* __restrict__ 
                                                        const float* __restrict__ bias, float* __restrict__ out,
                                                        int batch, int Cin, int Cout, int H, int W, int pix_per_warp) {
     extern __shared__ float s_w[];  // packed [Cout][tap][Cin]
-    ptx::pdl_trigger();
     for (int i = threadIdx.x; i < Cout * 9 * Cin / 4; i += blockDim.x)   // static weights: before the wait (Cin % 4 == 0)
         reinterpret_cast<float4*>(s_w)[i] = __ldg(reinterpret_cast<const float4*>(w) + i);
     __syncthreads();
-    ptx::pdl_wait();
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int hw = H * W, total = batch * hw;
     const int first = (blockIdx.x * 8 + warp) * pix_per_warp;
@@ -224,8 +216,6 @@ __global__ void __launch_bounds__(256) conv_out_kernel(const bf16* __restrict__ 
 // ---- nearest x2 upsample, NHWC, 8-channel vectors (fp32 or bf16 in, bf16 out) -----------------------
 template <int DT>
 __global__ void upsample2x_kernel(const void* __restrict__ x, bf16* __restrict__ out, int batch, int H, int W, int C8) {
-    ptx::pdl_trigger();
-    ptx::pdl_wait();
     const int64_t total = (int64_t)batch * 4 * H * W * C8;
     const int64_t stride = (int64_t)gridDim.x * blockDim.x;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += stride) {
@@ -244,8 +234,6 @@ __global__ void upsample2x_kernel(const void* __restrict__ x, bf16* __restrict__
 // ---- im2col for the stride-2 pad-1 3x3 Downsample2D conv --------------------------------------------
 template <int DT>
 __global__ void im2col_s2_kernel(const void* __restrict__ x, bf16* __restrict__ out, int batch, int H, int W, int C8, int pad) {
-    ptx::pdl_trigger();
-    ptx::pdl_wait();
     const int OH = H / 2, OW = W / 2;
     const int64_t total = (int64_t)batch * OH * OW * 9 * C8;
     const int64_t stride = (int64_t)gridDim.x * blockDim.x;
@@ -279,7 +267,7 @@ extern "C" int b200sd_timestep_embedding(const float* timesteps, float* out, int
     B200SD_REQUIRE(timesteps && out, "timestep_embedding: null pointer");
     B200SD_REQUIRE(batch > 0 && dim > 0 && dim % 2 == 0, "timestep_embedding: bad sizes");
     const int total = batch * dim / 2;
-    B200SD_CUDA(b200sd_launch(temb_kernel, dim3(ceil_div(total, 128)), dim3(128), 0, static_cast<cudaStream_t>(stream), timesteps, out, batch, dim));
+    temb_kernel<<<dim3(ceil_div(total, 128)), dim3(128), 0, static_cast<cudaStream_t>(stream)>>>(timesteps, out, batch, dim);
     COUNT_LAUNCH();
     B200SD_LAUNCH_CHECK();
     return B200SD_OK;
@@ -300,8 +288,8 @@ extern "C" int b200sd_small_linear(const float* in, const void* w_bf16, const fl
     if (gx > cap) gx = cap;
     dim3 grid(gx, ceil_div(batch, rows));
     auto kern = rows == 2 ? small_linear_kernel<2> : (rows == 4 ? small_linear_kernel<4> : small_linear_kernel<8>);
-    B200SD_CUDA(b200sd_launch(kern, dim3(grid), dim3(256), smem, static_cast<cudaStream_t>(stream), in, static_cast<const bf16*>(w_bf16), bias,
-                              out, batch, N, K, silu_in, silu_out));
+    kern<<<dim3(grid), dim3(256), smem, static_cast<cudaStream_t>(stream)>>>(in, static_cast<const bf16*>(w_bf16), bias,
+                              out, batch, N, K, silu_in, silu_out);
     COUNT_LAUNCH();
     B200SD_LAUNCH_CHECK();
     return B200SD_OK;
@@ -317,11 +305,9 @@ extern "C" int b200sd_conv_in(const float* x_nchw, const float* w, const float* 
     if (threads > 256) threads = 256;
     threads = ceil_div(threads, 32) * 32;
     if (out_dtype == B200SD_F32)
-        B200SD_CUDA(b200sd_launch(conv_in_kernel<B200SD_F32>, dim3(ceil_div(total, kCinPix)), dim3(threads), 0,
-                                  static_cast<cudaStream_t>(stream), x_nchw, w, bias, out_nhwc, batch, Cout, H, W));
+        conv_in_kernel<B200SD_F32><<<dim3(ceil_div(total, kCinPix)), dim3(threads), 0, static_cast<cudaStream_t>(stream)>>>(x_nchw, w, bias, out_nhwc, batch, Cout, H, W);
     else
-        B200SD_CUDA(b200sd_launch(conv_in_kernel<B200SD_BF16>, dim3(ceil_div(total, kCinPix)), dim3(threads), 0,
-                                  static_cast<cudaStream_t>(stream), x_nchw, w, bias, out_nhwc, batch, Cout, H, W));
+        conv_in_kernel<B200SD_BF16><<<dim3(ceil_div(total, kCinPix)), dim3(threads), 0, static_cast<cudaStream_t>(stream)>>>(x_nchw, w, bias, out_nhwc, batch, Cout, H, W);
     COUNT_LAUNCH();
     B200SD_LAUNCH_CHECK();
     return B200SD_OK;
@@ -338,8 +324,8 @@ extern "C" int b200sd_conv_out(const void* x_nhwc, const float* w, const float* 
     int ppw = ceil_div(total, b200sd_num_sms() * 2 * 8);
     if (ppw < 4) ppw = 4;
     const int blocks = ceil_div(total, ppw * 8);
-    B200SD_CUDA(b200sd_launch(conv_out_kernel, dim3(blocks), dim3(256), smem, static_cast<cudaStream_t>(stream), static_cast<const bf16*>(x_nhwc), w, bias,
-                                                                             out_nchw, batch, Cin, Cout, H, W, ppw));
+    conv_out_kernel<<<dim3(blocks), dim3(256), smem, static_cast<cudaStream_t>(stream)>>>(static_cast<const bf16*>(x_nhwc), w, bias,
+                                                                             out_nchw, batch, Cin, Cout, H, W, ppw);
     COUNT_LAUNCH();
     B200SD_LAUNCH_CHECK();
     return B200SD_OK;
@@ -348,8 +334,6 @@ extern "C" int b200sd_conv_out(const void* x_nhwc, const float* w, const float* 
 // [M][ld] fp32 (NHWC, the first C of ld columns) + bias -> NCHW fp32: the tail of the tensor-core conv_out
 __global__ void __launch_bounds__(256) nhwc_bias_to_nchw_kernel(const float* __restrict__ x, const float* __restrict__ bias,
                                                                 float* __restrict__ out, int total, int hw, int C, int ld) {
-    ptx::pdl_trigger();
-    ptx::pdl_wait();
     const int m = blockIdx.x * blockDim.x + threadIdx.x;
     if (m >= total) return;
     const int b = m / hw, pix = m - b * hw;
@@ -364,8 +348,8 @@ extern "C" int b200sd_nhwc_bias_to_nchw(const float* x, const float* bias, float
     B200SD_REQUIRE(x && bias && out_nchw, "nhwc_bias_to_nchw: null pointer");
     B200SD_REQUIRE(C >= 1 && C <= 8 && ld % 4 == 0 && ld >= (C > 4 ? 8 : 4) && batch > 0 && hw > 0, "nhwc_bias_to_nchw: C in 1..8, ld %% 4 == 0");
     const int total = batch * hw;
-    B200SD_CUDA(b200sd_launch(nhwc_bias_to_nchw_kernel, dim3(ceil_div(total, 256)), dim3(256), 0, static_cast<cudaStream_t>(stream), x, bias,
-                              out_nchw, total, hw, C, ld));
+    nhwc_bias_to_nchw_kernel<<<dim3(ceil_div(total, 256)), dim3(256), 0, static_cast<cudaStream_t>(stream)>>>(x, bias,
+                              out_nchw, total, hw, C, ld);
     COUNT_LAUNCH();
     B200SD_LAUNCH_CHECK();
     return B200SD_OK;
@@ -377,11 +361,9 @@ extern "C" int b200sd_upsample2x(const void* x, void* out, int batch, int H, int
     B200SD_REQUIRE(C % 8 == 0 && batch > 0 && H > 0 && W > 0, "upsample2x: bad sizes");
     const int64_t total = (int64_t)batch * 4 * H * W * (C / 8);
     if (in_dtype == B200SD_F32)
-        B200SD_CUDA(b200sd_launch(upsample2x_kernel<B200SD_F32>, dim3(ew_grid(total, 256)), dim3(256), 0,
-                                  static_cast<cudaStream_t>(stream), x, static_cast<bf16*>(out), batch, H, W, C / 8));
+        upsample2x_kernel<B200SD_F32><<<dim3(ew_grid(total, 256)), dim3(256), 0, static_cast<cudaStream_t>(stream)>>>(x, static_cast<bf16*>(out), batch, H, W, C / 8);
     else
-        B200SD_CUDA(b200sd_launch(upsample2x_kernel<B200SD_BF16>, dim3(ew_grid(total, 256)), dim3(256), 0,
-                                  static_cast<cudaStream_t>(stream), x, static_cast<bf16*>(out), batch, H, W, C / 8));
+        upsample2x_kernel<B200SD_BF16><<<dim3(ew_grid(total, 256)), dim3(256), 0, static_cast<cudaStream_t>(stream)>>>(x, static_cast<bf16*>(out), batch, H, W, C / 8);
     COUNT_LAUNCH();
     B200SD_LAUNCH_CHECK();
     return B200SD_OK;
@@ -399,11 +381,9 @@ extern "C" int b200sd_im2col_s2_pad(const void* x, void* out, int batch, int H, 
     B200SD_REQUIRE(C % 8 == 0 && batch > 0 && H % 2 == 0 && W % 2 == 0, "im2col_s2: bad sizes");
     const int64_t total = (int64_t)batch * (H / 2) * (W / 2) * 9 * (C / 8);
     if (in_dtype == B200SD_F32)
-        B200SD_CUDA(b200sd_launch(im2col_s2_kernel<B200SD_F32>, dim3(ew_grid(total, 256)), dim3(256), 0,
-                                  static_cast<cudaStream_t>(stream), x, static_cast<bf16*>(out), batch, H, W, C / 8, pad));
+        im2col_s2_kernel<B200SD_F32><<<dim3(ew_grid(total, 256)), dim3(256), 0, static_cast<cudaStream_t>(stream)>>>(x, static_cast<bf16*>(out), batch, H, W, C / 8, pad);
     else
-        B200SD_CUDA(b200sd_launch(im2col_s2_kernel<B200SD_BF16>, dim3(ew_grid(total, 256)), dim3(256), 0,
-                                  static_cast<cudaStream_t>(stream), x, static_cast<bf16*>(out), batch, H, W, C / 8, pad));
+        im2col_s2_kernel<B200SD_BF16><<<dim3(ew_grid(total, 256)), dim3(256), 0, static_cast<cudaStream_t>(stream)>>>(x, static_cast<bf16*>(out), batch, H, W, C / 8, pad);
     COUNT_LAUNCH();
     B200SD_LAUNCH_CHECK();
     return B200SD_OK;

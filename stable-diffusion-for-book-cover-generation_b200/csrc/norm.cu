@@ -4,7 +4,6 @@
 
 #include <algorithm>
 
-#include <cstdlib>
 
 #include "common.cuh"
 
@@ -45,8 +44,6 @@ __global__ void __launch_bounds__(1024) gn_stats_kernel(const void* __restrict__
     const int C8 = C / 8;
     const int cpg = C / groups;
     const int b = blockIdx.y, slab = blockIdx.x, slabs = gridDim.x;
-    ptx::pdl_trigger();
-    ptx::pdl_wait();
     const int vec = threadIdx.x % C8;
     const int prow = threadIdx.x / C8;
     const int c = vec * 8;
@@ -137,8 +134,6 @@ __global__ void __launch_bounds__(kGnThreads) gn_apply_kernel(const void* __rest
                                                               const float* __restrict__ mean_rstd, int hw,
                                                               int groups, int silu, int pix_per_block) {
     extern __shared__ float2 s_ab[];  // per-channel (scale, shift)
-    ptx::pdl_trigger();
-    ptx::pdl_wait();
     const int C = C0 + C1;
     const int cpg = C / groups;
     const int b = blockIdx.y;
@@ -211,8 +206,6 @@ __global__ void __launch_bounds__(512) gn_fused_kernel(const void* __restrict__ 
     const int c_base = set * Cg;
     float* s_part = gsm;
     float2* s_ab = reinterpret_cast<float2*>(gsm + 2 * R * Cg);
-    ptx::pdl_trigger();
-    ptx::pdl_wait();
     const int vec = threadIdx.x % VC, prow = threadIdx.x / VC;
     const bool active = prow < R;
     const int c = c_base + vec * 8;  // global channel of this thread's vector
@@ -342,8 +335,6 @@ __global__ void __launch_bounds__(512) gn_parts_kernel(const void* __restrict__ 
     const int c_base = set * Cg;
     float* s_tot = gsm;
     float2* s_ab = reinterpret_cast<float2*>(gsm + 2 * Cg);
-    ptx::pdl_trigger();
-    ptx::pdl_wait();
     // fold the partial rows: nq thread groups take every nq-th row (8 loads in flight each), then a fixed-order fold
     float* s_red = gsm + 4 * Cg;    // [nq][2 * Cg]
     const int nq = max(1, (int)blockDim.x / (2 * Cg));
@@ -425,8 +416,6 @@ template <int PAIRS_PER_LANE, int DT>
 __global__ void __launch_bounds__(256) layernorm_kernel(const void* __restrict__ x, const float* __restrict__ gamma,
                                                         const float* __restrict__ beta, bf16* __restrict__ out,
                                                         bf16* __restrict__ out_lo, int rows, int C, float eps) {
-    ptx::pdl_trigger();
-    ptx::pdl_wait();
     const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int lane = threadIdx.x & 31;
     if (warp >= rows) return;
@@ -489,8 +478,7 @@ extern "C" int b200sd_groupnorm_silu_split(const void* x0, const void* x1, int C
         // The single-kernel path keeps an image's pixels on at most 8 CTAs per channel set: right for the UNet (<= 2.6 M elements
         // per image, launch latency dominates), hopeless for the VAE's 256^2 / 512^2 levels (33 M elements on 32 CTAs measured
         // 832 us = 0.4 TB/s).  Large images take the two-kernel path below: 128 statistics slabs + 4 apply CTAs per SM.
-        static const long fused_max = [] { const char* e = getenv("B200SD_GN_FUSED_MAX"); return e ? atol(e) : 3000000L; }();
-        if ((Cg % 8) == 0 && groups % G == 0 && Cg / 8 <= 512 && (long)hw * C <= fused_max) {
+        if ((Cg % 8) == 0 && groups % G == 0 && Cg / 8 <= 512 && (long)hw * C <= 3000000L) {
             const int VC = Cg / 8;
             const int sets = groups / G;
             int CL = 1;
@@ -507,22 +495,15 @@ extern "C" int b200sd_groupnorm_silu_split(const void* x0, const void* x1, int C
             cfg.blockDim = dim3(threads);
             cfg.dynamicSmemBytes = smem;
             cfg.stream = s;
-            cudaLaunchAttribute attr[2];
-            int na = 0;
+            cudaLaunchAttribute attr[1];
             if (CL > 1) {
-                attr[na].id = cudaLaunchAttributeClusterDimension;
-                attr[na].val.clusterDim.x = CL;
-                attr[na].val.clusterDim.y = 1;
-                attr[na].val.clusterDim.z = 1;
-                ++na;
+                attr[0].id = cudaLaunchAttributeClusterDimension;
+                attr[0].val.clusterDim.x = CL;
+                attr[0].val.clusterDim.y = 1;
+                attr[0].val.clusterDim.z = 1;
+                cfg.attrs = attr;
+                cfg.numAttrs = 1;
             }
-            if (b200sd_pdl_enabled()) {
-                attr[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-                attr[na].val.programmaticStreamSerializationAllowed = 1;
-                ++na;
-            }
-            cfg.attrs = attr;
-            cfg.numAttrs = na;
             if (in_dtype == B200SD_F32)
                 B200SD_CUDA(cudaLaunchKernelEx(&cfg, gn_fused_kernel<B200SD_F32>, x0, x1, C0, C1, gamma, beta, static_cast<bf16*>(out),
                                                static_cast<bf16*>(raw_out), static_cast<bf16*>(out_lo), static_cast<bf16*>(raw_lo), hw, groups, G, CL, ppc, R, eps,
@@ -553,11 +534,11 @@ extern "C" int b200sd_groupnorm_silu_split(const void* x0, const void* x1, int C
     slabs = ceil_div(hw, pps);
     const size_t st_smem = (size_t)2 * rows_per_pass * C * sizeof(float);
     if (in_dtype == B200SD_F32)
-        B200SD_CUDA(b200sd_launch(gn_stats_kernel<B200SD_F32>, dim3(slabs, batch), dim3(threads), st_smem, s, x0, x1, C0, C1, partial,
-                                  mean_rstd, counters, hw, groups, pps, rows_per_pass, eps));
+        gn_stats_kernel<B200SD_F32><<<dim3(slabs, batch), dim3(threads), st_smem, s>>>(x0, x1, C0, C1, partial,
+                                  mean_rstd, counters, hw, groups, pps, rows_per_pass, eps);
     else
-        B200SD_CUDA(b200sd_launch(gn_stats_kernel<B200SD_BF16>, dim3(slabs, batch), dim3(threads), st_smem, s, x0, x1, C0, C1, partial,
-                                  mean_rstd, counters, hw, groups, pps, rows_per_pass, eps));
+        gn_stats_kernel<B200SD_BF16><<<dim3(slabs, batch), dim3(threads), st_smem, s>>>(x0, x1, C0, C1, partial,
+                                  mean_rstd, counters, hw, groups, pps, rows_per_pass, eps);
     COUNT_LAUNCH();
     B200SD_LAUNCH_CHECK();
     if (stats_out != nullptr)
@@ -568,13 +549,13 @@ extern "C" int b200sd_groupnorm_silu_split(const void* x0, const void* x1, int C
     if (ppb < min_ppb) ppb = min_ppb;
     blocks = ceil_div(hw, ppb);
     if (in_dtype == B200SD_F32)
-        B200SD_CUDA(b200sd_launch(gn_apply_kernel<B200SD_F32>, dim3(blocks, batch), dim3(kGnThreads), C * sizeof(float2), s, x0, x1, C0, C1,
+        gn_apply_kernel<B200SD_F32><<<dim3(blocks, batch), dim3(kGnThreads), C * sizeof(float2), s>>>(x0, x1, C0, C1,
                                   gamma, beta, static_cast<bf16*>(out), static_cast<bf16*>(raw_out), static_cast<bf16*>(out_lo), static_cast<bf16*>(raw_lo),
-                                  mean_rstd, hw, groups, silu, ppb));
+                                  mean_rstd, hw, groups, silu, ppb);
     else
-        B200SD_CUDA(b200sd_launch(gn_apply_kernel<B200SD_BF16>, dim3(blocks, batch), dim3(kGnThreads), C * sizeof(float2), s, x0, x1, C0, C1,
+        gn_apply_kernel<B200SD_BF16><<<dim3(blocks, batch), dim3(kGnThreads), C * sizeof(float2), s>>>(x0, x1, C0, C1,
                                   gamma, beta, static_cast<bf16*>(out), static_cast<bf16*>(raw_out), static_cast<bf16*>(out_lo), static_cast<bf16*>(raw_lo),
-                                  mean_rstd, hw, groups, silu, ppb));
+                                  mean_rstd, hw, groups, silu, ppb);
     COUNT_LAUNCH();
     B200SD_LAUNCH_CHECK();
     return B200SD_OK;
@@ -614,9 +595,9 @@ extern "C" int b200sd_layernorm_split(const void* x, const float* gamma, const f
 #define LN_CASE(P)                                                                                     \
     case P:                                                                                            \
         if (in_dtype == B200SD_F32)                                                                         \
-            B200SD_CUDA(b200sd_launch(layernorm_kernel<P, B200SD_F32>, dim3(blocks), dim3(256), 0, s, xi, gamma, beta, xo, xl, rows, C, eps)); \
+            layernorm_kernel<P, B200SD_F32><<<dim3(blocks), dim3(256), 0, s>>>(xi, gamma, beta, xo, xl, rows, C, eps); \
         else                                                                                                \
-            B200SD_CUDA(b200sd_launch(layernorm_kernel<P, B200SD_BF16>, dim3(blocks), dim3(256), 0, s, xi, gamma, beta, xo, xl, rows, C, eps)); \
+            layernorm_kernel<P, B200SD_BF16><<<dim3(blocks), dim3(256), 0, s>>>(xi, gamma, beta, xo, xl, rows, C, eps); \
         break;
     switch (C / 64) {
         LN_CASE(1) LN_CASE(2) LN_CASE(3) LN_CASE(4) LN_CASE(5) LN_CASE(6) LN_CASE(7) LN_CASE(8) LN_CASE(9) LN_CASE(10)
@@ -656,8 +637,7 @@ extern "C" int b200sd_groupnorm_silu_parts(const void* x0, const void* x1, int C
     const int Cg = G * cpg;
     if ((Cg % 8) != 0 || groups % G != 0 || Cg / 8 > 512) return B200SD_ERR_UNSUPPORTED;
     const int VC = Cg / 8, sets = groups / G;
-    static const int ctas_per_sm = [] { const char* e = getenv("B200SD_GN_CTAS_PER_SM"); return e ? atoi(e) : 2; }();
-    int slabs = ceil_div(b200sd_num_sms() * ctas_per_sm, batch * sets);
+    int slabs = ceil_div(b200sd_num_sms() * 2, batch * sets);   // two CTAs per SM
     if (slabs > hw / 32) slabs = hw / 32;
     if (slabs < 1) slabs = 1;
     const int ppc = ceil_div(hw, slabs);
@@ -670,13 +650,13 @@ extern "C" int b200sd_groupnorm_silu_parts(const void* x0, const void* x1, int C
     const size_t smem = ((size_t)4 * Cg + (size_t)std::max(threads, 2 * Cg)) * sizeof(float);
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     if (in_dtype == B200SD_F32)
-        B200SD_CUDA(b200sd_launch(gn_parts_kernel<B200SD_F32>, dim3(slabs, sets, batch), dim3(threads), smem, s, x0, x1, C0, C1, part0, ppi0,
+        gn_parts_kernel<B200SD_F32><<<dim3(slabs, sets, batch), dim3(threads), smem, s>>>(x0, x1, C0, C1, part0, ppi0,
                                   ld0, part1, ppi1, ld1, gamma, beta, static_cast<bf16*>(out), static_cast<bf16*>(raw_out), hw, groups, G,
-                                  ppc, R, eps, silu, stats_out));
+                                  ppc, R, eps, silu, stats_out);
     else
-        B200SD_CUDA(b200sd_launch(gn_parts_kernel<B200SD_BF16>, dim3(slabs, sets, batch), dim3(threads), smem, s, x0, x1, C0, C1, part0, ppi0,
+        gn_parts_kernel<B200SD_BF16><<<dim3(slabs, sets, batch), dim3(threads), smem, s>>>(x0, x1, C0, C1, part0, ppi0,
                                   ld0, part1, ppi1, ld1, gamma, beta, static_cast<bf16*>(out), static_cast<bf16*>(raw_out), hw, groups, G,
-                                  ppc, R, eps, silu, stats_out));
+                                  ppc, R, eps, silu, stats_out);
     COUNT_LAUNCH();
     B200SD_LAUNCH_CHECK();
     return B200SD_OK;

@@ -16,7 +16,6 @@
 // 4 fit) ran at 2.66 TB/s = 41 % of the measured copy bandwidth (profiles/r02c_elementwise_with_optimizers_v1.json).
 #include <atomic>
 #include <cmath>
-#include <cstdlib>
 
 #include "common.cuh"
 
@@ -28,9 +27,9 @@ namespace {
 constexpr int kBlock = 2048;      // values per quantisation block
 constexpr int kV = 4;             // values per thread
 constexpr int kThreads = kBlock / kV;     // 512: one CTA iteration = one quantisation block
-// resident CTAs per SM the kernel is compiled for: 3 -> 40 registers, 48 warps per SM; 4 -> 32 registers (24 B of spills), 64 warps.
-// B200SD_ADAM8_CTAS=3|4 selects at run time; the default is the faster one on B200 (profiles/r02c_adam8bit_variants.txt).
-constexpr int kDefaultCtasPerSm = 3;
+// resident CTAs per SM the kernel is compiled for: 3 -> 40 registers, 48 warps per SM.  4 (32 registers, 24 B of spills,
+// 64 warps) measured slower on B200: 420.9 vs 411.5 us per launch (profiles/r02c_adam8bit_variants_v3.txt).
+constexpr int kCtasPerSm = 3;
 constexpr int kModeSkip = -2;     // chunk_mode: frozen parameter / padding -- untouched
 constexpr int kMode8bit = -1;     // chunk_mode: moments stored as codes; >= 0: offset into the compact fp32 moments
 // lookup-table bins: q = (order-preserving key of x) >> 16.  Positive x in [2^-24, 1.0078): q in [0xB380, 0xBF80], everything
@@ -65,8 +64,7 @@ __device__ __forceinline__ int lut_bin_unsigned(float x) {       // x >= 0
 __device__ __forceinline__ float bin_low_pos(int bp) { return bp == 0 ? 0.f : __uint_as_float((uint32_t)(kPosBase + bp - 0x8000) << 16); }
 __device__ __forceinline__ float bin_low_neg(int b) { return __uint_as_float(((0xFFFFu - (uint32_t)(kNegBase + b)) << 16) | 0xFFFFu); }
 
-template <int CTAS>
-__global__ void __launch_bounds__(kThreads, CTAS) adamw8bit_kernel(float* __restrict__ p, float* __restrict__ g,
+__global__ void __launch_bounds__(kThreads, kCtasPerSm) adamw8bit_kernel(float* __restrict__ p, float* __restrict__ g,
                                                                          uint8_t* __restrict__ st1, uint8_t* __restrict__ st2,
                                                                          float* __restrict__ absmax1, float* __restrict__ absmax2,
                                                                          const float* __restrict__ qmap1,
@@ -79,8 +77,6 @@ __global__ void __launch_bounds__(kThreads, CTAS) adamw8bit_kernel(float* __rest
     __shared__ uint8_t lut1[2 * kNPos + 4], lut2[kNPos + 6];
     __shared__ float red1[kThreads / 32], red2[kThreads / 32];
     const int tid = threadIdx.x;
-    ptx::pdl_trigger();
-    ptx::pdl_wait();
     if (tid < 256) {
         q1[tid] = __ldg(qmap1 + tid);
         q2[tid] = __ldg(qmap2 + tid);
@@ -242,29 +238,16 @@ extern "C" int b200sd_adamw8bit_step(float* param, float* grad, uint8_t* state1,
     c.zero_grad = zero_grad;
     const int64_t nblocks = (n + kBlock - 1) / kBlock;
     // persistent grid: exactly the CTAs that are resident at once (a larger grid would run its tail at partial occupancy)
-    static const int variant = [] {
-        const char* e = getenv("B200SD_ADAM8_CTAS");
-        const int v = e ? atoi(e) : kDefaultCtasPerSm;
-        return v == 4 ? 4 : 3;
-    }();
-    static int resident[2] = {0, 0};
-    int& ctas_per_sm = resident[variant - 3];
+    static int ctas_per_sm = 0;
     if (ctas_per_sm == 0) {
         int v = 0;
-        if (variant == 4) B200SD_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&v, adamw8bit_kernel<4>, kThreads, 0));
-        else B200SD_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&v, adamw8bit_kernel<3>, kThreads, 0));
+        B200SD_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&v, adamw8bit_kernel, kThreads, 0));
         ctas_per_sm = v > 0 ? v : 1;
     }
     int64_t grid = (int64_t)b200sd_num_sms() * ctas_per_sm;
     if (grid > nblocks) grid = nblocks;
-    if (variant == 4)
-        B200SD_CUDA(b200sd_launch(adamw8bit_kernel<4>, dim3((unsigned)grid), dim3(kThreads), 0, static_cast<cudaStream_t>(stream), param,
-                                  grad, state1, state2, absmax1, absmax2, qmap1, qmap2, chunk_mode, small_exp_avg, small_exp_avg_sq,
-                                  static_cast<bf16*>(weights_bf16), n, nblocks, c));
-    else
-        B200SD_CUDA(b200sd_launch(adamw8bit_kernel<3>, dim3((unsigned)grid), dim3(kThreads), 0, static_cast<cudaStream_t>(stream), param,
-                                  grad, state1, state2, absmax1, absmax2, qmap1, qmap2, chunk_mode, small_exp_avg, small_exp_avg_sq,
-                                  static_cast<bf16*>(weights_bf16), n, nblocks, c));
+    adamw8bit_kernel<<<dim3((unsigned)grid), dim3(kThreads), 0, static_cast<cudaStream_t>(stream)>>>(param, grad, state1, state2,
+        absmax1, absmax2, qmap1, qmap2, chunk_mode, small_exp_avg, small_exp_avg_sq, static_cast<bf16*>(weights_bf16), n, nblocks, c);
     COUNT_LAUNCH();
     B200SD_LAUNCH_CHECK();
     return B200SD_OK;

@@ -33,8 +33,6 @@ __device__ __forceinline__ float block_reduce(float v, float* sh, bool is_max) {
 __global__ void __launch_bounds__(256) softmax_rows_kernel(const float* __restrict__ x, bf16* __restrict__ out, int L, int ldx,
                                                            int ldo, float scale_log2) {
     __shared__ float sh[8];
-    ptx::pdl_trigger();
-    ptx::pdl_wait();
     const float4* xr = reinterpret_cast<const float4*>(x + (size_t)blockIdx.x * ldx);
     const int L4 = L >> 2;
     float m = -INFINITY;
@@ -60,8 +58,6 @@ __global__ void __launch_bounds__(256) softmax_rows_kernel(const float* __restri
 // 1x1 convolution over a handful of channels, NCHW fp32 -> NCHW fp32 (quant_conv 8 -> 8, post_quant_conv 4 -> 4)
 __global__ void conv1x1_small_kernel(const float* __restrict__ x, const float* __restrict__ w, const float* __restrict__ bias,
                                      float* __restrict__ out, int batch, int Cin, int Cout, int hw) {
-    ptx::pdl_trigger();
-    ptx::pdl_wait();
     const int64_t total = (int64_t)batch * hw, stride = (int64_t)gridDim.x * blockDim.x;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += stride) {
         const int b = (int)(i / hw), p = (int)(i % hw);
@@ -79,8 +75,6 @@ __global__ void conv1x1_small_kernel(const float* __restrict__ x, const float* _
 // -30, 20)) * noise) * out_scale  (noise == NULL: the mode)
 __global__ void gaussian_sample_kernel(const float* __restrict__ moments, const float* __restrict__ noise, float* __restrict__ out,
                                        int batch, int C, int hw, float out_scale) {
-    ptx::pdl_trigger();
-    ptx::pdl_wait();
     const int64_t total = (int64_t)batch * C * hw, stride = (int64_t)gridDim.x * blockDim.x;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += stride) {
         const int64_t b = i / ((int64_t)C * hw), r = i % ((int64_t)C * hw);
@@ -106,8 +100,8 @@ extern "C" int b200sd_softmax_rows(const float* x, void* out_bf16, int rows, int
                                    b200sd_stream_t stream) {
     B200SD_REQUIRE(x && out_bf16 && rows > 0 && L > 0, "softmax_rows: bad arguments");
     B200SD_REQUIRE(L % 4 == 0 && ldx % 4 == 0 && ldo % 4 == 0, "softmax_rows: L / ldx / ldo must be multiples of 4");
-    B200SD_CUDA(b200sd_launch(softmax_rows_kernel, dim3(rows), dim3(256), 0, static_cast<cudaStream_t>(stream), x,
-                              static_cast<bf16*>(out_bf16), L, ldx, ldo, scale * 1.4426950408889634f));
+    softmax_rows_kernel<<<dim3(rows), dim3(256), 0, static_cast<cudaStream_t>(stream)>>>(x,
+                              static_cast<bf16*>(out_bf16), L, ldx, ldo, scale * 1.4426950408889634f);
     COUNT_LAUNCH();
     B200SD_LAUNCH_CHECK();
     return B200SD_OK;
@@ -117,8 +111,7 @@ extern "C" int b200sd_conv1x1_small(const float* x_nchw, const float* w, const f
                                     int Cout, int hw, b200sd_stream_t stream) {
     B200SD_REQUIRE(x_nchw && w && bias && out_nchw, "conv1x1_small: null pointer");
     B200SD_REQUIRE(batch > 0 && hw > 0 && Cin >= 1 && Cin <= 8 && Cout >= 1 && Cout <= 8, "conv1x1_small: 1..8 channels");
-    B200SD_CUDA(b200sd_launch(conv1x1_small_kernel, dim3(ew_grid((int64_t)batch * hw, 256)), dim3(256), 0,
-                              static_cast<cudaStream_t>(stream), x_nchw, w, bias, out_nchw, batch, Cin, Cout, hw));
+    conv1x1_small_kernel<<<dim3(ew_grid((int64_t)batch * hw, 256)), dim3(256), 0, static_cast<cudaStream_t>(stream)>>>(x_nchw, w, bias, out_nchw, batch, Cin, Cout, hw);
     COUNT_LAUNCH();
     B200SD_LAUNCH_CHECK();
     return B200SD_OK;
@@ -127,8 +120,7 @@ extern "C" int b200sd_conv1x1_small(const float* x_nchw, const float* w, const f
 extern "C" int b200sd_gaussian_sample(const float* moments, const float* noise, float* out, int batch, int C, int hw, float out_scale,
                                       b200sd_stream_t stream) {
     B200SD_REQUIRE(moments && out && batch > 0 && C > 0 && hw > 0, "gaussian_sample: bad arguments");
-    B200SD_CUDA(b200sd_launch(gaussian_sample_kernel, dim3(ew_grid((int64_t)batch * C * hw, 256)), dim3(256), 0,
-                              static_cast<cudaStream_t>(stream), moments, noise, out, batch, C, hw, out_scale));
+    gaussian_sample_kernel<<<dim3(ew_grid((int64_t)batch * C * hw, 256)), dim3(256), 0, static_cast<cudaStream_t>(stream)>>>(moments, noise, out, batch, C, hw, out_scale);
     COUNT_LAUNCH();
     B200SD_LAUNCH_CHECK();
     return B200SD_OK;

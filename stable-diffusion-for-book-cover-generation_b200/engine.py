@@ -15,8 +15,6 @@ Data flow per block (SURVEY.md App. A.2), each arrow = one kernel:
 """
 from __future__ import annotations
 
-import os
-
 import torch
 
 from . import ops
@@ -37,34 +35,10 @@ class Engine(Builder):
         self._ctx_key = ContextKey()
         self.debug = False      # when True (eager runs only) every tapped activation is cloned
         self.debug_out = {}
-        self.prefetch_kblocks = int(os.environ.get("B200SD_PREFETCH", "0"))     # k-blocks of the next layer staged in L2 (0 = off)
-        self.prefetch_weights = self.prefetch_kblocks > 0
-        self._prev_gemm, self._first_w = None, None
         with torch.cuda.device(device):
             self._build()
 
     # -- plan-building helpers --------------------------------------------------------------------
-    def gemm(self, plan, a0, w, out, **kw):
-        args = super().gemm(plan, a0, w, out, **kw)
-        if plan is self.plan and self.prefetch_weights:
-            # the weights of THIS layer are what the PREVIOUS tensor-core launch pulls into L2 while it runs: every layer's weights
-            # are cold in HBM when its kernel starts (1.7 GB stream through a 126 MB L2 once per step)
-            if self._prev_gemm is not None:
-                self._prev_gemm.prefetch, self._prev_gemm.prefetch_bytes = w.data_ptr(), self._prefetch_bytes(w)
-            else:
-                self._first_w = w
-            self._prev_gemm = args
-        return args
-
-    def _prefetch_bytes(self, w):
-        """How much of the next layer's weights the previous launch stages in L2.  Staging ALL of it was measured slower (the
-        prefetch stream competes with the running kernel's own, latency-critical loads: 5.01 vs 4.95 ms per step); what the next
-        kernel needs at once is its first k-blocks -- a contiguous prefix in the k-block-major layout ([K/64][N][64])."""
-        total = w.numel() * w.element_size()
-        if w.dim() == 3:
-            return min(total, self.prefetch_kblocks * w.shape[1] * w.shape[2] * w.element_size())
-        return total if self.prefetch_kblocks >= 1000 else 0
-
     def _tap(self, name, t, h, w):
         """Debug probe: snapshot activation `t` ([N*h*w, C] NHWC) as NCHW fp32 under `name`."""
         def op():
@@ -103,7 +77,7 @@ class Engine(Builder):
         # all 22 time_emb_proj heads at once: (N, 1280) x (19200, 1280)^T.  The CUDA-core small_linear re-reads the 49 MB of weights
         # per group of 8 batch rows (16 us at CFG batch 2, 154 us at batch 16); from 8 rows on it is one tensor-core GEMM
         # (rows beyond N are TMA zero fill) behind a SiLU + bf16 cast of the 1280-vector
-        self.large_batch = N >= int(os.environ.get("B200SD_LARGE_BATCH", "8"))
+        self.large_batch = N >= 8
         if self.large_batch:
             a16 = torch.empty(N, temb_dim, dtype=torch.bfloat16, device=dev)
             P.append(lambda: ops.cast_act(t_emb, a16, silu=True), "time_embed")
@@ -234,8 +208,6 @@ class Engine(Builder):
             P.append(lambda tmp=tmp: ops.nhwc_bias_to_nchw(tmp, wo["b"], self.out), "conv_io", 0, "conv_out: bias + NCHW")
         else:
             P.append(lambda t=t: ops.conv_out(t, wo["w"], wo["b"], self.out), "conv_io", 0, "conv_out")
-        if self._prev_gemm is not None and self._first_w is not None:   # the last layer stages the first layer of the next step
-            self._prev_gemm.prefetch, self._prev_gemm.prefetch_bytes = self._first_w.data_ptr(), self._prefetch_bytes(self._first_w)
         self.activation_bytes = pool.total
 
     # -- execution --------------------------------------------------------------------------------

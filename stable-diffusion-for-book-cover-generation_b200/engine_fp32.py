@@ -20,7 +20,6 @@ import torch
 
 from . import ops
 from .engine import Engine
-from .plan import Builder
 
 F32, BF16 = torch.float32, torch.bfloat16
 
@@ -46,8 +45,6 @@ def _pack_lin(w):       # (out, in[,1,1]) -> W1 [out][2 in] = [hi | hi], W2 [out
 
 class EngineF32(Engine):
     """Engine's inputs, context cache and execution over the fp32-accuracy plan built below."""
-
-    gemm = Builder.gemm     # no L2 weight prefetch chain (Engine.gemm): every contraction here is a pair of launches
 
     def _buf(self, rows, cols, dtype=F32):
         return torch.empty(rows, cols, dtype=dtype, device=self.device)

@@ -11,7 +11,6 @@ from ._lib import DgradArgs, GemmArgs, WgradArgs, B200SDError, check, lib
 
 F32, BF16 = 0, 1
 EPI_LINEAR, EPI_GEGLU = 0, 1
-_GN_RECOMPUTE = __import__("os").environ.get("B200SD_GN_FAST", "1") == "0"   # debug: GroupNorm backward recomputes its statistics
 
 
 def _up16(*ts):
@@ -229,10 +228,7 @@ def gemm(a0, w, out, *, a1=None, bias=None, rowbias=None, residual=None, conv=No
          epilogue=EPI_LINEAR, block_n=0, split_k=0, M=None, ldrb=0, launch=True, pair=0):
     """out[M, N] = [a0 | a1] @ w^T (+bias +rowbias +residual); conv=(batch, H, W) -> 3x3 pad-1 conv (NHWC)."""
     _chk(a0, a1, w, bias, rowbias, residual, out)
-    if w.dim() == 3:            # k-block-major weights [K/64][N][64] (packing.kblock_major)
-        N, K = w.shape[1], w.shape[0] * w.shape[2]
-    else:
-        N, K = w.shape
+    N, K = w.shape
     C0 = a0.shape[-1]
     C1 = a1.shape[-1] if a1 is not None else 0
     if M is None:
@@ -257,7 +253,6 @@ def gemm(a0, w, out, *, a1=None, bias=None, rowbias=None, residual=None, conv=No
     args.residual_dtype = _dt(residual) if residual is not None else BF16
     args.block_n, args.split_k = block_n, split_k
     args.pair = pair
-    args.w_layout = 1 if w.dim() == 3 else 0
     args.workspace, args.workspace_bytes = _p(ws), ws.numel()
     if not launch:
         return args
@@ -517,8 +512,6 @@ def adamw8bit_step(param, grad, state1, state2, absmax1, absmax2, qmap1, qmap2, 
 def groupnorm_silu_bwd(x0, x1, gamma, beta, dy, out0, out1, batch, hw, *, add_src=None, acc0=False, acc1=False,
                        dgamma=None, dbeta=None, groups=32, eps=1e-5, silu=True, mean_rstd=None):
     _chk(x0, x1, gamma, beta, dy, out0, out1, add_src, dgamma, dbeta, mean_rstd)
-    if _GN_RECOMPUTE:
-        mean_rstd = None
     ws = _workspace("gn_bwd", lib().b200sd_groupnorm_bwd_workspace_floats(batch) * 4, x0.device, zero=True)
     C0 = x0.shape[-1]
     C1 = x1.shape[-1] if x1 is not None else 0

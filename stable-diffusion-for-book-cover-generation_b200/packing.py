@@ -35,15 +35,6 @@ def pack_geglu(w: torch.Tensor, b: torch.Tensor, tile: int):
     return wp, bp
 
 
-def kblock_major(w: torch.Tensor) -> torch.Tensor:
-    """[N][K] -> [K/64][N][64] (B200SD_W_KBLOCK_MAJOR): the 64-wide k-blocks of all N rows stored together, so the weight
-    tile a GEMM CTA fetches per k-block (block_n rows x 128 B) is one contiguous run of DRAM instead of block_n pieces a whole
-    weight row apart.  ops.gemm recognises the layout by the 3-D shape."""
-    n, k = w.shape
-    assert k % 64 == 0
-    return w.reshape(n, k // 64, 64).permute(1, 0, 2).contiguous()
-
-
 def pack_conv_out_tc(w: torch.Tensor, pad_to: int = 32) -> torch.Tensor:
     """conv_out (Cout <= 4, Cin, 3, 3) fp32 -> bf16 [pad_to][9][2*Cin] for the tensor-core path: per tap [hi | lo] with
     hi = bf16(w), lo = bf16(w - hi), so that [x | x] . [hi | lo] restores the fp32 weights to ~2^-17 (the last layer of the network

@@ -41,9 +41,9 @@ def _captured_sampler(unet, scheduler, latents, ctx2, guidance_scale):
     if not (isinstance(unet, UNet2DConditionModel) and isinstance(scheduler, (DDIMScheduler, PNDMScheduler)) and latents.is_cuda
             and unet._precision == "bf16" and unet.use_cuda_graph and not unet.training):
         return None
-    from .sampler import CapturedSampler, default_lanes
+    from .sampler import CapturedSampler
     B, _, h, w = latents.shape
-    key = (type(scheduler).__name__, B, h, w, ctx2.shape[1], latents.device.index, float(guidance_scale), default_lanes(B),
+    key = (type(scheduler).__name__, B, h, w, ctx2.shape[1], latents.device.index, float(guidance_scale),
            tuple(scheduler.timesteps.tolist()), tuple(sorted((k, str(v)) for k, v in vars(scheduler.config).items())))
     cache = unet.__dict__.setdefault("_samplers", {})
     smp = cache.get(key)

@@ -90,8 +90,7 @@ class Builder:
 
     def gemm(self, plan, a0, w, out, *, rowbias_ptr=None, gn_hw=0, kind=None, name=None, **kw):
         """out = [a0 | a1] w^T (+ epilogue terms, see ops.gemm).  rowbias_ptr = (address, ld, rows per image) of a per-image bias
-        row; gn_hw > 0: `out` feeds a GroupNorm over gn_hw rows per image -- the epilogue also emits its column statistics.
-        Returns the GemmArgs (Engine points their prefetch fields at the next layer's weights)."""
+        row; gn_hw > 0: `out` feeds a GroupNorm over gn_hw rows per image -- the epilogue also emits its column statistics."""
         args = ops.gemm(a0, w, out, launch=False, **kw)
         if rowbias_ptr is not None:
             args.rowbias, args.ldrb, args.rows_per_image = rowbias_ptr
@@ -106,7 +105,6 @@ class Builder:
         k = "conv3x3" if args.conv_taps == 9 else "gemm"
         plan.append(lambda a=args: ops.gemm_run(a), kind or k, 2.0 * args.M * args.N * args.K,
                     name or f"{k} M{args.M} N{args.N} K{args.K}")
-        return args
 
     def dgrad(self, plan, dy, w, out, *, name=None, **kw):
         """out = dy (*) w (+ residual): the data gradient of gemm() (ops.gemm_dgrad)."""

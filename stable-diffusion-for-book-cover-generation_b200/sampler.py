@@ -26,20 +26,12 @@ the new latents -- what bench.py reports as `e2e`.
 """
 from __future__ import annotations
 
-import os
-
 import torch
 
 from . import ops
 from ._lib import B200SDError
 from .engine import Engine
 from .plan import run_plan
-
-
-def default_lanes(batch_images: int) -> int:
-    """1 (measured: concurrent CFG halves lose at every batch size, see the module docstring); B200SD_LANES overrides."""
-    env = os.environ.get("B200SD_LANES")
-    return int(env) if env else 1
 
 
 class CapturedSampler:
@@ -53,7 +45,7 @@ class CapturedSampler:
         if unet._precision != "bf16":
             raise B200SDError("CapturedSampler runs the bf16 plan")
         B = int(batch_images)
-        L = default_lanes(B) if lanes is None else int(lanes)
+        L = 1 if lanes is None else int(lanes)   # 1: see the module docstring
         if L < 1 or (L > 1 and (L % 2 or B % (L // 2))):
             raise ValueError(f"lanes={L} does not split the {2 * B}-sample CFG batch into whole sub-batches of one half")
         self.unet, self.scheduler, self.B, self.h, self.w, self.S, self.lanes = unet, scheduler, B, h, w, S_ctx, L

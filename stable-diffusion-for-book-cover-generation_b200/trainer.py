@@ -311,7 +311,6 @@ class Trainer:
         self.opt = None
         self.micro_steps = 0
         self.allreduce_enabled = True    # False: every rank steps on its local gradient (bench.py times the exposed communication)
-        self.pipelined_optimizer = __import__("os").environ.get("B200SD_PIPELINED_ADAMW", "1") != "0"
 
     def _prepare(self, device):
         from .autograd import ensure_flat
@@ -349,7 +348,7 @@ class Trainer:
         self.micro_steps += 1
         if sync:
             scale = 1.0 / (self.world * self.micro_steps)
-            if reduce_now and self.pipelined_optimizer:
+            if reduce_now:
                 # AdamW bucket by bucket, in the order the buckets were put on the wire: the update of the early buckets (the
                 # tail of the flat buffer, reduced while the backward was still running) overlaps the allreduce of the last
                 # ones, which used to be fully exposed; work.wait() makes the compute STREAM wait, not the host
@@ -361,8 +360,6 @@ class Trainer:
                     self.opt.step_range(a, b, grad_scale=scale, zero_grad=True)
                 self.opt.end_step()
             else:
-                if reduce_now:
-                    self.reducer.finish()
                 self.opt.step(grad_scale=scale, zero_grad=True)
             self.micro_steps = 0
         return loss.detach()

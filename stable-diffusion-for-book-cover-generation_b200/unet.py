@@ -373,16 +373,6 @@ class UNet2DConditionModel(nn.Module):
             if hasattr(b, "upsamplers"):
                 W[f"up{i}.us"] = dict(w=packing.pack_conv3x3(b.upsamplers[0].conv.weight.detach()),
                                       b=f32(b.upsamplers[0].conv.bias))
-        # weights are streamed from HBM once per step: store every tensor-core GEMM operand k-block-major so that a CTA's
-        # weight tile is one contiguous run of DRAM (opt-in with B200SD_W_KMAJOR=1: measured on B200 it changes nothing -- 5.142 vs 5.154 ms per step -- the deep-K layers are bound by per-SM operand streaming, not by DRAM page locality)
-        if os.environ.get("B200SD_W_KMAJOR", "0") == "1":
-            gemm_keys = ("w1", "w2", "wsc", "w_in", "w_out", "w_qkv", "w_o1", "w_q2", "w_kv2", "w_o2", "w_ff1", "w_ff2")
-            for prefix, d in W.items():
-                if prefix in ("conv_in", "conv_out", "temb", "tproj"):
-                    continue
-                for k in list(d.keys()):
-                    if k in gemm_keys or (k == "w" and (prefix.endswith(".ds") or prefix.endswith(".us"))):
-                        d[k] = packing.kblock_major(d[k])
         self._packed = W
         self._dirty = False
         self._param_versions = self._versions()

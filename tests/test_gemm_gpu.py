@@ -39,22 +39,25 @@ def test_gemm_plain(M, N, K):
 
 @pytest.mark.parametrize("M,N,K,conv", [(128, 1280, 5120, None), (512, 1280, 1280, None), (8192, 320, 320, None),
                                         (2048, 640, 9 * 640, (2, 32, 32)), (128, 1280, 9 * 1280, (2, 8, 8))])
-def test_gemm_kblock_major_weights(M, N, K, conv):
-    """B200SD_W_KBLOCK_MAJOR ([K/64][N][64], the DRAM-contiguous layout for streamed weights) == row-major, bit for bit."""
-    from b200sd import ops, packing
+def test_gemm_deep_k_f32(M, N, K, conv):
+    """fp32-output GEMM / conv3x3 (+bias) against fp32 torch math: small-M / deep-K layers (split-K) and a short-K one."""
+    from b200sd import ops
     _setup()
     torch.manual_seed(M + N + K)
     C = K // 9 if conv else K
     a = torch.randn(M, C, device=DEV).bfloat16()
     w = (torch.randn(N, K, device=DEV) / K ** 0.5).bfloat16()
     bias = torch.randn(N, device=DEV)
-    out0 = torch.empty(M, N, device=DEV, dtype=torch.float32)
-    out1 = torch.empty_like(out0)
-    ops.gemm(a, w, out0, bias=bias, conv=conv)
-    ops.gemm(a, packing.kblock_major(w), out1, bias=bias, conv=conv)
-    assert torch.equal(out0, out1)
+    out = torch.empty(M, N, device=DEV, dtype=torch.float32)
+    ops.gemm(a, w, out, bias=bias, conv=conv)
     if conv is None:
-        _close(out1, a.float() @ w.float().t() + bias, rel=1e-3)
+        want = a.float() @ w.float().t() + bias
+    else:
+        B, H, W = conv
+        x = a.float().reshape(B, H, W, C).permute(0, 3, 1, 2)
+        w_oihw = w.float().reshape(N, 3, 3, C).permute(0, 3, 1, 2)
+        want = F.conv2d(x, w_oihw, bias, padding=1).permute(0, 2, 3, 1).reshape(M, N)
+    _close(out, want, rel=1e-3)
 
 
 def test_gemm_f32_out_no_bias():

@@ -15,6 +15,6 @@ with torch.no_grad():
     m.use_cuda_graph = True
     g1 = m(x, t, ctx).sample; g2 = m(x, t, ctx).sample; g3 = m(x, t, ctx).sample
 s = float(e1.abs().max())
-print("PDL", os.environ.get("B200SD_PDL", "default"), "scale", s)
+print("scale", s)
 for n, a, b in (("eager-eager", e1, e2), ("eager-graph", e1, g1), ("graph-graph", g1, g2), ("graph-graph2", g2, g3)):
     print(f"{n:14s} max abs diff {float((a - b).abs().max()):.3e}  rel {float((a - b).abs().max()) / s:.3e}")

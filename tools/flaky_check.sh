@@ -1,3 +1,2 @@
 T="tests/test_blocks_gpu.py tests/test_unet_gpu.py::test_50_step_cfg_plms_sampling_cosine"
-echo "== default"; python -m pytest $T -x -q 2>&1 | grep -E "cosine|passed|failed"
-echo "== ATTN_TC=0"; B200SD_ATTN_TC=0 python -m pytest $T -x -q 2>&1 | grep -E "cosine|passed|failed"
+python -m pytest $T -x -q 2>&1 | grep -E "cosine|passed|failed"

@@ -32,5 +32,5 @@ for i in range(5):
     e1.record(); torch.cuda.synchronize()
     best = min(best, e0.elapsed_time(e1) / 4)
 fl = 4.0 * B * H * S * S * d
-print(f"variant {os.environ.get('B200SD_ATTN_FWD', 'default')} attention B{B} S{S} d{d} ramp{ramp}: {best * 1e3:.1f} us "
+print(f"attention B{B} S{S} d{d} ramp{ramp}: {best * 1e3:.1f} us "
       f"{fl / best / 1e9:.0f} TF/s  max-rel err {err:.2e}  lse err {lerr:.2e}")
