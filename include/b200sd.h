@@ -83,6 +83,23 @@ int b200sd_cfg_ddim_step_table(const void* eps_u, const void* eps_c, const void*
 int b200sd_cfg_plms_step_table(const float* eps_u, const float* eps_c, float* x, float* saved, float* ring, int64_t n,
                                float guidance, const float* table, const int* cursor, b200sd_stream_t stream);
 
+/* CFG combine fused with an ancestral (stochastic) update: DDPMScheduler.step, and DDIMScheduler.step with eta > 0:
+ *   eps = eps_u + g (eps_c - eps_u);  x0 = (x - sb_t eps) / sa_t;  if clip: x0 = clamp(x0, -1, 1)
+ *   out = c_x0 x0 + c_x x + c_e eps + (noise ? c_z noise : 0)
+ * noise: fp32, n elements, NULL = no noise term (DDPM's t = 0 step).  The host draws it from the caller's generator.
+ * x_dtype / eps_dtype: B200SD_F32 or B200SD_BF16; out has x_dtype.  out may alias x.
+ * Algorithmic bytes: 5 * n * 4 in fp32 (eps_u, eps_c, x, noise read; out written). */
+int b200sd_cfg_ancestral_step(const void* eps_u, const void* eps_c, const void* x, const float* noise, void* out,
+                              int64_t n, float guidance, float sa_t, float sb_t, float c_x0, float c_x, float c_e, float c_z,
+                              int clip, int eps_dtype, int x_dtype, b200sd_stream_t stream);
+
+/* The captured-sampler form of b200sd_cfg_ancestral_step (fp32; x is updated in place).  Per step one row of 8 floats of
+ * `table` (16-byte aligned), indexed by cursor[1]: sa_t sb_t c_x0 c_x c_e c_z noise_row clip.  noise_row = -1: this step adds
+ * no noise and `noise` is not read; otherwise z = noise + noise_row * n (`noise` is [n_noisy_steps][n] floats, filled by the
+ * host before the run).  `noise` may be NULL when no row names a noise row. */
+int b200sd_cfg_ancestral_step_table(const float* eps_u, const float* eps_c, float* x, const float* noise, int64_t n,
+                                    float guidance, const float* table, const int* cursor, b200sd_stream_t stream);
+
 /* CFG combine fused with the PLMS (PNDM skip_prk_steps=True) linear-multistep update:
  *   eps = eps_u + g (eps_c - eps_u);  e = w[0] eps + sum_{i<nhist} w[1+i] hist[i];
  *   out = cx * x - ce * e

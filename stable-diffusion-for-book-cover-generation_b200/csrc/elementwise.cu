@@ -422,6 +422,102 @@ extern "C" int b200sd_cfg_ddim_step_table(const void* eps_u, const void* eps_c, 
     return B200SD_OK;
 }
 
+// Ancestral samplers (DDPMScheduler; DDIMScheduler with eta > 0): the DDIM prediction of x0, then
+//   x' = c_x0 x0 + c_x x + c_e eps + c_z z
+// z ~ N(0, 1) is drawn by the host from the caller's torch.Generator, so the per-call and the captured loop consume the same
+// noise.  Table row (8 floats): sa_t sb_t c_x0 c_x c_e c_z noise_row clip; noise_row = -1: no noise term, z is not read.
+namespace {
+constexpr int kAncestralRow = 8;
+
+struct AncestralCoef {
+    float g, sa_t, sb_t, c_x0, c_x, c_e, c_z;
+    bool clip;
+};
+
+__device__ __forceinline__ float ancestral_one(float eu, float ec, float x, float z, bool cfg, bool has_z,
+                                               const AncestralCoef& c) {
+    const float e = cfg ? (eu + c.g * (ec - eu)) : eu;
+    float x0 = (x - c.sb_t * e) / c.sa_t;
+    if (c.clip) x0 = fminf(fmaxf(x0, -1.f), 1.f);
+    const float mean = c.c_x0 * x0 + c.c_x * x + c.c_e * e;
+    return has_z ? mean + c.c_z * z : mean;
+}
+
+// x and out may alias (the table form updates the latents in place): each element is read before it is written, by the
+// same thread.
+template <int EDT, int XDT>
+__global__ void __launch_bounds__(kThreads) cfg_ancestral_kernel(const void* __restrict__ eps_u,
+                                                                 const void* __restrict__ eps_c, const void* x,
+                                                                 const float* __restrict__ noise, void* out, int64_t n,
+                                                                 int64_t nvec, AncestralCoef c,
+                                                                 const float* __restrict__ table,
+                                                                 const int* __restrict__ cursor) {
+    if (table != nullptr) {
+        const float4* row = reinterpret_cast<const float4*>(table + (size_t)cursor[1] * kAncestralRow);
+        const float4 a = row[0], b = row[1];
+        c.sa_t = a.x, c.sb_t = a.y, c.c_x0 = a.z, c.c_x = a.w, c.c_e = b.x, c.c_z = b.y;
+        const int noise_row = (int)b.z;
+        noise = (noise_row < 0 || noise == nullptr) ? nullptr : noise + (size_t)noise_row * n;
+        c.clip = b.w != 0.f;
+    }
+    const bool cfg = eps_c != nullptr, has_z = noise != nullptr;
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < nvec; i += stride) {
+        float eu[8], ec[8], xv[8], z[8] = {}, o[8];
+        load8<EDT>(eps_u, i * 8, eu);
+        if (cfg) load8<EDT>(eps_c, i * 8, ec);
+        load8<XDT>(x, i * 8, xv);
+        if (has_z) load8<B200SD_F32>(noise, i * 8, z);
+#pragma unroll
+        for (int j = 0; j < 8; ++j) o[j] = ancestral_one(eu[j], ec[j], xv[j], z[j], cfg, has_z, c);
+        store8<XDT>(out, i * 8, o);
+    }
+    for (int64_t i = nvec * 8 + (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
+        const float eu = load1<EDT>(eps_u, i);
+        const float ec = cfg ? load1<EDT>(eps_c, i) : 0.f;
+        const float z = has_z ? noise[i] : 0.f;
+        store1<XDT>(out, i, ancestral_one(eu, ec, load1<XDT>(x, i), z, cfg, has_z, c));
+    }
+}
+}  // namespace
+
+extern "C" int b200sd_cfg_ancestral_step(const void* eps_u, const void* eps_c, const void* x, const float* noise, void* out,
+                                         int64_t n, float guidance, float sa_t, float sb_t, float c_x0, float c_x, float c_e,
+                                         float c_z, int clip, int eps_dtype, int x_dtype, b200sd_stream_t stream) {
+    B200SD_REQUIRE(eps_u && x && out, "cfg_ancestral_step: null pointer");
+    B200SD_REQUIRE(n >= 0, "cfg_ancestral_step: negative n");
+    B200SD_REQUIRE(dtype_ok(eps_dtype) && dtype_ok(x_dtype), "cfg_ancestral_step: bad dtype");
+    B200SD_REQUIRE(sa_t != 0.f, "cfg_ancestral_step: sa_t == 0");
+    const bool vec = aligned16(eps_u) && aligned16(eps_c) && aligned16(x) && aligned16(noise) && aligned16(out);
+    const int64_t nvec = vec ? n / 8 : 0;  // unaligned views take the scalar path
+    if (n == 0) return B200SD_OK;
+    AncestralCoef c{guidance, sa_t, sb_t, c_x0, c_x, c_e, c_z, clip != 0};
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    DISPATCH2(eps_dtype, x_dtype, cfg_ancestral_kernel, grid_for(vec ? n / 8 : n), s, eps_u, eps_c, x, noise, out, n, nvec, c,
+              (const float*)nullptr, (const int*)nullptr);
+    COUNT_LAUNCH();
+    B200SD_LAUNCH_CHECK();
+    return B200SD_OK;
+}
+
+extern "C" int b200sd_cfg_ancestral_step_table(const float* eps_u, const float* eps_c, float* x, const float* noise, int64_t n,
+                                               float guidance, const float* table, const int* cursor, b200sd_stream_t stream) {
+    B200SD_REQUIRE(eps_u && x && table && cursor, "cfg_ancestral_step_table: null pointer");
+    B200SD_REQUIRE(n >= 0, "cfg_ancestral_step_table: negative n");
+    B200SD_REQUIRE(aligned16(table), "cfg_ancestral_step_table: table must be 16-byte aligned");
+    // every noise row must be 16-byte aligned for the vector path: the base pointer and the row pitch n
+    const bool vec = aligned16(eps_u) && aligned16(eps_c) && aligned16(x) && aligned16(noise) && n % 4 == 0;
+    const int64_t nvec = vec ? n / 8 : 0;
+    if (n == 0) return B200SD_OK;
+    AncestralCoef c{guidance, 1.f, 0.f, 1.f, 0.f, 0.f, 0.f, false};
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    cfg_ancestral_kernel<B200SD_F32, B200SD_F32><<<dim3(grid_for(vec ? n / 8 : n)), dim3(kThreads), 0, s>>>(
+        eps_u, eps_c, x, noise, x, n, nvec, c, table, cursor);
+    COUNT_LAUNCH();
+    B200SD_LAUNCH_CHECK();
+    return B200SD_OK;
+}
+
 extern "C" int b200sd_cfg_plms_step(const void* eps_u, const void* eps_c, const void* x, void* out, void* eps_out,
                                     const void* hist0, const void* hist1, const void* hist2, const void* hist3,
                                     int nhist, const float* w_host5, int64_t n, float guidance, float cx, float ce,

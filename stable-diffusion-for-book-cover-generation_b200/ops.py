@@ -98,6 +98,29 @@ def cfg_ddim_step(eps_u, eps_c, x, guidance, sa_t, sb_t, sa_p, sb_p, out=None, e
     return out
 
 
+def cfg_ancestral_step(eps_u, eps_c, x, noise, guidance, sa_t, sb_t, c_x0, c_x, c_e, c_z, clip, out=None):
+    """DDPM / DDIM (eta > 0) update: c_x0 x0 + c_x x + c_e eps + c_z noise, x0 = (x - sb_t eps) / sa_t (clamped if clip).
+    noise: fp32 with x's size, or None for no noise term."""
+    eps_u, eps_c, x, half = _up16(eps_u, eps_c, x)
+    if half:
+        r = cfg_ancestral_step(eps_u.contiguous(), None if eps_c is None else eps_c.contiguous(), x.contiguous(), noise, guidance,
+                               sa_t, sb_t, c_x0, c_x, c_e, c_z, clip).half()
+        return r if out is None else out.copy_(r)
+    _chk(eps_u, eps_c, x, noise, out)
+    if out is None:
+        out = torch.empty_like(x)
+    if eps_c is not None and eps_c.shape != eps_u.shape:
+        raise ValueError("eps_u / eps_c shape mismatch")
+    if eps_u.numel() != x.numel():
+        raise ValueError(f"model_output {tuple(eps_u.shape)} and sample {tuple(x.shape)} sizes differ")
+    if noise is not None and (noise.dtype != torch.float32 or noise.numel() != x.numel()):
+        raise ValueError(f"noise must be float32 with {x.numel()} elements")
+    check(lib().b200sd_cfg_ancestral_step(_p(eps_u), _p(eps_c), _p(x), _p(noise), _p(out), x.numel(), float(guidance),
+                                          float(sa_t), float(sb_t), float(c_x0), float(c_x), float(c_e), float(c_z), int(bool(clip)),
+                                          _dt(eps_u), _dt(x), _stream()), "cfg_ancestral_step")
+    return out
+
+
 def cfg_plms_step(eps_u, eps_c, x, hist, weights, guidance, cx, ce, out=None, eps_out=None):
     eps_u, eps_c, x, half = _up16(eps_u, eps_c, x)
     if half:
@@ -128,6 +151,13 @@ def cfg_ddim_step_table(eps_u, eps_c, x, out, guidance, coef_table, cursor):
     """cfg_ddim_step() with the coefficients read from coef_table[cursor[0]] (fp32 tensors)"""
     check(lib().b200sd_cfg_ddim_step_table(_p(eps_u), _p(eps_c), _p(x), _p(out), None, x.numel(), float(guidance), _p(coef_table),
                                            _p(cursor), F32, F32, _stream()), "cfg_ddim_step_table")
+
+
+def cfg_ancestral_step_table(eps_u, eps_c, x, noise, guidance, coef_table, cursor):
+    """cfg_ancestral_step() with row coef_table[cursor[1]] (sa_t sb_t c_x0 c_x c_e c_z noise_row clip) and z = noise[noise_row]
+    (fp32 tensors); x is updated in place"""
+    check(lib().b200sd_cfg_ancestral_step_table(_p(eps_u), _p(eps_c), _p(x), _p(noise), x.numel(), float(guidance),
+                                                _p(coef_table), _p(cursor), _stream()), "cfg_ancestral_step_table")
 
 
 def cfg_plms_step_table(eps_u, eps_c, x, saved, ring, guidance, coef_table, cursor):

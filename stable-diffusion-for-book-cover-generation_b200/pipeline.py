@@ -5,20 +5,26 @@ callers pass the (2B, 77, 768) context `cat([uncond, cond])` and the initial lat
 Reference call sites: inference.py:175-176, 342-351; finetune_sd.py:264-271."""
 from __future__ import annotations
 
+import inspect
+
 import torch
 
 
 @torch.no_grad()
 def denoise_loop(unet, scheduler, latents, encoder_hidden_states_2b, num_inference_steps=50, guidance_scale=7.5,
-                 record=None):
+                 record=None, eta=0.0, generator=None):
     """latents (B,4,h,w) -> denoised latents (B,4,h,w).  One UNet call at batch 2B per step, then ONE
-    fused kernel for `eps_u + s (eps_c - eps_u)` + the scheduler update."""
+    fused kernel for `eps_u + s (eps_c - eps_u)` + the scheduler update.  As in diffusers, `eta` and `generator` reach only
+    a scheduler whose step takes them (eta: DDIM; generator: DDIM and DDPM)."""
     if encoder_hidden_states_2b.shape[0] != 2 * latents.shape[0]:
         raise ValueError("encoder_hidden_states must be cat([uncond, cond]) with batch 2B")
     scheduler.set_timesteps(num_inference_steps)
-    sampler = _captured_sampler(unet, scheduler, latents, encoder_hidden_states_2b, guidance_scale) if record is None else None
+    accepted = inspect.signature(scheduler.step_cfg).parameters
+    extra = {k: v for k, v in (("eta", eta), ("generator", generator)) if k in accepted}
+    sampler = (_captured_sampler(unet, scheduler, latents, encoder_hidden_states_2b, guidance_scale, extra.get("eta", 0.0))
+               if record is None else None)
     if sampler is not None:
-        return sampler.run(latents, encoder_hidden_states_2b).to(latents.dtype)
+        return sampler.run(latents, encoder_hidden_states_2b, generator).to(latents.dtype)
     latents = (latents * scheduler.init_noise_sigma).float().contiguous()
     x2 = torch.empty((2 * latents.shape[0],) + tuple(latents.shape[1:]), dtype=latents.dtype, device=latents.device)
     B = latents.shape[0]
@@ -29,21 +35,22 @@ def denoise_loop(unet, scheduler, latents, encoder_hidden_states_2b, num_inferen
         if record is not None:
             record.append(eps2[:B] + guidance_scale * (eps2[B:] - eps2[:B]))
         latents = scheduler.step_cfg(eps2.float() if eps2.dtype not in (torch.float32, torch.bfloat16) else eps2, t,
-                                     latents, guidance_scale).prev_sample
+                                     latents, guidance_scale, **extra).prev_sample
     return latents
 
 
-def _captured_sampler(unet, scheduler, latents, ctx2, guidance_scale):
+def _captured_sampler(unet, scheduler, latents, ctx2, guidance_scale, eta=0.0):
     """The whole-step CUDA graph (sampler.CapturedSampler) when the combination is covered: b200sd UNet on its bf16 plan with
-    CUDA graphs on, DDIM or PLMS, CUDA tensors.  Cached on the UNet per (geometry, schedule, guidance); None -> the per-call loop."""
-    from .schedulers import DDIMScheduler, PNDMScheduler
+    CUDA graphs on, DDIM, PLMS or DDPM, CUDA tensors.  Cached on the UNet per (geometry, schedule, guidance, eta); None -> the
+    per-call loop."""
+    from .schedulers import DDIMScheduler, DDPMScheduler, PNDMScheduler
     from .unet import UNet2DConditionModel
-    if not (isinstance(unet, UNet2DConditionModel) and isinstance(scheduler, (DDIMScheduler, PNDMScheduler)) and latents.is_cuda
-            and unet._precision == "bf16" and unet.use_cuda_graph and not unet.training):
+    if not (isinstance(unet, UNet2DConditionModel) and isinstance(scheduler, (DDIMScheduler, PNDMScheduler, DDPMScheduler))
+            and latents.is_cuda and unet._precision == "bf16" and unet.use_cuda_graph and not unet.training):
         return None
     from .sampler import CapturedSampler
     B, _, h, w = latents.shape
-    key = (type(scheduler).__name__, B, h, w, ctx2.shape[1], latents.device.index, float(guidance_scale),
+    key = (type(scheduler).__name__, B, h, w, ctx2.shape[1], latents.device.index, float(guidance_scale), float(eta),
            tuple(scheduler.timesteps.tolist()), tuple(sorted((k, str(v)) for k, v in vars(scheduler.config).items())))
     cache = unet.__dict__.setdefault("_samplers", {})
     smp = cache.get(key)
@@ -53,7 +60,7 @@ def _captured_sampler(unet, scheduler, latents, ctx2, guidance_scale):
     if smp is None:
         if len(cache) >= 4:
             cache.clear()          # each sampler owns a full set of activation buffers
-        smp = cache[key] = CapturedSampler(unet, scheduler, B, h, w, ctx2.shape[1], guidance_scale)
+        smp = cache[key] = CapturedSampler(unet, scheduler, B, h, w, ctx2.shape[1], guidance_scale, eta=eta)
     return smp
 
 
@@ -179,9 +186,8 @@ class StableDiffusionPipeline:
     def __call__(self, prompt=None, height=512, width=512, num_inference_steps=50, guidance_scale=7.5, negative_prompt=None,
                  eta=0.0, generator=None, latents=None, output_type="pil", return_dict=True, prompt_embeds=None, **kw):
         """inference.py:175-176, 342-351: `pipeline(prompts, height=, width=, num_inference_steps=50, guidance_scale=7.5,
-        latents=...)`.  `prompt_embeds` = cat([uncond, cond]) lets a caller without CLIP drive the hot path directly."""
-        if eta != 0.0:
-            raise NotImplementedError("eta != 0 is not on the reference path")
+        latents=...)`.  `prompt_embeds` = cat([uncond, cond]) lets a caller without CLIP drive the hot path directly.
+        `generator` draws the initial latents, then the step noise of DDPM / DDIM with eta > 0; `eta` reaches DDIM only."""
         if height % 8 or width % 8:
             raise ValueError(f"`height` and `width` have to be divisible by 8 but are {height} and {width}.")
         device = self.device
@@ -198,7 +204,8 @@ class StableDiffusionPipeline:
                                   else "cpu").to(device)
         elif tuple(latents.shape) != shape:
             raise ValueError(f"Unexpected latents shape, got {tuple(latents.shape)}, expected {shape}")
-        lat = denoise_loop(self.unet, self.scheduler, latents.to(device).float(), ctx2.float(), num_inference_steps, guidance_scale)
+        lat = denoise_loop(self.unet, self.scheduler, latents.to(device).float(), ctx2.float(), num_inference_steps, guidance_scale,
+                           eta=eta, generator=generator)
         if output_type == "latent" or self.vae is None:
             images = lat
         else:

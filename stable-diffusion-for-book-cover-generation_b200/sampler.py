@@ -1,4 +1,4 @@
-"""The whole denoising step of StableDiffusionPipeline.__call__ as ONE CUDA graph (DDIM or PLMS + classifier-free guidance).
+"""The whole denoising step of StableDiffusionPipeline.__call__ as ONE CUDA graph (DDIM, PLMS or DDPM + classifier-free guidance).
 
 Reference call sites: the loop inside `pipeline(...)` -- inference.py:175-176, 342-351; finetune_sd.py:264-271 -- i.e. per
 step `latent_model_input = cat([latents] * 2)`, `unet(...)`, `noise_pred_uncond + guidance_scale * (...)`, `scheduler.step`.
@@ -12,6 +12,10 @@ What the graph holds (nothing is launched eagerly between two steps, the host on
     cfg_ddim_step_table        latents <- DDIM(eps_u + g (eps_c - eps_u)), coefficients = table[cursor], in place
     (PNDMScheduler / PLMS: cfg_plms_step_table -- weights, eps-ring slots and the saved-sample flags of this call = table[cursor];
      the 4-deep eps history is a device ring, PNDM's repeated first timestep reads the sample saved by the first call)
+    (DDPMScheduler, or DDIMScheduler with eta > 0: cfg_ancestral_step_table -- coefficients and the noise row = table[cursor];
+     the noise of every stochastic step sits in a device table that `draw_noise` fills from the caller's generator before
+     the run, outside the graph, in the order the per-call loop draws it.  It holds n_noisy_steps * B*4*h*w floats: 3.3 MB
+     per image at 50 steps and 64x64 latents, 2.1 GB for 1000 DDPM steps at batch 32.)
 
 Lanes (`lanes` = 1, 2, or any even number that divides 2B into whole sub-batches of one half; default 1).  The two halves of
 the CFG batch never meet before the combine, so they can run as two independent launch chains reading the SAME latent buffer
@@ -35,11 +39,13 @@ from .plan import run_plan
 
 
 class CapturedSampler:
-    def __init__(self, unet, scheduler, batch_images, h, w, S_ctx=77, guidance_scale=7.5, lanes=None):
-        from .schedulers import DDIMScheduler, PNDMScheduler
-        if not isinstance(scheduler, (DDIMScheduler, PNDMScheduler)):
-            raise B200SDError("CapturedSampler covers DDIMScheduler and PNDMScheduler (PLMS)")
+    def __init__(self, unet, scheduler, batch_images, h, w, S_ctx=77, guidance_scale=7.5, lanes=None, eta=0.0):
+        from .schedulers import DDIMScheduler, DDPMScheduler, PNDMScheduler
+        if not isinstance(scheduler, (DDIMScheduler, PNDMScheduler, DDPMScheduler)):
+            raise B200SDError("CapturedSampler covers DDIMScheduler, PNDMScheduler (PLMS) and DDPMScheduler")
         self.plms = isinstance(scheduler, PNDMScheduler)
+        # eta reaches only DDIM, as in diffusers' pipeline
+        self.ancestral = isinstance(scheduler, DDPMScheduler) or (isinstance(scheduler, DDIMScheduler) and eta != 0.0)
         if scheduler.num_inference_steps is None:
             raise ValueError("call scheduler.set_timesteps(n) first")
         if unet._precision != "bf16":
@@ -67,6 +73,10 @@ class CapturedSampler:
                 self.coef_table = torch.tensor(scheduler.plms_plan(), **f32).contiguous()       # [calls][12]
                 self.saved = torch.zeros_like(self.latents)                                        # the first call's sample
                 self.ring = torch.zeros(4, self.latents.numel(), **f32)                            # eps history
+            elif self.ancestral:
+                rows, n_noisy = scheduler.ancestral_plan(eta)
+                self.coef_table = torch.tensor(rows, **f32).contiguous()                                   # [steps][8]
+                self.noise = torch.zeros(n_noisy, self.latents.numel(), **f32)
             else:
                 self.coef_table = torch.tensor([scheduler._coefs(int(t)) for t in ts], **f32).contiguous()
             self.cursor = torch.zeros(2, dtype=torch.int32, device=dev)
@@ -135,6 +145,10 @@ class CapturedSampler:
             ops.cfg_plms_step_table(self.eps[:B], self.eps[B:], self.latents, self.saved, self.ring, self.guidance, self.coef_table,
                                     self.cursor)
             return
+        if self.ancestral:
+            ops.cfg_ancestral_step_table(self.eps[:B], self.eps[B:], self.latents, self.noise, self.guidance, self.coef_table,
+                                         self.cursor)
+            return
         ops.cfg_ddim_step_table(self.eps[:B], self.eps[B:], self.latents, self.latents, self.guidance, self.coef_table, self.cursor)
 
     def _capture(self, body):
@@ -178,13 +192,24 @@ class CapturedSampler:
                 self.latents.copy_(keep)       # the warm-up run updated the latents in place
             self.graph.replay()
 
+    def draw_noise(self, generator=None):
+        """Fill the noise table of an ancestral sampler: one schedulers.step_noise draw per stochastic step, in step order --
+        the same numbers the per-call loop draws from the same generator."""
+        from .schedulers import step_noise
+        with torch.cuda.device(self.device):
+            for k in range(self.noise.shape[0]):
+                step_noise(self.latents, generator, out=self.noise[k].view(self.latents.shape))
+
     @torch.no_grad()
-    def run(self, latents, ctx2):
-        """latents (B,4,h,w) ~ N(0,1) -> denoised latents after scheduler.num_inference_steps steps"""
+    def run(self, latents, ctx2, generator=None):
+        """latents (B,4,h,w) ~ N(0,1) -> denoised latents after scheduler.num_inference_steps steps.  An ancestral sampler
+        first draws its step noise from `generator` (draw_noise)."""
         if self.unet._stale(self._pack_gen):
             raise B200SDError("the UNet's weights changed after this sampler was built: build a new CapturedSampler")
         self.set_context(ctx2.float())
         self.set_latents(latents.float() * self.scheduler.init_noise_sigma)
+        if self.ancestral:
+            self.draw_noise(generator)
         self.reset(0)
         for _ in range(self.n_steps):
             self.step()

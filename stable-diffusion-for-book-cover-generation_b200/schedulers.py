@@ -7,8 +7,12 @@
 
 Host side: timestep tables and per-step scalar coefficients (fp64 from the fp32 abar table).
 Device side: ONE fused kernel per step through the C ABI (b200sd_cfg_ddim_step /
-b200sd_cfg_plms_step / b200sd_add_noise).  `step_cfg` additionally fuses the pipeline's
+b200sd_cfg_plms_step / b200sd_cfg_ancestral_step / b200sd_add_noise).  `step_cfg` additionally fuses the pipeline's
 classifier-free-guidance combine into the same kernel.
+
+Ancestral sampling (DDPMScheduler.step, DDIMScheduler.step with eta > 0) follows diffusers 0.7.2's formulas; its noise is
+drawn by `step_noise` from the caller's generator.  Whether that noise stream is bit-equal to diffusers' own draws (which
+device, whether the 0.7.2 pipeline hands `generator` to `step`) is not claimed.
 """
 from __future__ import annotations
 
@@ -114,10 +118,91 @@ class _SchedulerBase:
         if model_output.numel() != sample.numel():
             raise ValueError("model_output and sample must have the same number of elements")
 
+    def _ancestral_step(self, eps_u, eps_c, sample, guidance, coefs, generator, out=None):
+        sa_t, sb_t, c_x0, c_x, c_e, c_z, noisy, clip = coefs
+        z = step_noise(sample, generator) if noisy else None
+        return ops.cfg_ancestral_step(eps_u, eps_c, sample.contiguous(), z, guidance, sa_t, sb_t, c_x0, c_x, c_e, c_z, clip,
+                                      out=out)
+
+    def ancestral_plan(self, eta=0.0):
+        """One row per timestep for b200sd_cfg_ancestral_step_table: sa_t sb_t c_x0 c_x c_e c_z noise_row clip, where
+        noise_row counts the steps that add noise (the order step_noise draws them in) and is -1 on a step that adds none.
+        Returns (rows, number of noise rows)."""
+        if self.num_inference_steps is None:
+            raise ValueError("call set_timesteps first")
+        rows, k = [], 0
+        for t in self.timesteps.tolist():
+            sa_t, sb_t, c_x0, c_x, c_e, c_z, noisy, clip = self._ancestral_coefs(t, eta)
+            rows.append([sa_t, sb_t, c_x0, c_x, c_e, c_z, float(k if noisy else -1), float(clip)])
+            k += noisy
+        return rows, k
+
+
+def step_noise(sample, generator=None, out=None):
+    """The noise of one stochastic step (DDPMScheduler.step, DDIMScheduler.step with eta > 0, and the captured sampler's
+    noise table): torch.randn(sample.shape, float32) from `generator` on the generator's device (the sample's when generator is
+    None), copied to the sample's device (or into `out`).  Steps draw in step order, and only steps that add noise draw."""
+    dev = generator.device if generator is not None else sample.device
+    z = torch.randn(tuple(sample.shape), generator=generator, dtype=torch.float32, device=dev)
+    if out is None:
+        if z.device == sample.device:
+            return z
+        out = torch.empty(z.shape, dtype=torch.float32, device=sample.device)
+    return out.copy_(z)
+
 
 class DDPMScheduler(_SchedulerBase):
-    """Only the training-time surface the reference uses: add_noise / num_train_timesteps."""
+    """The training-time surface the reference uses (add_noise / num_train_timesteps) and ancestral sampling, the scheduler
+    finetune_sd.py:517-537 saves with its pipeline.  set_timesteps / step follow diffusers 0.7.2's formulas, including its
+    previous-timestep rule abar[t - 1] at every step count.  Only `fixed_small` and `fixed_large` variances: the learned
+    ones need an 8-channel UNet output that SD v1.x does not have."""
     _defaults = dict(trained_betas=None, variance_type="fixed_small", clip_sample=True)
+
+    def __init__(self, *a, **kw):
+        super().__init__(*a, **kw)
+        self._b = self.betas.double().tolist()
+        self._a = self.alphas.double().tolist()
+
+    def set_timesteps(self, num_inference_steps, device=None):
+        if num_inference_steps < 1:
+            raise ValueError("num_inference_steps out of range")
+        if self.config.variance_type not in ("fixed_small", "fixed_large"):
+            raise NotImplementedError(f"variance_type={self.config.variance_type!r} is not implemented")
+        self.num_inference_steps = min(self.num_train_timesteps, num_inference_steps)
+        ts = np.arange(0, self.num_train_timesteps, self.num_train_timesteps // self.num_inference_steps)[::-1]
+        self.timesteps = torch.from_numpy(ts.copy().astype(np.int64))
+
+    def _ancestral_coefs(self, timestep, eta=0.0):
+        """(sa_t, sb_t, c_x0, c_x, c_e, c_z, adds_noise, clip) of one step, fp64 from the fp32 tables"""
+        t = int(timestep)
+        a_t = self._ac[t]
+        a_p = self._ac[t - 1] if t > 0 else 1.0
+        b_t, b_p = 1 - a_t, 1 - a_p
+        c_x0 = a_p ** 0.5 * self._b[t] / b_t
+        c_x = self._a[t] ** 0.5 * b_p / b_t
+        c_z = 0.0
+        if t > 0:
+            if self.config.variance_type == "fixed_small":
+                var = max(b_p / b_t * self._b[t], 1e-20)
+            elif self.config.variance_type == "fixed_large":
+                var = self._b[t]
+            else:
+                raise NotImplementedError(f"variance_type={self.config.variance_type!r} is not implemented")
+            c_z = var ** 0.5
+        return a_t ** 0.5, b_t ** 0.5, c_x0, c_x, 0.0, c_z, t > 0, bool(self.config.clip_sample)
+
+    def step(self, model_output, timestep, sample, generator=None, return_dict: bool = True):
+        self._check_step_args(model_output, sample)
+        prev = self._ancestral_step(model_output.contiguous(), None, sample, 0.0, self._ancestral_coefs(timestep), generator)
+        return SchedulerOutput(prev_sample=prev) if return_dict else (prev,)
+
+    def step_cfg(self, model_output_2b, timestep, sample, guidance_scale, out=None, generator=None):
+        """Fused `eps_u + s (eps_c - eps_u)` + DDPM update; model_output_2b is the (2B, ...) UNet output."""
+        B = sample.shape[0]
+        self._check_step_args(model_output_2b[:B], sample)
+        prev = self._ancestral_step(model_output_2b[:B], model_output_2b[B:], sample, guidance_scale,
+                                    self._ancestral_coefs(timestep), generator, out=out)
+        return SchedulerOutput(prev_sample=prev)
 
 
 class DDIMScheduler(_SchedulerBase):
@@ -144,17 +229,35 @@ class DDIMScheduler(_SchedulerBase):
         a_t, a_p = self._ac[t], self._alpha_prev(prev_t)
         return a_t ** 0.5, (1 - a_t) ** 0.5, a_p ** 0.5, (1 - a_p) ** 0.5
 
-    def step(self, model_output, timestep, sample, eta: float = 0.0, return_dict: bool = True, **kw):
-        if eta != 0.0:
-            raise NotImplementedError("eta != 0 is not on the reference path")
+    def _ancestral_coefs(self, timestep, eta):
+        """eta > 0 (diffusers 0.7.2): sigma = eta sqrt((1 - a_p) / (1 - a_t) (1 - a_t / a_p)), x' = sqrt(a_p) x0 +
+        sqrt(1 - a_p - sigma^2) eps + sigma z, with noise drawn on every step.  fp64 from the fp32 abar table."""
+        if not 0.0 <= eta <= 1.0:
+            raise ValueError(f"eta must be in [0, 1], got {eta}")
+        t = int(timestep)
+        prev_t = t - self.num_train_timesteps // self.num_inference_steps
+        a_t, a_p = self._ac[t], self._alpha_prev(prev_t)
+        var = (1 - a_p) / (1 - a_t) * (1 - a_t / a_p)
+        sigma = eta * var ** 0.5
+        return a_t ** 0.5, (1 - a_t) ** 0.5, a_p ** 0.5, 0.0, (1 - a_p - sigma ** 2) ** 0.5, sigma, True, False
+
+    def step(self, model_output, timestep, sample, eta: float = 0.0, return_dict: bool = True, generator=None, **kw):
         self._check_step_args(model_output, sample)
-        prev = ops.cfg_ddim_step(model_output.contiguous(), None, sample.contiguous(), 0.0, *self._coefs(timestep))
+        if eta == 0.0:
+            prev = ops.cfg_ddim_step(model_output.contiguous(), None, sample.contiguous(), 0.0, *self._coefs(timestep))
+        else:
+            prev = self._ancestral_step(model_output.contiguous(), None, sample, 0.0, self._ancestral_coefs(timestep, eta),
+                                        generator)
         return SchedulerOutput(prev_sample=prev) if return_dict else (prev,)
 
-    def step_cfg(self, model_output_2b, timestep, sample, guidance_scale, out=None):
+    def step_cfg(self, model_output_2b, timestep, sample, guidance_scale, out=None, eta: float = 0.0, generator=None):
         """Fused `eps_u + s (eps_c - eps_u)` + DDIM update; model_output_2b is the (2B, ...) UNet output."""
         self._check_step_args(model_output_2b[: sample.shape[0]], sample)
         B = sample.shape[0]
+        if eta != 0.0:
+            prev = self._ancestral_step(model_output_2b[:B], model_output_2b[B:], sample, guidance_scale,
+                                        self._ancestral_coefs(timestep, eta), generator, out=out)
+            return SchedulerOutput(prev_sample=prev)
         prev = ops.cfg_ddim_step(model_output_2b[:B], model_output_2b[B:], sample.contiguous(), guidance_scale,
                                  *self._coefs(timestep), out=out)
         return SchedulerOutput(prev_sample=prev)
