@@ -56,26 +56,24 @@ int b200sd_timer_elapsed_ms(int i, int j, float* ms);
  *   eps = eps_u + g (eps_c - eps_u);  x0 = (x - sb_t eps) / sa_t;  out = sa_p x0 + sb_p eps
  * Replaces the pipeline's `noise_pred_uncond + guidance_scale * (...)` and DDIMScheduler.step
  * (reference call sites inference.py:175-176, 386-387; SURVEY.md App. B.2/B.4).
- * eps_c == NULL -> no CFG (eps = eps_u).  eps_out (optional) receives the combined eps.
- * x_dtype / eps_dtype: B200SD_F32 or B200SD_BF16; out has x_dtype, eps_out has eps_dtype.
+ * eps_c == NULL -> no CFG (eps = eps_u).  eps_out must be NULL: since version 102 the combined eps is not written out and a
+ * non-NULL eps_out returns B200SD_ERR_INVALID.  This is b200sd_cfg_ancestral_step with c_x0 = sa_p, c_x = 0, c_e = sb_p, no
+ * noise and no clipping, whose error messages it returns.
+ * x_dtype / eps_dtype: B200SD_F32 or B200SD_BF16; out has x_dtype.  out may alias x.
  * Algorithmic bytes: 4 * n * elem (3 reads + 1 write). */
 int b200sd_cfg_ddim_step(const void* eps_u, const void* eps_c, const void* x, void* out, void* eps_out,
                          int64_t n, float guidance, float sa_t, float sb_t, float sa_p, float sb_p,
                          int eps_dtype, int x_dtype, b200sd_stream_t stream);
 
-/* Captured sampler: the whole denoising step (timestep -> UNet plan -> CFG + DDIM update) is ONE CUDA graph that is replayed
- * with no host-side arguments, so the step index lives on the device.  `cursor` is int[2]: [0] = next step, [1] = the step
- * being executed.  b200sd_sampler_advance opens a step: in_t[0..n_t) = timesteps[cursor[0]] (the UNet plan's timestep input),
- * cursor[1] = cursor[0], cursor[0] = (cursor[0] + 1) % n_steps.  b200sd_cfg_ddim_step_table closes it: the same kernel as
- * b200sd_cfg_ddim_step with (sa_t, sb_t, sa_p, sb_p) = coef_table[cursor[1]] ([n_steps][4] floats, 16-byte aligned).
- * out may alias x (elementwise).  Replaces the per-step Python of StableDiffusionPipeline.__call__'s loop
- * (reference call sites inference.py:175-176, 342-351). */
+/* Captured sampler: the whole denoising step (timestep -> UNet plan -> CFG + scheduler update) is ONE CUDA graph that is
+ * replayed with no host-side arguments, so the step index lives on the device.  `cursor` is int[2]: [0] = next step, [1] = the
+ * step being executed.  b200sd_sampler_advance opens a step: in_t[0..n_t) = timesteps[cursor[0]] (the UNet plan's timestep
+ * input), cursor[1] = cursor[0], cursor[0] = (cursor[0] + 1) % n_steps.  b200sd_cfg_ancestral_step_table (DDIM, DDPM) or
+ * b200sd_cfg_plms_step_table (PLMS) closes it with the coefficients of row cursor[1] of its table.  Replaces the per-step
+ * Python of StableDiffusionPipeline.__call__'s loop (reference call sites inference.py:175-176, 342-351). */
 int b200sd_sampler_advance(const float* timesteps, int n_steps, int* cursor, float* in_t, int n_t, b200sd_stream_t stream);
-int b200sd_cfg_ddim_step_table(const void* eps_u, const void* eps_c, const void* x, void* out, void* eps_out,
-                               int64_t n, float guidance, const float* coef_table, const int* cursor,
-                               int eps_dtype, int x_dtype, b200sd_stream_t stream);
 
-/* The PLMS counterpart of b200sd_cfg_ddim_step_table (fp32): x (the latents) is updated in place; `saved` (n floats) holds the
+/* The PLMS step of the captured sampler (fp32): x (the latents) is updated in place; `saved` (n floats) holds the
  * sample of the first call for PNDM's repeated first timestep; `ring` is the 4-deep eps history (4 * n floats).  Per call one
  * row of 12 floats of `table`, indexed by cursor[1]: w0 w1 w2 w3 | cx ce | h1 h2 h3 (ring slot of ets[-1], ets[-2], ets[-3];
  * -1 = unused) | out_slot (-1 = this call's eps is not kept) | x_from_saved | save_x.  The host fills the table by running
@@ -83,20 +81,21 @@ int b200sd_cfg_ddim_step_table(const void* eps_u, const void* eps_c, const void*
 int b200sd_cfg_plms_step_table(const float* eps_u, const float* eps_c, float* x, float* saved, float* ring, int64_t n,
                                float guidance, const float* table, const int* cursor, b200sd_stream_t stream);
 
-/* CFG combine fused with an ancestral (stochastic) update: DDPMScheduler.step, and DDIMScheduler.step with eta > 0:
+/* CFG combine fused with the affine update of DDPMScheduler.step and DDIMScheduler.step (any eta in [0, 1]):
  *   eps = eps_u + g (eps_c - eps_u);  x0 = (x - sb_t eps) / sa_t;  if clip: x0 = clamp(x0, -1, 1)
  *   out = c_x0 x0 + c_x x + c_e eps + (noise ? c_z noise : 0)
- * noise: fp32, n elements, NULL = no noise term (DDPM's t = 0 step).  The host draws it from the caller's generator.
+ * noise: fp32, n elements, NULL = no noise term (DDIM with eta = 0, DDPM's t = 0 step).  The host draws it from the caller's
+ * generator.
  * x_dtype / eps_dtype: B200SD_F32 or B200SD_BF16; out has x_dtype.  out may alias x.
  * Algorithmic bytes: 5 * n * 4 in fp32 (eps_u, eps_c, x, noise read; out written). */
 int b200sd_cfg_ancestral_step(const void* eps_u, const void* eps_c, const void* x, const float* noise, void* out,
                               int64_t n, float guidance, float sa_t, float sb_t, float c_x0, float c_x, float c_e, float c_z,
                               int clip, int eps_dtype, int x_dtype, b200sd_stream_t stream);
 
-/* The captured-sampler form of b200sd_cfg_ancestral_step (fp32; x is updated in place).  Per step one row of 8 floats of
- * `table` (16-byte aligned), indexed by cursor[1]: sa_t sb_t c_x0 c_x c_e c_z noise_row clip.  noise_row = -1: this step adds
- * no noise and `noise` is not read; otherwise z = noise + noise_row * n (`noise` is [n_noisy_steps][n] floats, filled by the
- * host before the run).  `noise` may be NULL when no row names a noise row. */
+/* The captured-sampler form of b200sd_cfg_ancestral_step (fp32; x is updated in place), for DDIM and DDPM.  Per step one row
+ * of 8 floats of `table` (16-byte aligned), indexed by cursor[1]: sa_t sb_t c_x0 c_x c_e c_z noise_row clip.  noise_row = -1:
+ * this step adds no noise and `noise` is not read; otherwise z = noise + noise_row * n (`noise` is [n_noisy_steps][n] floats,
+ * filled by the host before the run).  `noise` may be NULL when no row names a noise row. */
 int b200sd_cfg_ancestral_step_table(const float* eps_u, const float* eps_c, float* x, const float* noise, int64_t n,
                                     float guidance, const float* table, const int* cursor, b200sd_stream_t stream);
 

@@ -70,7 +70,6 @@ SIGNATURES = {
     "b200sd_gaussian_sample": (_i, [_vp, _vp, _vp, _i, _i, _i, _f, _vp]),
     "b200sd_sampler_advance": (_i, [_vp, _i, _vp, _vp, _i, _vp]),
     "b200sd_cfg_plms_step_table": (_i, [_vp, _vp, _vp, _vp, _vp, _i64, _f, _vp, _vp, _vp]),
-    "b200sd_cfg_ddim_step_table": (_i, [_vp, _vp, _vp, _vp, _vp, _i64, _f, _vp, _vp, _i, _i, _vp]),
     "b200sd_cfg_ancestral_step": (_i, [_vp, _vp, _vp, _vp, _vp, _i64, _f, _f, _f, _f, _f, _f, _f, _i, _i, _i, _vp]),
     "b200sd_cfg_ancestral_step_table": (_i, [_vp, _vp, _vp, _vp, _i64, _f, _vp, _vp, _vp]),
     "b200sd_cfg_plms_step": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, C.POINTER(C.c_float), _i64, _f, _f,

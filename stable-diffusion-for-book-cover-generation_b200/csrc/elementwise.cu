@@ -74,54 +74,6 @@ inline int grid_for(int64_t nvec) {
 }
 
 // ---------------------------------------------------------------------------------------------
-// CFG + DDIM
-// ---------------------------------------------------------------------------------------------
-struct DdimCoef {
-    float g, sa_t, sb_t, sa_p, sb_p;
-};
-
-__device__ __forceinline__ float ddim_one(float eu, float ec, float x, bool cfg, const DdimCoef& c, float& eps) {
-    eps = cfg ? (eu + c.g * (ec - eu)) : eu;
-    float x0 = (x - c.sb_t * eps) / c.sa_t;
-    return c.sa_p * x0 + c.sb_p * eps;
-}
-
-template <int EDT, int XDT>
-__global__ void __launch_bounds__(kThreads) cfg_ddim_kernel(const void* __restrict__ eps_u,
-                                                            const void* __restrict__ eps_c,
-                                                            const void* __restrict__ x, void* __restrict__ out,
-                                                            void* __restrict__ eps_out, int64_t n, int64_t nvec, DdimCoef c,
-                                                            const float4* __restrict__ coef_table, const int* __restrict__ cursor) {
-    if (coef_table != nullptr) {     // captured sampler: this step's coefficients come from a device table (b200sd_sampler_advance)
-        const float4 v = coef_table[cursor[1]];
-        c.sa_t = v.x, c.sb_t = v.y, c.sa_p = v.z, c.sb_p = v.w;
-    }
-    const bool cfg = eps_c != nullptr;
-    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < nvec; i += stride) {
-        float eu[8], ec[8], xv[8], o[8], e[8];
-        load8<EDT>(eps_u, i * 8, eu);
-        if (cfg) load8<EDT>(eps_c, i * 8, ec);
-        load8<XDT>(x, i * 8, xv);
-#pragma unroll
-        for (int j = 0; j < 8; ++j) o[j] = ddim_one(eu[j], ec[j], xv[j], cfg, c, e[j]);
-        store8<XDT>(out, i * 8, o);
-        if (eps_out) store8<EDT>(eps_out, i * 8, e);
-    }
-    // scalar tail (n % 8)
-    {
-        for (int64_t i = nvec * 8 + (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
-            float e;
-            float eu = load1<EDT>(eps_u, i);
-            float ec = cfg ? load1<EDT>(eps_c, i) : 0.f;
-            float o = ddim_one(eu, ec, load1<XDT>(x, i), cfg, c, e);
-            store1<XDT>(out, i, o);
-            if (eps_out) store1<EDT>(eps_out, i, e);
-        }
-    }
-}
-
-// ---------------------------------------------------------------------------------------------
 // CFG + PLMS
 // ---------------------------------------------------------------------------------------------
 struct PlmsArgs {
@@ -311,25 +263,6 @@ bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 
 
 static bool dtype_ok(int d) { return d == B200SD_F32 || d == B200SD_BF16; }
 
-extern "C" int b200sd_cfg_ddim_step(const void* eps_u, const void* eps_c, const void* x, void* out, void* eps_out,
-                                    int64_t n, float guidance, float sa_t, float sb_t, float sa_p, float sb_p,
-                                    int eps_dtype, int x_dtype, b200sd_stream_t stream) {
-    B200SD_REQUIRE(eps_u && x && out, "cfg_ddim_step: null pointer");
-    B200SD_REQUIRE(n >= 0, "cfg_ddim_step: negative n");
-    B200SD_REQUIRE(dtype_ok(eps_dtype) && dtype_ok(x_dtype), "cfg_ddim_step: bad dtype");
-    const bool vec = aligned16(eps_u) && aligned16(eps_c) && aligned16(x) && aligned16(out) && aligned16(eps_out);
-    const int64_t nvec = vec ? n / 8 : 0;  // unaligned views (odd slices) take the scalar path
-    B200SD_REQUIRE(sa_t != 0.f, "cfg_ddim_step: sa_t == 0");
-    if (n == 0) return B200SD_OK;
-    DdimCoef c{guidance, sa_t, sb_t, sa_p, sb_p};
-    cudaStream_t s = static_cast<cudaStream_t>(stream);
-    DISPATCH2(eps_dtype, x_dtype, cfg_ddim_kernel, grid_for(vec ? n / 8 : n), s, eps_u, eps_c, x, out, eps_out, n, nvec, c,
-              (const float4*)nullptr, (const int*)nullptr);
-    COUNT_LAUNCH();
-    B200SD_LAUNCH_CHECK();
-    return B200SD_OK;
-}
-
 // Captured sampler (one CUDA graph per denoising step, replayed with no host-side arguments): the step index lives on the
 // device.  cursor[0] = next step, cursor[1] = the step being executed.
 namespace {
@@ -403,26 +336,8 @@ extern "C" int b200sd_cfg_plms_step_table(const float* eps_u, const float* eps_c
     return B200SD_OK;
 }
 
-extern "C" int b200sd_cfg_ddim_step_table(const void* eps_u, const void* eps_c, const void* x, void* out, void* eps_out,
-                                          int64_t n, float guidance, const float* coef_table, const int* cursor,
-                                          int eps_dtype, int x_dtype, b200sd_stream_t stream) {
-    B200SD_REQUIRE(eps_u && x && out && coef_table && cursor, "cfg_ddim_step_table: null pointer");
-    B200SD_REQUIRE(n >= 0, "cfg_ddim_step_table: negative n");
-    B200SD_REQUIRE(dtype_ok(eps_dtype) && dtype_ok(x_dtype), "cfg_ddim_step_table: bad dtype");
-    B200SD_REQUIRE(aligned16(coef_table), "cfg_ddim_step_table: coef_table must be 16-byte aligned");
-    const bool vec = aligned16(eps_u) && aligned16(eps_c) && aligned16(x) && aligned16(out) && aligned16(eps_out);
-    const int64_t nvec = vec ? n / 8 : 0;
-    if (n == 0) return B200SD_OK;
-    DdimCoef c{guidance, 1.f, 0.f, 1.f, 0.f};
-    cudaStream_t s = static_cast<cudaStream_t>(stream);
-    DISPATCH2(eps_dtype, x_dtype, cfg_ddim_kernel, grid_for(vec ? n / 8 : n), s, eps_u, eps_c, x, out, eps_out, n, nvec, c,
-              reinterpret_cast<const float4*>(coef_table), cursor);
-    COUNT_LAUNCH();
-    B200SD_LAUNCH_CHECK();
-    return B200SD_OK;
-}
-
-// Ancestral samplers (DDPMScheduler; DDIMScheduler with eta > 0): the DDIM prediction of x0, then
+// DDIM (eta = 0 is c_x0 = sqrt(abar_prev), c_x = 0, c_e = sqrt(1 - abar_prev), no noise; eta > 0 adds sigma z) and DDPM:
+// the DDIM prediction of x0, then
 //   x' = c_x0 x0 + c_x x + c_e eps + c_z z
 // z ~ N(0, 1) is drawn by the host from the caller's torch.Generator, so the per-call and the captured loop consume the same
 // noise.  Table row (8 floats): sa_t sb_t c_x0 c_x c_e c_z noise_row clip; noise_row = -1: no noise term, z is not read.
@@ -498,6 +413,14 @@ extern "C" int b200sd_cfg_ancestral_step(const void* eps_u, const void* eps_c, c
     COUNT_LAUNCH();
     B200SD_LAUNCH_CHECK();
     return B200SD_OK;
+}
+
+extern "C" int b200sd_cfg_ddim_step(const void* eps_u, const void* eps_c, const void* x, void* out, void* eps_out,
+                                    int64_t n, float guidance, float sa_t, float sb_t, float sa_p, float sb_p,
+                                    int eps_dtype, int x_dtype, b200sd_stream_t stream) {
+    B200SD_REQUIRE(eps_out == nullptr, "cfg_ddim_step: eps_out is no longer supported and must be NULL");
+    return b200sd_cfg_ancestral_step(eps_u, eps_c, x, nullptr, out, n, guidance, sa_t, sb_t, sa_p, 0.f, sb_p, 0.f, 0, eps_dtype,
+                                     x_dtype, stream);
 }
 
 extern "C" int b200sd_cfg_ancestral_step_table(const float* eps_u, const float* eps_c, float* x, const float* noise, int64_t n,

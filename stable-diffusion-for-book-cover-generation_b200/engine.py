@@ -25,7 +25,7 @@ class Engine(Builder):
     def __init__(self, model, N, H, W, S_ctx, device, io=None):
         super().__init__(device)
         self.model, self.N, self.H, self.W, self.S = model, N, H, W, S_ctx
-        self._io = io           # LanedEngine: (in_sample, in_t, out) views of the parent's static buffers
+        self._io = io           # (in_sample, in_t, out): static buffers owned by the caller (CapturedSampler)
         cfg = model.config
         self.heads = cfg.attention_head_dim
         self.ctx_dim = cfg.cross_attention_dim

@@ -77,29 +77,27 @@ def launch_count() -> int:
 # ---------------------------------------------------------------------------------------------
 # scheduler / loss elementwise
 # ---------------------------------------------------------------------------------------------
-def cfg_ddim_step(eps_u, eps_c, x, guidance, sa_t, sb_t, sa_p, sb_p, out=None, eps_out=None):
+def cfg_ddim_step(eps_u, eps_c, x, guidance, sa_t, sb_t, sa_p, sb_p, out=None):
     eps_u, eps_c, x, half = _up16(eps_u, eps_c, x)
     if half:
-        if eps_out is not None:
-            raise B200SDError("cfg_ddim_step: eps_out is not supported with float16 inputs")
         r = cfg_ddim_step(eps_u.contiguous(), None if eps_c is None else eps_c.contiguous(), x.contiguous(), guidance, sa_t, sb_t,
                           sa_p, sb_p).half()
         return r if out is None else out.copy_(r)
-    _chk(eps_u, eps_c, x, out, eps_out)
+    _chk(eps_u, eps_c, x, out)
     if out is None:
         out = torch.empty_like(x)
     if eps_c is not None and eps_c.shape != eps_u.shape:
         raise ValueError("eps_u / eps_c shape mismatch")
     if eps_u.numel() != x.numel():
         raise ValueError(f"model_output {tuple(eps_u.shape)} and sample {tuple(x.shape)} sizes differ")
-    check(lib().b200sd_cfg_ddim_step(_p(eps_u), _p(eps_c), _p(x), _p(out), _p(eps_out), x.numel(), float(guidance),
+    check(lib().b200sd_cfg_ddim_step(_p(eps_u), _p(eps_c), _p(x), _p(out), None, x.numel(), float(guidance),
                                      float(sa_t), float(sb_t), float(sa_p), float(sb_p), _dt(eps_u), _dt(x), _stream()),
           "cfg_ddim_step")
     return out
 
 
 def cfg_ancestral_step(eps_u, eps_c, x, noise, guidance, sa_t, sb_t, c_x0, c_x, c_e, c_z, clip, out=None):
-    """DDPM / DDIM (eta > 0) update: c_x0 x0 + c_x x + c_e eps + c_z noise, x0 = (x - sb_t eps) / sa_t (clamped if clip).
+    """DDPM / DDIM update: c_x0 x0 + c_x x + c_e eps + c_z noise, x0 = (x - sb_t eps) / sa_t (clamped if clip).
     noise: fp32 with x's size, or None for no noise term."""
     eps_u, eps_c, x, half = _up16(eps_u, eps_c, x)
     if half:
@@ -145,12 +143,6 @@ def sampler_advance(t_table, cursor, in_t):
     """in_t[:] = t_table[cursor[0]]; cursor[0] += 1 (device-side step index of a captured denoising loop)"""
     check(lib().b200sd_sampler_advance(_p(t_table), t_table.numel(), _p(cursor), _p(in_t), in_t.numel(), _stream()),
           "sampler_advance")
-
-
-def cfg_ddim_step_table(eps_u, eps_c, x, out, guidance, coef_table, cursor):
-    """cfg_ddim_step() with the coefficients read from coef_table[cursor[0]] (fp32 tensors)"""
-    check(lib().b200sd_cfg_ddim_step_table(_p(eps_u), _p(eps_c), _p(x), _p(out), None, x.numel(), float(guidance), _p(coef_table),
-                                           _p(cursor), F32, F32, _stream()), "cfg_ddim_step_table")
 
 
 def cfg_ancestral_step_table(eps_u, eps_c, x, noise, guidance, coef_table, cursor):
@@ -427,7 +419,7 @@ def groupnorm_silu(x0, x1, gamma, beta, out, batch, hw, groups=32, eps=1e-5, sil
     _chk(x0, x1, gamma, beta, out, raw_out, stats_out)
     if x1 is not None and x1.dtype != x0.dtype:
         raise B200SDError("groupnorm: both sources must have the same dtype")
-    ws = _workspace(("gn", _stream()), lib().b200sd_groupnorm_workspace_floats(batch) * 4, x0.device)   # per stream: lanes run concurrently
+    ws = _workspace(("gn", _stream()), lib().b200sd_groupnorm_workspace_floats(batch) * 4, x0.device)
     C0 = x0.shape[-1]
     C1 = x1.shape[-1] if x1 is not None else 0
     check(lib().b200sd_groupnorm_silu_stats(_p(x0), _p(x1), C0, C1, _p(gamma), _p(beta), _p(out), _p(raw_out), _p(ws),

@@ -6,23 +6,15 @@ step `latent_model_input = cat([latents] * 2)`, `unet(...)`, `noise_pred_uncond 
 What the graph holds (nothing is launched eagerly between two steps, the host only calls cudaGraphLaunch):
 
     sampler_advance            in_t <- timesteps[cursor]; cursor += 1            (device-side step index)
-      fork ──> lane 0: UNet plan over the UNCONDITIONAL half of the batch  ──┐
-           └─> lane 1: UNet plan over the CONDITIONAL half                 ──┤  (lanes: independent launch chains on
-      join <──────────────────────────────────────────────────────────────────┘   forked streams of the same graph)
-    cfg_ddim_step_table        latents <- DDIM(eps_u + g (eps_c - eps_u)), coefficients = table[cursor], in place
+    UNet plan                  over the CFG batch [uncond | cond], one launch chain
+    cfg_ancestral_step_table   latents <- c_x0 x0 + c_x x + c_e eps (+ c_z z), eps = eps_u + g (eps_c - eps_u), coefficients and
+                               the noise row = table[cursor], in place.  DDIMScheduler (eta = 0: no noise rows; eta > 0) and
+                               DDPMScheduler.  The noise of every stochastic step sits in a device table that `draw_noise` fills
+                               from the caller's generator before the run, outside the graph, in the order the per-call loop
+                               draws it.  It holds n_noisy_steps * B*4*h*w floats: 3.3 MB per image at 50 steps and 64x64
+                               latents, 2.1 GB for 1000 DDPM steps at batch 32.
     (PNDMScheduler / PLMS: cfg_plms_step_table -- weights, eps-ring slots and the saved-sample flags of this call = table[cursor];
      the 4-deep eps history is a device ring, PNDM's repeated first timestep reads the sample saved by the first call)
-    (DDPMScheduler, or DDIMScheduler with eta > 0: cfg_ancestral_step_table -- coefficients and the noise row = table[cursor];
-     the noise of every stochastic step sits in a device table that `draw_noise` fills from the caller's generator before
-     the run, outside the graph, in the order the per-call loop draws it.  It holds n_noisy_steps * B*4*h*w floats: 3.3 MB
-     per image at 50 steps and 64x64 latents, 2.1 GB for 1000 DDPM steps at batch 32.)
-
-Lanes (`lanes` = 1, 2, or any even number that divides 2B into whole sub-batches of one half; default 1).  The two halves of
-the CFG batch never meet before the combine, so they can run as two independent launch chains reading the SAME latent buffer
-and the same weights.  Measured on B200 (profiles/r02b_lanes_sweep.txt): it LOSES at every batch -- 1 image 5.05 -> 5.67 ms
-per step, 2 images 7.14 -> 7.58 (4 lanes 9.39), 4 images 11.15 -> 11.82, 8 images 20.14 -> 20.94 -- because the GEMM split
-policy already spreads a half batch over the whole machine (smaller M -> more K slices), so the two chains contend for the
-same SMs and each streams the weights on its own.  Kept as a tested option, off by default.
 
 `host_step()` is the same graph with the host on both ends: H2D memcpy nodes for the latents and the text context out of
 pinned host buffers, the context K/V projections (the context may change every call), the step, and a D2H memcpy node of
@@ -43,18 +35,16 @@ class CapturedSampler:
         from .schedulers import DDIMScheduler, DDPMScheduler, PNDMScheduler
         if not isinstance(scheduler, (DDIMScheduler, PNDMScheduler, DDPMScheduler)):
             raise B200SDError("CapturedSampler covers DDIMScheduler, PNDMScheduler (PLMS) and DDPMScheduler")
+        if lanes not in (None, 1):
+            raise ValueError(f"lanes={lanes}: the step runs the CFG batch as one launch chain.  Concurrent per-half chains were "
+                             "slower at every batch size measured (profiles/r02b_lanes_sweep.txt) and were removed")
         self.plms = isinstance(scheduler, PNDMScheduler)
-        # eta reaches only DDIM, as in diffusers' pipeline
-        self.ancestral = isinstance(scheduler, DDPMScheduler) or (isinstance(scheduler, DDIMScheduler) and eta != 0.0)
         if scheduler.num_inference_steps is None:
             raise ValueError("call scheduler.set_timesteps(n) first")
         if unet._precision != "bf16":
             raise B200SDError("CapturedSampler runs the bf16 plan")
         B = int(batch_images)
-        L = 1 if lanes is None else int(lanes)   # 1: see the module docstring
-        if L < 1 or (L > 1 and (L % 2 or B % (L // 2))):
-            raise ValueError(f"lanes={L} does not split the {2 * B}-sample CFG batch into whole sub-batches of one half")
-        self.unet, self.scheduler, self.B, self.h, self.w, self.S, self.lanes = unet, scheduler, B, h, w, S_ctx, L
+        self.unet, self.scheduler, self.B, self.h, self.w, self.S, self.lanes = unet, scheduler, B, h, w, S_ctx, 1
         self.guidance = float(guidance_scale)
         dev = self.device = unet.device
         unet._ensure_packed()
@@ -63,6 +53,7 @@ class CapturedSampler:
         f32 = dict(dtype=torch.float32, device=dev)
         with torch.cuda.device(dev):
             self.latents = torch.zeros(B, cfg.in_channels, h, w, **f32)        # updated in place by every step
+            self.x2 = torch.zeros(2 * B, cfg.in_channels, h, w, **f32)         # [latents | latents], the UNet's input
             self.eps = torch.zeros(2 * B, cfg.out_channels, h, w, **f32)       # [uncond | cond] noise predictions
             self.in_t = torch.zeros(2 * B, **f32)
             self.ctx = torch.zeros(2 * B, S_ctx, cfg.cross_attention_dim, **f32)
@@ -73,87 +64,42 @@ class CapturedSampler:
                 self.coef_table = torch.tensor(scheduler.plms_plan(), **f32).contiguous()       # [calls][12]
                 self.saved = torch.zeros_like(self.latents)                                        # the first call's sample
                 self.ring = torch.zeros(4, self.latents.numel(), **f32)                            # eps history
-            elif self.ancestral:
-                rows, n_noisy = scheduler.ancestral_plan(eta)
+            else:
+                rows, n_noisy = scheduler.ancestral_plan(eta)          # eta reaches only DDIM, as in diffusers' pipeline
                 self.coef_table = torch.tensor(rows, **f32).contiguous()                                   # [steps][8]
                 self.noise = torch.zeros(n_noisy, self.latents.numel(), **f32)
-            else:
-                self.coef_table = torch.tensor([scheduler._coefs(int(t)) for t in ts], **f32).contiguous()
             self.cursor = torch.zeros(2, dtype=torch.int32, device=dev)
-            self.streams = [torch.cuda.Stream(device=dev) for _ in range(L)]
-            # lane l of L > 1: half = l // (L/2) (0 = unconditional), images [j*c, (j+1)*c) of that half
-            self.engines, self._slices = [], []
-            if L == 1:
-                self.x2 = torch.zeros(2 * B, cfg.in_channels, h, w, **f32)
-                with torch.cuda.stream(self.streams[0]):
-                    self.engines.append(Engine(unet, 2 * B, h, w, S_ctx, dev, io=(self.x2, self.in_t, self.eps)))
-                self._slices.append((0, 2 * B))
-            else:
-                per, c = L // 2, B // (L // 2)
-                for l in range(L):
-                    half, j = divmod(l, per)
-                    lo = half * B + j * c
-                    io = (self.latents[j * c:(j + 1) * c], self.in_t[lo:lo + c], self.eps[lo:lo + c])
-                    # built under the lane's own stream: the split-K workspace of the GEMMs is per (device, stream)
-                    with torch.cuda.stream(self.streams[l]):
-                        self.engines.append(Engine(unet, c, h, w, S_ctx, dev, io=io))
-                    self._slices.append((lo, lo + c))
+            self.stream = torch.cuda.Stream(device=dev)
+            # built under the capture stream: the split-K workspace of the GEMMs is per (device, stream)
+            with torch.cuda.stream(self.stream):
+                self.engines = [Engine(unet, 2 * B, h, w, S_ctx, dev, io=(self.x2, self.in_t, self.eps))]
             self.graph = None
             self.host_graph = None
             self.kernels_per_step = 0
             self._ctx_key = None
 
     # -- building blocks ----------------------------------------------------------------------------
-    def _fork_join(self, fn):
-        """Run fn(lane) for every lane: lane 0 on the current stream, the others on their own streams forked from / joined
-        into it with events (inside a capture these become the graph's parallel branches)."""
-        cur = torch.cuda.current_stream()
-        if self.lanes == 1:
-            fn(0)
-            return
-        ev = torch.cuda.Event()
-        ev.record(cur)
-        done = []
-        for l in range(1, self.lanes):
-            st = self.streams[l]
-            st.wait_event(ev)
-            with torch.cuda.stream(st):
-                fn(l)
-                e = torch.cuda.Event()
-                e.record(st)
-            done.append(e)
-        fn(0)
-        for e in done:
-            cur.wait_event(e)
-
     def _project_context(self):
-        def lane(l):
-            eng = self.engines[l]
-            lo, hi = self._slices[l]
-            eng.in_ctx.copy_(self.ctx[lo:hi].reshape(-1, self.ctx.shape[-1]))
-            run_plan(eng.ctx_plan)
-        self._fork_join(lane)
+        eng = self.engines[0]
+        eng.in_ctx.copy_(self.ctx.reshape(-1, self.ctx.shape[-1]))
+        run_plan(eng.ctx_plan)
 
     def _step_ops(self):
         ops.sampler_advance(self.t_table, self.cursor, self.in_t)
-        if self.lanes == 1:
-            self.x2[:self.B].copy_(self.latents)
-            self.x2[self.B:].copy_(self.latents)
-        self._fork_join(lambda l: run_plan(self.engines[l].plan))
         B = self.B
+        self.x2[:B].copy_(self.latents)
+        self.x2[B:].copy_(self.latents)
+        run_plan(self.engines[0].plan)
         if self.plms:
             ops.cfg_plms_step_table(self.eps[:B], self.eps[B:], self.latents, self.saved, self.ring, self.guidance, self.coef_table,
                                     self.cursor)
-            return
-        if self.ancestral:
+        else:
             ops.cfg_ancestral_step_table(self.eps[:B], self.eps[B:], self.latents, self.noise, self.guidance, self.coef_table,
                                          self.cursor)
-            return
-        ops.cfg_ddim_step_table(self.eps[:B], self.eps[B:], self.latents, self.latents, self.guidance, self.coef_table, self.cursor)
 
     def _capture(self, body):
         """Warm up `body` on the capture stream (lazy one-time setup: function attributes, per-stream workspaces), then capture."""
-        s0 = self.streams[0]
+        s0 = self.stream
         s0.wait_stream(torch.cuda.current_stream())
         with torch.cuda.stream(s0):
             body()
@@ -193,8 +139,8 @@ class CapturedSampler:
             self.graph.replay()
 
     def draw_noise(self, generator=None):
-        """Fill the noise table of an ancestral sampler: one schedulers.step_noise draw per stochastic step, in step order --
-        the same numbers the per-call loop draws from the same generator."""
+        """Fill the noise table: one schedulers.step_noise draw per stochastic step, in step order -- the same numbers the
+        per-call loop draws from the same generator.  DDIM with eta = 0 draws nothing."""
         from .schedulers import step_noise
         with torch.cuda.device(self.device):
             for k in range(self.noise.shape[0]):
@@ -202,13 +148,13 @@ class CapturedSampler:
 
     @torch.no_grad()
     def run(self, latents, ctx2, generator=None):
-        """latents (B,4,h,w) ~ N(0,1) -> denoised latents after scheduler.num_inference_steps steps.  An ancestral sampler
+        """latents (B,4,h,w) ~ N(0,1) -> denoised latents after scheduler.num_inference_steps steps.  A stochastic sampler
         first draws its step noise from `generator` (draw_noise)."""
         if self.unet._stale(self._pack_gen):
             raise B200SDError("the UNet's weights changed after this sampler was built: build a new CapturedSampler")
         self.set_context(ctx2.float())
         self.set_latents(latents.float() * self.scheduler.init_noise_sigma)
-        if self.ancestral:
+        if not self.plms:
             self.draw_noise(generator)
         self.reset(0)
         for _ in range(self.n_steps):

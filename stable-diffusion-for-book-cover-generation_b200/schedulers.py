@@ -6,8 +6,8 @@
     DDPMScheduler.from_config(path, subfolder="scheduler").add_noise(...)     finetune_sd.py:335-336, 473
 
 Host side: timestep tables and per-step scalar coefficients (fp64 from the fp32 abar table).
-Device side: ONE fused kernel per step through the C ABI (b200sd_cfg_ddim_step /
-b200sd_cfg_plms_step / b200sd_cfg_ancestral_step / b200sd_add_noise).  `step_cfg` additionally fuses the pipeline's
+Device side: ONE fused kernel per step through the C ABI (b200sd_cfg_ancestral_step for DDIM and DDPM /
+b200sd_cfg_plms_step / b200sd_add_noise).  `step_cfg` additionally fuses the pipeline's
 classifier-free-guidance combine into the same kernel.
 
 Ancestral sampling (DDPMScheduler.step, DDIMScheduler.step with eta > 0) follows diffusers 0.7.2's formulas; its noise is
@@ -223,15 +223,10 @@ class DDIMScheduler(_SchedulerBase):
         ts = (np.arange(0, num_inference_steps) * ratio).round()[::-1].copy().astype(np.int64)
         self.timesteps = torch.from_numpy(ts + self.config.steps_offset)
 
-    def _coefs(self, timestep):
-        t = int(timestep)
-        prev_t = t - self.num_train_timesteps // self.num_inference_steps
-        a_t, a_p = self._ac[t], self._alpha_prev(prev_t)
-        return a_t ** 0.5, (1 - a_t) ** 0.5, a_p ** 0.5, (1 - a_p) ** 0.5
-
-    def _ancestral_coefs(self, timestep, eta):
-        """eta > 0 (diffusers 0.7.2): sigma = eta sqrt((1 - a_p) / (1 - a_t) (1 - a_t / a_p)), x' = sqrt(a_p) x0 +
-        sqrt(1 - a_p - sigma^2) eps + sigma z, with noise drawn on every step.  fp64 from the fp32 abar table."""
+    def _ancestral_coefs(self, timestep, eta=0.0):
+        """diffusers 0.7.2: sigma = eta sqrt((1 - a_p) / (1 - a_t) (1 - a_t / a_p)), x' = sqrt(a_p) x0 + sqrt(1 - a_p - sigma^2)
+        eps + sigma z, with noise drawn on every step when eta > 0.  At eta = 0 this is the deterministic DDIM update
+        sqrt(a_p) x0 + sqrt(1 - a_p) eps.  fp64 from the fp32 abar table."""
         if not 0.0 <= eta <= 1.0:
             raise ValueError(f"eta must be in [0, 1], got {eta}")
         t = int(timestep)
@@ -239,27 +234,19 @@ class DDIMScheduler(_SchedulerBase):
         a_t, a_p = self._ac[t], self._alpha_prev(prev_t)
         var = (1 - a_p) / (1 - a_t) * (1 - a_t / a_p)
         sigma = eta * var ** 0.5
-        return a_t ** 0.5, (1 - a_t) ** 0.5, a_p ** 0.5, 0.0, (1 - a_p - sigma ** 2) ** 0.5, sigma, True, False
+        return a_t ** 0.5, (1 - a_t) ** 0.5, a_p ** 0.5, 0.0, (1 - a_p - sigma ** 2) ** 0.5, sigma, eta > 0, False
 
     def step(self, model_output, timestep, sample, eta: float = 0.0, return_dict: bool = True, generator=None, **kw):
         self._check_step_args(model_output, sample)
-        if eta == 0.0:
-            prev = ops.cfg_ddim_step(model_output.contiguous(), None, sample.contiguous(), 0.0, *self._coefs(timestep))
-        else:
-            prev = self._ancestral_step(model_output.contiguous(), None, sample, 0.0, self._ancestral_coefs(timestep, eta),
-                                        generator)
+        prev = self._ancestral_step(model_output.contiguous(), None, sample, 0.0, self._ancestral_coefs(timestep, eta), generator)
         return SchedulerOutput(prev_sample=prev) if return_dict else (prev,)
 
     def step_cfg(self, model_output_2b, timestep, sample, guidance_scale, out=None, eta: float = 0.0, generator=None):
         """Fused `eps_u + s (eps_c - eps_u)` + DDIM update; model_output_2b is the (2B, ...) UNet output."""
-        self._check_step_args(model_output_2b[: sample.shape[0]], sample)
         B = sample.shape[0]
-        if eta != 0.0:
-            prev = self._ancestral_step(model_output_2b[:B], model_output_2b[B:], sample, guidance_scale,
-                                        self._ancestral_coefs(timestep, eta), generator, out=out)
-            return SchedulerOutput(prev_sample=prev)
-        prev = ops.cfg_ddim_step(model_output_2b[:B], model_output_2b[B:], sample.contiguous(), guidance_scale,
-                                 *self._coefs(timestep), out=out)
+        self._check_step_args(model_output_2b[:B], sample)
+        prev = self._ancestral_step(model_output_2b[:B], model_output_2b[B:], sample, guidance_scale,
+                                    self._ancestral_coefs(timestep, eta), generator, out=out)
         return SchedulerOutput(prev_sample=prev)
 
 
@@ -283,34 +270,47 @@ class PNDMScheduler(_SchedulerBase):
         self.timesteps = torch.from_numpy(plms.astype(np.int64))
         self.ets, self.counter, self.cur_sample = [], 0, None
 
-    def _plms(self, eps_u, eps_c, timestep, sample, guidance, out=None):
-        self._check_step_args(eps_u, sample)
+    def _plms_call(self, counter, timestep, ets):
+        """diffusers' step_plms (skip_prk_steps=True) for call number `counter` at `timestep`, given `ets`, the eps history
+        kept so far (tensors for `_plms`, ring slots for `plms_plan`).  Returns (ets, keep_eps, w, hist, cx, ce, save_x,
+        from_saved): ets trimmed to the entries later calls may read; whether this call's eps joins the history; the weights
+        of this call's eps and of the history entries `hist` (newest first); cx, ce of _get_prev_sample; whether this call's
+        sample is saved (the first call) or the saved sample is the one updated (the second call re-does the first timestep)."""
         t = int(timestep)
         ratio = self.num_train_timesteps // self.num_inference_steps
         prev_t = t - ratio
-        keep_eps = self.counter != 1
+        keep_eps = counter != 1
         if keep_eps:
-            self.ets = self.ets[-3:]
-            n_after = len(self.ets) + 1
+            ets = ets[-3:]
+            n_after = len(ets) + 1
         else:
             prev_t, t = t, t + ratio
-            n_after = len(self.ets)
-        if n_after == 1 and self.counter == 0:
-            w, hist, x = [1.0], [], sample
-            self.cur_sample = sample.clone()    # the caller may recycle its latent buffers (step_cfg(out=...))
-        elif n_after == 1 and self.counter == 1:
-            w, hist, x = [0.5, 0.5], [self.ets[-1]], self.cur_sample
-            self.cur_sample = None
+            n_after = len(ets)
+        save_x = from_saved = False
+        if n_after == 1 and counter == 0:
+            w, hist, save_x = [1.0], [], True
+        elif n_after == 1 and counter == 1:
+            w, hist, from_saved = [0.5, 0.5], [ets[-1]], True
         elif n_after == 2:
-            w, hist, x = [1.5, -0.5], [self.ets[-1]], sample
+            w, hist = [1.5, -0.5], [ets[-1]]
         elif n_after == 3:
-            w, hist, x = [23 / 12, -16 / 12, 5 / 12], [self.ets[-1], self.ets[-2]], sample
+            w, hist = [23 / 12, -16 / 12, 5 / 12], [ets[-1], ets[-2]]
         else:
-            w, hist, x = [55 / 24, -59 / 24, 37 / 24, -9 / 24], [self.ets[-1], self.ets[-2], self.ets[-3]], sample
+            w, hist = [55 / 24, -59 / 24, 37 / 24, -9 / 24], [ets[-1], ets[-2], ets[-3]]
         a_t, a_p = self._ac[t], self._alpha_prev(prev_t)
         b_t, b_p = 1 - a_t, 1 - a_p
         cx = (a_p / a_t) ** 0.5
         ce = (a_p - a_t) / (a_t * b_p ** 0.5 + (a_t * b_t * a_p) ** 0.5)
+        return ets, keep_eps, w, hist, cx, ce, save_x, from_saved
+
+    def _plms(self, eps_u, eps_c, timestep, sample, guidance, out=None):
+        self._check_step_args(eps_u, sample)
+        self.ets, keep_eps, w, hist, cx, ce, save_x, from_saved = self._plms_call(self.counter, timestep, self.ets)
+        x = sample
+        if save_x:
+            self.cur_sample = sample.clone()    # the caller may recycle its latent buffers (step_cfg(out=...))
+        elif from_saved:
+            x, self.cur_sample = self.cur_sample, None
         eps_out = torch.empty_like(eps_u) if keep_eps else None
         if eps_u.dtype == torch.float16:      # fp16 pipelines: the eps history is kept in fp32
             eps_u, eps_c = eps_u.float(), (None if eps_c is None else eps_c.float())
@@ -328,43 +328,19 @@ class PNDMScheduler(_SchedulerBase):
     def plms_plan(self):
         """The whole call sequence of one sampling run as data: one row per UNet call for b200sd_cfg_plms_step_table
         (w0 w1 w2 w3 | cx ce | ring slots of ets[-1], ets[-2], ets[-3] | slot this call's eps goes to | x_from_saved | save_x).
-        It is `_plms`'s counter logic run once on the host with a 4-slot eps ring instead of tensors, so that
+        It is `_plms_call` run once on the host with a 4-slot eps ring instead of tensors, so that
         sampler.CapturedSampler can replay every call as the same CUDA graph (the step index lives on the device)."""
         if self.num_inference_steps is None:
             raise ValueError("call set_timesteps first")
-        ratio = self.num_train_timesteps // self.num_inference_steps
         rows, ets = [], []
         for counter, timestep in enumerate(self.timesteps.tolist()):
-            t = int(timestep)
-            prev_t = t - ratio
-            keep_eps = counter != 1
-            if keep_eps:
-                ets = ets[-3:]
-                n_after = len(ets) + 1
-            else:
-                prev_t, t = t, t + ratio
-                n_after = len(ets)
-            from_saved = save_x = 0.0
-            if n_after == 1 and counter == 0:
-                w, hist, save_x = [1.0], [], 1.0
-            elif n_after == 1 and counter == 1:
-                w, hist, from_saved = [0.5, 0.5], [ets[-1]], 1.0
-            elif n_after == 2:
-                w, hist = [1.5, -0.5], [ets[-1]]
-            elif n_after == 3:
-                w, hist = [23 / 12, -16 / 12, 5 / 12], [ets[-1], ets[-2]]
-            else:
-                w, hist = [55 / 24, -59 / 24, 37 / 24, -9 / 24], [ets[-1], ets[-2], ets[-3]]
-            a_t, a_p = self._ac[t], self._alpha_prev(prev_t)
-            b_t, b_p = 1 - a_t, 1 - a_p
-            cx = (a_p / a_t) ** 0.5
-            ce = (a_p - a_t) / (a_t * b_p ** 0.5 + (a_t * b_t * a_p) ** 0.5)
+            ets, keep_eps, w, hist, cx, ce, save_x, from_saved = self._plms_call(counter, timestep, ets)
             slot = -1
             if keep_eps:
                 slot = next(k for k in range(4) if k not in ets)       # ets holds <= 3 live slots here
                 ets.append(slot)
             rows.append(w + [0.0] * (4 - len(w)) + [cx, ce] + [float(h) for h in hist] + [-1.0] * (3 - len(hist))
-                        + [float(slot), from_saved, save_x])
+                        + [float(slot), float(from_saved), float(save_x)])
         return rows
 
     def step(self, model_output, timestep, sample, return_dict: bool = True, **kw):

@@ -132,7 +132,7 @@ def test_captured_sampler_50_steps(models, kind):
         oracle.to("cpu")
     sch, _, _ = _pair(kind)
     smp = CapturedSampler(ours, sch, 1, 64, 64, 77, 7.5, eta=eta)
-    assert smp.ancestral and smp.noise.shape == (49 if kind == "ddpm" else 50, 4 * 64 * 64)
+    assert smp.noise.shape == (49 if kind == "ddpm" else 50, 4 * 64 * 64)
     got = smp.run(lat.to(DEV), ctx2.to(DEV), generator=torch.Generator().manual_seed(0)).cpu()
     cos = _cos(got, want)
     print(f"{kind}: captured vs fp32 oracle loop cosine {cos:.6f}")
@@ -154,8 +154,7 @@ def test_captured_sampler_50_steps(models, kind):
     assert smp.kernels_per_step == ref_smp.kernels_per_step > 0
 
 
-@pytest.mark.parametrize("lanes", [1, 2])
-def test_captured_ddpm_batched_portrait_tiny_net(lanes):
+def test_captured_ddpm_batched_portrait_tiny_net():
     from b200sd.sampler import CapturedSampler
     from b200sd.unet import UNet2DConditionModel
     from oracle.unet_ref import TINY_OVERRIDES, make_oracle_unet
@@ -169,10 +168,10 @@ def test_captured_ddpm_batched_portrait_tiny_net(lanes):
     sch, ref, _ = _pair("ddpm", 6)
     with torch.no_grad():
         want = A.denoise_loop(oracle, ref, lat, ctx2, 6, 7.5, generator=torch.Generator().manual_seed(5))
-    got = CapturedSampler(ours, sch, 2, 48, 32, 77, 7.5, lanes=lanes).run(lat.to(DEV), ctx2.to(DEV),
-                                                                           generator=torch.Generator().manual_seed(5)).cpu()
+    got = CapturedSampler(ours, sch, 2, 48, 32, 77, 7.5, lanes=1).run(lat.to(DEV), ctx2.to(DEV),
+                                                                       generator=torch.Generator().manual_seed(5)).cpu()
     cos = _cos(got, want)
-    assert cos >= 0.999, f"lanes={lanes}: cosine {cos:.6f}"
+    assert cos >= 0.999, f"cosine {cos:.6f}"
 
 
 # ---------------------------------------------------------------------------------------------------
@@ -219,7 +218,7 @@ def test_pipeline_ddim_eta1(tmp_path):
     ctx2 = torch.randn(4, 77, 64, generator=torch.Generator().manual_seed(4)).to(DEV)
     out = pipe(prompt_embeds=ctx2, height=256, width=256, num_inference_steps=6, guidance_scale=7.5, eta=1.0,
                generator=torch.Generator("cuda").manual_seed(0), output_type="latent")
-    assert any(smp.ancestral for smp in pipe.unet._samplers.values())
+    assert any(smp.noise.shape[0] > 0 for smp in pipe.unet._samplers.values())
     want = _per_call(pipe.unet, DDIMScheduler(**_DDIM_KW), ctx2, torch.Generator("cuda").manual_seed(0), eta=1.0)
     cos = _cos(out.images, want)
     assert cos >= 0.9999, cos

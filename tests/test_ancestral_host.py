@@ -93,6 +93,33 @@ def test_ddim_eta_rows_match_oracle(eta, set_alpha_to_one):
         assert noise_row == k and clip_flag == 0.0
 
 
+@pytest.mark.parametrize("n", [50, 1000])
+@pytest.mark.parametrize("set_alpha_to_one", [True, False])
+def test_ddim_eta0_rows_are_the_deterministic_ddim_update(n, set_alpha_to_one):
+    """At eta = 0 the affine row is DDIM's update, sqrt(a_p) x0 + sqrt(1 - a_p) eps, with no x term, no noise and no clipping:
+    sa_t, sb_t, c_x0, c_e equal sa_t, sb_t, sa_p, sb_p of DDIM's closed form below (what b200sd_cfg_ddim_step takes), exactly
+    in fp64 and after rounding to the fp32 the kernel receives."""
+    from b200sd.schedulers import DDIMScheduler
+    ours = DDIMScheduler(**_KW, clip_sample=False, set_alpha_to_one=set_alpha_to_one)
+    ours.set_timesteps(n)
+
+    def ddim_coefs(t):
+        prev_t = t - ours.num_train_timesteps // ours.num_inference_steps
+        a_t, a_p = ours._ac[t], ours._ac[prev_t] if prev_t >= 0 else ours._final_alpha
+        return a_t ** 0.5, (1 - a_t) ** 0.5, a_p ** 0.5, (1 - a_p) ** 0.5
+
+    rows, n_noisy = ours.ancestral_plan(0.0)
+    assert n_noisy == 0 and len(rows) == n
+    for row, t in zip(rows, ours.timesteps.tolist()):
+        sa_t, sb_t, c_x0, c_x, c_e, c_z, noisy, clip = ours._ancestral_coefs(t, 0.0)
+        assert c_x == 0.0 and c_z == 0.0 and not noisy and not clip
+        want = ddim_coefs(t)
+        assert (sa_t, sb_t, c_x0, c_e) == want
+        f32 = lambda v: torch.tensor(v, dtype=torch.float32).tolist()
+        assert f32([sa_t, sb_t, c_x0, c_e]) == f32(list(want))
+        assert f32(row) == f32([*want[:3], 0.0, want[3], 0.0, -1.0, 0.0])
+
+
 def test_ddim_eta_out_of_range_raises():
     from b200sd.schedulers import DDIMScheduler
     s = DDIMScheduler(**_KW, clip_sample=False, set_alpha_to_one=False)

@@ -274,7 +274,7 @@ def test_context_cache_is_not_fooled_by_address_reuse(models):
 
 
 # ---------------------------------------------------------------------------------------------------
-# CapturedSampler: the whole denoising step as one CUDA graph, CFG halves on concurrent lanes
+# CapturedSampler: the whole denoising step as one CUDA graph
 # ---------------------------------------------------------------------------------------------------
 _DDIM_KW = dict(beta_start=0.00085, beta_end=0.012, beta_schedule="scaled_linear", clip_sample=False, set_alpha_to_one=False)
 
@@ -295,20 +295,19 @@ def oracle_50_step(models):
     return lat, ctx2, want.cpu()
 
 
-@pytest.mark.parametrize("lanes", [1, 2])
-def test_captured_sampler_50_steps_vs_oracle(models, oracle_50_step, lanes):
+def test_captured_sampler_50_steps_vs_oracle(models, oracle_50_step):
     """BASELINE config 2 through the one-graph-per-step sampler (what bench.py times): 50-step latents cosine >= 0.999 vs the
-    fp32 oracle loop, with the two CFG halves on one lane and on two concurrent lanes."""
+    fp32 oracle loop."""
     from b200sd.sampler import CapturedSampler
     from b200sd.schedulers import DDIMScheduler
     _oracle, ours = models
     lat, ctx2, want = oracle_50_step
     sch = DDIMScheduler(**_DDIM_KW)
     sch.set_timesteps(50)
-    smp = CapturedSampler(ours, sch, 1, 64, 64, 77, 7.5, lanes=lanes)
+    smp = CapturedSampler(ours, sch, 1, 64, 64, 77, 7.5, lanes=1)
     got = smp.run(lat.to(DEV), ctx2.to(DEV)).cpu()
     cos = float(torch.nn.functional.cosine_similarity(got.flatten(), want.flatten(), dim=0))
-    assert cos >= 0.999, f"lanes={lanes}: 50-step latents cosine {cos:.6f}"
+    assert cos >= 0.999, f"50-step latents cosine {cos:.6f}"
     # the same sampler object again, other latents first: no state leaks between runs (cursor, context K/V, latents)
     smp.run(torch.randn(1, 4, 64, 64).to(DEV), ctx2.flip(0).to(DEV))
     again = smp.run(lat.to(DEV), ctx2.to(DEV)).cpu()
@@ -375,10 +374,8 @@ def test_captured_sampler_refuses_stale_weights(models):
             w.sub_(1.0)
 
 
-@pytest.mark.parametrize("lanes", [1, 2, 4])
-def test_captured_sampler_batched_portrait_tiny_net(lanes):
-    """2 images (UNet batch 4) at a portrait geometry on the reduced-width network: lanes 1 / 2 / 4 (sub-batches of one CFG
-    half) all reproduce the oracle loop."""
+def test_captured_sampler_batched_portrait_tiny_net():
+    """2 images (UNet batch 4) at a portrait geometry on the reduced-width network reproduce the oracle loop."""
     from b200sd.sampler import CapturedSampler
     from b200sd.schedulers import DDIMScheduler
     from b200sd.unet import UNet2DConditionModel
@@ -395,9 +392,11 @@ def test_captured_sampler_batched_portrait_tiny_net(lanes):
         want = R.denoise_loop(oracle, R.DDIMSchedulerRef(clip_sample=False, set_alpha_to_one=False), lat, ctx2, 6, 7.5)
     sch = DDIMScheduler(**_DDIM_KW)
     sch.set_timesteps(6)
-    got = CapturedSampler(ours, sch, 2, 48, 32, 77, 7.5, lanes=lanes).run(lat.to(DEV), ctx2.to(DEV)).cpu()
+    got = CapturedSampler(ours, sch, 2, 48, 32, 77, 7.5, lanes=1).run(lat.to(DEV), ctx2.to(DEV)).cpu()
     cos = float(torch.nn.functional.cosine_similarity(got.flatten(), want.flatten(), dim=0))
-    assert cos >= 0.999, f"lanes={lanes}: cosine {cos:.6f}"
+    assert cos >= 0.999, f"cosine {cos:.6f}"
+    with pytest.raises(ValueError, match="lanes=2"):
+        CapturedSampler(ours, sch, 2, 48, 32, 77, 7.5, lanes=2)
 
 
 def test_captured_sampler_plms_51_calls_vs_oracle_and_per_call_loop(models):

@@ -61,7 +61,7 @@ def step_times(unet, B, steps, repeats):
             for name, smp in smps.items():
                 smp.set_context(ctx2)
                 smp.set_latents(lat)
-                if smp.ancestral:
+                if smp.noise.shape[0]:
                     smp.draw_noise(torch.Generator(DEV).manual_seed(0))
                 smp.reset(0)
                 torch.cuda.synchronize()
