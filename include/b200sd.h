@@ -116,6 +116,20 @@ int b200sd_add_noise(const void* x0, const void* noise, const int64_t* timesteps
                      const float* sb_table, void* out, int batch, int64_t per_sample, int num_train_timesteps,
                      int dtype, b200sd_stream_t stream);
 
+/* The masking step of legacy inpainting (diffusers 0.7.2 StableDiffusionInpaintPipelineLegacy), run after every scheduler step
+ * at loop timestep t, fp32 and in place:
+ *   x = m (sa[t] x0 + sb[t] noise) + (1 - m) x
+ * x, x0 (the init latents before noising), noise (the init noise) and m (1 = keep, not binarised) all have n elements: the
+ * host expands the mask to the latents' shape.  sa_table / sb_table: float[num_train_timesteps], the tables of
+ * b200sd_add_noise; t is clamped to [0, num_train_timesteps).  Algorithmic bytes: 5 * n * 4 (x, x0, noise, m read; x written).
+ * b200sd_inpaint_blend takes t by value; b200sd_inpaint_blend_table (the captured sampler) reads t = t_table[cursor[1]] on the
+ * device, the timestep table and cursor of b200sd_sampler_advance. */
+int b200sd_inpaint_blend(float* x, const float* x0, const float* noise, const float* mask, int64_t n, int64_t timestep,
+                         const float* sa_table, const float* sb_table, int num_train_timesteps, b200sd_stream_t stream);
+int b200sd_inpaint_blend_table(float* x, const float* x0, const float* noise, const float* mask, int64_t n,
+                               const float* t_table, const int* cursor, const float* sa_table, const float* sb_table,
+                               int num_train_timesteps, b200sd_stream_t stream);
+
 /* F.mse_loss(pred, target, "none").mean([1,2,3]).mean() (finetune_sd.py:483-484) == global mean.
  * loss_out: float[1]; workspace: float[b200sd_mse_workspace_floats()]. */
 int b200sd_mse_workspace_floats(void);

@@ -1,7 +1,8 @@
 """b200sd -- B200-native (sm_100a) SD v1.x UNet denoise hot path behind the diffusers class surface.
 
 Public surface (mirrors what finetune_sd.py / inference.py / StableDiffusionPipeline touch):
-    UNet2DConditionModel, DDIMScheduler, PNDMScheduler, DDPMScheduler, StableDiffusionPipeline, denoise_loop, mse_loss,
+    UNet2DConditionModel, DDIMScheduler, PNDMScheduler, DDPMScheduler, StableDiffusionPipeline,
+    StableDiffusionImg2ImgPipeline, StableDiffusionInpaintPipelineLegacy (image-to-image, legacy inpainting), denoise_loop, mse_loss,
     CapturedSampler (the whole denoising step as one CUDA graph), CLIPTextModel (transformers' surface, own kernels),
     AutoencoderKL (diffusers' surface, own kernels)
 """
@@ -17,6 +18,8 @@ def __getattr__(name):  # lazy: importing the package must not require torch.cud
         "DDPMScheduler": "b200sd.schedulers",
         "denoise_loop": "b200sd.pipeline",
         "StableDiffusionPipeline": "b200sd.pipeline",
+        "StableDiffusionImg2ImgPipeline": "b200sd.pipeline",
+        "StableDiffusionInpaintPipelineLegacy": "b200sd.pipeline",
         "mse_loss": "b200sd.ops",
         "CapturedSampler": "b200sd.sampler",
         "CLIPTextModel": "b200sd.clip",

@@ -75,6 +75,8 @@ SIGNATURES = {
     "b200sd_cfg_plms_step": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, C.POINTER(C.c_float), _i64, _f, _f,
                                   _f, _i, _i, _vp]),
     "b200sd_add_noise": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i, _i64, _i, _i, _vp]),
+    "b200sd_inpaint_blend": (_i, [_vp, _vp, _vp, _vp, _i64, _i64, _vp, _vp, _i, _vp]),
+    "b200sd_inpaint_blend_table": (_i, [_vp, _vp, _vp, _vp, _i64, _vp, _vp, _vp, _vp, _i, _vp]),
     "b200sd_mse_workspace_floats": (_i, []),
     "b200sd_mse_loss_fwd": (_i, [_vp, _vp, _vp, _vp, _i64, _i, _i, _vp]),
     "b200sd_mse_loss_bwd": (_i, [_vp, _vp, _vp, _vp, _i64, _i, _i, _vp]),

@@ -490,6 +490,66 @@ extern "C" int b200sd_add_noise(const void* x0, const void* noise, const int64_t
     return B200SD_OK;
 }
 
+// Legacy inpainting (diffusers 0.7.2 StableDiffusionInpaintPipelineLegacy), after every scheduler step at loop timestep t:
+//   x <- m (sa[t] x0 + sb[t] z) + (1 - m) x
+// i.e. the kept region is re-noised from the original latents with the same noise every step.  m, x0, z have x's full shape
+// (the host expands the mask).  The timestep comes by value or, in the captured sampler, from t_table[cursor[1]].
+namespace {
+__global__ void __launch_bounds__(kThreads) inpaint_blend_kernel(float* x, const float* __restrict__ x0,
+                                                                 const float* __restrict__ z, const float* __restrict__ m,
+                                                                 const float* __restrict__ sa_table,
+                                                                 const float* __restrict__ sb_table, int T, int64_t t,
+                                                                 const float* __restrict__ t_table,
+                                                                 const int* __restrict__ cursor, int64_t n, int64_t nvec) {
+    if (t_table != nullptr) t = (int64_t)t_table[cursor[1]];
+    t = t < 0 ? 0 : (t >= T ? T - 1 : t);
+    const float sa = __ldg(sa_table + t), sb = __ldg(sb_table + t);
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < nvec; i += stride) {
+        float xv[8], a[8], e[8], mv[8], o[8];
+        load8<B200SD_F32>(x, i * 8, xv);
+        load8<B200SD_F32>(x0, i * 8, a);
+        load8<B200SD_F32>(z, i * 8, e);
+        load8<B200SD_F32>(m, i * 8, mv);
+#pragma unroll
+        for (int j = 0; j < 8; ++j) o[j] = mv[j] * (sa * a[j] + sb * e[j]) + (1.f - mv[j]) * xv[j];
+        store8<B200SD_F32>(x, i * 8, o);
+    }
+    for (int64_t i = nvec * 8 + (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride)
+        x[i] = m[i] * (sa * x0[i] + sb * z[i]) + (1.f - m[i]) * x[i];
+}
+
+int inpaint_blend_launch(float* x, const float* x0, const float* noise, const float* mask, int64_t n, int64_t timestep,
+                         const float* t_table, const int* cursor, const float* sa_table, const float* sb_table,
+                         int num_train_timesteps, b200sd_stream_t stream) {
+    B200SD_REQUIRE(x && x0 && noise && mask && sa_table && sb_table, "inpaint_blend: null pointer");
+    B200SD_REQUIRE(n >= 0 && num_train_timesteps > 0, "inpaint_blend: bad sizes");
+    const bool vec = aligned16(x) && aligned16(x0) && aligned16(noise) && aligned16(mask);
+    const int64_t nvec = vec ? n / 8 : 0;
+    if (n == 0) return B200SD_OK;
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    inpaint_blend_kernel<<<dim3(grid_for(vec ? n / 8 : n)), dim3(kThreads), 0, s>>>(
+        x, x0, noise, mask, sa_table, sb_table, num_train_timesteps, timestep, t_table, cursor, n, nvec);
+    COUNT_LAUNCH();
+    B200SD_LAUNCH_CHECK();
+    return B200SD_OK;
+}
+}  // namespace
+
+extern "C" int b200sd_inpaint_blend(float* x, const float* x0, const float* noise, const float* mask, int64_t n,
+                                    int64_t timestep, const float* sa_table, const float* sb_table, int num_train_timesteps,
+                                    b200sd_stream_t stream) {
+    return inpaint_blend_launch(x, x0, noise, mask, n, timestep, nullptr, nullptr, sa_table, sb_table, num_train_timesteps,
+                                stream);
+}
+
+extern "C" int b200sd_inpaint_blend_table(float* x, const float* x0, const float* noise, const float* mask, int64_t n,
+                                          const float* t_table, const int* cursor, const float* sa_table, const float* sb_table,
+                                          int num_train_timesteps, b200sd_stream_t stream) {
+    B200SD_REQUIRE(t_table && cursor, "inpaint_blend_table: null pointer");
+    return inpaint_blend_launch(x, x0, noise, mask, n, 0, t_table, cursor, sa_table, sb_table, num_train_timesteps, stream);
+}
+
 extern "C" int b200sd_mse_workspace_floats(void) { return kMsePartials + 4; }
 
 extern "C" int b200sd_mse_loss_fwd(const void* pred, const void* target, float* loss_out, float* workspace,

@@ -178,6 +178,32 @@ def add_noise(x0, noise, timesteps, sa_table, sb_table, out=None):
     return out
 
 
+def _blend_args(x, x0, noise, mask, sa_table, sb_table):
+    _chk(x, x0, noise, mask, sa_table, sb_table)
+    for t in (x, x0, noise, mask, sa_table, sb_table):
+        if t.dtype != torch.float32:
+            raise B200SDError("inpaint_blend is fp32")
+    if not x.shape == x0.shape == noise.shape == mask.shape:
+        raise ValueError("inpaint_blend: x, x0, noise and mask must have the same shape (expand the mask first)")
+    return _p(x), _p(x0), _p(noise), _p(mask), x.numel()
+
+
+def inpaint_blend(x, x0, noise, mask, timestep, sa_table, sb_table):
+    """x <- mask (sa[t] x0 + sb[t] noise) + (1 - mask) x in place (legacy inpainting's masking step at loop timestep t)"""
+    args = _blend_args(x, x0, noise, mask, sa_table, sb_table)
+    check(lib().b200sd_inpaint_blend(*args, int(timestep), _p(sa_table), _p(sb_table), sa_table.numel(), _stream()),
+          "inpaint_blend")
+    return x
+
+
+def inpaint_blend_table(x, x0, noise, mask, t_table, cursor, sa_table, sb_table):
+    """inpaint_blend() at t = t_table[cursor[1]], read on the device (the captured sampler's step)"""
+    args = _blend_args(x, x0, noise, mask, sa_table, sb_table)
+    check(lib().b200sd_inpaint_blend_table(*args, _p(t_table), _p(cursor), _p(sa_table), _p(sb_table), sa_table.numel(),
+                                           _stream()), "inpaint_blend_table")
+    return x
+
+
 def mse_loss_fwd(pred, target):
     _chk(pred, target)
     if pred.shape != target.shape:

@@ -15,6 +15,11 @@ What the graph holds (nothing is launched eagerly between two steps, the host on
                                latents, 2.1 GB for 1000 DDPM steps at batch 32.
     (PNDMScheduler / PLMS: cfg_plms_step_table -- weights, eps-ring slots and the saved-sample flags of this call = table[cursor];
      the 4-deep eps history is a device ring, PNDM's repeated first timestep reads the sample saved by the first call)
+    inpaint_blend_table        inpaint mode only: latents <- m (sa[t] x0 + sb[t] z) + (1 - m) latents at t = timesteps[cursor],
+                               the masking step of legacy inpainting; x0, z and m are buffers `run(blend=...)` fills
+
+A run that starts partway through the schedule (img2img, inpainting: `start` = t_start) holds only the executed steps in its
+timestep, coefficient and noise tables, so its graph is launch for launch the text-to-image graph.
 
 `host_step()` is the same graph with the host on both ends: H2D memcpy nodes for the latents and the text context out of
 pinned host buffers, the context K/V projections (the context may change every call), the step, and a D2H memcpy node of
@@ -31,7 +36,8 @@ from .plan import run_plan
 
 
 class CapturedSampler:
-    def __init__(self, unet, scheduler, batch_images, h, w, S_ctx=77, guidance_scale=7.5, lanes=None, eta=0.0):
+    def __init__(self, unet, scheduler, batch_images, h, w, S_ctx=77, guidance_scale=7.5, lanes=None, eta=0.0, start=0,
+                 inpaint=False):
         from .schedulers import DDIMScheduler, DDPMScheduler, PNDMScheduler
         if not isinstance(scheduler, (DDIMScheduler, PNDMScheduler, DDPMScheduler)):
             raise B200SDError("CapturedSampler covers DDIMScheduler, PNDMScheduler (PLMS) and DDPMScheduler")
@@ -57,17 +63,23 @@ class CapturedSampler:
             self.eps = torch.zeros(2 * B, cfg.out_channels, h, w, **f32)       # [uncond | cond] noise predictions
             self.in_t = torch.zeros(2 * B, **f32)
             self.ctx = torch.zeros(2 * B, S_ctx, cfg.cross_attention_dim, **f32)
-            ts = [float(t) for t in scheduler.timesteps.tolist()]
+            ts = [float(t) for t in scheduler.timesteps.tolist()[start:]]
+            if not ts:
+                raise ValueError(f"start={start} leaves no step of the {len(scheduler.timesteps)}-step schedule")
             self.n_steps = len(ts)
             self.t_table = torch.tensor(ts, **f32)
             if self.plms:
-                self.coef_table = torch.tensor(scheduler.plms_plan(), **f32).contiguous()       # [calls][12]
+                self.coef_table = torch.tensor(scheduler.plms_plan(start), **f32).contiguous()  # [calls][12]
                 self.saved = torch.zeros_like(self.latents)                                        # the first call's sample
                 self.ring = torch.zeros(4, self.latents.numel(), **f32)                            # eps history
             else:
-                rows, n_noisy = scheduler.ancestral_plan(eta)          # eta reaches only DDIM, as in diffusers' pipeline
+                rows, n_noisy = scheduler.ancestral_plan(eta, start)   # eta reaches only DDIM, as in diffusers' pipeline
                 self.coef_table = torch.tensor(rows, **f32).contiguous()                                   # [steps][8]
                 self.noise = torch.zeros(n_noisy, self.latents.numel(), **f32)
+            self.inpaint = bool(inpaint)
+            if self.inpaint:         # the init latents before noising, the init noise and the keep-mask, latents-shaped
+                self.init_orig, self.blend_noise, self.mask = (torch.zeros_like(self.latents) for _ in range(3))
+                self.noise_tables = scheduler._noise_tables(dev)
             self.cursor = torch.zeros(2, dtype=torch.int32, device=dev)
             self.stream = torch.cuda.Stream(device=dev)
             # built under the capture stream: the split-K workspace of the GEMMs is per (device, stream)
@@ -96,6 +108,9 @@ class CapturedSampler:
         else:
             ops.cfg_ancestral_step_table(self.eps[:B], self.eps[B:], self.latents, self.noise, self.guidance, self.coef_table,
                                          self.cursor)
+        if self.inpaint:
+            ops.inpaint_blend_table(self.latents, self.init_orig, self.blend_noise, self.mask, self.t_table, self.cursor,
+                                    *self.noise_tables)
 
     def _capture(self, body):
         """Warm up `body` on the capture stream (lazy one-time setup: function attributes, per-stream workspaces), then capture."""
@@ -115,7 +130,7 @@ class CapturedSampler:
 
     # -- public surface -----------------------------------------------------------------------------
     def reset(self, step=0):
-        """the next step() executes scheduler.timesteps[step]"""
+        """the next step() executes scheduler.timesteps[start + step]"""
         self.cursor.copy_(torch.tensor([step % self.n_steps, 0], dtype=torch.int32))
 
     def set_context(self, ctx2):
@@ -146,12 +161,24 @@ class CapturedSampler:
             for k in range(self.noise.shape[0]):
                 step_noise(self.latents, generator, out=self.noise[k].view(self.latents.shape))
 
+    def set_blend(self, init_orig, noise, mask):
+        """inpaint mode: the init latents before noising, the init noise (both (B,4,h,w)) and the keep-mask (broadcastable to
+        them; 1 = keep) that every step's blend reads"""
+        if not self.inpaint:
+            raise ValueError("this sampler was built without inpaint=True")
+        for buf, t in ((self.init_orig, init_orig), (self.blend_noise, noise), (self.mask, mask)):
+            buf.copy_(t.float().expand_as(buf))
+
     @torch.no_grad()
-    def run(self, latents, ctx2, generator=None):
-        """latents (B,4,h,w) ~ N(0,1) -> denoised latents after scheduler.num_inference_steps steps.  A stochastic sampler
-        first draws its step noise from `generator` (draw_noise)."""
+    def run(self, latents, ctx2, generator=None, blend=None):
+        """latents (B,4,h,w) -> denoised latents after the steps timesteps[start:].  A stochastic sampler first draws its step
+        noise from `generator` (draw_noise).  An inpainting sampler needs blend=(init_orig, noise, mask) (set_blend)."""
         if self.unet._stale(self._pack_gen):
             raise B200SDError("the UNet's weights changed after this sampler was built: build a new CapturedSampler")
+        if (blend is not None) != self.inpaint:
+            raise ValueError("blend=(init_orig, noise, mask) is required in inpaint mode and only there")
+        if blend is not None:
+            self.set_blend(*blend)
         self.set_context(ctx2.float())
         self.set_latents(latents.float() * self.scheduler.init_noise_sigma)
         if not self.plms:

@@ -124,14 +124,26 @@ class _SchedulerBase:
         return ops.cfg_ancestral_step(eps_u, eps_c, sample.contiguous(), z, guidance, sa_t, sb_t, c_x0, c_x, c_e, c_z, clip,
                                       out=out)
 
-    def ancestral_plan(self, eta=0.0):
-        """One row per timestep for b200sd_cfg_ancestral_step_table: sa_t sb_t c_x0 c_x c_e c_z noise_row clip, where
-        noise_row counts the steps that add noise (the order step_noise draws them in) and is -1 on a step that adds none.
-        Returns (rows, number of noise rows)."""
+    def img2img_start(self, num_inference_steps, strength):
+        """set_timesteps(n), then where diffusers 0.7.2's img2img / legacy inpainting pipelines enter the schedule for `strength`:
+        (t_start, t_noise).  The loop runs over timesteps[t_start:] (possibly empty) and the init latents are noised to
+        t_noise = timesteps[-init_timestep] -- timesteps[0] when init_timestep is 0, as in 0.7.2."""
+        if not 0 <= strength <= 1:
+            raise ValueError(f"The value of strength should in [0.0, 1.0] but is {strength}")
+        self.set_timesteps(num_inference_steps)
+        offset = getattr(self.config, "steps_offset", 0)
+        init_timestep = min(int(num_inference_steps * strength) + offset, num_inference_steps)
+        t_noise = int(self.timesteps[-init_timestep])
+        return max(num_inference_steps - init_timestep + offset, 0), t_noise
+
+    def ancestral_plan(self, eta=0.0, start=0):
+        """One row per timestep of timesteps[start:] for b200sd_cfg_ancestral_step_table: sa_t sb_t c_x0 c_x c_e c_z noise_row
+        clip, where noise_row counts the executed steps that add noise (the order step_noise draws them in) and is -1 on a step
+        that adds none.  Returns (rows, number of noise rows)."""
         if self.num_inference_steps is None:
             raise ValueError("call set_timesteps first")
         rows, k = [], 0
-        for t in self.timesteps.tolist():
+        for t in self.timesteps.tolist()[start:]:
             sa_t, sb_t, c_x0, c_x, c_e, c_z, noisy, clip = self._ancestral_coefs(t, eta)
             rows.append([sa_t, sb_t, c_x0, c_x, c_e, c_z, float(k if noisy else -1), float(clip)])
             k += noisy
@@ -325,15 +337,16 @@ class PNDMScheduler(_SchedulerBase):
         self.counter += 1
         return SchedulerOutput(prev_sample=prev)
 
-    def plms_plan(self):
-        """The whole call sequence of one sampling run as data: one row per UNet call for b200sd_cfg_plms_step_table
-        (w0 w1 w2 w3 | cx ce | ring slots of ets[-1], ets[-2], ets[-3] | slot this call's eps goes to | x_from_saved | save_x).
-        It is `_plms_call` run once on the host with a 4-slot eps ring instead of tensors, so that
-        sampler.CapturedSampler can replay every call as the same CUDA graph (the step index lives on the device)."""
+    def plms_plan(self, start=0):
+        """The whole call sequence of one sampling run over timesteps[start:] as data: one row per UNet call for
+        b200sd_cfg_plms_step_table (w0 w1 w2 w3 | cx ce | ring slots of ets[-1], ets[-2], ets[-3] | slot this call's eps goes to |
+        x_from_saved | save_x).  It is `_plms_call` run once on the host with a 4-slot eps ring instead of tensors, so that
+        sampler.CapturedSampler can replay every call as the same CUDA graph (the step index lives on the device).  The call
+        counter starts at 0 on timesteps[start], as the per-call loop's does after set_timesteps."""
         if self.num_inference_steps is None:
             raise ValueError("call set_timesteps first")
         rows, ets = [], []
-        for counter, timestep in enumerate(self.timesteps.tolist()):
+        for counter, timestep in enumerate(self.timesteps.tolist()[start:]):
             ets, keep_eps, w, hist, cx, ce, save_x, from_saved = self._plms_call(counter, timestep, ets)
             slot = -1
             if keep_eps:

@@ -62,8 +62,11 @@ class DiagonalGaussianDistribution:
         return torch.exp(self.logvar)
 
     def sample(self, generator=None):
+        """mean + std * noise, the noise drawn on the generator's device (the moments' when there is none), as the pipelines
+        draw their latents"""
         p = self.parameters
-        noise = torch.randn(self.mean.shape, generator=generator, device=p.device, dtype=torch.float32)
+        dev = p.device if generator is None else generator.device
+        noise = torch.randn(self.mean.shape, generator=generator, device=dev, dtype=torch.float32).to(p.device)
         out = torch.empty_like(noise)
         ops.gaussian_sample(p.float().contiguous(), noise, out)
         return out.to(p.dtype)
