@@ -130,6 +130,32 @@ int b200sd_inpaint_blend_table(float* x, const float* x0, const float* noise, co
                                const float* t_table, const int* cursor, const float* sa_table, const float* sb_table,
                                int num_train_timesteps, b200sd_stream_t stream);
 
+/* CFG combine fused with the step of diffusers 0.7.2's sigma-space schedulers (LMSDiscreteScheduler, EulerDiscreteScheduler,
+ * EulerAncestralDiscreteScheduler), in 0.7.2's order of operations, every operation separately rounded (no FMA contraction):
+ *   eps = eps_u + g (eps_c - eps_u);  x0 = x - sigma eps;  d = (x - x0) / sigma
+ *   out = x + (((c0 d + c1 hist1) + c2 hist2) + c3 hist3)  (+ sigma_up noise)
+ * Euler: c0 = sigma_next - sigma.  Euler-a: c0 = sigma_down - sigma, noise = the step's N(0, 1) draw.  LMS: the linear-multistep
+ * coefficients, hist1..3 = the derivatives of the previous steps, newest first.  A NULL hist term or noise is left out.
+ * d_out (optional) receives d.  eps_dtype: B200SD_F32 or B200SD_BF16; x, noise, hist, out and d_out are fp32.  out may alias x.
+ * Algorithmic bytes: (4 + number of non-NULL of eps_c, noise, hist1..3, d_out) * n * 4 in fp32. */
+int b200sd_cfg_sigma_step(const void* eps_u, const void* eps_c, const float* x, const float* noise, float* out, float* d_out,
+                          const float* hist1, const float* hist2, const float* hist3, int64_t n, float guidance, float sigma,
+                          float c0, float c1, float c2, float c3, float sigma_up, int eps_dtype, b200sd_stream_t stream);
+
+/* The captured-sampler form of b200sd_cfg_sigma_step (fp32; x is updated in place).  Per step one row of 12 floats of `table`
+ * (16-byte aligned), indexed by cursor[1]: sigma | c0 c1 c2 c3 | h1 h2 h3 (ring slots of the history terms; -1 = unused) |
+ * out_slot (ring slot d is written to; -1 = not kept) | noise_row (-1 = none) | sigma_up | in_div.  `ring` is [4][n] floats
+ * (the LMS derivative history; may be NULL when no row names a slot), `noise` [n_noise_rows][n] floats filled by the host
+ * before the run (may be NULL when no row names a noise row). */
+int b200sd_cfg_sigma_step_table(const float* eps_u, const float* eps_c, float* x, float* ring, const float* noise, int64_t n,
+                                float guidance, const float* table, const int* cursor, b200sd_stream_t stream);
+
+/* The UNet input of a sigma-space captured step: x2[0..n) = x2[n..2n) = x / in_div with in_div = table[cursor[1]].in_div
+ * (column 11 of the b200sd_cfg_sigma_step_table row), i.e. scheduler.scale_model_input(cat([x, x]), t).  A true division, bit
+ * for bit what torch computes for a tensor divided by a tensor. */
+int b200sd_sampler_scale_input(const float* x, float* x2, int64_t n, const float* table, const int* cursor,
+                               b200sd_stream_t stream);
+
 /* F.mse_loss(pred, target, "none").mean([1,2,3]).mean() (finetune_sd.py:483-484) == global mean.
  * loss_out: float[1]; workspace: float[b200sd_mse_workspace_floats()]. */
 int b200sd_mse_workspace_floats(void);

@@ -1,7 +1,8 @@
 """b200sd -- B200-native (sm_100a) SD v1.x UNet denoise hot path behind the diffusers class surface.
 
 Public surface (mirrors what finetune_sd.py / inference.py / StableDiffusionPipeline touch):
-    UNet2DConditionModel, DDIMScheduler, PNDMScheduler, DDPMScheduler, StableDiffusionPipeline,
+    UNet2DConditionModel, DDIMScheduler, PNDMScheduler, DDPMScheduler, LMSDiscreteScheduler, EulerDiscreteScheduler,
+    EulerAncestralDiscreteScheduler, StableDiffusionPipeline,
     StableDiffusionImg2ImgPipeline, StableDiffusionInpaintPipelineLegacy (image-to-image, legacy inpainting), denoise_loop, mse_loss,
     CapturedSampler (the whole denoising step as one CUDA graph), CLIPTextModel (transformers' surface, own kernels),
     AutoencoderKL (diffusers' surface, own kernels)
@@ -16,6 +17,9 @@ def __getattr__(name):  # lazy: importing the package must not require torch.cud
         "DDIMScheduler": "b200sd.schedulers",
         "PNDMScheduler": "b200sd.schedulers",
         "DDPMScheduler": "b200sd.schedulers",
+        "LMSDiscreteScheduler": "b200sd.schedulers",
+        "EulerDiscreteScheduler": "b200sd.schedulers",
+        "EulerAncestralDiscreteScheduler": "b200sd.schedulers",
         "denoise_loop": "b200sd.pipeline",
         "StableDiffusionPipeline": "b200sd.pipeline",
         "StableDiffusionImg2ImgPipeline": "b200sd.pipeline",

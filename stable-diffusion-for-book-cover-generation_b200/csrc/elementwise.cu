@@ -550,6 +550,163 @@ extern "C" int b200sd_inpaint_blend_table(float* x, const float* x0, const float
     return inpaint_blend_launch(x, x0, noise, mask, n, 0, t_table, cursor, sa_table, sb_table, num_train_timesteps, stream);
 }
 
+// The sigma-space schedulers of diffusers 0.7.2 (LMSDiscreteScheduler, EulerDiscreteScheduler, EulerAncestralDiscreteScheduler),
+// with the CFG combine, in 0.7.2's own order of operations:
+//   e = eps_u + g (eps_c - eps_u);  x0 = x - sigma e;  d = (x - x0) / sigma
+//   out = x + (((c0 d + c1 d[-1]) + c2 d[-2]) + c3 d[-3])  (+ sigma_up z)
+// Every product, sum and the quotient is a separately rounded __f*_rn so that nvcc cannot contract them into FMAs torch does
+// not do, and d is not simplified to e.  Euler: c0 = sigma_next - sigma.  Euler-a: c0 = sigma_down - sigma plus the noise
+// term.  LMS: up to 4 terms over the derivative history, which the captured sampler keeps in a 4-slot device ring.
+// Table row (12 floats): sigma | c0 c1 c2 c3 | h1 h2 h3 (ring slots of d[-1], d[-2], d[-3]; -1 = unused) | out_slot (ring slot
+// this step's d goes to, -1 = not kept) | noise_row (-1 = none) | sigma_up | in_div (the model-input divisor (sigma^2 + 1)^0.5).
+namespace {
+constexpr int kSigmaRow = 12;
+
+struct SigmaCoef {
+    float g, sigma, c0, c1, c2, c3, sigma_up;
+};
+
+__device__ __forceinline__ float sigma_one(float eu, float ec, float x, float z, float h1, float h2, float h3, bool cfg,
+                                           bool has_h1, bool has_h2, bool has_h3, bool has_z, const SigmaCoef& c, float& d) {
+    const float e = cfg ? __fadd_rn(eu, __fmul_rn(c.g, __fsub_rn(ec, eu))) : eu;
+    const float x0 = __fsub_rn(x, __fmul_rn(c.sigma, e));
+    d = __fdiv_rn(__fsub_rn(x, x0), c.sigma);
+    float acc = __fmul_rn(c.c0, d);
+    if (has_h1) acc = __fadd_rn(acc, __fmul_rn(c.c1, h1));
+    if (has_h2) acc = __fadd_rn(acc, __fmul_rn(c.c2, h2));
+    if (has_h3) acc = __fadd_rn(acc, __fmul_rn(c.c3, h3));
+    const float out = __fadd_rn(x, acc);
+    return has_z ? __fadd_rn(out, __fmul_rn(z, c.sigma_up)) : out;
+}
+
+// x and out may alias (the table form updates the latents in place): each element is read before it is written, by the same
+// thread.  d_out never aliases a history row (the table names distinct ring slots).
+template <int EDT>
+__global__ void __launch_bounds__(kThreads) cfg_sigma_kernel(const void* __restrict__ eps_u, const void* __restrict__ eps_c,
+                                                             const float* x, const float* noise, float* out, float* d_out,
+                                                             const float* h1, const float* h2, const float* h3, int64_t n,
+                                                             int64_t nvec, SigmaCoef c, const float* __restrict__ table,
+                                                             const int* __restrict__ cursor, float* ring) {
+    if (table != nullptr) {
+        const float4* row = reinterpret_cast<const float4*>(table + (size_t)cursor[1] * kSigmaRow);
+        const float4 a = row[0], b = row[1], r2 = row[2];
+        c.sigma = a.x, c.c0 = a.y, c.c1 = a.z, c.c2 = a.w, c.c3 = b.x;
+        const int s1 = (int)b.y, s2 = (int)b.z, s3 = (int)b.w, slot = (int)r2.x, noise_row = (int)r2.y;
+        c.sigma_up = r2.z;
+        h1 = s1 < 0 ? nullptr : ring + (size_t)s1 * n;
+        h2 = s2 < 0 ? nullptr : ring + (size_t)s2 * n;
+        h3 = s3 < 0 ? nullptr : ring + (size_t)s3 * n;
+        d_out = slot < 0 ? nullptr : ring + (size_t)slot * n;
+        noise = (noise_row < 0 || noise == nullptr) ? nullptr : noise + (size_t)noise_row * n;
+    }
+    const bool cfg = eps_c != nullptr, has_z = noise != nullptr;
+    const bool b1 = h1 != nullptr, b2 = h2 != nullptr, b3 = h3 != nullptr;
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < nvec; i += stride) {
+        float eu[8], ec[8], xv[8], z[8] = {}, p1[8] = {}, p2[8] = {}, p3[8] = {}, o[8], d[8];
+        load8<EDT>(eps_u, i * 8, eu);
+        if (cfg) load8<EDT>(eps_c, i * 8, ec);
+        load8<B200SD_F32>(x, i * 8, xv);
+        if (has_z) load8<B200SD_F32>(noise, i * 8, z);
+        if (b1) load8<B200SD_F32>(h1, i * 8, p1);
+        if (b2) load8<B200SD_F32>(h2, i * 8, p2);
+        if (b3) load8<B200SD_F32>(h3, i * 8, p3);
+#pragma unroll
+        for (int j = 0; j < 8; ++j)
+            o[j] = sigma_one(eu[j], ec[j], xv[j], z[j], p1[j], p2[j], p3[j], cfg, b1, b2, b3, has_z, c, d[j]);
+        store8<B200SD_F32>(out, i * 8, o);
+        if (d_out) store8<B200SD_F32>(d_out, i * 8, d);
+    }
+    for (int64_t i = nvec * 8 + (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
+        float d;
+        const float eu = load1<EDT>(eps_u, i);
+        const float ec = cfg ? load1<EDT>(eps_c, i) : 0.f;
+        const float o = sigma_one(eu, ec, x[i], has_z ? noise[i] : 0.f, b1 ? h1[i] : 0.f, b2 ? h2[i] : 0.f, b3 ? h3[i] : 0.f,
+                                  cfg, b1, b2, b3, has_z, c, d);
+        out[i] = o;
+        if (d_out) d_out[i] = d;
+    }
+}
+
+// x2[0:n] = x2[n:2n] = x / in_div, in_div = table[cursor[1]].in_div: the CFG batch's UNet input, scaled as
+// scale_model_input scales it.  A true division, as torch's tensor-by-tensor division, not a multiply by the reciprocal.
+__global__ void __launch_bounds__(kThreads) sampler_scale_input_kernel(const float* __restrict__ x, float* __restrict__ x2,
+                                                                       int64_t n, int64_t nvec, const float* __restrict__ table,
+                                                                       const int* __restrict__ cursor) {
+    const float div = table[(size_t)cursor[1] * kSigmaRow + 11];
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < nvec; i += stride) {
+        float4 v = __ldg(reinterpret_cast<const float4*>(x) + i);
+        v = make_float4(__fdiv_rn(v.x, div), __fdiv_rn(v.y, div), __fdiv_rn(v.z, div), __fdiv_rn(v.w, div));
+        reinterpret_cast<float4*>(x2)[i] = v;
+        reinterpret_cast<float4*>(x2 + n)[i] = v;
+    }
+    for (int64_t i = nvec * 4 + (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
+        const float v = __fdiv_rn(x[i], div);
+        x2[i] = v;
+        x2[n + i] = v;
+    }
+}
+}  // namespace
+
+extern "C" int b200sd_cfg_sigma_step(const void* eps_u, const void* eps_c, const float* x, const float* noise, float* out,
+                                     float* d_out, const float* hist1, const float* hist2, const float* hist3, int64_t n,
+                                     float guidance, float sigma, float c0, float c1, float c2, float c3, float sigma_up,
+                                     int eps_dtype, b200sd_stream_t stream) {
+    B200SD_REQUIRE(eps_u && x && out, "cfg_sigma_step: null pointer");
+    B200SD_REQUIRE(n >= 0, "cfg_sigma_step: negative n");
+    B200SD_REQUIRE(dtype_ok(eps_dtype), "cfg_sigma_step: bad dtype");
+    B200SD_REQUIRE(sigma != 0.f, "cfg_sigma_step: sigma == 0");
+    const bool vec = aligned16(eps_u) && aligned16(eps_c) && aligned16(x) && aligned16(noise) && aligned16(out) &&
+                     aligned16(d_out) && aligned16(hist1) && aligned16(hist2) && aligned16(hist3);
+    const int64_t nvec = vec ? n / 8 : 0;  // unaligned views take the scalar path
+    if (n == 0) return B200SD_OK;
+    SigmaCoef c{guidance, sigma, c0, c1, c2, c3, sigma_up};
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    if (eps_dtype == B200SD_F32)
+        cfg_sigma_kernel<B200SD_F32><<<dim3(grid_for(vec ? n / 8 : n)), dim3(kThreads), 0, s>>>(
+            eps_u, eps_c, x, noise, out, d_out, hist1, hist2, hist3, n, nvec, c, nullptr, nullptr, nullptr);
+    else
+        cfg_sigma_kernel<B200SD_BF16><<<dim3(grid_for(vec ? n / 8 : n)), dim3(kThreads), 0, s>>>(
+            eps_u, eps_c, x, noise, out, d_out, hist1, hist2, hist3, n, nvec, c, nullptr, nullptr, nullptr);
+    COUNT_LAUNCH();
+    B200SD_LAUNCH_CHECK();
+    return B200SD_OK;
+}
+
+extern "C" int b200sd_cfg_sigma_step_table(const float* eps_u, const float* eps_c, float* x, float* ring, const float* noise,
+                                           int64_t n, float guidance, const float* table, const int* cursor,
+                                           b200sd_stream_t stream) {
+    B200SD_REQUIRE(eps_u && x && table && cursor, "cfg_sigma_step_table: null pointer");
+    B200SD_REQUIRE(n >= 0, "cfg_sigma_step_table: negative n");
+    B200SD_REQUIRE(aligned16(table), "cfg_sigma_step_table: table must be 16-byte aligned");
+    // every ring and noise row must be 16-byte aligned for the vector path: the base pointers and the row pitch n
+    const bool vec = aligned16(eps_u) && aligned16(eps_c) && aligned16(x) && aligned16(ring) && aligned16(noise) && n % 4 == 0;
+    const int64_t nvec = vec ? n / 8 : 0;
+    if (n == 0) return B200SD_OK;
+    SigmaCoef c{guidance, 1.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    cfg_sigma_kernel<B200SD_F32><<<dim3(grid_for(vec ? n / 8 : n)), dim3(kThreads), 0, s>>>(
+        eps_u, eps_c, x, noise, x, nullptr, nullptr, nullptr, nullptr, n, nvec, c, table, cursor, ring);
+    COUNT_LAUNCH();
+    B200SD_LAUNCH_CHECK();
+    return B200SD_OK;
+}
+
+extern "C" int b200sd_sampler_scale_input(const float* x, float* x2, int64_t n, const float* table, const int* cursor,
+                                          b200sd_stream_t stream) {
+    B200SD_REQUIRE(x && x2 && table && cursor, "sampler_scale_input: null pointer");
+    B200SD_REQUIRE(n >= 0, "sampler_scale_input: negative n");
+    const bool vec = aligned16(x) && aligned16(x2) && n % 4 == 0;
+    const int64_t nvec = vec ? n / 4 : 0;
+    if (n == 0) return B200SD_OK;
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    sampler_scale_input_kernel<<<dim3(grid_for(vec ? n / 4 : n)), dim3(kThreads), 0, s>>>(x, x2, n, nvec, table, cursor);
+    COUNT_LAUNCH();
+    B200SD_LAUNCH_CHECK();
+    return B200SD_OK;
+}
+
 extern "C" int b200sd_mse_workspace_floats(void) { return kMsePartials + 4; }
 
 extern "C" int b200sd_mse_loss_fwd(const void* pred, const void* target, float* loss_out, float* workspace,

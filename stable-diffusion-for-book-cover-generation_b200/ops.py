@@ -204,6 +204,45 @@ def inpaint_blend_table(x, x0, noise, mask, t_table, cursor, sa_table, sb_table)
     return x
 
 
+def cfg_sigma_step(eps_u, eps_c, x, guidance, sigma, coefs, hist=(), noise=None, sigma_up=0.0, out=None, d_out=None):
+    """Step of the sigma-space schedulers (LMS, Euler, Euler-a): d = (x - (x - sigma eps)) / sigma, eps the CFG combine;
+    out = x + sum(coefs[k] * [d, *hist][k]) (+ sigma_up noise).  hist: up to 3 earlier derivatives, newest first.  eps fp32 or
+    bf16; x, hist, noise, out and d_out (receives d) fp32."""
+    _chk(eps_u, eps_c, x, noise, out, d_out, *hist)
+    if len(coefs) != len(hist) + 1 or len(hist) > 3:
+        raise ValueError(f"cfg_sigma_step: {len(coefs)} coefficients for {len(hist)} history terms (up to 3)")
+    for t in (x, noise, out, d_out, *hist):
+        if t is not None and (t.dtype != torch.float32 or t.numel() != x.numel()):
+            raise ValueError(f"cfg_sigma_step: x, noise, history, out and d_out must be float32 with {x.numel()} elements")
+    if eps_c is not None and eps_c.shape != eps_u.shape:
+        raise ValueError("eps_u / eps_c shape mismatch")
+    if eps_u.numel() != x.numel():
+        raise ValueError(f"model_output {tuple(eps_u.shape)} and sample {tuple(x.shape)} sizes differ")
+    if out is None:
+        out = torch.empty_like(x)
+    c = [float(v) for v in coefs] + [0.0] * (4 - len(coefs))
+    hp = [_p(h) for h in hist] + [None] * (3 - len(hist))
+    check(lib().b200sd_cfg_sigma_step(_p(eps_u), _p(eps_c), _p(x), _p(noise), _p(out), _p(d_out), hp[0], hp[1], hp[2],
+                                      x.numel(), float(guidance), float(sigma), *c, float(sigma_up), _dt(eps_u), _stream()),
+          "cfg_sigma_step")
+    return out
+
+
+def cfg_sigma_step_table(eps_u, eps_c, x, ring, noise, guidance, coef_table, cursor):
+    """cfg_sigma_step() with row coef_table[cursor[1]] (sigma | c0..c3 | h1 h2 h3 | out_slot | noise_row | sigma_up | in_div):
+    history from / derivative to the 4-slot `ring`, z = noise[noise_row] (fp32 tensors); x is updated in place"""
+    check(lib().b200sd_cfg_sigma_step_table(_p(eps_u), _p(eps_c), _p(x), _p(ring), _p(noise), x.numel(), float(guidance),
+                                            _p(coef_table), _p(cursor), _stream()), "cfg_sigma_step_table")
+
+
+def sampler_scale_input(x, x2, coef_table, cursor):
+    """x2[:B] = x2[B:] = x / in_div of row coef_table[cursor[1]] (fp32): the scaled UNet input of a sigma-space captured step"""
+    if x2.numel() != 2 * x.numel():
+        raise ValueError("sampler_scale_input: x2 must hold two copies of x")
+    check(lib().b200sd_sampler_scale_input(_p(x), _p(x2), x.numel(), _p(coef_table), _p(cursor), _stream()),
+          "sampler_scale_input")
+
+
 def mse_loss_fwd(pred, target):
     _chk(pred, target)
     if pred.shape != target.shape:

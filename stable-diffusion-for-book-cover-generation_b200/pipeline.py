@@ -55,11 +55,12 @@ def denoise_loop(unet, scheduler, latents, encoder_hidden_states_2b, num_inferen
 
 def _captured_sampler(unet, scheduler, latents, ctx2, guidance_scale, eta=0.0, start=0, inpaint=False):
     """The whole-step CUDA graph (sampler.CapturedSampler) when the combination is covered: b200sd UNet on its bf16 plan with
-    CUDA graphs on, DDIM, PLMS or DDPM, CUDA tensors.  Cached on the UNet per (geometry, schedule, guidance, eta, start step,
-    inpaint mode); None -> the per-call loop."""
-    from .schedulers import DDIMScheduler, DDPMScheduler, PNDMScheduler
+    CUDA graphs on, DDIM, PLMS, DDPM, LMS, Euler or Euler-ancestral, CUDA tensors.  Cached on the UNet per (geometry, schedule,
+    guidance, eta, start step, inpaint mode); None -> the per-call loop."""
+    from .schedulers import SIGMA_SCHEDULERS, DDIMScheduler, DDPMScheduler, PNDMScheduler
     from .unet import UNet2DConditionModel
-    if not (isinstance(unet, UNet2DConditionModel) and isinstance(scheduler, (DDIMScheduler, PNDMScheduler, DDPMScheduler))
+    if not (isinstance(unet, UNet2DConditionModel)
+            and isinstance(scheduler, (DDIMScheduler, PNDMScheduler, DDPMScheduler, *SIGMA_SCHEDULERS))
             and latents.is_cuda and unet._precision == "bf16" and unet.use_cuda_graph and not unet.training):
         return None
     from .sampler import CapturedSampler
@@ -90,7 +91,8 @@ import json
 import os
 from types import SimpleNamespace
 
-_SCHEDULERS = ("DDIMScheduler", "PNDMScheduler", "DDPMScheduler")
+_SCHEDULERS = ("DDIMScheduler", "PNDMScheduler", "DDPMScheduler", "LMSDiscreteScheduler", "EulerDiscreteScheduler",
+               "EulerAncestralDiscreteScheduler")
 
 
 class StableDiffusionPipelineOutput(SimpleNamespace):
@@ -171,7 +173,7 @@ class StableDiffusionPipeline:
             with open(os.path.join(path, "scheduler", "scheduler_config.json")) as f:
                 cls_name = json.load(f).get("_class_name", cls_name)
             if cls_name not in _SCHEDULERS:
-                raise ValueError(f"scheduler class {cls_name!r} is not on the reference path ({', '.join(_SCHEDULERS)})")
+                raise ValueError(f"scheduler class {cls_name!r} is not implemented ({', '.join(_SCHEDULERS)} are)")
             kw = {"skip_prk_steps": True} if cls_name == "PNDMScheduler" else {}
             scheduler = getattr(S, cls_name).from_config(path, subfolder="scheduler", **kw)
         tokenizer, text_encoder = overrides.pop("tokenizer", None), overrides.pop("text_encoder", None)
@@ -289,6 +291,10 @@ class StableDiffusionImg2ImgPipeline(StableDiffusionPipeline):
 
     def _from_image(self, prompt, init_image, mask_image, strength, num_inference_steps, guidance_scale, negative_prompt, eta,
                     generator, output_type, return_dict, prompt_embeds):
+        from .schedulers import SIGMA_SCHEDULERS
+        if isinstance(self.scheduler, SIGMA_SCHEDULERS):
+            # 0.7.2 noises the init latents in sigma space there; the blend kernel indexes integer timesteps
+            raise NotImplementedError(f"{type(self).__name__} with {type(self.scheduler).__name__} is not implemented")
         t_start, t_noise = self.scheduler.img2img_start(num_inference_steps, strength)     # checks strength first
         if init_image is None or self.vae is None:
             raise ValueError("image-to-image needs an init_image and a vae")

@@ -1,4 +1,5 @@
-"""The whole denoising step of StableDiffusionPipeline.__call__ as ONE CUDA graph (DDIM, PLMS or DDPM + classifier-free guidance).
+"""The whole denoising step of StableDiffusionPipeline.__call__ as ONE CUDA graph (DDIM, PLMS, DDPM, LMS, Euler or Euler-ancestral +
+classifier-free guidance).
 
 Reference call sites: the loop inside `pipeline(...)` -- inference.py:175-176, 342-351; finetune_sd.py:264-271 -- i.e. per
 step `latent_model_input = cat([latents] * 2)`, `unet(...)`, `noise_pred_uncond + guidance_scale * (...)`, `scheduler.step`.
@@ -15,6 +16,10 @@ What the graph holds (nothing is launched eagerly between two steps, the host on
                                latents, 2.1 GB for 1000 DDPM steps at batch 32.
     (PNDMScheduler / PLMS: cfg_plms_step_table -- weights, eps-ring slots and the saved-sample flags of this call = table[cursor];
      the 4-deep eps history is a device ring, PNDM's repeated first timestep reads the sample saved by the first call)
+    (LMS / Euler / Euler-ancestral: sampler_scale_input replaces the two latents copies -- x2 = [latents | latents] / in_div, the
+     model-input scaling of the sigma-space schedulers -- and cfg_sigma_step_table closes the step: sigma, the update weights,
+     the LMS derivative-ring slots, the noise row and sigma_up = table[cursor].  The 4-slot derivative ring exists for LMS only,
+     the noise table (one row per step, the last one included) for Euler-ancestral only.)
     inpaint_blend_table        inpaint mode only: latents <- m (sa[t] x0 + sb[t] z) + (1 - m) latents at t = timesteps[cursor],
                                the masking step of legacy inpainting; x0, z and m are buffers `run(blend=...)` fills
 
@@ -38,13 +43,18 @@ from .plan import run_plan
 class CapturedSampler:
     def __init__(self, unet, scheduler, batch_images, h, w, S_ctx=77, guidance_scale=7.5, lanes=None, eta=0.0, start=0,
                  inpaint=False):
-        from .schedulers import DDIMScheduler, DDPMScheduler, PNDMScheduler
-        if not isinstance(scheduler, (DDIMScheduler, PNDMScheduler, DDPMScheduler)):
-            raise B200SDError("CapturedSampler covers DDIMScheduler, PNDMScheduler (PLMS) and DDPMScheduler")
+        from .schedulers import SIGMA_SCHEDULERS, DDIMScheduler, DDPMScheduler, PNDMScheduler
+        if not isinstance(scheduler, (DDIMScheduler, PNDMScheduler, DDPMScheduler, *SIGMA_SCHEDULERS)):
+            raise B200SDError("CapturedSampler covers DDIMScheduler, PNDMScheduler (PLMS), DDPMScheduler, LMSDiscreteScheduler, "
+                              "EulerDiscreteScheduler and EulerAncestralDiscreteScheduler")
         if lanes not in (None, 1):
             raise ValueError(f"lanes={lanes}: the step runs the CFG batch as one launch chain.  Concurrent per-half chains were "
                              "slower at every batch size measured (profiles/r02b_lanes_sweep.txt) and were removed")
         self.plms = isinstance(scheduler, PNDMScheduler)
+        self.sigma = isinstance(scheduler, SIGMA_SCHEDULERS)
+        if self.sigma and (start != 0 or inpaint):
+            raise ValueError(f"{type(scheduler).__name__}: image-to-image and inpainting (start != 0, inpaint=True) are not "
+                             "implemented for the sigma-space schedulers")
         if scheduler.num_inference_steps is None:
             raise ValueError("call scheduler.set_timesteps(n) first")
         if unet._precision != "bf16":
@@ -72,6 +82,12 @@ class CapturedSampler:
                 self.coef_table = torch.tensor(scheduler.plms_plan(start), **f32).contiguous()  # [calls][12]
                 self.saved = torch.zeros_like(self.latents)                                        # the first call's sample
                 self.ring = torch.zeros(4, self.latents.numel(), **f32)                            # eps history
+            elif self.sigma:
+                rows, n_noisy = scheduler.sigma_plan()
+                self.coef_table = torch.tensor(rows, **f32).contiguous()                                   # [steps][12]
+                keeps = any(r[8] >= 0 for r in rows)                                                       # LMS
+                self.ring = torch.zeros(4 if keeps else 0, self.latents.numel(), **f32)                  # derivative history
+                self.noise = torch.zeros(n_noisy, self.latents.numel(), **f32)                           # Euler-ancestral
             else:
                 rows, n_noisy = scheduler.ancestral_plan(eta, start)   # eta reaches only DDIM, as in diffusers' pipeline
                 self.coef_table = torch.tensor(rows, **f32).contiguous()                                   # [steps][8]
@@ -99,10 +115,16 @@ class CapturedSampler:
     def _step_ops(self):
         ops.sampler_advance(self.t_table, self.cursor, self.in_t)
         B = self.B
-        self.x2[:B].copy_(self.latents)
-        self.x2[B:].copy_(self.latents)
+        if self.sigma:
+            ops.sampler_scale_input(self.latents, self.x2, self.coef_table, self.cursor)
+        else:
+            self.x2[:B].copy_(self.latents)
+            self.x2[B:].copy_(self.latents)
         run_plan(self.engines[0].plan)
-        if self.plms:
+        if self.sigma:
+            ops.cfg_sigma_step_table(self.eps[:B], self.eps[B:], self.latents, self.ring if self.ring.numel() else None,
+                                     self.noise if self.noise.numel() else None, self.guidance, self.coef_table, self.cursor)
+        elif self.plms:
             ops.cfg_plms_step_table(self.eps[:B], self.eps[B:], self.latents, self.saved, self.ring, self.guidance, self.coef_table,
                                     self.cursor)
         else:
@@ -155,7 +177,7 @@ class CapturedSampler:
 
     def draw_noise(self, generator=None):
         """Fill the noise table: one schedulers.step_noise draw per stochastic step, in step order -- the same numbers the
-        per-call loop draws from the same generator.  DDIM with eta = 0 draws nothing."""
+        per-call loop draws from the same generator.  DDIM with eta = 0, LMS and Euler draw nothing."""
         from .schedulers import step_noise
         with torch.cuda.device(self.device):
             for k in range(self.noise.shape[0]):

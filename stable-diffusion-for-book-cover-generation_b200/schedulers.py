@@ -7,7 +7,7 @@
 
 Host side: timestep tables and per-step scalar coefficients (fp64 from the fp32 abar table).
 Device side: ONE fused kernel per step through the C ABI (b200sd_cfg_ancestral_step for DDIM and DDPM /
-b200sd_cfg_plms_step / b200sd_add_noise).  `step_cfg` additionally fuses the pipeline's
+b200sd_cfg_plms_step / b200sd_cfg_sigma_step for LMS, Euler and Euler-ancestral / b200sd_add_noise).  `step_cfg` additionally fuses the pipeline's
 classifier-free-guidance combine into the same kernel.
 
 Ancestral sampling (DDPMScheduler.step, DDIMScheduler.step with eta > 0) follows diffusers 0.7.2's formulas; its noise is
@@ -363,3 +363,213 @@ class PNDMScheduler(_SchedulerBase):
     def step_cfg(self, model_output_2b, timestep, sample, guidance_scale, out=None):
         B = sample.shape[0]
         return self._plms(model_output_2b[:B], model_output_2b[B:], timestep, sample, guidance_scale, out=out)
+
+
+# ---------------------------------------------------------------------------------------------------
+# The sigma-space family of diffusers 0.7.2 (scheduling_lms_discrete.py, scheduling_euler_discrete.py,
+# scheduling_euler_ancestral_discrete.py).  They sample the variance-exploding ODE x_VE = x_VP / sqrt(abar): the UNet input is
+# scaled by 1 / sqrt(sigma^2 + 1) and the timesteps are fractional.  One step rule (`_sigma_call`) serves the per-call step and
+# the captured sampler's table (`sigma_plan`); the device work is one fused kernel, b200sd_cfg_sigma_step.
+# ---------------------------------------------------------------------------------------------------
+class _SigmaSchedulerBase(_SchedulerBase):
+    """sigmas = ((1 - abar) / abar) ** 0.5 in fp32; set_timesteps(n): timesteps = linspace(0, T - 1, n)[::-1] (float64), sigmas
+    interpolated at them plus a final 0, fp32.  A timestep is looked up by exact match in `timesteps`."""
+    _defaults = dict(trained_betas=None)
+    _keeps_history = False
+
+    def __init__(self, *a, **kw):
+        super().__init__(*a, **kw)
+        T = self.num_train_timesteps
+        self._train_sigmas = (((1 - self.alphas_cumprod) / self.alphas_cumprod) ** 0.5).numpy()
+        self.sigmas = torch.from_numpy(np.concatenate([self._train_sigmas[::-1], [0.0]]).astype(np.float32))
+        self.init_noise_sigma = float(self.sigmas.max())
+        self._set_schedule(np.linspace(0, T - 1, T, dtype=float)[::-1].copy(), self.sigmas)
+        self.num_inference_steps = None
+
+    def _set_schedule(self, timesteps, sigmas):
+        self.timesteps = torch.from_numpy(timesteps)
+        self.sigmas = sigmas
+        self._sig = sigmas.numpy()
+        self._step_index = {t: i for i, t in enumerate(timesteps.tolist())}
+        self._in_div = (sigmas ** 2 + 1) ** 0.5           # fp32, as scale_model_input computes it
+        self._in_div_dev = {}
+        self._lms_cache = {}
+        self._derivs = []
+
+    def set_timesteps(self, num_inference_steps, device=None):
+        if num_inference_steps < 1:
+            raise ValueError("num_inference_steps out of range")
+        self.num_inference_steps = num_inference_steps
+        T = self.num_train_timesteps
+        ts = np.linspace(0, T - 1, num_inference_steps, dtype=float)[::-1].copy()
+        sig = np.interp(ts, np.arange(0, len(self._train_sigmas)), self._train_sigmas)
+        self._set_schedule(ts, torch.from_numpy(np.concatenate([sig, [0.0]]).astype(np.float32)))
+
+    def _index(self, timestep):
+        i = self._step_index.get(float(timestep))
+        if i is None:
+            raise ValueError(f"timestep {float(timestep)!r} is not in this scheduler's timesteps")
+        return i
+
+    def scale_model_input(self, sample, timestep):
+        """sample / ((sigma ** 2 + 1) ** 0.5): a true division by a tensor on the sample's device"""
+        i = self._index(timestep)
+        key = str(sample.device)
+        if key not in self._in_div_dev:
+            self._in_div_dev[key] = self._in_div.to(sample.device)
+        return sample / self._in_div_dev[key][i]
+
+    def add_noise(self, original_samples, noise, timesteps):
+        raise NotImplementedError(f"{type(self).__name__}.add_noise (sigma-space noising) is not implemented")
+
+    def img2img_start(self, num_inference_steps, strength):
+        raise NotImplementedError(f"image-to-image and inpainting with {type(self).__name__} are not implemented")
+
+    # -- the step rule ----------------------------------------------------------------------------
+    def _coefs(self, i, order, sig):
+        """(weights of [d, d[-1], ...], adds noise, sigma_up) of step i"""
+        raise NotImplementedError
+
+    def _sigma_call(self, i, hist, order=4, sig=None):
+        """The decisions of step index i given `hist`, the derivatives kept by earlier steps (tensors for the per-call step, ring
+        slots for `sigma_plan`), oldest first.  Returns (hist, sigma, coefs, used, keep_d, noisy, sigma_up): hist trimmed to the
+        entries this and later steps may read; the weights `coefs` of this step's derivative and of the history entries `used`
+        (newest first); whether this step's derivative joins the history; whether it adds sigma_up * z.  `sig` (default: this
+        schedule's fp32 sigmas) may be another sigma sequence, e.g. in float64."""
+        if not 1 <= order <= 4:
+            raise ValueError(f"order must be in 1..4, got {order}")
+        sig = self._sig if sig is None else sig
+        coefs, noisy, sigma_up = self._coefs(i, order, sig)
+        keep = self._keeps_history and order > 1
+        hist = list(hist)[max(0, len(hist) - (order - 1)):] if keep else []
+        used = hist[::-1][:len(coefs) - 1]
+        return hist, sig[i], coefs[:len(used) + 1], used, keep, noisy, sigma_up
+
+    def sigma_plan(self, order=4):
+        """The whole run as rows for b200sd_cfg_sigma_step_table: sigma | c0 c1 c2 c3 | h1 h2 h3 (ring slots, -1 unused) |
+        out_slot | noise_row (-1 none) | sigma_up | in_div.  `_sigma_call` run once on the host with a 4-slot ring instead of
+        tensors; noise rows are numbered in step order, as the per-call step draws.  Returns (rows, number of noise rows)."""
+        if self.num_inference_steps is None:
+            raise ValueError("call set_timesteps first")
+        rows, hist, k = [], [], 0
+        for i in range(len(self.timesteps)):
+            hist, sigma, coefs, used, keep, noisy, sigma_up = self._sigma_call(i, hist, order)
+            slot = next(s for s in range(4) if s not in hist) if keep else -1
+            rows.append([float(sigma)] + [float(c) for c in coefs] + [0.0] * (4 - len(coefs))
+                        + [float(h) for h in used] + [-1.0] * (3 - len(used))
+                        + [float(slot), float(k if noisy else -1), float(sigma_up), float(self._in_div[i])])
+            if keep:
+                hist.append(slot)
+            k += noisy
+        return rows, k
+
+    def _sigma_step(self, eps_u, eps_c, timestep, sample, guidance, generator=None, out=None, order=4):
+        self._check_step_args(eps_u, sample)
+        i = self._index(timestep)
+        self._derivs, sigma, coefs, used, keep, noisy, sigma_up = self._sigma_call(i, self._derivs, order)
+        if eps_u.dtype == torch.float16:      # fp16 pipelines: computed in fp32, the result cast back
+            eps_u, eps_c = eps_u.float(), (None if eps_c is None else eps_c.float())
+        x = sample.float().contiguous()
+        z = step_noise(x, generator) if noisy else None
+        d = torch.empty_like(x) if keep else None
+        fits = out is not None and out.dtype == torch.float32 and out.is_contiguous()
+        prev = ops.cfg_sigma_step(eps_u.contiguous(), None if eps_c is None else eps_c.contiguous(), x, guidance, sigma, coefs,
+                                  used, z, sigma_up, out=out if fits else None, d_out=d)
+        if keep:
+            self._derivs.append(d)
+        if out is not None and not fits:
+            prev = out.copy_(prev)
+        elif prev.dtype != sample.dtype:
+            prev = prev.to(sample.dtype)
+        return SchedulerOutput(prev_sample=prev)
+
+
+def _lms_coefficient(sig, order, t, current_order):
+    """0.7.2's get_lms_coefficient: the integral of the Lagrange basis polynomial over [sigma[t], sigma[t + 1]], with the
+    integrand evaluated in sig's precision (fp32 there: the sigmas are fp32 tensors)"""
+    from scipy import integrate
+
+    def lms_derivative(tau):
+        prod = 1.0
+        for k in range(order):
+            if current_order == k:
+                continue
+            prod *= (tau - sig[t - k]) / (sig[t - current_order] - sig[t - k])
+        return prod
+
+    return integrate.quad(lms_derivative, float(sig[t]), float(sig[t + 1]), epsrel=1e-4)[0]
+
+
+class LMSDiscreteScheduler(_SigmaSchedulerBase):
+    """diffusers 0.7.2 LMSDiscreteScheduler: linear multistep of order min(step index + 1, order) over the ODE derivatives."""
+    _keeps_history = True
+
+    def _coefs(self, i, order, sig):
+        o = min(i + 1, order)
+        if sig is not self._sig:
+            return [_lms_coefficient(sig, o, i, k) for k in range(o)], False, 0.0
+        key = (o, i)
+        if key not in self._lms_cache:
+            self._lms_cache[key] = [_lms_coefficient(sig, o, i, k) for k in range(o)]
+        return self._lms_cache[key], False, 0.0
+
+    def step(self, model_output, timestep, sample, order: int = 4, return_dict: bool = True):
+        out = self._sigma_step(model_output, None, timestep, sample, 0.0, order=order)
+        return out if return_dict else (out.prev_sample,)
+
+    def step_cfg(self, model_output_2b, timestep, sample, guidance_scale, out=None, order: int = 4):
+        """Fused `eps_u + s (eps_c - eps_u)` + LMS update; model_output_2b is the (2B, ...) UNet output."""
+        B = sample.shape[0]
+        return self._sigma_step(model_output_2b[:B], model_output_2b[B:], timestep, sample, guidance_scale, out=out, order=order)
+
+
+class EulerDiscreteScheduler(_SigmaSchedulerBase):
+    """diffusers 0.7.2 EulerDiscreteScheduler with s_churn = 0 (x' = x + (sigma_next - sigma) d).  It draws no noise; 0.7.2
+    draws a tensor it does not use on every step, so the generator's state afterwards differs from diffusers'."""
+
+    def _coefs(self, i, order, sig):
+        return [sig[i + 1] - sig[i]], False, 0.0
+
+    def _check_churn(self, timestep, s_churn, s_tmin, s_tmax):
+        sigma = float(self._sig[self._index(timestep)])
+        gamma = min(s_churn / (len(self._sig) - 1), 2 ** 0.5 - 1) if s_tmin <= sigma <= s_tmax else 0.0
+        if gamma > 0:
+            raise NotImplementedError("EulerDiscreteScheduler with s_churn > 0 is not implemented")
+
+    def step(self, model_output, timestep, sample, s_churn: float = 0.0, s_tmin: float = 0.0, s_tmax: float = float("inf"),
+             s_noise: float = 1.0, generator=None, return_dict: bool = True):
+        self._check_churn(timestep, s_churn, s_tmin, s_tmax)
+        out = self._sigma_step(model_output, None, timestep, sample, 0.0)
+        return out if return_dict else (out.prev_sample,)
+
+    def step_cfg(self, model_output_2b, timestep, sample, guidance_scale, out=None, s_churn: float = 0.0, s_tmin: float = 0.0,
+                 s_tmax: float = float("inf"), s_noise: float = 1.0, generator=None):
+        """Fused `eps_u + s (eps_c - eps_u)` + Euler update; model_output_2b is the (2B, ...) UNet output."""
+        self._check_churn(timestep, s_churn, s_tmin, s_tmax)
+        B = sample.shape[0]
+        return self._sigma_step(model_output_2b[:B], model_output_2b[B:], timestep, sample, guidance_scale, out=out)
+
+
+class EulerAncestralDiscreteScheduler(_SigmaSchedulerBase):
+    """diffusers 0.7.2 EulerAncestralDiscreteScheduler: x' = x + (sigma_down - sigma) d + sigma_up z with
+    sigma_up = (sigma_to^2 (sigma_from^2 - sigma_to^2) / sigma_from^2) ** 0.5, sigma_down = (sigma_to^2 - sigma_up^2) ** 0.5.
+    Every step, the last one included (sigma_up = 0 there), draws one `step_noise` from the caller's generator."""
+
+    def _coefs(self, i, order, sig):
+        sf, st = sig[i], sig[i + 1]
+        sigma_up = np.sqrt(st * st * (sf * sf - st * st) / (sf * sf))
+        sigma_down = np.sqrt(st * st - sigma_up * sigma_up)
+        return [sigma_down - sf], True, sigma_up
+
+    def step(self, model_output, timestep, sample, generator=None, return_dict: bool = True):
+        out = self._sigma_step(model_output, None, timestep, sample, 0.0, generator=generator)
+        return out if return_dict else (out.prev_sample,)
+
+    def step_cfg(self, model_output_2b, timestep, sample, guidance_scale, out=None, generator=None):
+        """Fused `eps_u + s (eps_c - eps_u)` + Euler-ancestral update; model_output_2b is the (2B, ...) UNet output."""
+        B = sample.shape[0]
+        return self._sigma_step(model_output_2b[:B], model_output_2b[B:], timestep, sample, guidance_scale, generator=generator,
+                                out=out)
+
+
+SIGMA_SCHEDULERS = (LMSDiscreteScheduler, EulerDiscreteScheduler, EulerAncestralDiscreteScheduler)
