@@ -675,7 +675,9 @@ def split_hi_lo(x, hi, lo):
 
 def groupnorm_silu_split(x0, x1, gamma, beta, out, out_lo, batch, hw, groups=32, eps=1e-5, silu=True, raw_out=None, raw_lo=None):
     _chk(x0, x1, gamma, beta, out, out_lo, raw_out, raw_lo)
-    ws = _workspace("gn", lib().b200sd_groupnorm_workspace_floats(batch) * 4, x0.device)
+    if x1 is not None and x1.dtype != x0.dtype:
+        raise B200SDError("groupnorm: both sources must have the same dtype")
+    ws = _workspace(("gn", _stream()), lib().b200sd_groupnorm_workspace_floats(batch) * 4, x0.device)
     C0 = x0.shape[-1]
     C1 = x1.shape[-1] if x1 is not None else 0
     check(lib().b200sd_groupnorm_silu_split(_p(x0), _p(x1), C0, C1, _p(gamma), _p(beta), _p(out), _p(out_lo), _p(raw_out),
