@@ -235,6 +235,10 @@ int b200sd_gemm(const b200sd_gemm_args* args, b200sd_stream_t stream);
  * [b * parts_per_image, (b + 1) * parts_per_image) of total_parts.  parts_per_image == 0: not available for this shape
  * (output tiles straddle images, bf16 output, ...) -- leave gn_part NULL and use b200sd_groupnorm_silu. */
 int b200sd_gemm_gn_layout(const b200sd_gemm_args* args, int hw, int* parts_per_image, int* total_parts);
+/* The launch b200sd_gemm would make for these arguments (same tiling decision; nothing is launched).  fields[10] =
+ * {kernel (0 one tile per CTA, 1 persistent, 2 persistent split-K), cluster split_k, persistent K slices (0 = none), CTA pair,
+ *  block_n, m_tiles, n_tiles, rows_valid, tile_n (images per conv tile), tiles_x}. */
+int b200sd_gemm_describe(const b200sd_gemm_args* args, int* fields);
 
 /* ---- backward GEMMs (autograd.backward through the UNet, finetune_sd.py:494; SURVEY.md row A9) ----
  * Same tcgen05 pipeline as b200sd_gemm; the operands that the forward read K-major are read MN-major

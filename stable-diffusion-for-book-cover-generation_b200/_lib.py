@@ -89,6 +89,7 @@ SIGNATURES = {
     "b200sd_geglu_tile": (_i, [_i]),
     "b200sd_gemm": (_i, [C.POINTER(GemmArgs), _vp]),
     "b200sd_gemm_gn_layout": (_i, [C.POINTER(GemmArgs), _i, C.POINTER(C.c_int), C.POINTER(C.c_int)]),
+    "b200sd_gemm_describe": (_i, [C.POINTER(GemmArgs), C.POINTER(C.c_int)]),
     "b200sd_groupnorm_silu_parts": (_i, [_vp, _vp, _i, _i, _vp, _i, _i, _vp, _i, _i, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _f, _i,
                                          _i, _vp]),
     "b200sd_gemm_dgrad": (_i, [C.POINTER(DgradArgs), _vp]),

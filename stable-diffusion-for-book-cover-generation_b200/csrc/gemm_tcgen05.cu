@@ -1630,6 +1630,32 @@ extern "C" int b200sd_gemm_gn_layout(const b200sd_gemm_args* a, int hw, int* par
     return B200SD_OK;
 }
 
+// Which kernel and tiling b200sd_gemm would launch for these arguments (same gemm_tiling call; launches nothing).
+extern "C" int b200sd_gemm_describe(const b200sd_gemm_args* a, int* f) {
+    B200SD_REQUIRE(a && f, "gemm_describe: bad arguments");
+    B200SD_REQUIRE(a->conv_taps == 1 || a->conv_taps == 9, "gemm_describe: conv_taps must be 1 or 9");
+    KParams p;
+    memset(&p, 0, sizeof(p));
+    p.M = a->M;
+    p.N = a->N;
+    p.num_k_blocks = a->K / BLOCK_K;
+    p.conv = a->conv_taps == 9;
+    int m_tiles = 0, n_tiles = 0;
+    const int rc = gemm_tiling(a, p, &m_tiles, &n_tiles);
+    if (rc) return rc;
+    f[0] = p.persist ? (p.psplit > 1 ? 2 : 1) : 0;
+    f[1] = p.split_k;
+    f[2] = p.psplit;
+    f[3] = p.pair;
+    f[4] = p.block_n;
+    f[5] = m_tiles;
+    f[6] = n_tiles;
+    f[7] = p.rows_valid;
+    f[8] = p.tile_n;
+    f[9] = p.tiles_x;
+    return B200SD_OK;
+}
+
 // ------------------------------------------------------------------------------------------------
 // backward entry points (same kernel, MN-major operand modes)
 // ------------------------------------------------------------------------------------------------

@@ -351,6 +351,20 @@ def gemm_run(args):
     check(lib().b200sd_gemm(C.byref(args), _stream()), "gemm")
 
 
+_GEMM_PATH_FIELDS = ("kernel", "split_k", "psplit", "pair", "block_n", "m_tiles", "n_tiles", "rows_valid", "tile_n", "tiles_x")
+_GEMM_KERNELS = ("tile", "persistent", "persistent-split")
+
+
+def gemm_path(args) -> dict:
+    """The kernel and tiling gemm_run(args) would launch (b200sd_gemm_describe: the launch's own decision, nothing launched).
+    kernel is "tile" (one output tile per CTA), "persistent" or "persistent-split" (its K-sliced mode)."""
+    f = (C.c_int * len(_GEMM_PATH_FIELDS))()
+    check(lib().b200sd_gemm_describe(C.byref(args), f), "gemm_describe")
+    d = dict(zip(_GEMM_PATH_FIELDS, f))
+    d["kernel"] = _GEMM_KERNELS[d["kernel"]]
+    return d
+
+
 class GnParts:
     """Column statistics a GEMM writes next to its fp32 output (GemmArgs.gn_part) for the GroupNorm that consumes it:
     buf [total_parts][2][N] floats; image b owns partial rows [b * ppi, (b + 1) * ppi)."""
