@@ -156,6 +156,13 @@ int b200sd_cfg_sigma_step_table(const float* eps_u, const float* eps_c, float* x
 int b200sd_sampler_scale_input(const float* x, float* x2, int64_t n, const float* table, const int* cursor,
                                b200sd_stream_t stream);
 
+/* The UNet input of a captured step of the 9-channel inpainting UNet: x2[n] = [latents[n mod B] | cond[n mod B]] / in_div for
+ * n in [0, 2B), all NCHW fp32: latents (B, c_lat, hw), cond (B, c_cond, hw) = [mask | masked-image latents], x2
+ * (2B, c_lat + c_cond, hw).  in_div as in b200sd_sampler_scale_input when `table` is given (a true division); table == NULL
+ * (DDIM, PLMS, DDPM): a plain copy, and cursor may be NULL.  diffusers 0.7.2's order: concatenate, then scale_model_input. */
+int b200sd_sampler_inpaint_input(const float* latents, const float* cond, float* x2, int batch, int c_lat, int c_cond,
+                                 int64_t hw, const float* table, const int* cursor, b200sd_stream_t stream);
+
 /* F.mse_loss(pred, target, "none").mean([1,2,3]).mean() (finetune_sd.py:483-484) == global mean.
  * loss_out: float[1]; workspace: float[b200sd_mse_workspace_floats()]. */
 int b200sd_mse_workspace_floats(void);
@@ -283,7 +290,8 @@ typedef struct b200sd_wgrad_args {
 int b200sd_gemm_wgrad(const b200sd_wgrad_args* args, b200sd_stream_t stream);
 
 /* Direct 3x3 convs at the ends of the UNet (degenerate GEMM shapes, CUDA cores):
- * conv_in : NCHW fp32 (batch, Cin=4, H, W) -> NHWC bf16 (batch*H*W, Cout); w fp32 packed [Cout][ky][kx][Cin].
+ * conv_in : NCHW fp32 (batch, Cin, H, W) -> NHWC bf16 or fp32 (batch*H*W, Cout); Cin = 4 (latents) or 9 (the inpainting
+ *           UNet's latents | mask | masked-image latents); w fp32 packed [Cout][ky][kx][Cin].
  * conv_out: NHWC bf16 (batch*H*W, Cin) -> NCHW fp32 (batch, Cout<=4, H, W); w fp32 packed [Cout][ky][kx][Cin]. */
 int b200sd_conv_in(const float* x_nchw, const float* w, const float* bias, void* out_nhwc, int batch, int Cin,
                    int Cout, int H, int W, int out_dtype, b200sd_stream_t stream);

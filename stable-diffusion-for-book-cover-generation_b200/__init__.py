@@ -3,7 +3,8 @@
 Public surface (mirrors what finetune_sd.py / inference.py / StableDiffusionPipeline touch):
     UNet2DConditionModel, DDIMScheduler, PNDMScheduler, DDPMScheduler, LMSDiscreteScheduler, EulerDiscreteScheduler,
     EulerAncestralDiscreteScheduler, StableDiffusionPipeline,
-    StableDiffusionImg2ImgPipeline, StableDiffusionInpaintPipelineLegacy (image-to-image, legacy inpainting), denoise_loop, mse_loss,
+    StableDiffusionImg2ImgPipeline, StableDiffusionInpaintPipelineLegacy (image-to-image, legacy inpainting),
+    StableDiffusionInpaintPipeline (the 9-channel inpainting UNet), denoise_loop, mse_loss,
     CapturedSampler (the whole denoising step as one CUDA graph), CLIPTextModel (transformers' surface, own kernels),
     AutoencoderKL (diffusers' surface, own kernels)
 """
@@ -24,6 +25,7 @@ def __getattr__(name):  # lazy: importing the package must not require torch.cud
         "StableDiffusionPipeline": "b200sd.pipeline",
         "StableDiffusionImg2ImgPipeline": "b200sd.pipeline",
         "StableDiffusionInpaintPipelineLegacy": "b200sd.pipeline",
+        "StableDiffusionInpaintPipeline": "b200sd.pipeline",
         "mse_loss": "b200sd.ops",
         "CapturedSampler": "b200sd.sampler",
         "CLIPTextModel": "b200sd.clip",

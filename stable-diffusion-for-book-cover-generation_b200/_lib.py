@@ -80,6 +80,7 @@ SIGNATURES = {
     "b200sd_cfg_sigma_step": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _f, _f, _f, _f, _f, _f, _f, _i, _vp]),
     "b200sd_cfg_sigma_step_table": (_i, [_vp, _vp, _vp, _vp, _vp, _i64, _f, _vp, _vp, _vp]),
     "b200sd_sampler_scale_input": (_i, [_vp, _vp, _i64, _vp, _vp, _vp]),
+    "b200sd_sampler_inpaint_input": (_i, [_vp, _vp, _vp, _i, _i, _i, _i64, _vp, _vp, _vp]),
     "b200sd_mse_workspace_floats": (_i, []),
     "b200sd_mse_loss_fwd": (_i, [_vp, _vp, _vp, _vp, _i64, _i, _i, _vp]),
     "b200sd_mse_loss_bwd": (_i, [_vp, _vp, _vp, _vp, _i64, _i, _i, _vp]),

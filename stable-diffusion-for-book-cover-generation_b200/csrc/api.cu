@@ -41,7 +41,7 @@ cudaError_t b200sd_opt_in_smem_impl(const void* kernel, int bytes, bool max_carv
     configured[key] = bytes;
     return cudaSuccess;
 }
-extern "C" int b200sd_version(void) { return 105; }
+extern "C" int b200sd_version(void) { return 106; }
 extern "C" int64_t b200sd_launch_count(void) { return g_b200sd_launches.load(); }
 
 // ---- in-graph timers: events recorded with cudaEventRecordExternal, so that a captured plan can carry a timestamp between

@@ -647,6 +647,32 @@ __global__ void __launch_bounds__(kThreads) sampler_scale_input_kernel(const flo
         x2[n + i] = v;
     }
 }
+
+// The UNet input of a captured step of the 9-channel inpainting UNet: x2[n] = [lat[n mod B] | cond[n mod B]] / in_div for
+// n in [0, 2B), NCHW -- diffusers 0.7.2's cat([latents] * 2), cat with the mask and the masked-image latents, then
+// scale_model_input, in one pass.  in_div as in sampler_scale_input_kernel (a true division); no table: no division.
+// T = float4 moves 4 pixels of one channel plane (hw % 4 == 0), `plane` counts T elements.
+__device__ __forceinline__ float div_rn(float v, float d) { return __fdiv_rn(v, d); }
+__device__ __forceinline__ float4 div_rn(float4 v, float d) {
+    return make_float4(__fdiv_rn(v.x, d), __fdiv_rn(v.y, d), __fdiv_rn(v.z, d), __fdiv_rn(v.w, d));
+}
+
+template <typename T>
+__global__ void __launch_bounds__(kThreads) sampler_inpaint_input_kernel(const T* __restrict__ lat, const T* __restrict__ cond,
+                                                                         T* __restrict__ x2, int batch, int c_lat, int c_cond,
+                                                                         int64_t plane, const float* __restrict__ table,
+                                                                         const int* __restrict__ cursor) {
+    const float div = table != nullptr ? table[(size_t)cursor[1] * kSigmaRow + 11] : 1.f;
+    const int64_t n_lat = c_lat * plane, n_cond = c_cond * plane, per = n_lat + n_cond;
+    const int64_t total = 2 * batch * per;
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += stride) {
+        const int64_t n = i / per, r = i - n * per, b = n % batch;
+        T v = r < n_lat ? __ldg(lat + b * n_lat + r) : __ldg(cond + b * n_cond + (r - n_lat));
+        if (table != nullptr) v = div_rn(v, div);
+        x2[i] = v;
+    }
+}
 }  // namespace
 
 extern "C" int b200sd_cfg_sigma_step(const void* eps_u, const void* eps_c, const float* x, const float* noise, float* out,
@@ -702,6 +728,26 @@ extern "C" int b200sd_sampler_scale_input(const float* x, float* x2, int64_t n, 
     if (n == 0) return B200SD_OK;
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     sampler_scale_input_kernel<<<dim3(grid_for(vec ? n / 4 : n)), dim3(kThreads), 0, s>>>(x, x2, n, nvec, table, cursor);
+    COUNT_LAUNCH();
+    B200SD_LAUNCH_CHECK();
+    return B200SD_OK;
+}
+
+extern "C" int b200sd_sampler_inpaint_input(const float* latents, const float* cond, float* x2, int batch, int c_lat,
+                                            int c_cond, int64_t hw, const float* table, const int* cursor,
+                                            b200sd_stream_t stream) {
+    B200SD_REQUIRE(latents && cond && x2, "sampler_inpaint_input: null pointer");
+    B200SD_REQUIRE(table == nullptr || cursor != nullptr, "sampler_inpaint_input: a table needs the cursor");
+    B200SD_REQUIRE(batch > 0 && c_lat > 0 && c_cond > 0 && hw > 0, "sampler_inpaint_input: bad sizes");
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    const int64_t total = 2 * (int64_t)batch * (c_lat + c_cond) * hw;
+    if (aligned16(latents) && aligned16(cond) && aligned16(x2) && hw % 4 == 0)
+        sampler_inpaint_input_kernel<float4><<<dim3(grid_for(total / 4)), dim3(kThreads), 0, s>>>(
+            reinterpret_cast<const float4*>(latents), reinterpret_cast<const float4*>(cond), reinterpret_cast<float4*>(x2), batch,
+            c_lat, c_cond, hw / 4, table, cursor);
+    else
+        sampler_inpaint_input_kernel<float><<<dim3(grid_for(total)), dim3(kThreads), 0, s>>>(latents, cond, x2, batch, c_lat,
+                                                                                            c_cond, hw, table, cursor);
     COUNT_LAUNCH();
     B200SD_LAUNCH_CHECK();
     return B200SD_OK;

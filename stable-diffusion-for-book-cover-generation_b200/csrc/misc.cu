@@ -1,5 +1,5 @@
 // b200sd -- the small kernels around the GEMMs: timestep embedding, time-MLP linears, the two
-// degenerate convs at the ends of the UNet (4 -> 320 and 320 -> 4 channels), nearest x2 upsample
+// degenerate convs at the ends of the UNet (4 or 9 -> 320 and 320 -> 4 channels), nearest x2 upsample
 // and the stride-2 im2col of the three Downsample2D convs.
 #include <atomic>
 
@@ -97,18 +97,26 @@ __global__ void __launch_bounds__(256) small_linear_kernel(const float* __restri
     }
 }
 
-// ---- conv_in: NCHW fp32 (Cin = 4) -> NHWC bf16; thread = output-channel pair, block = 32 pixels ---
+// ---- conv_in: NCHW fp32 (Cin = 4 or 9) -> NHWC; thread = kCo output channels, block = 32 pixels ----------------
+// Cin = 4 (SD latents, the VAE's image and latent inputs): a channel pair per thread, 2 x 36 weights in registers.
+// Cin = 9 (the inpainting UNet: latents | mask | masked-image latents): one channel per thread, 81 weights in registers -- a
+// pair would hold 162 and spill.  Every output is one chain in the same order for both: bias first, then tap-major,
+// channel-minor.  So a 9-channel weight whose channels 4..8 are zero adds exact zeros and reproduces the 4-channel result.
 constexpr int kCinPix = 32;
-template <int ODT>
+template <int Cin>
+__host__ __device__ constexpr int conv_in_co() { return Cin <= 4 ? 2 : 1; }
+
+template <int Cin, int ODT>
 __global__ void conv_in_kernel(const float* __restrict__ x, const float* __restrict__ w, const float* __restrict__ bias,
                                void* __restrict__ out, int batch, int Cout, int H, int W) {
-    constexpr int Cin = 4;
-    __shared__ float patch[kCinPix][9 * Cin];
+    constexpr int kTaps = 9 * Cin;
+    constexpr int kCo = conv_in_co<Cin>();
+    __shared__ float patch[kCinPix][kTaps];
     const int hw = H * W;
     const int pix0 = blockIdx.x * kCinPix;
     const int total = batch * hw;
-    for (int i = threadIdx.x; i < kCinPix * 9 * Cin; i += blockDim.x) {
-        const int pl = i / (9 * Cin), r = i % (9 * Cin);
+    for (int i = threadIdx.x; i < kCinPix * kTaps; i += blockDim.x) {
+        const int pl = i / kTaps, r = i % kTaps;
         const int tap = r / Cin, c = r % Cin;
         const int pix = pix0 + pl;
         float v = 0.f;
@@ -120,31 +128,56 @@ __global__ void conv_in_kernel(const float* __restrict__ x, const float* __restr
         patch[pl][r] = v;
     }
     __syncthreads();
-    for (int co2 = threadIdx.x; co2 < Cout / 2; co2 += blockDim.x) {
-        const int co = co2 * 2;
-        float w0[9 * Cin], w1[9 * Cin];
+    for (int cg = threadIdx.x; cg < Cout / kCo; cg += blockDim.x) {
+        const int co = cg * kCo;
+        float wr[kCo][kTaps], bv[kCo];
 #pragma unroll
-        for (int r = 0; r < 9 * Cin; ++r) {  // packed [Cout][tap][Cin]
-            w0[r] = __ldg(w + (size_t)co * 9 * Cin + r);
-            w1[r] = __ldg(w + (size_t)(co + 1) * 9 * Cin + r);
+        for (int k = 0; k < kCo; ++k) {
+#pragma unroll
+            for (int r = 0; r < kTaps; ++r) wr[k][r] = __ldg(w + (size_t)(co + k) * kTaps + r);   // packed [Cout][tap][Cin]
+            bv[k] = bias[co + k];
         }
-        const float b0 = bias[co], b1 = bias[co + 1];
         for (int pl = 0; pl < kCinPix; ++pl) {
             const int pix = pix0 + pl;
             if (pix >= total) break;
-            float a0 = b0, a1 = b1;
+            float a[kCo];
 #pragma unroll
-            for (int r = 0; r < 9 * Cin; ++r) {
+            for (int k = 0; k < kCo; ++k) a[k] = bv[k];
+#pragma unroll
+            for (int r = 0; r < kTaps; ++r) {
                 const float v = patch[pl][r];
-                a0 += w0[r] * v;
-                a1 += w1[r] * v;
+#pragma unroll
+                for (int k = 0; k < kCo; ++k) a[k] += wr[k][r] * v;
             }
-            if constexpr (ODT == B200SD_F32)
-                *reinterpret_cast<float2*>(static_cast<float*>(out) + (size_t)pix * Cout + co) = make_float2(a0, a1);
-            else
-                *reinterpret_cast<uint32_t*>(static_cast<bf16*>(out) + (size_t)pix * Cout + co) = pack_bf16x2(a0, a1);
+            if constexpr (kCo == 2) {
+                if constexpr (ODT == B200SD_F32)
+                    *reinterpret_cast<float2*>(static_cast<float*>(out) + (size_t)pix * Cout + co) = make_float2(a[0], a[1]);
+                else
+                    *reinterpret_cast<uint32_t*>(static_cast<bf16*>(out) + (size_t)pix * Cout + co) = pack_bf16x2(a[0], a[1]);
+            } else {
+                if constexpr (ODT == B200SD_F32)
+                    static_cast<float*>(out)[(size_t)pix * Cout + co] = a[0];
+                else
+                    static_cast<bf16*>(out)[(size_t)pix * Cout + co] = __float2bfloat16_rn(a[0]);
+            }
         }
     }
+}
+
+template <int Cin>
+void launch_conv_in(const float* x, const float* w, const float* bias, void* out, int batch, int Cout, int H, int W,
+                    int out_dtype, cudaStream_t s) {
+    // Cin = 4: up to 256 threads of channel pairs (160 for the UNet's 320 channels); Cin = 9: the UNet's 320 channels in one pass
+    constexpr int kCo = conv_in_co<Cin>();
+    int threads = Cout / kCo;
+    const int cap = kCo == 2 ? 256 : 320;
+    if (threads > cap) threads = cap;
+    threads = ceil_div(threads, 32) * 32;
+    const dim3 grid(ceil_div(batch * H * W, kCinPix));
+    if (out_dtype == B200SD_F32)
+        conv_in_kernel<Cin, B200SD_F32><<<grid, dim3(threads), 0, s>>>(x, w, bias, out, batch, Cout, H, W);
+    else
+        conv_in_kernel<Cin, B200SD_BF16><<<grid, dim3(threads), 0, s>>>(x, w, bias, out, batch, Cout, H, W);
 }
 
 // ---- conv_out: NHWC bf16 (Cin = 320) -> NCHW fp32 (Cout = 4); warp per pixel, lanes over channels -
@@ -298,16 +331,13 @@ extern "C" int b200sd_small_linear(const float* in, const void* w_bf16, const fl
 extern "C" int b200sd_conv_in(const float* x_nchw, const float* w, const float* bias, void* out_nhwc, int batch, int Cin,
                               int Cout, int H, int W, int out_dtype, b200sd_stream_t stream) {
     B200SD_REQUIRE(x_nchw && w && bias && out_nhwc, "conv_in: null pointer");
-    B200SD_REQUIRE(Cin == 4, "conv_in: only Cin == 4 (SD latent) is supported, got %d", Cin);
+    B200SD_REQUIRE(Cin == 4 || Cin == 9, "conv_in: Cin must be 4 (SD latents) or 9 (inpainting UNet), got %d", Cin);
     B200SD_REQUIRE(Cout % 2 == 0 && batch > 0 && H > 0 && W > 0, "conv_in: bad sizes");
-    const int total = batch * H * W;
-    int threads = Cout / 2;
-    if (threads > 256) threads = 256;
-    threads = ceil_div(threads, 32) * 32;
-    if (out_dtype == B200SD_F32)
-        conv_in_kernel<B200SD_F32><<<dim3(ceil_div(total, kCinPix)), dim3(threads), 0, static_cast<cudaStream_t>(stream)>>>(x_nchw, w, bias, out_nhwc, batch, Cout, H, W);
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    if (Cin == 4)
+        launch_conv_in<4>(x_nchw, w, bias, out_nhwc, batch, Cout, H, W, out_dtype, s);
     else
-        conv_in_kernel<B200SD_BF16><<<dim3(ceil_div(total, kCinPix)), dim3(threads), 0, static_cast<cudaStream_t>(stream)>>>(x_nchw, w, bias, out_nhwc, batch, Cout, H, W);
+        launch_conv_in<9>(x_nchw, w, bias, out_nhwc, batch, Cout, H, W, out_dtype, s);
     COUNT_LAUNCH();
     B200SD_LAUNCH_CHECK();
     return B200SD_OK;

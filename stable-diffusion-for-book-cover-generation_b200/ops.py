@@ -243,6 +243,24 @@ def sampler_scale_input(x, x2, coef_table, cursor):
           "sampler_scale_input")
 
 
+def sampler_inpaint_input(latents, cond, x2, coef_table=None, cursor=None):
+    """x2[n] = [latents[n mod B] | cond[n mod B]] for n in [0, 2B), divided by in_div of row coef_table[cursor[1]] when a table is
+    given (fp32 NCHW): the input of a captured step of the 9-channel inpainting UNet, concatenated then scaled as in 0.7.2"""
+    _chk(latents, cond, x2, coef_table, cursor)
+    B, c_lat, h, w = latents.shape
+    c_cond = cond.shape[1]
+    if tuple(cond.shape) != (B, c_cond, h, w) or tuple(x2.shape) != (2 * B, c_lat + c_cond, h, w):
+        raise ValueError(f"sampler_inpaint_input: latents {tuple(latents.shape)}, cond {tuple(cond.shape)} and x2 {tuple(x2.shape)} "
+                         "do not fit together")
+    if any(t is not None and t.dtype != torch.float32 for t in (latents, cond, x2, coef_table)):
+        raise B200SDError("sampler_inpaint_input is fp32")
+    if (coef_table is None) != (cursor is None):
+        raise ValueError("sampler_inpaint_input: pass coef_table and cursor together")
+    check(lib().b200sd_sampler_inpaint_input(_p(latents), _p(cond), _p(x2), B, c_lat, c_cond, h * w, _p(coef_table), _p(cursor),
+                                             _stream()), "sampler_inpaint_input")
+    return x2
+
+
 def mse_loss_fwd(pred, target):
     _chk(pred, target)
     if pred.shape != target.shape:

@@ -14,16 +14,27 @@ from . import ops
 
 @torch.no_grad()
 def denoise_loop(unet, scheduler, latents, encoder_hidden_states_2b, num_inference_steps=50, guidance_scale=7.5,
-                 record=None, eta=0.0, generator=None, start=0, blend=None):
+                 record=None, eta=0.0, generator=None, start=0, blend=None, cond=None):
     """latents (B,4,h,w) -> denoised latents (B,4,h,w).  One UNet call at batch 2B per step, then ONE
     fused kernel for `eps_u + s (eps_c - eps_u)` + the scheduler update.  As in diffusers, `eta` and `generator` reach only
     a scheduler whose step takes them (eta: DDIM; generator: DDIM and DDPM).
 
     img2img / legacy inpainting: the loop runs over timesteps[start:] (no step when that is empty).  blend=(init_orig, noise,
     mask) adds legacy inpainting's masking step after every scheduler step at loop timestep t:
-    latents = mask * add_noise(init_orig, noise, t) + (1 - mask) * latents, mask broadcastable to the latents (1 = keep)."""
+    latents = mask * add_noise(init_orig, noise, t) + (1 - mask) * latents, mask broadcastable to the latents (1 = keep).
+
+    9-channel inpainting UNet: cond = cat([mask, masked_image_latents], 1) (B, 5, h, w) joins every step's UNet input in
+    diffusers 0.7.2's order -- cat([latents] * 2), cat with cat([cond] * 2) along the channels, then scale_model_input."""
     if encoder_hidden_states_2b.shape[0] != 2 * latents.shape[0]:
         raise ValueError("encoder_hidden_states must be cat([uncond, cond]) with batch 2B")
+    in_channels = getattr(getattr(unet, "config", None), "in_channels", latents.shape[1])
+    n_cond = in_channels - latents.shape[1]
+    if (cond is None) != (n_cond == 0) or (cond is not None and tuple(cond.shape) != (latents.shape[0], n_cond) + tuple(latents.shape[2:])):
+        raise ValueError(f"a UNet with in_channels={in_channels} takes {latents.shape[1]}-channel latents and "
+                         + (f"cond (B, {n_cond}, h, w) = [mask | masked-image latents], got "
+                            f"{None if cond is None else tuple(cond.shape)}" if n_cond else "no cond"))
+    if cond is not None and (start != 0 or blend is not None):
+        raise ValueError("the 9-channel inpainting UNet runs the full schedule from noise: no start step and no blend")
     scheduler.set_timesteps(num_inference_steps)
     timesteps = scheduler.timesteps.tolist()[start:]
     accepted = inspect.signature(scheduler.step_cfg).parameters
@@ -32,7 +43,8 @@ def denoise_loop(unet, scheduler, latents, encoder_hidden_states_2b, num_inferen
                                  start, blend is not None)
                if record is None and timesteps else None)
     if sampler is not None:
-        return sampler.run(latents, encoder_hidden_states_2b, generator, blend=blend).to(latents.dtype)
+        cond_args = None if cond is None else (cond[:, :1], cond[:, 1:])
+        return sampler.run(latents, encoder_hidden_states_2b, generator, blend=blend, cond=cond_args).to(latents.dtype)
     latents = (latents * scheduler.init_noise_sigma).float().contiguous()
     if blend is not None:
         init_orig, noise, mask = (t.to(latents.device).float() for t in blend)
@@ -40,10 +52,12 @@ def denoise_loop(unet, scheduler, latents, encoder_hidden_states_2b, num_inferen
         tables = scheduler._noise_tables(latents.device)
     x2 = torch.empty((2 * latents.shape[0],) + tuple(latents.shape[1:]), dtype=latents.dtype, device=latents.device)
     B = latents.shape[0]
+    cond2 = None if cond is None else torch.cat([cond.to(latents.device, latents.dtype)] * 2)
     for t in timesteps:
         x2[:B].copy_(latents)
         x2[B:].copy_(latents)
-        eps2 = unet(scheduler.scale_model_input(x2, t), t, encoder_hidden_states_2b).sample
+        x_in = x2 if cond2 is None else torch.cat([x2, cond2], dim=1)
+        eps2 = unet(scheduler.scale_model_input(x_in, t), t, encoder_hidden_states_2b).sample
         if record is not None:
             record.append(eps2[:B] + guidance_scale * (eps2[B:] - eps2[:B]))
         latents = scheduler.step_cfg(eps2.float() if eps2.dtype not in (torch.float32, torch.bfloat16) else eps2, t,
@@ -99,12 +113,23 @@ class StableDiffusionPipelineOutput(SimpleNamespace):
     """`.images` (list of PIL images, or a tensor for output_type "pt" / "latent") and `.nsfw_content_detected` (None)."""
 
 
+_INPAINT_CHANNELS = 4 + 1 + 4      # latents | mask | masked-image latents: the UNet of diffusers' StableDiffusionInpaintPipeline
+
+
+def _latent_channels(unet):
+    """the channel count of the latents `unet` denoises; a 9-channel inpainting UNet has no place in the 4-channel pipelines"""
+    if unet.in_channels == _INPAINT_CHANNELS:
+        raise ValueError(f"this UNet has in_channels={_INPAINT_CHANNELS} (an inpainting UNet): use StableDiffusionInpaintPipeline")
+    return unet.in_channels
+
+
 class StableDiffusionPipeline:
     """Same constructor keywords, `save_pretrained` / `from_pretrained` directory layout (`model_index.json` + one sub-folder
     per component) and `__call__` signature as diffusers 0.7.2's pipeline.  `safety_checker` / `feature_extractor` are
     accepted and ignored (the reference always passes `safety_checker=None`: inference.py:407, 427; utils.py:190, 225, 250)."""
 
     config_name = "model_index.json"
+    _saved_class_name = "StableDiffusionPipeline"     # model_index.json's _class_name
 
     def __init__(self, vae=None, text_encoder=None, tokenizer=None, unet=None, scheduler=None, safety_checker=None,
                  feature_extractor=None):
@@ -143,7 +168,7 @@ class StableDiffusionPipeline:
     # -- (de)serialisation in the diffusers directory layout -----------------------------------------
     def save_pretrained(self, path, safe_serialization=False):
         os.makedirs(path, exist_ok=True)
-        index = {"_class_name": "StableDiffusionPipeline", "_diffusers_version": "0.7.2"}
+        index = {"_class_name": self._saved_class_name, "_diffusers_version": "0.7.2"}
         for name, obj in self.components.items():
             if obj is None:
                 index[name] = [None, None]
@@ -235,7 +260,7 @@ class StableDiffusionPipeline:
         device = self.device
         ctx2 = self._context(prompt, negative_prompt, prompt_embeds)
         B = ctx2.shape[0] // 2
-        shape = (B, self.unet.in_channels, height // 8, width // 8)
+        shape = (B, _latent_channels(self.unet), height // 8, width // 8)
         if latents is None:
             latents = _randn(shape, generator, device)
         elif tuple(latents.shape) != shape:
@@ -306,7 +331,7 @@ class StableDiffusionImg2ImgPipeline(StableDiffusionPipeline):
         B = ctx2.shape[0] // 2
         if image.shape[0] not in (1, B):
             raise ValueError(f"init_image has batch {image.shape[0]}; it must be 1 or the prompt count {B}")
-        shape = (B, self.unet.in_channels, image.shape[2] // 8, image.shape[3] // 8)
+        shape = (B, _latent_channels(self.unet), image.shape[2] // 8, image.shape[3] // 8)
         mask = None
         if mask_image is not None:
             mask = mask_image if isinstance(mask_image, torch.Tensor) else preprocess_mask(mask_image)
@@ -336,3 +361,82 @@ class StableDiffusionInpaintPipelineLegacy(StableDiffusionImg2ImgPipeline):
             raise ValueError("mask_image is required")
         return self._from_image(prompt, init_image, mask_image, strength, num_inference_steps, guidance_scale, negative_prompt,
                                 eta, generator, output_type, return_dict, prompt_embeds)
+
+
+# ---------------------------------------------------------------------------------------------------
+# diffusers 0.7.2's StableDiffusionInpaintPipeline: the dedicated inpainting checkpoint, a UNet with in_channels = 9 that sees
+# the mask and the masked image's latents at every step.  It starts from pure noise over the full schedule (no strength).
+# ---------------------------------------------------------------------------------------------------
+def prepare_mask_and_masked_image(image, mask):
+    """0.7.2's prepare_mask_and_masked_image -> (mask (1|B, 1, H, W) in {0, 1}, masked image (1|B, 3, H, W) in [-1, 1]).
+    PIL image: "RGB", NCHW, / 127.5 - 1, not resized.  PIL mask: "L", / 255.  Tensors: an image in [-1, 1] and a mask in [0, 1].
+    The mask is binarised (< 0.5 -> 0, >= 0.5 -> 1; white = 1 = repaint) and the masked image keeps the pixels where it is 0."""
+    import numpy as np
+    if isinstance(image, torch.Tensor):
+        image = image.float()
+    else:
+        arr = np.array(image.convert("RGB"))[None].transpose(0, 3, 1, 2)
+        image = torch.from_numpy(arr.copy()).to(dtype=torch.float32) / 127.5 - 1.0
+    if isinstance(mask, torch.Tensor):
+        mask = mask.float()
+    else:
+        mask = torch.from_numpy((np.array(mask.convert("L")).astype(np.float32) / 255.0)[None, None].copy())
+    if image.dim() != 4 or mask.dim() != 4 or image.shape[2:] != mask.shape[2:]:
+        raise ValueError(f"image (B, 3, H, W) and mask_image (B, 1, H, W) must have the same height and width, got "
+                         f"{tuple(image.shape)} and {tuple(mask.shape)}")
+    mask = torch.where(mask < 0.5, torch.zeros_like(mask), torch.ones_like(mask))
+    masked_image = image * (mask.to(image.device) < 0.5)
+    return mask, masked_image
+
+
+def latent_mask(mask, h, w):
+    """the inpainting mask at latent size h x w: F.interpolate's default mode (nearest), as 0.7.2 resizes it"""
+    import torch.nn.functional as F
+    return F.interpolate(mask, size=(h, w))
+
+
+class StableDiffusionInpaintPipeline(StableDiffusionPipeline):
+    """diffusers 0.7.2's inpainting pipeline on a UNet with in_channels = 9: `pipe(prompt, image=, mask_image=, height=512,
+    width=512, ...)`.  image: a PIL image or a (1 or B, 3, H, W) tensor in [-1, 1]; mask_image: a PIL image or a (1 or B, 1, H,
+    W) tensor in [0, 1], white (>= 0.5) = repaint.  Both must already be height x width.  Every step's UNet input is
+    [latents | mask | masked-image latents], the mask nearest-resized to the latents; the run draws from `generator` the initial
+    latents, then the masked image's posterior sample, then the step noise."""
+
+    _saved_class_name = "StableDiffusionInpaintPipeline"
+
+    @torch.no_grad()
+    def __call__(self, prompt=None, image=None, mask_image=None, height=512, width=512, num_inference_steps=50,
+                 guidance_scale=7.5, negative_prompt=None, eta=0.0, generator=None, latents=None, output_type="pil",
+                 return_dict=True, prompt_embeds=None):
+        if height % 8 or width % 8:
+            raise ValueError(f"`height` and `width` have to be divisible by 8 but are {height} and {width}.")
+        if self.unet.in_channels != _INPAINT_CHANNELS:
+            raise ValueError(f"Incorrect configuration settings! The config of `pipeline.unet` expects "
+                             f"{self.unet.in_channels} input channels, but 4 (latents) + 1 (mask) + 4 (masked image latents) "
+                             f"= {_INPAINT_CHANNELS} are passed: StableDiffusionInpaintPipeline needs the 9-channel inpainting UNet")
+        if image is None or mask_image is None or self.vae is None:
+            raise ValueError("inpainting needs an image, a mask_image and a vae")
+        mask, masked_image = prepare_mask_and_masked_image(image, mask_image)
+        if masked_image.dim() != 4 or masked_image.shape[1] != 3 or tuple(masked_image.shape[2:]) != (height, width):
+            raise ValueError(f"image must be (B, 3, {height}, {width}) (height x width; it is not resized), got "
+                             f"{tuple(masked_image.shape)}")
+        if mask.dim() != 4 or mask.shape[1] != 1 or tuple(mask.shape[2:]) != (height, width):
+            raise ValueError(f"mask_image must be (B, 1, {height}, {width}) (height x width; it is not resized), got {tuple(mask.shape)}")
+        device = self.device
+        ctx2 = self._context(prompt, negative_prompt, prompt_embeds)
+        B = ctx2.shape[0] // 2
+        for name, t in (("image", image), ("mask_image", mask)):
+            if isinstance(t, torch.Tensor) and t.shape[0] not in (1, B):
+                raise ValueError(f"{name} has batch {t.shape[0]}; it must be 1 or the prompt count {B}")
+        shape = (B, self.unet.config.out_channels, height // 8, width // 8)
+        if latents is None:
+            latents = _randn(shape, generator, device)                      # first draw: the initial latents
+        elif tuple(latents.shape) != shape:
+            raise ValueError(f"Unexpected latents shape, got {tuple(latents.shape)}, expected {shape}")
+        mask = latent_mask(mask, *shape[2:])
+        vae_dtype = next(self.vae.parameters()).dtype
+        masked_latents = 0.18215 * self.vae.encode(masked_image.to(device, vae_dtype)).latent_dist.sample(generator).float()
+        cond = torch.cat([mask.to(device).expand(B, -1, -1, -1), masked_latents.expand(B, -1, -1, -1)], dim=1).contiguous()
+        lat = denoise_loop(self.unet, self.scheduler, latents.to(device).float(), ctx2.float(), num_inference_steps, guidance_scale,
+                           eta=eta, generator=generator, cond=cond)
+        return self._output(lat, output_type, return_dict)

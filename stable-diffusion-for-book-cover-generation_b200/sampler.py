@@ -22,6 +22,10 @@ What the graph holds (nothing is launched eagerly between two steps, the host on
      the noise table (one row per step, the last one included) for Euler-ancestral only.)
     inpaint_blend_table        inpaint mode only: latents <- m (sa[t] x0 + sb[t] z) + (1 - m) latents at t = timesteps[cursor],
                                the masking step of legacy inpainting; x0, z and m are buffers `run(blend=...)` fills
+    (9-channel inpainting UNet (in_channels = out_channels + 5): sampler_inpaint_input replaces the two latents copies and
+     sampler_scale_input -- x2 = [latents | cond | latents | cond] (/ in_div for the sigma-space schedulers), the UNet input of
+     diffusers 0.7.2's StableDiffusionInpaintPipeline, concatenated before it is scaled.  cond = [mask | masked-image latents]
+     (B, 5, h, w) is a buffer `run(cond=...)` fills; the latents, the step and every scheduler buffer keep out_channels.)
 
 A run that starts partway through the schedule (img2img, inpainting: `start` = t_start) holds only the executed steps in its
 timestep, coefficient and noise tables, so its graph is launch for launch the text-to-image graph.
@@ -57,6 +61,14 @@ class CapturedSampler:
                              "implemented for the sigma-space schedulers")
         if scheduler.num_inference_steps is None:
             raise ValueError("call scheduler.set_timesteps(n) first")
+        cfg = unet.config
+        self.n_cond = cfg.in_channels - cfg.out_channels     # 5 for the inpainting UNet: mask | masked-image latents
+        if self.n_cond not in (0, 5):
+            raise ValueError(f"a UNet with in_channels={cfg.in_channels}, out_channels={cfg.out_channels} is neither a text-to-image "
+                             "nor an inpainting UNet")
+        if self.n_cond and (start != 0 or inpaint):
+            raise ValueError("the 9-channel inpainting UNet runs the full schedule from noise: start != 0 and the legacy "
+                             "masking step (inpaint=True) do not apply to it")
         if unet._precision != "bf16":
             raise B200SDError("CapturedSampler runs the bf16 plan")
         B = int(batch_images)
@@ -65,11 +77,11 @@ class CapturedSampler:
         dev = self.device = unet.device
         unet._ensure_packed()
         self._pack_gen = unet._pack_gen
-        cfg = unet.config
         f32 = dict(dtype=torch.float32, device=dev)
         with torch.cuda.device(dev):
-            self.latents = torch.zeros(B, cfg.in_channels, h, w, **f32)        # updated in place by every step
-            self.x2 = torch.zeros(2 * B, cfg.in_channels, h, w, **f32)         # [latents | latents], the UNet's input
+            self.latents = torch.zeros(B, cfg.out_channels, h, w, **f32)       # updated in place by every step
+            self.x2 = torch.zeros(2 * B, cfg.in_channels, h, w, **f32)         # [latents | latents] (+ cond), the UNet's input
+            self.cond = torch.zeros(B, self.n_cond, h, w, **f32) if self.n_cond else None   # [mask | masked-image latents]
             self.eps = torch.zeros(2 * B, cfg.out_channels, h, w, **f32)       # [uncond | cond] noise predictions
             self.in_t = torch.zeros(2 * B, **f32)
             self.ctx = torch.zeros(2 * B, S_ctx, cfg.cross_attention_dim, **f32)
@@ -115,7 +127,10 @@ class CapturedSampler:
     def _step_ops(self):
         ops.sampler_advance(self.t_table, self.cursor, self.in_t)
         B = self.B
-        if self.sigma:
+        if self.n_cond:
+            table = (self.coef_table, self.cursor) if self.sigma else (None, None)
+            ops.sampler_inpaint_input(self.latents, self.cond, self.x2, *table)
+        elif self.sigma:
             ops.sampler_scale_input(self.latents, self.x2, self.coef_table, self.cursor)
         else:
             self.x2[:B].copy_(self.latents)
@@ -191,16 +206,33 @@ class CapturedSampler:
         for buf, t in ((self.init_orig, init_orig), (self.blend_noise, noise), (self.mask, mask)):
             buf.copy_(t.float().expand_as(buf))
 
+    def set_cond(self, mask, masked_latents):
+        """9-channel UNet: the mask (B or 1, 1, h, w) and the masked-image latents (B or 1, 4, h, w) that every step's UNet input
+        carries after the latents"""
+        if not self.n_cond:
+            raise ValueError("cond=(mask, masked_latents) is for a 9-channel inpainting UNet")
+        B, h, w = self.B, self.h, self.w
+        if tuple(mask.shape[1:]) != (1, h, w) or tuple(masked_latents.shape[1:]) != (self.n_cond - 1, h, w):
+            raise ValueError(f"cond: mask must be (B, 1, {h}, {w}) and masked_latents (B, {self.n_cond - 1}, {h}, {w}), got "
+                             f"{tuple(mask.shape)} and {tuple(masked_latents.shape)}")
+        self.cond[:, :1].copy_(mask.float().expand(B, 1, h, w))
+        self.cond[:, 1:].copy_(masked_latents.float().expand(B, self.n_cond - 1, h, w))
+
     @torch.no_grad()
-    def run(self, latents, ctx2, generator=None, blend=None):
+    def run(self, latents, ctx2, generator=None, blend=None, cond=None):
         """latents (B,4,h,w) -> denoised latents after the steps timesteps[start:].  A stochastic sampler first draws its step
-        noise from `generator` (draw_noise).  An inpainting sampler needs blend=(init_orig, noise, mask) (set_blend)."""
+        noise from `generator` (draw_noise).  An inpainting sampler needs blend=(init_orig, noise, mask) (set_blend), a 9-channel
+        UNet cond=(mask, masked_latents) (set_cond)."""
         if self.unet._stale(self._pack_gen):
             raise B200SDError("the UNet's weights changed after this sampler was built: build a new CapturedSampler")
         if (blend is not None) != self.inpaint:
             raise ValueError("blend=(init_orig, noise, mask) is required in inpaint mode and only there")
+        if (cond is not None) != bool(self.n_cond):
+            raise ValueError("cond=(mask, masked_latents) is required with a 9-channel inpainting UNet and only there")
         if blend is not None:
             self.set_blend(*blend)
+        if cond is not None:
+            self.set_cond(*cond)
         self.set_context(ctx2.float())
         self.set_latents(latents.float() * self.scheduler.init_noise_sigma)
         if not self.plms:

@@ -475,17 +475,20 @@ class UNet2DConditionModel(nn.Module):
     def forward(self, sample, timestep, encoder_hidden_states, return_dict: bool = True):
         if sample.dim() != 4 or sample.shape[1] != self.in_channels:
             raise ValueError(f"sample must be (N, {self.in_channels}, H, W), got {tuple(sample.shape)}")
+        ctx = encoder_hidden_states
+        needs_grad = torch.is_grad_enabled() and (
+            sample.requires_grad or ctx.requires_grad or any(p.requires_grad for p in self.parameters()) and self.training)
+        if needs_grad and self.in_channels != 4:
+            raise NotImplementedError(f"training a UNet with in_channels={self.in_channels} is not implemented (the inpainting "
+                                      "UNet runs inference only): call it under torch.no_grad() or in eval mode")
         if not sample.is_cuda:
             raise B200SDError("b200sd.UNet2DConditionModel runs on CUDA only (no CPU fallback)")
         N, _, H, Wd = sample.shape
         n_down = len(self.config.block_out_channels) - 1
         if H % (1 << n_down) or Wd % (1 << n_down):
             raise ValueError(f"H and W must be multiples of {1 << n_down}")
-        ctx = encoder_hidden_states
         if ctx.dim() != 3 or ctx.shape[0] != N or ctx.shape[2] != self.config.cross_attention_dim:
             raise ValueError(f"encoder_hidden_states must be ({N}, S, {self.config.cross_attention_dim}), got {tuple(ctx.shape)}")
-        needs_grad = torch.is_grad_enabled() and (
-            sample.requires_grad or ctx.requires_grad or any(p.requires_grad for p in self.parameters()) and self.training)
         if needs_grad:
             from .autograd import unet_forward_train
             out = unet_forward_train(self, sample, timestep, ctx)
