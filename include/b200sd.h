@@ -77,7 +77,8 @@ int b200sd_sampler_advance(const float* timesteps, int n_steps, int* cursor, flo
  * sample of the first call for PNDM's repeated first timestep; `ring` is the 4-deep eps history (4 * n floats).  Per call one
  * row of 12 floats of `table`, indexed by cursor[1]: w0 w1 w2 w3 | cx ce | h1 h2 h3 (ring slot of ets[-1], ets[-2], ets[-3];
  * -1 = unused) | out_slot (-1 = this call's eps is not kept) | x_from_saved | save_x.  The host fills the table by running
- * PNDMScheduler's counter logic once (sampler.py); reference call site utils.py:222-224. */
+ * PNDMScheduler's counter logic once (PNDMScheduler.plms_plan); reference call site utils.py:222-224.  Runs the kernel of
+ * b200sd_cfg_plms_step, so a row computes bit for bit what b200sd_cfg_plms_step computes with the same history, weights and x. */
 int b200sd_cfg_plms_step_table(const float* eps_u, const float* eps_c, float* x, float* saved, float* ring, int64_t n,
                                float guidance, const float* table, const int* cursor, b200sd_stream_t stream);
 

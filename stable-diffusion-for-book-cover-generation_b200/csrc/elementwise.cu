@@ -74,56 +74,6 @@ inline int grid_for(int64_t nvec) {
 }
 
 // ---------------------------------------------------------------------------------------------
-// CFG + PLMS
-// ---------------------------------------------------------------------------------------------
-struct PlmsArgs {
-    const void* hist[4];
-    float w[5];
-    int nhist;
-    float g, cx, ce;
-};
-
-template <int EDT, int XDT>
-__global__ void __launch_bounds__(kThreads) cfg_plms_kernel(const void* __restrict__ eps_u,
-                                                            const void* __restrict__ eps_c,
-                                                            const void* __restrict__ x, void* __restrict__ out,
-                                                            void* __restrict__ eps_out, int64_t n, int64_t nvec, PlmsArgs a) {
-    const bool cfg = eps_c != nullptr;
-    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < nvec; i += stride) {
-        float eu[8], ec[8], xv[8], e[8], acc[8], o[8];
-        load8<EDT>(eps_u, i * 8, eu);
-        if (cfg) load8<EDT>(eps_c, i * 8, ec);
-        load8<XDT>(x, i * 8, xv);
-#pragma unroll
-        for (int j = 0; j < 8; ++j) {
-            e[j] = cfg ? (eu[j] + a.g * (ec[j] - eu[j])) : eu[j];
-            acc[j] = a.w[0] * e[j];
-        }
-        for (int h = 0; h < a.nhist; ++h) {
-            float hv[8];
-            load8<EDT>(a.hist[h], i * 8, hv);
-#pragma unroll
-            for (int j = 0; j < 8; ++j) acc[j] += a.w[1 + h] * hv[j];
-        }
-#pragma unroll
-        for (int j = 0; j < 8; ++j) o[j] = a.cx * xv[j] - a.ce * acc[j];
-        store8<XDT>(out, i * 8, o);
-        if (eps_out) store8<EDT>(eps_out, i * 8, e);
-    }
-    {
-        for (int64_t i = nvec * 8 + (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
-            float eu = load1<EDT>(eps_u, i);
-            float e = cfg ? (eu + a.g * (load1<EDT>(eps_c, i) - eu)) : eu;
-            float acc = a.w[0] * e;
-            for (int h = 0; h < a.nhist; ++h) acc += a.w[1 + h] * load1<EDT>(a.hist[h], i);
-            store1<XDT>(out, i, a.cx * load1<XDT>(x, i) - a.ce * acc);
-            if (eps_out) store1<EDT>(eps_out, i, e);
-        }
-    }
-}
-
-// ---------------------------------------------------------------------------------------------
 // add_noise
 // ---------------------------------------------------------------------------------------------
 template <int DT>
@@ -290,47 +240,121 @@ extern "C" int b200sd_sampler_advance(const float* timesteps, int n_steps, int* 
     return B200SD_OK;
 }
 
-// Captured PLMS step: everything that changes from call to call -- the linear-multistep weights, which slots of the 4-deep eps
-// ring hold the history, where this call's eps goes, whether x is the running sample or the one saved by the first call
-// (PNDM's second call re-does the first timestep), the two scalars of _get_prev_sample -- is one row of a device table indexed
-// by the cursor.  Row layout (12 floats): w0 w1 w2 w3 | cx ce | h1 h2 h3 (ring slots, -1 = unused) | out_slot (-1 = not
-// kept) | x_from_saved | save_x.
+// CFG + PLMS (PNDMScheduler with skip_prk_steps=True): e = eps_u + g (eps_c - eps_u), out = cx x - ce (w0 e + w1 hist[0] + ...),
+// history newest first, each rounding spelled out (fmaf, __fmul_rn) so that nvcc cannot contract the two loops differently.
+// The per-call form passes weights and history pointers by value; the captured form reads them from row cursor[1] of a table,
+// with the 4-deep eps ring slot this call's eps goes to and the sample saved by PNDM's first call, which the second re-does.
+// Row (12 floats): w0 w1 w2 w3 | cx ce | h1 h2 h3 (ring slots, -1 = unused) | out_slot (-1 = not kept) | x_from_saved | save_x.
 namespace {
 constexpr int kPlmsRow = 12;
-__global__ void __launch_bounds__(kThreads) cfg_plms_table_kernel(const float* __restrict__ eps_u, const float* __restrict__ eps_c,
-                                                                  float* __restrict__ x, float* __restrict__ saved,
-                                                                  float* __restrict__ ring, int64_t n, float g,
-                                                                  const float* __restrict__ table, const int* __restrict__ cursor) {
-    const float* row = table + (size_t)cursor[1] * kPlmsRow;
-    const float w0 = row[0], w1 = row[1], w2 = row[2], w3 = row[3], cx = row[4], ce = row[5];
-    const int h1 = (int)row[6], h2 = (int)row[7], h3 = (int)row[8], slot = (int)row[9];
-    const bool from_saved = row[10] != 0.f, save_x = row[11] != 0.f;
+
+struct PlmsCoef {
+    float g, cx, ce, w[5];
+};
+
+// The sample is read from x_src (x, or `saved` on an x_from_saved row); a save_x row copies x to `saved`.  x and out may alias
+// (the table form updates the latents in place), and so may x_src and `saved`: each element is read before it is written, by
+// the same thread.  eps_out is never one of the history rows (the table names distinct ring slots).
+template <int EDT, int XDT>
+__global__ void __launch_bounds__(kThreads) cfg_plms_kernel(const void* __restrict__ eps_u, const void* __restrict__ eps_c,
+                                                            const void* x, void* out, void* eps_out, const void* h0,
+                                                            const void* h1, const void* h2, const void* h3, int64_t n,
+                                                            int64_t nvec, PlmsCoef c, const float* __restrict__ table,
+                                                            const int* __restrict__ cursor, float* ring, float* saved) {
+    const void* hist[4] = {h0, h1, h2, h3};
+    const void* x_src = x;
+    float* save = nullptr;
+    if (table != nullptr) {
+        const float* row = table + (size_t)cursor[1] * kPlmsRow;
+        auto slot = [&](int k) -> float* { const int s = (int)row[k]; return s < 0 ? nullptr : ring + (size_t)s * n; };
+        c = PlmsCoef{c.g, row[4], row[5], {row[0], row[1], row[2], row[3], 0.f}};
+#pragma unroll
+        for (int k = 0; k < 3; ++k) hist[k] = slot(6 + k);
+        eps_out = slot(9);
+        if (row[10] != 0.f) x_src = saved;
+        if (row[11] != 0.f) save = saved;
+    }
     const bool cfg = eps_c != nullptr;
     const int64_t stride = (int64_t)gridDim.x * blockDim.x;
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
-        const float eu = eps_u[i];
-        const float e = cfg ? (eu + g * (eps_c[i] - eu)) : eu;
-        float acc = w0 * e;
-        if (h1 >= 0) acc = fmaf(w1, ring[(size_t)h1 * n + i], acc);
-        if (h2 >= 0) acc = fmaf(w2, ring[(size_t)h2 * n + i], acc);
-        if (h3 >= 0) acc = fmaf(w3, ring[(size_t)h3 * n + i], acc);
-        const float cur = x[i];
-        const float xv = from_saved ? saved[i] : cur;
-        if (save_x) saved[i] = cur;
-        x[i] = cx * xv - ce * acc;
-        if (slot >= 0) ring[(size_t)slot * n + i] = e;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < nvec; i += stride) {
+        float eu[8], ec[8], xv[8], e[8], acc[8], o[8];
+        load8<EDT>(eps_u, i * 8, eu);
+        if (cfg) load8<EDT>(eps_c, i * 8, ec);
+        load8<XDT>(x_src, i * 8, xv);
+        if (save) {
+            load8<XDT>(x, i * 8, o);
+            store8<B200SD_F32>(save, i * 8, o);
+        }
+#pragma unroll
+        for (int j = 0; j < 8; ++j) {
+            e[j] = cfg ? fmaf(c.g, ec[j] - eu[j], eu[j]) : eu[j];
+            acc[j] = __fmul_rn(c.w[0], e[j]);
+        }
+#pragma unroll
+        for (int h = 0; h < 4; ++h) {
+            if (hist[h] == nullptr) continue;
+            float hv[8];
+            load8<EDT>(hist[h], i * 8, hv);
+#pragma unroll
+            for (int j = 0; j < 8; ++j) acc[j] = fmaf(c.w[1 + h], hv[j], acc[j]);
+        }
+#pragma unroll
+        for (int j = 0; j < 8; ++j) o[j] = fmaf(c.cx, xv[j], -__fmul_rn(c.ce, acc[j]));
+        store8<XDT>(out, i * 8, o);
+        if (eps_out) store8<EDT>(eps_out, i * 8, e);
+    }
+    for (int64_t i = nvec * 8 + (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
+        const float eu = load1<EDT>(eps_u, i);
+        const float e = cfg ? fmaf(c.g, load1<EDT>(eps_c, i) - eu, eu) : eu;
+        float acc = __fmul_rn(c.w[0], e);
+#pragma unroll
+        for (int h = 0; h < 4; ++h)
+            if (hist[h] != nullptr) acc = fmaf(c.w[1 + h], load1<EDT>(hist[h], i), acc);
+        const float xv = load1<XDT>(x_src, i);
+        if (save) save[i] = load1<XDT>(x, i);
+        store1<XDT>(out, i, fmaf(c.cx, xv, -__fmul_rn(c.ce, acc)));
+        if (eps_out) store1<EDT>(eps_out, i, e);
     }
 }
 }  // namespace
+
+extern "C" int b200sd_cfg_plms_step(const void* eps_u, const void* eps_c, const void* x, void* out, void* eps_out,
+                                    const void* hist0, const void* hist1, const void* hist2, const void* hist3,
+                                    int nhist, const float* w_host5, int64_t n, float guidance, float cx, float ce,
+                                    int eps_dtype, int x_dtype, b200sd_stream_t stream) {
+    B200SD_REQUIRE(eps_u && x && out && w_host5, "cfg_plms_step: null pointer");
+    B200SD_REQUIRE(nhist >= 0 && nhist <= 4, "cfg_plms_step: nhist out of range");
+    B200SD_REQUIRE(dtype_ok(eps_dtype) && dtype_ok(x_dtype), "cfg_plms_step: bad dtype");
+    const void* hist[4] = {hist0, hist1, hist2, hist3};
+    bool vec = aligned16(eps_u) && aligned16(eps_c) && aligned16(x) && aligned16(out) && aligned16(eps_out);
+    for (int i = 0; i < 4; ++i) {
+        B200SD_REQUIRE(i >= nhist || hist[i] != nullptr, "cfg_plms_step: null history pointer");
+        if (i >= nhist) hist[i] = nullptr;  // the kernel reads the non-null ones
+        vec = vec && aligned16(hist[i]);
+    }
+    const int64_t nvec = vec ? n / 8 : 0;  // unaligned views take the scalar path
+    const PlmsCoef c{guidance, cx, ce, {w_host5[0], w_host5[1], w_host5[2], w_host5[3], w_host5[4]}};
+    if (n == 0) return B200SD_OK;
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    DISPATCH2(eps_dtype, x_dtype, cfg_plms_kernel, grid_for(vec ? n / 8 : n), s, eps_u, eps_c, x, out, eps_out, hist[0], hist[1],
+              hist[2], hist[3], n, nvec, c, (const float*)nullptr, (const int*)nullptr, (float*)nullptr, (float*)nullptr);
+    COUNT_LAUNCH();
+    B200SD_LAUNCH_CHECK();
+    return B200SD_OK;
+}
 
 extern "C" int b200sd_cfg_plms_step_table(const float* eps_u, const float* eps_c, float* x, float* saved, float* ring, int64_t n,
                                           float guidance, const float* table, const int* cursor, b200sd_stream_t stream) {
     B200SD_REQUIRE(eps_u && x && saved && ring && table && cursor, "cfg_plms_step_table: null pointer");
     B200SD_REQUIRE(n >= 0, "cfg_plms_step_table: negative n");
+    // every ring row must be 16-byte aligned for the vector path: the base pointers and the row pitch n
+    const bool vec = aligned16(eps_u) && aligned16(eps_c) && aligned16(x) && aligned16(saved) && aligned16(ring) && n % 4 == 0;
+    const int64_t nvec = vec ? n / 8 : 0;
     if (n == 0) return B200SD_OK;
+    const PlmsCoef c{guidance, 1.f, 0.f, {1.f, 0.f, 0.f, 0.f, 0.f}};  // all but g come from the table
     cudaStream_t s = static_cast<cudaStream_t>(stream);
-    cfg_plms_table_kernel<<<dim3(grid_for(n)), dim3(kThreads), 0, s>>>(eps_u, eps_c, x, saved, ring, n, guidance,
-                              table, cursor);
+    cfg_plms_kernel<B200SD_F32, B200SD_F32><<<dim3(grid_for(vec ? n / 8 : n)), dim3(kThreads), 0, s>>>(
+        eps_u, eps_c, x, x, nullptr, nullptr, nullptr, nullptr, nullptr, n, nvec, c, table, cursor, ring, saved);
     COUNT_LAUNCH();
     B200SD_LAUNCH_CHECK();
     return B200SD_OK;
@@ -436,31 +460,6 @@ extern "C" int b200sd_cfg_ancestral_step_table(const float* eps_u, const float* 
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     cfg_ancestral_kernel<B200SD_F32, B200SD_F32><<<dim3(grid_for(vec ? n / 8 : n)), dim3(kThreads), 0, s>>>(
         eps_u, eps_c, x, noise, x, n, nvec, c, table, cursor);
-    COUNT_LAUNCH();
-    B200SD_LAUNCH_CHECK();
-    return B200SD_OK;
-}
-
-extern "C" int b200sd_cfg_plms_step(const void* eps_u, const void* eps_c, const void* x, void* out, void* eps_out,
-                                    const void* hist0, const void* hist1, const void* hist2, const void* hist3,
-                                    int nhist, const float* w_host5, int64_t n, float guidance, float cx, float ce,
-                                    int eps_dtype, int x_dtype, b200sd_stream_t stream) {
-    B200SD_REQUIRE(eps_u && x && out && w_host5, "cfg_plms_step: null pointer");
-    B200SD_REQUIRE(nhist >= 0 && nhist <= 4, "cfg_plms_step: nhist out of range");
-    B200SD_REQUIRE(dtype_ok(eps_dtype) && dtype_ok(x_dtype), "cfg_plms_step: bad dtype");
-    PlmsArgs a;
-    a.hist[0] = hist0; a.hist[1] = hist1; a.hist[2] = hist2; a.hist[3] = hist3;
-    bool vec = aligned16(eps_u) && aligned16(eps_c) && aligned16(x) && aligned16(out) && aligned16(eps_out);
-    for (int i = 0; i < nhist; ++i) {
-        B200SD_REQUIRE(a.hist[i] != nullptr, "cfg_plms_step: null history pointer");
-        vec = vec && aligned16(a.hist[i]);
-    }
-    const int64_t nvec = vec ? n / 8 : 0;
-    for (int i = 0; i < 5; ++i) a.w[i] = w_host5[i];
-    a.nhist = nhist; a.g = guidance; a.cx = cx; a.ce = ce;
-    if (n == 0) return B200SD_OK;
-    cudaStream_t s = static_cast<cudaStream_t>(stream);
-    DISPATCH2(eps_dtype, x_dtype, cfg_plms_kernel, grid_for(vec ? n / 8 : n), s, eps_u, eps_c, x, out, eps_out, n, nvec, a);
     COUNT_LAUNCH();
     B200SD_LAUNCH_CHECK();
     return B200SD_OK;

@@ -78,22 +78,8 @@ def launch_count() -> int:
 # scheduler / loss elementwise
 # ---------------------------------------------------------------------------------------------
 def cfg_ddim_step(eps_u, eps_c, x, guidance, sa_t, sb_t, sa_p, sb_p, out=None):
-    eps_u, eps_c, x, half = _up16(eps_u, eps_c, x)
-    if half:
-        r = cfg_ddim_step(eps_u.contiguous(), None if eps_c is None else eps_c.contiguous(), x.contiguous(), guidance, sa_t, sb_t,
-                          sa_p, sb_p).half()
-        return r if out is None else out.copy_(r)
-    _chk(eps_u, eps_c, x, out)
-    if out is None:
-        out = torch.empty_like(x)
-    if eps_c is not None and eps_c.shape != eps_u.shape:
-        raise ValueError("eps_u / eps_c shape mismatch")
-    if eps_u.numel() != x.numel():
-        raise ValueError(f"model_output {tuple(eps_u.shape)} and sample {tuple(x.shape)} sizes differ")
-    check(lib().b200sd_cfg_ddim_step(_p(eps_u), _p(eps_c), _p(x), _p(out), None, x.numel(), float(guidance),
-                                     float(sa_t), float(sb_t), float(sa_p), float(sb_p), _dt(eps_u), _dt(x), _stream()),
-          "cfg_ddim_step")
-    return out
+    """DDIM update at eta = 0: sa_p x0 + sb_p eps, x0 = (x - sb_t eps) / sa_t"""
+    return cfg_ancestral_step(eps_u, eps_c, x, None, guidance, sa_t, sb_t, sa_p, 0.0, sb_p, 0.0, False, out=out)
 
 
 def cfg_ancestral_step(eps_u, eps_c, x, noise, guidance, sa_t, sb_t, c_x0, c_x, c_e, c_z, clip, out=None):

@@ -10,6 +10,7 @@ import inspect
 import torch
 
 from . import ops
+from .schedulers import SCHEDULERS
 
 
 @torch.no_grad()
@@ -71,11 +72,9 @@ def _captured_sampler(unet, scheduler, latents, ctx2, guidance_scale, eta=0.0, s
     """The whole-step CUDA graph (sampler.CapturedSampler) when the combination is covered: b200sd UNet on its bf16 plan with
     CUDA graphs on, DDIM, PLMS, DDPM, LMS, Euler or Euler-ancestral, CUDA tensors.  Cached on the UNet per (geometry, schedule,
     guidance, eta, start step, inpaint mode); None -> the per-call loop."""
-    from .schedulers import SIGMA_SCHEDULERS, DDIMScheduler, DDPMScheduler, PNDMScheduler
     from .unet import UNet2DConditionModel
-    if not (isinstance(unet, UNet2DConditionModel)
-            and isinstance(scheduler, (DDIMScheduler, PNDMScheduler, DDPMScheduler, *SIGMA_SCHEDULERS))
-            and latents.is_cuda and unet._precision == "bf16" and unet.use_cuda_graph and not unet.training):
+    if not (isinstance(unet, UNet2DConditionModel) and hasattr(scheduler, "captured_step") and latents.is_cuda
+            and unet._precision == "bf16" and unet.use_cuda_graph and not unet.training):
         return None
     from .sampler import CapturedSampler
     B, _, h, w = latents.shape
@@ -105,8 +104,7 @@ import json
 import os
 from types import SimpleNamespace
 
-_SCHEDULERS = ("DDIMScheduler", "PNDMScheduler", "DDPMScheduler", "LMSDiscreteScheduler", "EulerDiscreteScheduler",
-               "EulerAncestralDiscreteScheduler")
+_SCHEDULERS = tuple(cls.__name__ for cls in SCHEDULERS)
 
 
 class StableDiffusionPipelineOutput(SimpleNamespace):
@@ -316,10 +314,6 @@ class StableDiffusionImg2ImgPipeline(StableDiffusionPipeline):
 
     def _from_image(self, prompt, init_image, mask_image, strength, num_inference_steps, guidance_scale, negative_prompt, eta,
                     generator, output_type, return_dict, prompt_embeds):
-        from .schedulers import SIGMA_SCHEDULERS
-        if isinstance(self.scheduler, SIGMA_SCHEDULERS):
-            # 0.7.2 noises the init latents in sigma space there; the blend kernel indexes integer timesteps
-            raise NotImplementedError(f"{type(self).__name__} with {type(self.scheduler).__name__} is not implemented")
         t_start, t_noise = self.scheduler.img2img_start(num_inference_steps, strength)     # checks strength first
         if init_image is None or self.vae is None:
             raise ValueError("image-to-image needs an init_image and a vae")

@@ -47,20 +47,13 @@ from .plan import run_plan
 class CapturedSampler:
     def __init__(self, unet, scheduler, batch_images, h, w, S_ctx=77, guidance_scale=7.5, lanes=None, eta=0.0, start=0,
                  inpaint=False):
-        from .schedulers import SIGMA_SCHEDULERS, DDIMScheduler, DDPMScheduler, PNDMScheduler
-        if not isinstance(scheduler, (DDIMScheduler, PNDMScheduler, DDPMScheduler, *SIGMA_SCHEDULERS)):
-            raise B200SDError("CapturedSampler covers DDIMScheduler, PNDMScheduler (PLMS), DDPMScheduler, LMSDiscreteScheduler, "
-                              "EulerDiscreteScheduler and EulerAncestralDiscreteScheduler")
+        if not hasattr(scheduler, "captured_step"):
+            raise B200SDError("CapturedSampler covers the schedulers of b200sd.schedulers: DDIMScheduler, PNDMScheduler (PLMS), "
+                              "DDPMScheduler, LMSDiscreteScheduler, EulerDiscreteScheduler and EulerAncestralDiscreteScheduler")
         if lanes not in (None, 1):
             raise ValueError(f"lanes={lanes}: the step runs the CFG batch as one launch chain.  Concurrent per-half chains were "
                              "slower at every batch size measured (profiles/r02b_lanes_sweep.txt) and were removed")
-        self.plms = isinstance(scheduler, PNDMScheduler)
-        self.sigma = isinstance(scheduler, SIGMA_SCHEDULERS)
-        if self.sigma and (start != 0 or inpaint):
-            raise ValueError(f"{type(scheduler).__name__}: image-to-image and inpainting (start != 0, inpaint=True) are not "
-                             "implemented for the sigma-space schedulers")
-        if scheduler.num_inference_steps is None:
-            raise ValueError("call scheduler.set_timesteps(n) first")
+        plan = scheduler.captured_step(eta, start, inpaint)     # eta reaches only DDIM, as in diffusers' pipeline
         cfg = unet.config
         self.n_cond = cfg.in_channels - cfg.out_channels     # 5 for the inpainting UNet: mask | masked-image latents
         if self.n_cond not in (0, 5):
@@ -90,20 +83,12 @@ class CapturedSampler:
                 raise ValueError(f"start={start} leaves no step of the {len(scheduler.timesteps)}-step schedule")
             self.n_steps = len(ts)
             self.t_table = torch.tensor(ts, **f32)
-            if self.plms:
-                self.coef_table = torch.tensor(scheduler.plms_plan(start), **f32).contiguous()  # [calls][12]
-                self.saved = torch.zeros_like(self.latents)                                        # the first call's sample
-                self.ring = torch.zeros(4, self.latents.numel(), **f32)                            # eps history
-            elif self.sigma:
-                rows, n_noisy = scheduler.sigma_plan()
-                self.coef_table = torch.tensor(rows, **f32).contiguous()                                   # [steps][12]
-                keeps = any(r[8] >= 0 for r in rows)                                                       # LMS
-                self.ring = torch.zeros(4 if keeps else 0, self.latents.numel(), **f32)                  # derivative history
-                self.noise = torch.zeros(n_noisy, self.latents.numel(), **f32)                           # Euler-ancestral
-            else:
-                rows, n_noisy = scheduler.ancestral_plan(eta, start)   # eta reaches only DDIM, as in diffusers' pipeline
-                self.coef_table = torch.tensor(rows, **f32).contiguous()                                   # [steps][8]
-                self.noise = torch.zeros(n_noisy, self.latents.numel(), **f32)
+            self.coef_table = torch.tensor(plan.rows, **f32).contiguous()         # one row per step
+            self.noise = torch.zeros(plan.n_noise, self.latents.numel(), **f32)
+            self.ring = torch.zeros(plan.ring_slots, self.latents.numel(), **f32)
+            self.saved = torch.zeros_like(self.latents) if "saved" in plan.buffers else None
+            self._scale_input, self._step = plan.scale_input, plan.step
+            self._step_buffers = tuple(getattr(self, b) for b in plan.buffers)
             self.inpaint = bool(inpaint)
             if self.inpaint:         # the init latents before noising, the init noise and the keep-mask, latents-shaped
                 self.init_orig, self.blend_noise, self.mask = (torch.zeros_like(self.latents) for _ in range(3))
@@ -128,23 +113,15 @@ class CapturedSampler:
         ops.sampler_advance(self.t_table, self.cursor, self.in_t)
         B = self.B
         if self.n_cond:
-            table = (self.coef_table, self.cursor) if self.sigma else (None, None)
+            table = (self.coef_table, self.cursor) if self._scale_input else (None, None)
             ops.sampler_inpaint_input(self.latents, self.cond, self.x2, *table)
-        elif self.sigma:
+        elif self._scale_input:
             ops.sampler_scale_input(self.latents, self.x2, self.coef_table, self.cursor)
         else:
             self.x2[:B].copy_(self.latents)
             self.x2[B:].copy_(self.latents)
         run_plan(self.engines[0].plan)
-        if self.sigma:
-            ops.cfg_sigma_step_table(self.eps[:B], self.eps[B:], self.latents, self.ring if self.ring.numel() else None,
-                                     self.noise if self.noise.numel() else None, self.guidance, self.coef_table, self.cursor)
-        elif self.plms:
-            ops.cfg_plms_step_table(self.eps[:B], self.eps[B:], self.latents, self.saved, self.ring, self.guidance, self.coef_table,
-                                    self.cursor)
-        else:
-            ops.cfg_ancestral_step_table(self.eps[:B], self.eps[B:], self.latents, self.noise, self.guidance, self.coef_table,
-                                         self.cursor)
+        self._step(self.eps[:B], self.eps[B:], self.latents, *self._step_buffers, self.guidance, self.coef_table, self.cursor)
         if self.inpaint:
             ops.inpaint_blend_table(self.latents, self.init_orig, self.blend_noise, self.mask, self.t_table, self.cursor,
                                     *self.noise_tables)
@@ -192,7 +169,7 @@ class CapturedSampler:
 
     def draw_noise(self, generator=None):
         """Fill the noise table: one schedulers.step_noise draw per stochastic step, in step order -- the same numbers the
-        per-call loop draws from the same generator.  DDIM with eta = 0, LMS and Euler draw nothing."""
+        per-call loop draws from the same generator.  DDIM with eta = 0, PLMS, LMS and Euler draw nothing."""
         from .schedulers import step_noise
         with torch.cuda.device(self.device):
             for k in range(self.noise.shape[0]):
@@ -235,8 +212,7 @@ class CapturedSampler:
             self.set_cond(*cond)
         self.set_context(ctx2.float())
         self.set_latents(latents.float() * self.scheduler.init_noise_sigma)
-        if not self.plms:
-            self.draw_noise(generator)
+        self.draw_noise(generator)
         self.reset(0)
         for _ in range(self.n_steps):
             self.step()

@@ -19,6 +19,7 @@ from __future__ import annotations
 import json
 import os
 from types import SimpleNamespace
+from typing import Callable, NamedTuple
 
 import numpy as np
 import torch
@@ -28,6 +29,20 @@ from . import ops
 
 class SchedulerOutput(SimpleNamespace):
     pass
+
+
+class CapturedStep(NamedTuple):
+    """How sampler.CapturedSampler runs one scheduler (`captured_step`): the rows of its device coefficient table (one per
+    executed step), the number of noise rows `draw_noise` fills, the slots of its history ring (0 or 4), whether the UNet input
+    is the latents divided by the row's in_div (sampler_scale_input), and the ops.*_table call that closes the step.  `buffers`
+    names the sampler's buffers ("noise", "ring", "saved": PNDM's saved sample) that `step` takes after the latents, in its
+    argument order."""
+    rows: list
+    n_noise: int
+    ring_slots: int
+    scale_input: bool
+    step: Callable
+    buffers: tuple
 
 
 def _betas(num_train_timesteps, beta_start, beta_end, beta_schedule):
@@ -148,6 +163,12 @@ class _SchedulerBase:
             rows.append([sa_t, sb_t, c_x0, c_x, c_e, c_z, float(k if noisy else -1), float(clip)])
             k += noisy
         return rows, k
+
+    def captured_step(self, eta=0.0, start=0, inpaint=False):
+        """CapturedSampler's step for DDIM (any eta) and DDPM over timesteps[start:]: ancestral_plan's rows, its noise table.
+        Legacy inpainting (`inpaint`) adds a blend after the step and changes nothing here."""
+        rows, n_noise = self.ancestral_plan(eta, start)
+        return CapturedStep(rows, n_noise, 0, False, ops.cfg_ancestral_step_table, ("noise",))
 
 
 def step_noise(sample, generator=None, out=None):
@@ -356,6 +377,10 @@ class PNDMScheduler(_SchedulerBase):
                         + [float(slot), float(from_saved), float(save_x)])
         return rows
 
+    def captured_step(self, eta=0.0, start=0, inpaint=False):
+        """PLMS over timesteps[start:]: plms_plan's rows, the 4-slot eps ring and the sample saved by the first call"""
+        return CapturedStep(self.plms_plan(start), 0, 4, False, ops.cfg_plms_step_table, ("saved", "ring"))
+
     def step(self, model_output, timestep, sample, return_dict: bool = True, **kw):
         out = self._plms(model_output.contiguous(), None, timestep, sample, 0.0)
         return out if return_dict else (out.prev_sample,)
@@ -423,6 +448,7 @@ class _SigmaSchedulerBase(_SchedulerBase):
         raise NotImplementedError(f"{type(self).__name__}.add_noise (sigma-space noising) is not implemented")
 
     def img2img_start(self, num_inference_steps, strength):
+        # 0.7.2 noises the init latents in sigma space here; add_noise and the inpainting blend index integer timesteps
         raise NotImplementedError(f"image-to-image and inpainting with {type(self).__name__} are not implemented")
 
     # -- the step rule ----------------------------------------------------------------------------
@@ -462,6 +488,15 @@ class _SigmaSchedulerBase(_SchedulerBase):
                 hist.append(slot)
             k += noisy
         return rows, k
+
+    def captured_step(self, eta=0.0, start=0, inpaint=False):
+        """The full schedule only: sigma_plan's rows, the derivative ring of LMS, the noise table of Euler-ancestral, and the
+        UNet input divided by in_div"""
+        if start != 0 or inpaint:
+            raise ValueError(f"{type(self).__name__}: image-to-image and inpainting (start != 0, inpaint=True) are not "
+                             "implemented for the sigma-space schedulers")
+        rows, n_noise = self.sigma_plan()
+        return CapturedStep(rows, n_noise, 4 if self._keeps_history else 0, True, ops.cfg_sigma_step_table, ("ring", "noise"))
 
     def _sigma_step(self, eps_u, eps_c, timestep, sample, guidance, generator=None, out=None, order=4):
         self._check_step_args(eps_u, sample)
@@ -572,4 +607,5 @@ class EulerAncestralDiscreteScheduler(_SigmaSchedulerBase):
                                 out=out)
 
 
-SIGMA_SCHEDULERS = (LMSDiscreteScheduler, EulerDiscreteScheduler, EulerAncestralDiscreteScheduler)
+SCHEDULERS = (DDIMScheduler, PNDMScheduler, DDPMScheduler, LMSDiscreteScheduler, EulerDiscreteScheduler,
+              EulerAncestralDiscreteScheduler)

@@ -169,3 +169,42 @@ def test_plms_kernel_reproduces_diffusers_full_loop_known_answer(variant):
     for t in plms_timesteps:
         sample = sch.step(dummy_model(sample, int(t)).contiguous(), int(t), sample, return_dict=False)[0]   # diffusers' tuple form
     _check_sched("pndm", variant, sample.cpu())
+
+
+@pytest.mark.parametrize("n, offset", [(2 * 4 * 64 * 64, 0), (3 * 5 * 7, 0), (4 * 3 * 5, 0), (2 * 4 * 64 * 64, 1)])
+@pytest.mark.parametrize("from_image", [False, True])
+def test_plms_table_kernel_equals_per_call_kernel_bit_for_bit(n, offset, from_image):
+    """Every row of plms_plan() and of plms_plan(t_start), PNDM's saved-sample rows 0 and 1 included, on cfg_plms_step_table
+    against cfg_plms_step fed with the same history tensors, weights, cx / ce and sample: the latents, the saved sample and the
+    eps written to the ring bit for bit.  n = 105 runs the scalar tail, n = 60 the vector path plus a 4-element tail, and
+    buffers one float past 16-byte alignment the scalar path."""
+    from b200sd import ops
+    from b200sd.schedulers import PNDMScheduler
+    sch = PNDMScheduler(beta_start=0.00085, beta_end=0.012, beta_schedule="scaled_linear", skip_prk_steps=True, steps_offset=1)
+    start = sch.img2img_start(50, 0.6)[0] if from_image else 0
+    sch.set_timesteps(50)
+    table = torch.tensor(sch.plms_plan(start), dtype=torch.float32, device=_dev())
+    g = torch.Generator(_dev()).manual_seed(1)
+
+    def buf(rows, like=None):      # rows x n floats, `offset` floats into their storage
+        t = torch.randn(rows * n + offset, generator=g, device=_dev())[offset:].view(rows, n)
+        return t if like is None else t.copy_(like.view(rows, n))
+
+    x, saved, ring = buf(1)[0], buf(1)[0], buf(4)
+    cursor = torch.zeros(2, dtype=torch.int32, device=_dev())
+    for k, row in enumerate(table.tolist()):
+        w, cx, ce, slots, out_slot, from_saved, save_x = row[:4], row[4], row[5], row[6:9], int(row[9]), row[10], row[11]
+        assert (k < 2) == bool(save_x or from_saved)
+        eu, ec = buf(1)[0], buf(1)[0]
+        hist = [ring[int(s)] for s in slots if s >= 0]
+        eps = buf(1)[0] if out_slot >= 0 else None
+        want = ops.cfg_plms_step(eu, ec, saved if from_saved else x, hist, w[:len(hist) + 1], 7.5, cx, ce, eps_out=eps)
+        want_saved = x if save_x else saved
+        cursor[1] = k
+        got, got_saved, got_ring = buf(1, x)[0], buf(1, saved)[0], buf(4, ring)
+        ops.cfg_plms_step_table(eu, ec, got, got_saved, got_ring, 7.5, table, cursor)
+        assert torch.equal(got, want), f"row {k}"
+        assert torch.equal(got_saved, want_saved), f"row {k}: saved sample"
+        for s in range(4):
+            assert torch.equal(got_ring[s], eps if s == out_slot else ring[s]), f"row {k}: ring slot {s}"
+        x, saved, ring = got, got_saved, got_ring
